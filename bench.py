@@ -32,6 +32,22 @@ import numpy as np  # noqa: E402
 METRIC = "series-samples/sec (and % HBM roofline) for Batch.Run at 1/2/4/8 B200 vs host Go"
 UNIT = "series-samples/s"
 SEED = 20261018
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: the result records of the last timed step, one float64 <path>/<name>.npy per field (lags and series
+    indices are exact in float64), so that two builds can be compared output for output.  Above DUMP_BYTES in all, a
+    fixed, seeded sample of the records is written, and the record numbers it kept go to sample_rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float64).ravel() for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    keep = (DUMP_BYTES - 4096) // (8 * (len(arrays) + 1))         # 4096: room for the .npy headers
+    if n * 8 * len(arrays) > DUMP_BYTES - 4096:
+        rows = np.sort(np.random.default_rng(SEED).choice(n, keep, replace=False))
+        arrays = dict({k: v[rows] for k, v in arrays.items()}, sample_rows=rows.astype(np.float64))
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 def workload(args):
@@ -110,17 +126,17 @@ class ClockSampler(threading.Thread):
 
 
 def cpu_arm(args, Y, ref, steps, warmup, nthreads):
-    """The reference algorithm on the host cores: the C oracle port (go-muse itself is Go and
-    cannot be built here).  Returns (series-samples/s, ms per step)."""
+    """The reference algorithm on the host cores: the C oracle port of go-muse's Batch.Run path.
+    Returns (series-samples/s, ms per step, the last step's (scores, lags, series indices))."""
     from oracle import c_oracle as co
     S, N = Y.shape
     for _ in range(max(0, warmup)):
         co.batch_run(ref, Y, None, args.max_lag, args.top_n, args.threshold, 0, nthreads)
     t0 = time.perf_counter()
     for _ in range(steps):
-        co.batch_run(ref, Y, None, args.max_lag, args.top_n, args.threshold, 0, nthreads)
+        out = co.batch_run(ref, Y, None, args.max_lag, args.top_n, args.threshold, 0, nthreads)
     dt = (time.perf_counter() - t0) / steps
-    return S * N / dt, dt * 1e3
+    return S * N / dt, dt * 1e3, out
 
 
 def run_reference(args):
@@ -134,7 +150,9 @@ def run_reference(args):
     n_rows = min(args.series, args.cpu_sample)
     Y = co.synth_rows(SEED, 0, n_rows, args.length)
     ref = co.synth_reference(SEED, args.length)
-    value, ms = cpu_arm(args, Y, ref, args.steps, args.warmup, cores)
+    value, ms, out = cpu_arm(args, Y, ref, args.steps, args.warmup, cores)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"scores": out[0], "lags": out[1], "series_idx": out[2]})
     sample = "first %d of the %d series of the workload per step (bounded so the run ends in minutes)" % (n_rows, args.series)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -266,6 +284,11 @@ def run_c5(args, mb, torch, dist, rank, local_rank, world, mode):
             "gpu_launches": int(args.steps * n_groups * 12),
             "clocks": clocks, "top": {"score": float(out[0][0][0]) if len(out[0][0]) else None, "n": int(len(out[0][0]))},
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"query": np.concatenate([np.full(len(o[0]), q) for q, o in enumerate(out)]),
+                                             "scores": np.concatenate([o[0] for o in out]),
+                                             "lags": np.concatenate([o[1] for o in out]),
+                                             "series_idx": np.concatenate([o[2] for o in out])})
         print(json.dumps(line), flush=True)
     store.close()
 
@@ -298,7 +321,12 @@ def main():
                          "(adversarial for the screening: nearly every score lies within the slack of the cut-off)")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: --series per GPU (the metric's configuration); strong: --series in total, sharded over the GPUs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the results of the last one as DIR/<name>.npy (float64; a seeded "
+                         "sample of them above 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     dflt = {"c3": (1_000_000, 1440, 60), "c4": (1_250_000, 10080, 240), "c5": (1_000_000, 1440, 60)}[args.workload]
     args.series = args.series if args.series is not None else dflt[0]
     args.length = args.length if args.length is not None else dflt[1]
@@ -537,6 +565,8 @@ def main():
             "roofline": roofline, "cpu_baseline": cpu, "e2e": e2e, "gpu_launches": launches, "clocks": clocks,
             "top": {"score": float(out[0][0]) if len(out[0]) else None, "n": int(len(out[0]))},
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"scores": out[0], "lags": out[1], "series_idx": out[2]})
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()

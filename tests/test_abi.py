@@ -94,11 +94,11 @@ def test_facade_labels_group_results(kats):
     assert out == [] and math.isnan(mean)
 
 
-def test_kernel_phases_on_cpu():
+def test_kernel_phases_on_cpu(tmp_path):
     """The per-thread phases of the CUDA kernels, compiled as host code and run for all
     'threads' of a series, against a direct O(n^2) long-double cross correlation."""
     import subprocess
-    exe = "/tmp/muse_emulate_kernel"
+    exe = str(tmp_path / "muse_emulate_kernel")
     subprocess.check_call(["g++", "-O1", "-std=c++17", "-I", os.path.join(ROOT, "go-muse_b200", "csrc"),
                            os.path.join(ROOT, "tests", "cpp", "emulate_kernel.cpp"), "-o", exe])
     out = subprocess.run([exe], capture_output=True, text=True)
@@ -106,12 +106,12 @@ def test_kernel_phases_on_cpu():
     assert "ALL OK" in out.stdout
 
 
-def test_big_kernel_phases_on_cpu():
+def test_big_kernel_phases_on_cpu(tmp_path):
     """score_screen_big_kernel's phases (n = 4096 .. 16384: mirror-paired last pass, split and conj(Y)*X in
     registers, transposed inverse) run thread by thread on the CPU against a double-precision FFT: the bound
     sum |Y||X| / n and the maxima of |cc| inside and outside the lag window."""
     import subprocess
-    exe = "/tmp/muse_emulate_big"
+    exe = str(tmp_path / "muse_emulate_big")
     subprocess.check_call(["g++", "-O2", "-std=c++17", "-I", os.path.join(ROOT, "go-muse_b200", "csrc"),
                            "-I", "/usr/local/cuda/include", os.path.join(ROOT, "tests", "cpp", "emulate_big.cpp"), "-o", exe])
     out = subprocess.run([exe], capture_output=True, text=True)
@@ -119,12 +119,12 @@ def test_big_kernel_phases_on_cpu():
     assert out.stdout.count(" ok") == 10 and "FAIL" not in out.stdout
 
 
-def test_wide_kernel_phases_on_cpu():
+def test_wide_kernel_phases_on_cpu(tmp_path):
     """score_screen_wide_kernel's phases (n = 16384 on 512 threads: radix 16, 16, 16 and a mirror-paired radix-2 pass,
     split and conj(Y)*X in registers, transposed inverse 2, 16, 16, 16) thread by thread on the CPU against a
     double-precision FFT."""
     import subprocess
-    exe = "/tmp/muse_emulate_wide"
+    exe = str(tmp_path / "muse_emulate_wide")
     subprocess.check_call(["g++", "-O2", "-std=c++17", "-I", os.path.join(ROOT, "go-muse_b200", "csrc"),
                            "-I", "/usr/local/cuda/include", os.path.join(ROOT, "tests", "cpp", "emulate_wide.cpp"), "-o", exe])
     out = subprocess.run([exe], capture_output=True, text=True)
