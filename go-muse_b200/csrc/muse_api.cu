@@ -2603,6 +2603,9 @@ struct muse_exchange {
     size_t merge_bytes;               // one allocation behind merge.hkeys
     unsigned long long *d_nlocal;     // grouped runs: representatives of this shard
     PartialRec *d_out;                // [capacity] merged top_n
+    // muse_multi_run_exchange, allocated on its first call: this rank's per-query lists of one step, device and pinned host
+    // ([capacity] records, [MUSE_MULTI_GROUP] counts; the host copy then receives the [world] flag words of the step)
+    unsigned char *d_send, *h_send;
 };
 
 static size_t exchange_bytes(int world, int64_t capacity) {
@@ -2696,7 +2699,9 @@ extern "C" void muse_exchange_destroy(muse_exchange *x) {
     cudaFree(x->d_done);
     cudaFree(x->d_status);
     cudaFree(x->merge.hkeys);
+    cudaFree(x->d_send);
     if (x->h_recs) cudaFreeHost(x->h_recs);
+    if (x->h_send) cudaFreeHost(x->h_send);
     delete x;
 }
 
@@ -2825,6 +2830,160 @@ extern "C" int muse_batch_run_exchange(muse_batch *b, muse_exchange *x, int64_t 
                                        int32_t sign_filter, int32_t mode, double *scores, int64_t *lags, int64_t *series_idx,
                                        int64_t *n_out) {
     return muse_batch_run_exchange_ex(b, x, nullptr, 0, max_lag, top_n, threshold, sign_filter, mode, scores, lags, series_idx, n_out);
+}
+
+// ---- many references against a sharded store (ungrouped) ----------------------------------------------------------------
+// Send table of one step: [MUSE_MULTI_GROUP] record counts, then [capacity] records (q * top_n + j), so that the counts and
+// the step's records go to the device in ONE copy.  The pinned copy has [world] flag words behind it (read back per step).
+static size_t multi_send_bytes(const muse_exchange *x) {
+    return (size_t)MUSE_MULTI_GROUP * sizeof(long long) + (size_t)x->capacity * sizeof(PartialRec);
+}
+
+static int multi_send_alloc(muse_exchange *x) {
+    if (!x->d_send) CU(cudaMalloc(&x->d_send, multi_send_bytes(x)));
+    if (!x->h_send) CU(cudaHostAlloc((void **)&x->h_send, multi_send_bytes(x) + (size_t)x->world * sizeof(unsigned long long), cudaHostAllocDefault));
+    return MUSE_OK;
+}
+
+// Steps of q_step = min(MUSE_MULTI_GROUP, capacity / top_n) queries, one epoch each: muse_multi_run on the shard, this rank's
+// lists into the send table, push to every rank, wait for every rank's flag, per-query merge on the device, merged lists back.
+// The number of steps depends only on n_refs, top_n and the capacity, which every rank shares.  Every check that could fail
+// on one rank alone comes before the first epoch; a local failure after that still takes part in its step, with the failure
+// marker instead of records, so that every rank leaves in that same step.
+extern "C" int muse_multi_run_exchange(muse_group *g, muse_exchange *x, const double *refs, int64_t n_refs, int64_t ref_len,
+                                       int64_t max_lag, int64_t top_n, double threshold, int32_t sign_filter, int32_t mode,
+                                       double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out) {
+    if (!g || !x || (!refs && n_refs > 0) || !n_out) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run_exchange: NULL argument");
+    if (n_refs < 0 || top_n < 0)
+        return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run_exchange: n_refs %lld, top_n %lld", (long long)n_refs, (long long)top_n);
+    if (top_n > 0 && (!scores || !lags || !series_idx)) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run_exchange: NULL output");
+    if (x->ctx != g->ctx) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run_exchange: exchange and store belong to different contexts");
+    if (!x->opened) return fail(MUSE_ERR_INVALID_ARG, "muse_exchange_open_peers has not been called");
+    if (top_n > x->capacity) return fail(MUSE_ERR_INVALID_ARG, "exchange capacity %lld < top_n %lld", (long long)x->capacity, (long long)top_n);
+    if (ref_len != g->N)      // muse_batch.go:24-28
+        return fail(MUSE_ERR_LENGTH_MISMATCH, "reference has length %lld, the comparison group %lld", (long long)ref_len, (long long)g->N);
+    muse_ctx *ctx = x->ctx;
+    if (top_n == 0)           // nothing to exchange: every rank's answer (no records; -1 for a std-zero reference) is the same
+        return muse_multi_run(ctx, g, refs, n_refs, ref_len, nullptr, 0, max_lag, 0, threshold, sign_filter, mode, scores, lags,
+                              series_idx, n_out);
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const int64_t q_step = std::min<int64_t>(MUSE_MULTI_GROUP, x->capacity / top_n);
+    int local_rc = multi_send_alloc(x);          // a failure from here on is this rank's failure in the current step
+    for (int64_t q0 = 0; q0 < n_refs; q0 += q_step) {
+        const int nq = (int)std::min<int64_t>(q_step, n_refs - q0);
+        double *sc = scores + (size_t)q0 * (size_t)top_n;
+        int64_t *lg = lags + (size_t)q0 * (size_t)top_n, *ix = series_idx + (size_t)q0 * (size_t)top_n, *no = n_out + q0;
+        long long *h_cnt = reinterpret_cast<long long *>(x->h_send);
+        PartialRec *h_tab = reinterpret_cast<PartialRec *>(x->h_send + (size_t)MUSE_MULTI_GROUP * sizeof(long long));
+        const unsigned long long *h_flags = reinterpret_cast<const unsigned long long *>(x->h_send + multi_send_bytes(x));
+        if (local_rc == MUSE_OK)
+            local_rc = muse_multi_run(ctx, g, refs + (size_t)q0 * (size_t)ref_len, nq, ref_len, nullptr, 0, max_lag, top_n, threshold,
+                                      sign_filter, mode, sc, lg, ix, no);
+        if (local_rc == MUSE_OK) {
+            for (int q = 0; q < nq; q++) {
+                h_cnt[q] = std::max<int64_t>(no[q], 0);
+                for (int64_t k = 0; k < h_cnt[q]; k++) {
+                    const size_t i = (size_t)q * (size_t)top_n + (size_t)k;
+                    h_tab[i] = PartialRec{(unsigned long long)ix[i], sc[i], (long long)ix[i], (int)lg[i], 0};
+                }
+            }
+            const cudaError_t e = cudaMemcpyAsync(x->d_send, x->h_send, (size_t)MUSE_MULTI_GROUP * sizeof(long long) + (size_t)nq * (size_t)top_n * sizeof(PartialRec),
+                                                  cudaMemcpyHostToDevice, st);
+            if (e != cudaSuccess) {
+                (void)cudaGetLastError();
+                local_rc = fail(MUSE_ERR_CUDA, "muse_multi_run_exchange: send table: %s", cudaGetErrorString(e));
+            }
+        }
+        x->epoch++;
+        const int par = (int)(x->epoch & 1ull);
+        ExchangePeers ex;
+        memset(&ex, 0, sizeof(ex));
+        for (int r = 0; r < x->world; r++) {
+            ex.recs[r] = reinterpret_cast<PartialRec *>(x->peer_base[r] + (size_t)par * x->recs_bytes);
+            ex.flags[r] = reinterpret_cast<unsigned long long *>(x->peer_base[r] + 2 * x->recs_bytes) + (size_t)par * x->world;
+        }
+        ex.world = x->world;
+        ex.rank = x->rank;
+        ex.epoch = x->epoch;
+        ex.done_blocks = x->d_done;
+        const long long total = (long long)nq * top_n;
+        const unsigned pblocks = (unsigned)std::max<long long>(1, std::min<long long>((total + 255) / 256, (long long)ctx->sm_count * 4));
+        const long long *d_cnt = reinterpret_cast<const long long *>(x->d_send);
+        const PartialRec *d_tab = reinterpret_cast<const PartialRec *>(x->d_send + (size_t)MUSE_MULTI_GROUP * sizeof(long long));
+        multi_records_push_kernel<<<pblocks, 256, 0, st>>>(d_tab, d_cnt, nq, (long long)top_n, (long long)x->capacity,
+                                                           local_rc != MUSE_OK ? 1 : 0, ex);
+        // ~10 s at ~2 GHz, as muse_batch_run_exchange_ex
+        exchange_wait_kernel<<<1, 32, 0, st>>>(ex.flags[x->rank], x->world, x->epoch, 20000000000ll, x->d_status);
+        multi_merge_kernel<<<(unsigned)nq, 256, 0, st>>>(ex.recs[x->rank], x->world, (long long)x->capacity, (long long)top_n, x->d_out, nullptr);
+        CU(cudaGetLastError());
+        int *h_status = reinterpret_cast<int *>(x->h_recs + (size_t)x->capacity * sizeof(muse_partial));
+        CU(cudaMemcpyAsync(x->h_recs, x->d_out, sizeof(muse_partial) * (size_t)total, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(h_status, x->d_status, sizeof(int), cudaMemcpyDeviceToHost, st));
+        if (x->h_send)      // (absent only when its allocation was this rank's failure)
+            CU(cudaMemcpyAsync((void *)h_flags, ex.flags[x->rank], sizeof(unsigned long long) * (size_t)x->world, cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        if (local_rc != MUSE_OK) return local_rc;
+        if (*h_status) {
+            CU(cudaMemsetAsync(x->d_status, 0, sizeof(int), st));
+            return fail(MUSE_ERR_CUDA, "muse_multi_run_exchange: a peer did not deliver its records within the time limit");
+        }
+        for (int r = 0; r < x->world; r++)
+            if ((h_flags[r] & 0xffffffffull) == MUSE_EXCHANGE_RANK_FAILED)
+                return fail(MUSE_ERR_CUDA, "muse_multi_run_exchange: rank %d failed", r);
+        const muse_partial *recs = reinterpret_cast<const muse_partial *>(x->h_recs);
+        for (int q = 0; q < nq; q++) {
+            if (no[q] < 0) continue;      // std(ref) == 0 on every rank (muse_batch.go:38-41)
+            const size_t row = (size_t)q * (size_t)top_n;
+            int64_t k = 0;
+            for (; k < top_n && recs[row + k].flags == 0; k++) {
+                sc[row + k] = recs[row + k].score;
+                lg[row + k] = recs[row + k].lag;
+                ix[row + k] = recs[row + k].series_idx;
+            }
+            no[q] = k;
+        }
+    }
+    return MUSE_OK;
+}
+
+// The merge of muse_multi_run_exchange on lists already gathered into device memory (e.g. by an NCCL all-gather).
+extern "C" int muse_merge_partials_many(muse_ctx *ctx, const muse_partial *d_parts, int32_t world, int64_t n_refs, int64_t top_n,
+                                        double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out) {
+    if (!ctx || !n_out) return fail(MUSE_ERR_INVALID_ARG, "muse_merge_partials_many: NULL argument");
+    if (world < 1 || n_refs < 0 || top_n < 0)
+        return fail(MUSE_ERR_INVALID_ARG, "muse_merge_partials_many: world %d, n_refs %lld, top_n %lld", world, (long long)n_refs, (long long)top_n);
+    if (n_refs > 0 && top_n > 0 && (!d_parts || !scores || !lags || !series_idx))
+        return fail(MUSE_ERR_INVALID_ARG, "muse_merge_partials_many: NULL records or output");
+    if (n_refs > 0x7fffffffll) return fail(MUSE_ERR_INVALID_ARG, "muse_merge_partials_many: n_refs %lld", (long long)n_refs);
+    for (int64_t q = 0; q < n_refs; q++) n_out[q] = 0;
+    if (n_refs == 0 || top_n == 0) return MUSE_OK;
+    CU(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const size_t n_rec = (size_t)n_refs * (size_t)top_n;
+    unsigned char *d = nullptr;
+    CU(cudaMalloc(&d, n_rec * sizeof(PartialRec) + (size_t)n_refs * sizeof(long long)));
+    PartialRec *d_out = reinterpret_cast<PartialRec *>(d);
+    long long *d_n = reinterpret_cast<long long *>(d_out + n_rec);
+    std::vector<muse_partial> h(n_rec);
+    auto body = [&]() -> int {
+        multi_merge_kernel<<<(unsigned)n_refs, 256, 0, st>>>(reinterpret_cast<const PartialRec *>(d_parts), world, (long long)(n_refs * top_n),
+                                                             (long long)top_n, d_out, d_n);
+        CU(cudaGetLastError());
+        CU(cudaMemcpyAsync(h.data(), d_out, n_rec * sizeof(PartialRec), cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(n_out, d_n, (size_t)n_refs * sizeof(long long), cudaMemcpyDeviceToHost, st));
+        CU(cudaStreamSynchronize(st));
+        return MUSE_OK;
+    };
+    const int rc = body();
+    cudaFree(d);
+    if (rc) return rc;
+    for (size_t i = 0; i < n_rec; i++) {
+        scores[i] = h[i].score;
+        lags[i] = h[i].lag;
+        series_idx[i] = h[i].series_idx;
+    }
+    return MUSE_OK;
 }
 
 extern "C" int muse_batch_last_timing(const muse_batch *cb, muse_timing *out) {

@@ -470,6 +470,100 @@ __global__ void exchange_wait_kernel(const unsigned long long *flags, int world,
     if (!ok) *status = 1;
 }
 
+// ---- many references against a sharded store: every shard's per-query top-N lists in ONE exchange step -----------------
+// The send table holds q_step lists of top_n records (what muse_multi_run returns for the step's queries on this shard,
+// sorted by (|score| desc, global index asc)) followed by the q_step record counts.  Record j of query q goes to
+// [q * top_n + j] of slot [rank] of every rank's receive buffer; j >= count[q] is padding (flags = 1).  failed != 0: this
+// rank's local run failed after the step began -- it stores no records and releases the failure marker instead, so that its
+// peers return in the same step rather than wait for records that never come.
+// Low 32 bits of a flag word that mark a failed sender (0xffffffff already means "take the host path").
+#define MUSE_EXCHANGE_RANK_FAILED 0xfffffffeull
+__global__ void __launch_bounds__(256)
+multi_records_push_kernel(const PartialRec *__restrict__ table, const long long *__restrict__ counts, int q_step, long long top_n,
+                          long long capacity, int failed, ExchangePeers ex) {
+    const long long total = (long long)q_step * top_n;
+    const long long slot0 = (long long)ex.rank * capacity;
+    if (!failed) {
+        for (long long g = (long long)blockIdx.x * blockDim.x + threadIdx.x; g < total; g += (long long)gridDim.x * blockDim.x) {
+            const long long q = g / top_n, j = g - q * top_n;
+            const PartialRec rec = j < counts[q] ? table[g] : PartialRec{0ull, 0.0, 0ll, 0, 1};
+            for (int d = 0; d < ex.world; d++) ex.recs[d][slot0 + g] = rec;
+        }
+    }
+    // last block of the grid: everything this GPU stored is ordered before the flags it releases
+    __shared__ bool last;
+    __threadfence_system();
+    __syncthreads();
+    if (threadIdx.x == 0) last = (atomicAdd(ex.done_blocks, 1u) == gridDim.x - 1);
+    __syncthreads();
+    if (!last) return;
+    __threadfence_system();
+    const unsigned long long word = (ex.epoch << 32) | (failed ? MUSE_EXCHANGE_RANK_FAILED : (unsigned long long)total);
+    if (threadIdx.x < ex.world) st_release_sys_u64(&ex.flags[threadIdx.x][ex.rank], word);
+    if (threadIdx.x == 0) *ex.done_blocks = 0u;
+}
+
+// a precedes b in (|score| desc, global series index asc), the order of results.go:81-85 with ties by index
+__device__ __forceinline__ bool rec_precedes(const PartialRec &a, const PartialRec &b) {
+    const double sa = fabs(a.score), sb = fabs(b.score);
+    return sa > sb || (sa == sb && a.series_idx < b.series_idx);
+}
+
+// Per-query merge of `world` sorted lists into the global top_n: one CTA per query (blockIdx.x).  List r of query q starts at
+// recs[r * rank_stride + q * top_n] -- the exchange's receive buffer ([world][capacity]) and a gathered array
+// ([world][n_refs][top_n]) have that same layout.  Each list is valid records in order, then padding (flags != 0), so a
+// record's place in the merged order is its own index plus, in every other list, the number of records before it: one
+// binary search per list, O(world * top_n * log top_n) per query and no shared-memory bound on top_n.  Equal keys in two
+// lists (not produced by disjoint shards) go to the lower rank first, so positions stay distinct.  The lists were filtered on
+// their shards: no filter here.  out[q * top_n ..] gets the merged list padded with flags = 1; n_out[q] (may be NULL) its length.
+__device__ __forceinline__ long long list_count_before(const PartialRec *__restrict__ list, long long top_n, const PartialRec &x,
+                                                       bool or_equal) {
+    long long lo = 0, hi = top_n;      // first k whose record does not come before x (padding never does)
+    while (lo < hi) {
+        const long long mid = (lo + hi) >> 1;
+        const PartialRec y = list[mid];
+        const bool before = y.flags == 0 && (rec_precedes(y, x) || (or_equal && !rec_precedes(x, y)));
+        if (before) lo = mid + 1;
+        else hi = mid;
+    }
+    return lo;
+}
+
+__global__ void __launch_bounds__(256)
+multi_merge_kernel(const PartialRec *__restrict__ recs, int world, long long rank_stride, long long top_n,
+                   PartialRec *__restrict__ out, long long *__restrict__ n_out) {
+    const long long q = blockIdx.x;
+    const PartialRec *base = recs + q * top_n;
+    PartialRec *o = out + q * top_n;
+    __shared__ unsigned long long total;
+    if (threadIdx.x == 0) total = 0ull;
+    __syncthreads();
+    for (int r = threadIdx.x; r < world; r += blockDim.x) {     // valid records of list r: the first padding record
+        const PartialRec *list = base + (long long)r * rank_stride;
+        long long lo = 0, hi = top_n;
+        while (lo < hi) {
+            const long long mid = (lo + hi) >> 1;
+            if (list[mid].flags == 0) lo = mid + 1;
+            else hi = mid;
+        }
+        atomicAdd(&total, (unsigned long long)lo);
+    }
+    for (long long g = threadIdx.x; g < (long long)world * top_n; g += blockDim.x) {
+        const int r = (int)(g / top_n);
+        const long long j = g - (long long)r * top_n;
+        const PartialRec x = base[(long long)r * rank_stride + j];
+        if (x.flags != 0) continue;
+        long long pos = j;
+        for (int s = 0; s < world && pos < top_n; s++)
+            if (s != r) pos += list_count_before(base + (long long)s * rank_stride, top_n, x, s < r);
+        if (pos < top_n) o[pos] = x;
+    }
+    __syncthreads();
+    const long long n = (long long)total < top_n ? (long long)total : top_n;
+    for (long long k = n + threadIdx.x; k < top_n; k += blockDim.x) o[k] = PartialRec{0ull, 0.0, 0ll, 0, 1};
+    if (threadIdx.x == 0 && n_out) n_out[q] = n;
+}
+
 // ---- grouped shards: every group representative (unfiltered, SURVEY F2) pushed to every GPU ------------------------
 // Flags carry (epoch << 32) | record count of the sender (0xffffffff: more representatives than the buffer holds).
 // One thread per series: the representative of its group (lowest index among the members holding the group max,

@@ -147,3 +147,69 @@ func (b *Batch) RunSharded(e *Exchange, groupByLabels []string) ([]ShardScore, e
 	}
 	return out, nil
 }
+
+// RunManySharded is RunMany over the whole sharded group (without groupByLabels): refs[q] is scored against the series of
+// every process, and scores[q] -- identical on every process, best first, filled as RunSharded fills its result -- is what a
+// single-process RunMany over the whole group puts into results[q].  results supply the settings (the same MaxLag, TopN,
+// Threshold and SignFilter on every Results) and are left untouched.  A constant reference gets NewBatch's error in errs[q].
+// Every process calls it with the same references and settings; a process whose shard holds no series takes part all the
+// same.  One call runs the queries in steps of up to 256, each one exchange step (muse_multi_run_exchange).
+func RunManySharded(e *Exchange, refs []*Series, comp *Group, results []*Results) (errs []error, scores [][]ShardScore, err error) {
+	if len(refs) != len(results) {
+		return nil, nil, fmt.Errorf("%d references but %d results", len(refs), len(results))
+	}
+	errs = make([]error, len(refs))
+	scores = make([][]ShardScore, len(refs))
+	if len(refs) == 0 {
+		return errs, scores, nil
+	}
+	if len(comp.series) == 0 && comp.n == 0 { // an empty shard: its store takes the references' length
+		comp.n = refs[0].Length()
+	}
+	n := comp.Length()
+	r0 := results[0]
+	rows := make([]float64, 0, len(refs)*n)
+	for q, ref := range refs {
+		if ref.Length() != n {
+			return nil, nil, fmt.Errorf("%s does not have the same length as the comparison group", ref.UID())
+		}
+		if rq := results[q]; rq.MaxLag != r0.MaxLag || rq.TopN != r0.TopN || rq.Threshold != r0.Threshold || rq.SignFilter != r0.SignFilter {
+			return nil, nil, fmt.Errorf("RunManySharded needs the same MaxLag, TopN, Threshold and SignFilter on every Results")
+		}
+		rows = append(rows, ref.Values()...)
+	}
+	if r0.TopN < 1 {
+		return errs, scores, nil
+	}
+	if err := comp.syncDevice(); err != nil {
+		return nil, nil, err
+	}
+	topN := r0.TopN
+	sc := make([]float64, len(refs)*topN)
+	lags := make([]int64, len(refs)*topN)
+	idx := make([]int64, len(refs)*topN)
+	nOut := make([]int64, len(refs))
+	rc := C.muse_multi_run_exchange(comp.store, e.x, (*C.double)(unsafe.Pointer(&rows[0])), C.int64_t(len(refs)), C.int64_t(n),
+		C.int64_t(r0.MaxLag), C.int64_t(topN), C.double(r0.Threshold), C.int32_t(r0.SignFilter), C.MUSE_MODE_AUTO,
+		(*C.double)(unsafe.Pointer(&sc[0])), (*C.int64_t)(unsafe.Pointer(&lags[0])),
+		(*C.int64_t)(unsafe.Pointer(&idx[0])), (*C.int64_t)(unsafe.Pointer(&nOut[0])))
+	if rc != C.MUSE_OK {
+		return nil, nil, lastError(rc)
+	}
+	for q := range refs {
+		if nOut[q] < 0 {
+			errs[q] = fmt.Errorf("Invalid input query, %v", "Standard deviation of zero")
+			continue
+		}
+		out := make([]ShardScore, int(nOut[q]))
+		for i := range out {
+			k := q*topN + i
+			out[i] = ShardScore{Index: idx[k], Lag: int(lags[k]), PercentScore: sc[k]}
+			if local := idx[k] - comp.shardFirst; local >= 0 && local < int64(len(comp.series)) {
+				out[i].Labels = comp.series[local].Labels()
+			}
+		}
+		scores[q] = out
+	}
+	return errs, scores, nil
+}

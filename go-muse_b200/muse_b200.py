@@ -167,6 +167,9 @@ ABI = {
                                           _dp, _ip64, _ip64, _ip64]),
     "muse_batch_run_exchange_ex": (C.c_int, [_vp, _vp, _ip32, C.c_int32, C.c_int64, C.c_int64, C.c_double, C.c_int32, C.c_int32,
                                              _dp, _ip64, _ip64, _ip64]),
+    "muse_multi_run_exchange": (C.c_int, [_vp, _vp, _dp, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_double, C.c_int32,
+                                          C.c_int32, _dp, _ip64, _ip64, _ip64]),
+    "muse_merge_partials_many": (C.c_int, [_vp, _vp, C.c_int32, C.c_int64, C.c_int64, _dp, _ip64, _ip64, _ip64]),
     "muse_batch_partial_capacity": (C.c_int64, [_vp, _ip32, C.c_int32, C.c_int64]),
     "muse_merge_partials": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_int64, C.c_double, C.c_int32,
                                       _dp, _ip64, _ip64, _ip64]),
@@ -442,6 +445,39 @@ def multi_run(store: "DeviceStore", refs, key_cols: Sequence[int], max_lag: int,
         return sc[:Q], lg[:Q], ix[:Q], n_out[:Q]
     return [None if n_out[q] < 0 else (sc[q, :n_out[q]].copy(), lg[q, :n_out[q]].copy(), ix[q, :n_out[q]].copy())
             for q in range(Q)]
+
+
+def multi_records(sc: np.ndarray, lg: np.ndarray, ix: np.ndarray, n_out: np.ndarray) -> np.ndarray:
+    """multi_run(raw=True) outputs as [Q, top_n] muse_partial records: row q holds query q's list in its order
+    (group_key = global series index), padded with flags = 1 -- the layout muse_merge_partials_many merges."""
+    Q, top_n = sc.shape
+    rec = np.zeros((Q, top_n), dtype=PARTIAL_DTYPE)
+    valid = np.arange(top_n)[None, :] < np.maximum(n_out, 0)[:, None]
+    rec["group_key"] = np.where(valid, ix, 0).astype(np.uint64)
+    rec["score"] = np.where(valid, sc, 0.0)
+    rec["series_idx"] = np.where(valid, ix, 0)
+    rec["lag"] = np.where(valid, lg, 0).astype(np.int32)
+    rec["flags"] = np.where(valid, 0, 1)
+    return rec
+
+
+def merge_partials_many(ctx: Context, d_parts: int, world: int, n_refs: int, top_n: int):
+    """muse_merge_partials_many: merge the per-query lists of `world` shards, gathered in DEVICE memory at address d_parts as
+    [world][n_refs][top_n] records (multi_records of each shard), into the global top_n of every query.  Returns
+    (scores[Q, top_n], lags[Q, top_n], series_idx[Q, top_n], n_out[Q])."""
+    cap = max(1, int(top_n))
+    sc = np.zeros((max(n_refs, 1), cap))
+    lg = np.zeros((max(n_refs, 1), cap), dtype=np.int64)
+    ix = np.zeros((max(n_refs, 1), cap), dtype=np.int64)
+    n_out = np.zeros(max(n_refs, 1), dtype=np.int64)
+    _check(lib().muse_merge_partials_many(ctx.h, _vp(d_parts), world, n_refs, top_n, _d(sc), lg.ctypes.data_as(_ip64),
+                                          ix.ctypes.data_as(_ip64), n_out.ctypes.data_as(_ip64)))
+    return sc[:n_refs], lg[:n_refs], ix[:n_refs], n_out[:n_refs]
+
+
+def _triples(sc, lg, ix, n_out):
+    return [None if n_out[q] < 0 else (sc[q, :n_out[q]].copy(), lg[q, :n_out[q]].copy(), ix[q, :n_out[q]].copy())
+            for q in range(len(n_out))]
 
 
 def multi_last_stats(ctx: Context) -> Tuple[int, int]:
@@ -882,6 +918,28 @@ def allgather_merge_device(batch: DeviceBatch, max_lag: int, top_n: int, thresho
     return merge_partials(allp, max_lag, top_n, threshold, sign_filter)
 
 
+def allgather_merge_many(store: DeviceStore, refs, max_lag: int, top_n: int, threshold: float, sign_filter: int = 0,
+                         mode: int = MODE_AUTO):
+    """Many references against a sharded store without the peer-memory exchange (CUDA IPC closed): multi_run on this rank's
+    shard, its per-query lists as records in device memory, ONE NCCL all-gather, then the per-query merge on the device
+    (muse_merge_partials_many).  Returns what Exchange.run_many returns -- identical on every rank."""
+    import torch
+    import torch.distributed as dist
+
+    world = dist.get_world_size()
+    sc, lg, ix, n_out = multi_run(store, refs, [], max_lag, top_n, threshold, sign_filter, mode=mode, raw=True)
+    Q = len(n_out)
+    if Q == 0 or top_n < 1:
+        return _triples(sc, lg, ix, n_out)
+    mine = torch.from_numpy(multi_records(sc, lg, ix, n_out).view(np.uint8).reshape(-1)).cuda()
+    allr = torch.empty(world * mine.numel(), dtype=torch.uint8, device=mine.device)
+    dist.all_gather_into_tensor(allr, mine)
+    torch.cuda.current_stream().synchronize()
+    msc, mlg, mix, mn = merge_partials_many(store.ctx, allr.data_ptr(), world, Q, top_n)
+    mn = np.where(n_out < 0, -1, mn)          # std(ref) == 0: the same on every rank
+    return _triples(msc, mlg, mix, mn)
+
+
 class Exchange:
     """muse_exchange: the shard's top_n records go into every rank's receive buffer over NVLink peer memory,
     written by the selection kernel itself (no library collective on the data path).  Setup exchanges the CUDA
@@ -939,6 +997,23 @@ class Exchange:
         _check(rc)
         k = int(n_out.value)
         return sc[:k], lg[:k], ix[:k]
+
+    def run_many(self, store: DeviceStore, refs, max_lag: int, top_n: int, threshold: float, sign_filter: int = 0,
+                 mode: int = MODE_AUTO):
+        """muse_multi_run_exchange: every row of refs against the WHOLE sharded store (ungrouped), as multi_run on one store
+        holding every shard would return it -- one (scores, lags, series_idx) triple per reference, None where the reference
+        has zero std -- identical on every rank.  Every rank passes the same refs and arguments."""
+        R = np.ascontiguousarray(refs, dtype=np.float64)
+        assert R.ndim == 2
+        Q, cap = R.shape[0], max(1, int(top_n))
+        sc = np.zeros((max(Q, 1), cap))
+        lg = np.zeros((max(Q, 1), cap), dtype=np.int64)
+        ix = np.zeros((max(Q, 1), cap), dtype=np.int64)
+        n_out = np.zeros(max(Q, 1), dtype=np.int64)
+        _check(lib().muse_multi_run_exchange(store.h, self.h, _d(R), Q, R.shape[1], max_lag, top_n, threshold, sign_filter, mode,
+                                             _d(sc), lg.ctypes.data_as(_ip64), ix.ctypes.data_as(_ip64),
+                                             n_out.ctypes.data_as(_ip64)))
+        return _triples(sc[:Q], lg[:Q], ix[:Q], n_out[:Q])
 
     def close(self):
         if self.h:

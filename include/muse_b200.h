@@ -205,10 +205,13 @@ int  muse_batch_xcorr(muse_batch *b, int64_t local_index, double *cc, int32_t *s
  * :99-130) return, in one call.  refs: host rows [n_refs][ref_len]; outputs: row q of scores / lags / series_idx
  * (capacity top_n each row) and n_out[q] = results of query q, or -1 when reference q has std == 0
  * (muse_batch.go:38-41: NewBatch fails for that query only).  Arguments as muse_batch_run_ex.
- * For FFT length 2048, ungrouped, unsigned runs over >= 16384 series the store is read and every series
- * transformed ONCE per 16 references (score_screen_multi_kernel: per-query bounds, second stage and running
- * cut-off; each query then finishes on the exact fp64 kernel like a single run) -- results identical to the
- * separate runs; other shapes are served as separate batches on the resident store. */
+ * For FFT length 2048, ungrouped, unsigned runs over >= 16384 series (any size in MUSE_MODE_SCREEN; more than one
+ * reference, top_n <= series / 4)
+ * the screening bounds of up to 256 references at a time are ONE bf16 contraction on the tensor cores (tcgen05.mma,
+ * muse_multi_bounds_tc), the second stages of all of them one launch over the store, and each query then finishes
+ * on the exact fp64 kernel like a single run -- results identical to the separate runs.  MUSE_MULTI_TC=0 takes the
+ * fp32 multi-query kernel instead (16 references per pass over the store).  Other shapes are served as separate
+ * batches on the resident store. */
 int  muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, int64_t n_refs, int64_t ref_len,
                     const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n, double threshold,
                     int32_t sign_filter, int32_t mode,
@@ -285,6 +288,27 @@ int  muse_batch_run_exchange(muse_batch *b, muse_exchange *x, int64_t max_lag, i
 int  muse_batch_run_exchange_ex(muse_batch *b, muse_exchange *x, const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag,
                                 int64_t top_n, double threshold, int32_t sign_filter, int32_t mode,
                                 double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out);
+/* Many references against a sharded store (ungrouped): what muse_multi_run writes on ONE store holding every shard -- row q
+ * of scores / lags / series_idx (capacity top_n each row, global series indices), n_out[q] results or -1 when reference q has
+ * std == 0 -- identical on every rank.  The queries go in steps of min(256, capacity / top_n), one exchange epoch each:
+ * muse_multi_run on this shard, its per-query top_n lists pushed into every rank's receive buffer, then a per-query merge on
+ * the device.  Contract: every rank passes the same references and arguments, and every rank's exchange has the same
+ * capacity (the number of steps follows from n_refs, top_n and the capacity alone).  Argument errors (NULLs, top_n > capacity,
+ * an exchange whose peers are not open, store and exchange on different contexts, ref_len) are reported before any step
+ * begins.  A rank whose local run fails during a step still completes the step with a failure marker and returns its own
+ * error; its peers return MUSE_ERR_CUDA ("rank r failed") in that same step.  A sticky CUDA error (a faulted context) cannot
+ * be published this way: the peers then return MUSE_ERR_CUDA after the exchange's time limit.  A shard with no series
+ * takes part and contributes no records. */
+int  muse_multi_run_exchange(muse_group *g, muse_exchange *x, const double *refs, int64_t n_refs, int64_t ref_len,
+                             int64_t max_lag, int64_t top_n, double threshold, int32_t sign_filter, int32_t mode,
+                             double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out);
+/* The merge of muse_multi_run_exchange for lists gathered by the caller (e.g. an NCCL all-gather, where CUDA IPC is closed).
+ * d_parts: DEVICE memory on the context's device, [world][n_refs][top_n] records -- every rank's muse_multi_run rows as
+ * muse_partial records (group_key = series_idx, flags 0), each row sorted as muse_multi_run returns it and padded with
+ * flags = 1.  Outputs (host) as muse_multi_run; n_out[q] = merged records (a std-zero reference has none: its -1 comes from
+ * the caller's own muse_multi_run).  Runs on the context's stream and synchronises it. */
+int  muse_merge_partials_many(muse_ctx *ctx, const muse_partial *d_parts, int32_t world, int64_t n_refs, int64_t top_n,
+                              double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out);
 /* Upper bound on the records run_partial can emit for these arguments. */
 int64_t muse_batch_partial_capacity(muse_batch *b, const int32_t *key_cols, int32_t n_key_cols,
                                     int64_t top_n);
