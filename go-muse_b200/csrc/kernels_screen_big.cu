@@ -1,12 +1,8 @@
 // kernels_screen_big.cu -- instantiations of score_screen_big_kernel (muse_screen_big.cuh), n = 4096 .. 16384.
 #include <algorithm>
-#include <cstdlib>
-
-#define MUSE_WIDE_KERNEL
 
 #include "muse_launch.h"
 #include "muse_screen_big.cuh"
-#include "muse_screen_wide.cuh"
 
 namespace muse {
 
@@ -26,31 +22,10 @@ static cudaError_t launch_screen_big_t(const ScreenParams &p, int sm_count, cuda
     return cudaGetLastError();
 }
 
-// n = 16384 on 512 threads per series (muse_screen_wide.cuh)
-cudaError_t launch_screen_wide(const ScreenParams &p, int sm_count, cudaStream_t st) {
-    using C = ScreenWideCfg;
-    auto kern = score_screen_wide_kernel;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM);
-    if (e != cudaSuccess) return e;
-    int per_sm = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, C::T, C::SMEM);
-    if (e != cudaSuccess) return e;
-    if (per_sm < 1) per_sm = 1;
-    const int64_t blocks = std::min<int64_t>(p.count, (int64_t)sm_count * per_sm);
-    kern<<<(unsigned)blocks, C::T, C::SMEM, st>>>(p);
-    return cudaGetLastError();
-}
-
-#ifndef MUSE_BIG_MINB13
-#define MUSE_BIG_MINB13 2      // blocks of 256 threads per SM at n = 16384 (3 = an 80-register cap: measured, see DESIGN.md)
-#endif
-
 cudaError_t launch_screen_big(int log2m, const ScreenParams &p, int sm_count, cudaStream_t st) {
     switch (log2m) {
-        case 13: {      // one instantiation per number of rows that hold samples (kernels_screen_big13_*.cu); MUSE_BIG13_GENERIC=1:
-                        // the run-time version, for A/B runs
-            static const bool generic = getenv("MUSE_BIG13_GENERIC") != nullptr;
-            if (generic) return launch_screen_big_t<13, MUSE_BIG_MINB13>(p, sm_count, st);
+        case 13: {      // one instantiation per number of rows that hold samples (kernels_screen_big13_*.cu), MUSE_BIG_MINB13
+                        // blocks of 256 threads per SM (2; 3 = an 80-register cap: measured, see DESIGN.md)
             const int nz = (((p.N + 1) >> 1) + ScreenBigCfg<13>::T - 1) / ScreenBigCfg<13>::T;
             if (nz >= 29) return launch_screen_big13_d(nz, p, sm_count, st);
             if (nz >= 25) return launch_screen_big13_c(nz, p, sm_count, st);

@@ -58,8 +58,10 @@ extern "C" const char *muse_version(void) { return "muse_b200 0.1 (sm_100a)"; }
 // cudaHostAlloc of these cost milliseconds to seconds (measured: a NewBatch + Run + destroy cycle per
 // request spent 3 s in cudaFree/cudaFreeHost once in four) while the run itself takes 2.7 ms.
 #define MUSE_MAX_LABEL_KEYS 64   // label-key columns of a store (the facade adds one all-absent column)
-#define MUSE_SCRATCH_POOL 272   // scratch sets kept per context: a multi-query launch has up to MUSE_MULTI_GROUP batches alive at once
+#define MUSE_SCRATCH_POOL 272   // scratch sets kept per context (MUSE_MULTI_GROUP + MUSE_MULTI_SEPARATE): room for the batches
+                                // of a tensor-core launch group and of a group of separate batches in muse_multi_run
 #define MUSE_MULTI_GROUP 256    // queries of one launch of the tensor-core multi-query path (== TcCfg::TN == RefineMultiCfg::QMAX)
+#define MUSE_MULTI_SEPARATE 16  // queries of one group of separate batches in muse_multi_run (one upload, one round trip)
 struct RunScratch {
     int64_t scratch_cap;
     double *d_score;
@@ -92,14 +94,12 @@ struct RunScratch {
     cd *Xt, *twM, *twn;
     cf *twp_f;                        // fp32 screening pass: per-pass twiddles
     cf *twi_f;                        // n = 4096 .. 16384: twiddle tables of muse_screen_big.cuh
-    cf *twide_f;                      // n = 16384: twiddle tables of muse_screen_wide.cuh
     float2 *swtw;                     // split twiddles exp(-2*pi*i*k/n), k < M/2, fp32
     float4 *sw_f;                     // fused kernels: (twn, A[k], A[M-k]) per k < M/2
     float4 *sx_f;                     // fused refinement: (Xt[k], Xt[M-k]) in fp32 per k < M/2
     float *sb_f;                      // warp / sub-warp kernels: sqrt(2 (A[k]^2 + A[M-k]^2)) rounded up per k < M/2
     float *d_mid;                     // [0] std-zero flag of the reference (as float bits), [1] A[M/2], [2..3] Xt[M/2] in fp32
     cudaEvent_t ev[4];
-    cudaStream_t aux;                 // the batch's own stream: the tails of the queries of a multi-query launch run side by side
 };
 
 struct muse_ctx {
@@ -122,8 +122,8 @@ struct muse_ctx {
     int64_t mt_top_n;               // result records per query the two buffers were sized for
     cudaEvent_t mt_ev[5];           // stage boundaries of the last multi-query launch group: start, magnitudes, bounds, second stages, end
     int64_t multi_refined, multi_rescored;      // totals of the last muse_multi_run (second stages, fp64 re-scorings)
-    void *d_multi_q;                // query table of score_screen_multi_kernel (ScreenMultiCfg::QC entries)
-    double *d_multi_refs;           // [QC][d_multi_ld] reference rows of a multi-query launch, pad columns kept zero
+    void *d_multi_q;                // query table of refine_multi_kernel (MUSE_MULTI_GROUP entries)
+    double *d_multi_refs;           // [MUSE_MULTI_GROUP][d_multi_ld] reference rows of a muse_multi_run group, pad columns kept zero
     int64_t d_multi_ld, d_multi_n;
 };
 
@@ -153,8 +153,7 @@ struct muse_batch : RunScratch {
     muse_timing timing;
     int timing_pending;    // the last run was queued without a final synchronisation (muse_batch_run_partial_device)
     int fused_run;         // 1: score_fused, 2: score_fused_grouped (d_counters[2] = exact list length, [3] = refined)
-    int prescreened;       // d_U and the cut-off state were filled by score_screen_multi_kernel: the next fused run starts at its tail
-    int use_aux;           // queue this batch's work on its own stream (RunScratch::aux) instead of the context's
+    int prescreened;       // d_U and the cut-off state were filled by the tensor-core multi-query path: the next fused run starts at its tail
     int signed_run;        // the current run keeps the sign of the scores (muse.go:72-76)
     // n > MUSE_MAX_FUSED_FFT_LEN: Stockham passes through global memory (kernels_long.cu); Xt holds n entries, twM the n twiddles
     int is_long;
@@ -163,13 +162,7 @@ struct muse_batch : RunScratch {
     long long long_pairs;  // pairs of series per chunk d_long was sized for
 };
 
-static inline cudaStream_t bstream(const muse_batch *b) { return b->use_aux ? b->aux : b->ctx->stream; }
-// timing events of a run: not recorded for the batches of a multi-query launch (nobody reads their timings, and five
-// calls per query are a fifth of what the host issues for one)
-#define TIMING_EVENT(b, i, st)                             \
-    do {                                                   \
-        if (!(b)->use_aux) CU(cudaEventRecord((b)->ev[i], st)); \
-    } while (0)
+static inline cudaStream_t bstream(const muse_batch *b) { return b->ctx->stream; }
 
 struct DeviceGuard {
     int prev;
@@ -210,9 +203,8 @@ static void scratch_free(RunScratch &r) {
     cudaFree(r.d_gmax); cudaFree(r.d_hkeys); cudaFree(r.d_gidx);
     cudaFree(r.d_flag); cudaFree(r.d_counters); cudaFree(r.d_sel); cudaFree(r.d_cut);
     cudaFree(r.d_ref); cudaFree(r.Xt); cudaFree(r.twM); cudaFree(r.twn);
-    cudaFree(r.twp_f); cudaFree(r.twi_f); cudaFree(r.twide_f); cudaFree(r.swtw); cudaFree(r.sw_f); cudaFree(r.sx_f); cudaFree(r.sb_f); cudaFree(r.d_mid);
+    cudaFree(r.twp_f); cudaFree(r.twi_f); cudaFree(r.swtw); cudaFree(r.sw_f); cudaFree(r.sx_f); cudaFree(r.sb_f); cudaFree(r.d_mid);
     for (int i = 0; i < 4; i++) if (r.ev[i]) cudaEventDestroy(r.ev[i]);
-    if (r.aux) cudaStreamDestroy(r.aux);
     if (r.h_pin) cudaFreeHost(r.h_pin);
     memset(&r, 0, sizeof(r));
 }
@@ -700,16 +692,9 @@ static int64_t next_pow2(int64_t v) {   // == nextPowOf2 (xcorr.go:19-24) for 1 
 // fp32 tables of the screening kernel; leaves screen_ok = 0 when the shape has no screening kernel
 // n = 128 .. 16384: kernels with the fused fp32 second stage (several series per warp up to 1024, one warp per series at 2048,
 // one block per series above)
-static bool block_small();
-static int screen_is_fused(int log2m) { return log2m >= (block_small() ? 8 : 6) && log2m <= 13; }
+static int screen_is_fused(int log2m) { return log2m >= 6 && log2m <= 13; }
 static int screen_is_big(int log2m) { return log2m >= 11 && log2m <= 13; }      // muse_screen_big.cuh
 static int screen_log2m_supported(int log2m) { return screen_is_fused(log2m); }
-// n = 128 .. 1024: several series per warp (muse_screen_sub.cuh); MUSE_BLOCK_SMALL=1 keeps round 1's block kernel for A/B runs
-static bool block_small() {
-    static const bool v = getenv("MUSE_BLOCK_SMALL") != nullptr;
-    return v;
-}
-static int screen_log2p(int log2m) { return (log2m >= 10 || !block_small()) ? 5 : (log2m == 9 ? 4 : 3); }
 
 // The per-reference tables of the fp32 kernels, from Xt on the device: weights of the bound
 // A[k] = |Xt[k]| * (1 at DC and Nyquist, else 2) rounded UP (the bound must not shrink), one 16-byte entry per
@@ -750,9 +735,9 @@ static int ensure_ref_tables(muse_batch *b, int64_t ld) {
     const bool want_screen = screen_log2m_supported(b->log2m);
     if (b->tab_n == n && (b->tab_screen || !want_screen)) return MUSE_OK;
     if (b->is_long) {      // the reference's transform has n entries, the twiddles are generated on the device
-        cudaFree(b->Xt); cudaFree(b->twM); cudaFree(b->twn); cudaFree(b->twp_f); cudaFree(b->twi_f); cudaFree(b->twide_f); cudaFree(b->swtw); cudaFree(b->sw_f); cudaFree(b->sx_f); cudaFree(b->sb_f);
+        cudaFree(b->Xt); cudaFree(b->twM); cudaFree(b->twn); cudaFree(b->twp_f); cudaFree(b->twi_f); cudaFree(b->swtw); cudaFree(b->sw_f); cudaFree(b->sx_f); cudaFree(b->sb_f);
         b->Xt = b->twM = b->twn = nullptr;
-        b->twp_f = b->twi_f = b->twide_f = nullptr; b->swtw = nullptr; b->sw_f = b->sx_f = nullptr; b->sb_f = nullptr;
+        b->twp_f = b->twi_f = nullptr; b->swtw = nullptr; b->sw_f = b->sx_f = nullptr; b->sb_f = nullptr;
         b->tab_n = 0;
         b->tab_screen = 0;
         CU(cudaMalloc(&b->Xt, sizeof(cd) * (size_t)n));
@@ -761,9 +746,9 @@ static int ensure_ref_tables(muse_batch *b, int64_t ld) {
         b->tab_n = n;
         return MUSE_OK;
     }
-    cudaFree(b->Xt); cudaFree(b->twM); cudaFree(b->twn); cudaFree(b->twp_f); cudaFree(b->twi_f); cudaFree(b->twide_f); cudaFree(b->swtw); cudaFree(b->sw_f); cudaFree(b->sx_f); cudaFree(b->sb_f);
+    cudaFree(b->Xt); cudaFree(b->twM); cudaFree(b->twn); cudaFree(b->twp_f); cudaFree(b->twi_f); cudaFree(b->swtw); cudaFree(b->sw_f); cudaFree(b->sx_f); cudaFree(b->sb_f);
     b->Xt = b->twM = b->twn = nullptr;
-    b->twp_f = b->twi_f = b->twide_f = nullptr; b->swtw = nullptr; b->sw_f = b->sx_f = nullptr; b->sb_f = nullptr;
+    b->twp_f = b->twi_f = nullptr; b->swtw = nullptr; b->sw_f = b->sx_f = nullptr; b->sb_f = nullptr;
     b->tab_n = 0;
     b->tab_screen = 0;
     const long double PI2 = 6.283185307179586476925286766559005768L;
@@ -780,7 +765,7 @@ static int ensure_ref_tables(muse_batch *b, int64_t ld) {
     CU(cudaMalloc(&b->twn, sizeof(cd) * (size_t)(M / 2 + 1)));
     CU(cudaMemcpyAsync(b->twM, twM.data(), sizeof(cd) * twM.size(), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(b->twn, twn.data(), sizeof(cd) * (size_t)(M / 2 + 1), cudaMemcpyHostToDevice, st));
-    std::vector<cf> twp, twi, twide;
+    std::vector<cf> twp, twi;
     std::vector<float2> swtw;
     if (want_screen) {
         if (screen_is_big(b->log2m)) {
@@ -790,17 +775,9 @@ static int ensure_ref_tables(muse_batch *b, int64_t ld) {
             });
             CU(cudaMalloc(&b->twi_f, sizeof(cf) * twi.size()));
             CU(cudaMemcpyAsync(b->twi_f, twi.data(), sizeof(cf) * twi.size(), cudaMemcpyHostToDevice, st));
-            if (b->log2m == 13 && getenv("MUSE_WIDE13")) {
-                twide.resize(ScreenWideCfg::TW_TOTAL);
-                fill_wide_twiddles(twide.data(), [&](long long num, long long den) {
-                    return cf{(float)cosl(-PI2 * num / den), (float)sinl(-PI2 * num / den)};
-                });
-                CU(cudaMalloc(&b->twide_f, sizeof(cf) * twide.size()));
-                CU(cudaMemcpyAsync(b->twide_f, twide.data(), sizeof(cf) * twide.size(), cudaMemcpyHostToDevice, st));
-            }
         }
         twp.resize((size_t)M + 64);
-        fill_pass_twiddles(b->log2m, screen_log2p(b->log2m), twp.data(), [&](long long num, long long den) {
+        fill_pass_twiddles(b->log2m, 5, twp.data(), [&](long long num, long long den) {      // radix-32 passes in every screening kernel
             return cf{(float)cosl(-PI2 * num / den), (float)sinl(-PI2 * num / den)};
         });
         swtw.resize((size_t)M / 2);
@@ -1369,20 +1346,12 @@ static int run_select(muse_batch *b, const RunArgs &a, int apply_filter, int64_t
 
 static cudaError_t launch_screen(const muse_batch *b, const ScreenParams &p, cudaStream_t st) {
     if (b->log2m == 10) return launch_screen_warp(p, b->ctx->sm_count, st);
-    // MUSE_WIDE13=1: the 512-thread, 64-register variant for n = 16384 (muse_screen_wide.cuh).  Measured SLOWER than the
-    // 256-thread kernel (56.8 ms against 45.9 ms per 1.25 M x 10080): both issue at 39 % of peak, so its 24 % more
-    // instructions decide; kept as the measured record of that design, off by default.
-    if (b->log2m == 13 && b->twide_f && getenv("MUSE_WIDE13")) {
-        ScreenParams pw = p;
-        pw.twi = b->twide_f;
-        return launch_screen_wide(pw, b->ctx->sm_count, st);
-    }
     if (screen_is_big(b->log2m)) return launch_screen_big(b->log2m, p, b->ctx->sm_count, st);
     if (b->log2m == 6) return launch_screen_sub1(p, b->ctx->sm_count, st);
     if (b->log2m == 7) return launch_screen_sub2(p, b->ctx->sm_count, st);
-    if (b->log2m == 8 && !block_small()) return launch_screen_sub3(p, b->ctx->sm_count, st);
-    if (b->log2m == 9 && !block_small()) return launch_screen_sub4(p, b->ctx->sm_count, st);
-    return launch_screen_block(b->log2m, p, b->ctx->sm_count, st);
+    if (b->log2m == 8) return launch_screen_sub3(p, b->ctx->sm_count, st);
+    if (b->log2m == 9) return launch_screen_sub4(p, b->ctx->sm_count, st);
+    return cudaErrorInvalidValue;
 }
 
 static int ensure_lower(muse_batch *b) {
@@ -1579,7 +1548,7 @@ static int score_fused(muse_batch *b, const RunArgs &a) {
     ScreenParams sp = screen_params(b);
     const float thr_lo = a.threshold > 0 ? (float)a.threshold * 0.999999f : 0.f;   // never above the fp64 threshold
     int rc = MUSE_OK;
-    if (b->prescreened) {      // muse_multi_run: this query's bounds and cut-off came out of the multi-query launch
+    if (b->prescreened) {      // muse_multi_run: this query's bounds and cut-off came out of the tensor-core launch group
         b->prescreened = 0;
     } else {
         rc = arm_refinement(b, sp, thr_lo, a.max_lag, a.top_n, a.threshold);
@@ -1587,7 +1556,7 @@ static int score_fused(muse_batch *b, const RunArgs &a) {
         CU(launch_screen(b, sp, st));
         b->timing.n_launches += 2;
     }
-    TIMING_EVENT(b, 1, st);
+    CU(cudaEventRecord(b->ev[1], st));
     if (!a.list_only) CU(cudaMemsetAsync(b->d_score, 0xff, sizeof(double) * (size_t)S, st));      // NaN = "cannot be in the result"
     const unsigned blocks = (unsigned)((S + 255) / 256);
     survivors_cut_kernel<<<blocks, 256, 0, st>>>(b->d_U, S, b->d_cut, b->d_list, b->d_counters + 2);
@@ -1631,14 +1600,14 @@ static int score_fused_grouped(muse_batch *b, const RunArgs &a) {
     }
     CU(launch_screen(b, sp, st));
     b->timing.n_launches += 2;
-    TIMING_EVENT(b, 1, st);
+    CU(cudaEventRecord(b->ev[1], st));
     CU(cudaMemsetAsync(b->d_score, 0xff, sizeof(double) * (size_t)S, st));      // NaN = "not its group's representative"
     if (!running) {
         group_lower_bound_kernel<<<blocks, 256, 0, st>>>(gt, kc, b->d_L, S, b->d_slot);
         b->timing.n_launches++;
     }
     const unsigned *cut_bits = nullptr;
-    if (running && a.group_cut && a.top_n > 0 && a.top_n < 0x7fffffff && !getenv("MUSE_NO_GROUP_CUT")) {
+    if (running && a.group_cut && a.top_n > 0 && a.top_n < 0x7fffffff) {
         group_uncertain_kernel<<<blocks, 256, 0, st>>>(gt, b->d_U, b->d_W, S, b->d_slot);
         group_cut_count_kernel<<<(unsigned)((gt.slots + 255) / 256), 256, 0, st>>>(gt, a.threshold, b->d_cut + 4);
         group_cut_find_kernel<<<1, 32, 0, st>>>(b->d_cut + 4, (int)a.top_n, b->d_cut);
@@ -1679,7 +1648,7 @@ static int run_scores(muse_batch *b, const RunArgs &a) {
     b->timing_pending = 0;
     b->signed_run = a.signed_scores ? 1 : 0;
     cudaStream_t st = bstream(b);
-    TIMING_EVENT(b, 0, st);
+    CU(cudaEventRecord(b->ev[0], st));
     CU(cudaMemsetAsync(b->d_counters, 0, sizeof(unsigned long long) * 4, st));
     // screening needs: a kernel for this FFT size, an ungrouped unsigned run, a sign filter that
     // unsigned scores can pass, and a store big enough to be worth two extra round trips
@@ -1695,7 +1664,7 @@ static int run_scores(muse_batch *b, const RunArgs &a) {
         b->fused_run = 2;          // statistics as a fused run; its exact list is already complete
         rc = score_fused_grouped(b, a);
         if (rc) return rc;
-        TIMING_EVENT(b, 2, st);
+        CU(cudaEventRecord(b->ev[2], st));
         return MUSE_OK;
     }
     if (screen) {
@@ -1703,19 +1672,18 @@ static int run_scores(muse_batch *b, const RunArgs &a) {
         b->fused_run = 1;
         rc = score_fused(b, a);
         if (rc) return rc;
-        TIMING_EVENT(b, 2, st);
+        CU(cudaEventRecord(b->ev[2], st));
         return MUSE_OK;
     }
     b->timing.mode = MUSE_MODE_EXACT;
     rc = score_exact_all(b, a.signed_scores, nullptr, b->g->size);
     if (rc) return rc;
-    TIMING_EVENT(b, 1, st);
-    TIMING_EVENT(b, 2, st);
+    CU(cudaEventRecord(b->ev[1], st));
+    CU(cudaEventRecord(b->ev[2], st));
     return MUSE_OK;
 }
 
-// Elapsed times between the run's events.  The batches of a multi-query launch record none (TIMING_EVENT), so there is
-// nothing to read for them; a failed query of an event must not stay behind as the runtime's last error.
+// Elapsed times between the run's events; a failed query of an event must not stay behind as the runtime's last error.
 static void read_timing_events(muse_batch *b) {
     float *out[4] = {&b->timing.total_ms, &b->timing.score_ms, &b->timing.rescore_ms, &b->timing.select_ms};
     const int from[4] = {0, 0, 1, 2}, to[4] = {3, 1, 2, 3};
@@ -1727,10 +1695,6 @@ static void read_timing_events(muse_batch *b) {
 }
 
 static int finish_timing(muse_batch *b) {
-    if (b->use_aux) {      // a query of a multi-query launch: no events were recorded for this run
-        CU(cudaStreamSynchronize(bstream(b)));
-        return MUSE_OK;
-    }
     cudaStream_t st = bstream(b);
     CU(cudaEventRecord(b->ev[3], st));
     CU(cudaEventSynchronize(b->ev[3]));
@@ -1740,11 +1704,10 @@ static int finish_timing(muse_batch *b) {
 
 static int queue_topn_records(muse_batch *b, const RunArgs &a, muse_partial *d_out, int64_t capacity);
 
-// Ungrouped runs with a device-side top-N, in two halves so that several batches can share ONE synchronisation
-// (muse_multi_run): queue = scores, filter, rank, copy of the top_n records into the batch's pinned mailbox;
-// finish (after the stream has been synchronised) = read the mailbox, or -- when the candidate list was too long for
-// the device-side select, or the fused path's exact launch did not cover its list -- finish on the host path from
-// the scores already on the device.
+// Ungrouped runs with a device-side top-N, in two halves: queue = scores, filter, rank, copy of the top_n records into
+// the batch's pinned mailbox; finish (after the stream has been synchronised) = read the mailbox, or -- when the
+// candidate list was too long for the device-side select, or the fused path's exact launch did not cover its list --
+// finish on the host path from the scores already on the device.
 static bool device_topn_applies(const muse_batch *b, const RunArgs &a) {
     return a.n_key_cols == 0 && a.top_n > 0 && a.top_n <= 65536 && b->g->size > 0;
 }
@@ -1755,7 +1718,7 @@ static int device_topn_queue(muse_batch *b, const RunArgs &a) {
     if (rc) return rc;
     cudaStream_t st = bstream(b);
     CU(cudaMemcpyAsync(b->h_pin + 64, d_rec, sizeof(muse_partial) * (size_t)a.top_n, cudaMemcpyDeviceToHost, st));
-    TIMING_EVENT(b, 3, st);
+    CU(cudaEventRecord(b->ev[3], st));
     return MUSE_OK;
 }
 
@@ -1770,7 +1733,6 @@ static int device_topn_finish(muse_batch *b, const RunArgs &a, double *scores, i
             series_idx[k] = h_rec[k].series_idx;
         }
         *n_out = k;
-        if (b->use_aux) return MUSE_OK;            // a query of a multi-query launch: no timing events were recorded
         muse_timing t;
         return muse_batch_last_timing(b, &t);      // settles timing_pending (events are complete)
     }
@@ -1888,8 +1850,8 @@ static int queue_topn_records(muse_batch *b, const RunArgs &a_in, muse_partial *
     CU(cudaGetLastError());
     // statistics and the end-of-run event are picked up by muse_batch_last_timing
     CU(cudaMemcpyAsync(b->h_pin, b->d_counters, sizeof(unsigned long long) * 4, cudaMemcpyDeviceToHost, st));
-    TIMING_EVENT(b, 3, st);
-    b->timing_pending = b->use_aux ? 0 : 1;
+    CU(cudaEventRecord(b->ev[3], st));
+    b->timing_pending = 1;
     return MUSE_OK;
 }
 
@@ -2024,56 +1986,6 @@ extern "C" int muse_merge_partials(const muse_partial *parts, int64_t n_parts, i
 // ------------------------------------------------------------------------------------
 // many reference queries against one resident store (SURVEY 8f rank 2, BASELINE.json configs[4])
 // ------------------------------------------------------------------------------------
-// Round-1 form: one NewBatch + Run per reference on the resident slab, inside the library -- the store, its
-// row statistics and the run scratch (context pool) are shared, results of query q land in row q of the
-// outputs.  Every query still streams the slab once (HBM-bound, 2.3 ms per 1 M x 1440 series); the multi-query
-// bound pass that reads the slab once for ALL queries is DESIGN.md section 8's next step.
-// Up to ScreenMultiCfg::QC queries in ONE pass over the slab: every batch gets its cut-off state armed, the
-// multi-query kernel fills each batch's bounds (d_U) and cut-off, and each batch is marked `prescreened` so that
-// its next fused run starts at the tail (survivors -> exact fp64 kernel -> filter -> top-N).
-static int tc_bounds_queue(muse_ctx *ctx, muse_group *g, muse_batch **bs, int nq);
-
-static int screen_multi(muse_ctx *ctx, muse_batch **bs, int nq, int64_t max_lag, int64_t top_n, double threshold, bool tensor_cores) {
-    cudaStream_t st = ctx->stream;
-    std::vector<MultiQuery> hq((size_t)nq);
-    ScreenParams sp0;
-    const float thr_lo = threshold > 0 ? (float)threshold * 0.999999f : 0.f;
-    for (int q = 0; q < nq; q++) {
-        muse_batch *b = bs[q];
-        int rc = ensure_scratch(b);
-        if (rc) return rc;
-        ScreenParams sp = screen_params(b);
-        rc = arm_refinement(b, sp, thr_lo, max_lag, top_n, threshold);
-        if (rc) return rc;
-        if (q == 0) sp0 = sp;
-        MultiQuery &m = hq[(size_t)q];
-        memset(&m, 0, sizeof(m));
-        m.sw = b->sw_f;
-        m.sx = b->sx_f;
-        m.x_mid = b->x_mid;
-        m.a_mid = b->a_mid;
-        m.cut = b->d_cut;
-        m.out_U = b->d_U;
-    }
-    // the query table lives with the context (stream-ordered reuse: copy and launch go down the same stream; a copy
-    // from pageable memory has left the host buffer when the call returns), so nothing here waits for the kernel
-    if (!ctx->d_multi_q) CU(cudaMalloc(&ctx->d_multi_q, sizeof(MultiQuery) * (size_t)MUSE_MULTI_GROUP));
-    MultiQuery *d_q = static_cast<MultiQuery *>(ctx->d_multi_q);
-    CU(cudaMemcpyAsync(d_q, hq.data(), sizeof(MultiQuery) * (size_t)nq, cudaMemcpyHostToDevice, st));
-    if (tensor_cores) {
-        // bounds of all queries as one bf16 contraction on the tensor cores, then ONE pass over the store for the second
-        // stages of all of them
-        int rc = tc_bounds_queue(ctx, bs[0]->g, bs, nq);
-        if (rc) return rc;
-        if (!ctx->d_multi_next) CU(cudaMalloc(&ctx->d_multi_next, sizeof(unsigned)));
-        CU(launch_refine_multi(sp0, d_q, nq, ctx->sm_count, ctx->d_multi_next, st));
-    } else {
-        CU(launch_screen_multi(sp0, d_q, nq, ctx->sm_count, st));
-    }
-    for (int q = 0; q < nq; q++) bs[q]->prescreened = 1;
-    return MUSE_OK;
-}
-
 // The bounds of up to TcCfg::TN queries (batches bs[0 .. nq), FFT length 2048, tables built) against the whole store, as
 // one bf16 contraction on the tensor cores: magnitudes of every series -> tiles, the queries' weights -> tiles, GEMM with
 // the bound's epilogue into every batch's d_U.  Everything is queued on the context's stream.
@@ -2412,23 +2324,21 @@ extern "C" int muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, 
     if (top_n > 0 && (!scores || !lags || !series_idx)) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run: NULL output");
     if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run: bad key columns");
     CU(cudaSetDevice(ctx->device));
-    // the one-pass multi-query kernel exists for the shape the single-query warp kernel serves (FFT length 2048,
-    // ungrouped, unsigned scores, a sign filter unsigned scores can pass, a store worth screening, a device-side
-    // top-N); everything else is n_refs x (NewBatch + Run) on the resident store
+    // the tensor-core path (multi_run_tc_group, up to MUSE_MULTI_GROUP queries per pass over the store) exists for the
+    // shape the single-query warp kernel serves (FFT length 2048, ungrouped, unsigned scores, a sign filter unsigned
+    // scores can pass, a store worth screening, a device-side top-N); everything else -- and a group of one query -- is
+    // NewBatch + Run per reference on the resident store: the store, its row statistics and the run scratch (context
+    // pool) are shared, and results of query q land in row q of the outputs
     const bool one_pass = n_key_cols == 0 && mode != MUSE_MODE_EXACT && sign_filter != MUSE_SIGN_NEG && ref_len == g->N &&
                           next_pow2(ref_len) == 2048 && top_n > 0 && top_n <= 65536 &&
                           top_n * 4 <= g->size && (g->size >= 16384 || mode == MUSE_MODE_SCREEN) && n_refs > 1;
-    // the bounds of a launch's queries: one bf16 contraction on the tensor cores for up to 256 queries at a time
-    // (MUSE_MULTI_TC=0: the fp32 kernel, 16 queries per pass over the store)
     ctx->multi_refined = ctx->multi_rescored = 0;
-    const char *tc_env = getenv("MUSE_MULTI_TC");
-    const bool tensor_cores = one_pass && !(tc_env && atoi(tc_env) == 0);
-    const int QC = tensor_cores ? MUSE_MULTI_GROUP : ScreenMultiCfg::QC;
+    const int QC = one_pass ? MUSE_MULTI_GROUP : MUSE_MULTI_SEPARATE;
     std::vector<muse_batch *> bs((size_t)QC), made((size_t)QC);
     std::vector<int64_t> which((size_t)QC);
     for (int64_t q0 = 0; q0 < n_refs; q0 += QC) {
         const int nq = (int)std::min<int64_t>(QC, n_refs - q0);
-        if (tensor_cores && nq > 1) {
+        if (one_pass && nq > 1) {
             int rct = multi_run_tc_group(ctx, g, refs + (size_t)q0 * (size_t)ref_len, nq, ref_len, max_lag, top_n, threshold, sign_filter,
                                          scores + (size_t)q0 * (size_t)top_n, lags + (size_t)q0 * (size_t)top_n,
                                          series_idx + (size_t)q0 * (size_t)top_n, n_out + q0);
@@ -2437,7 +2347,7 @@ extern "C" int muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, 
         }
         int live = 0, rc = MUSE_OK;
         int n_made = 0;
-        // the references of the launch: ONE upload (rows at the slab's pitch, pad columns zero), then queued back to
+        // the references of the group: ONE upload (rows at the slab's pitch, pad columns zero), then queued back to
         // back, ONE round trip
         if (ref_len == g->N && (ctx->d_multi_ld != g->ld || ctx->d_multi_n != g->N)) {
             cudaFree(ctx->d_multi_refs);
@@ -2474,42 +2384,10 @@ extern "C" int muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, 
                 which[live++] = q0 + i;
             }
         }
-        bool queued = false;
-        if (rc == MUSE_OK && one_pass && live > 1) {
-            rc = screen_multi(ctx, bs.data(), live, max_lag, top_n, threshold, tensor_cores);
-            // the tails of the queries are independent and small (a few thousand series each): every batch queues its
-            // tail on its own stream behind the multi-query kernel, so they share the GPU instead of taking turns
-            cudaEvent_t screened = nullptr;
-            cudaError_t e = cudaEventCreateWithFlags(&screened, cudaEventDisableTiming);
-            if (e == cudaSuccess) e = cudaEventRecord(screened, ctx->stream);
-            for (int i = 0; i < live && rc == MUSE_OK && e == cudaSuccess; i++) {
-                muse_batch *b = bs[i];
-                if (!b->aux) e = cudaStreamCreateWithFlags(&b->aux, cudaStreamNonBlocking);
-                if (e == cudaSuccess) e = cudaStreamWaitEvent(b->aux, screened, 0);
-                if (e != cudaSuccess) break;
-                b->use_aux = 1;
-                RunArgs a{nullptr, 0, max_lag, top_n, threshold, sign_filter, MUSE_MODE_SCREEN, 0};
-                rc = device_topn_queue(b, a);
-            }
-            for (int i = 0; i < live; i++)
-                if (bs[i]->use_aux && cudaStreamSynchronize(bs[i]->aux) != cudaSuccess && e == cudaSuccess) e = cudaErrorUnknown;
-            if (screened) cudaEventDestroy(screened);
-            if (e != cudaSuccess && rc == MUSE_OK) rc = fail(MUSE_ERR_CUDA, "muse_multi_run: %s", cudaGetErrorString(e));
-            queued = rc == MUSE_OK;
-        }
         for (int i = 0; i < live; i++) {
             const int64_t q = which[i];
-            if (rc == MUSE_OK && queued) {
-                RunArgs a{nullptr, 0, max_lag, top_n, threshold, sign_filter, MUSE_MODE_SCREEN, 0};
-                n_out[q] = 0;
-                rc = device_topn_finish(bs[i], a, scores + (size_t)q * (size_t)top_n, lags + (size_t)q * (size_t)top_n,
-                                        series_idx + (size_t)q * (size_t)top_n, n_out + q);
-                const unsigned long long *h_n = reinterpret_cast<const unsigned long long *>(bs[i]->h_pin);
-                ctx->multi_rescored += (int64_t)h_n[2];
-                ctx->multi_refined += (int64_t)h_n[3];
-            } else if (rc == MUSE_OK)
-                rc = muse_batch_run_ex(bs[i], key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter,
-                                       bs[i]->prescreened ? MUSE_MODE_SCREEN : mode, 0,
+            if (rc == MUSE_OK)
+                rc = muse_batch_run_ex(bs[i], key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0,
                                        scores ? scores + (size_t)q * (size_t)top_n : nullptr, lags ? lags + (size_t)q * (size_t)top_n : nullptr,
                                        series_idx ? series_idx + (size_t)q * (size_t)top_n : nullptr, n_out + q);
             muse_batch_destroy(bs[i]);

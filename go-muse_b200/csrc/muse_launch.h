@@ -6,8 +6,6 @@
 
 #include "muse_exact.cuh"
 #include "muse_screen_big.cuh"
-#include "muse_screen_wide.cuh"
-#include "muse_screen_block.cuh"
 #include "muse_screen_sub.cuh"
 #include "muse_screen_multi.cuh"
 #include "muse_bounds_tc.cuh"
@@ -20,9 +18,8 @@ cudaError_t launch_exact_batch(int mode, const ExactParams *d_table, int nq, int
 // points per thread of the exact kernel for each FFT size (fixes the twiddle layout of ExactParams::twM)
 inline int exact_log2p(int log2m) { return log2m < 4 ? log2m : 4; }
 
-// fp32 screening + fused second stage: warp kernel (n = 2048), block kernel (n = 512, 1024, 4096 .. 16384)
+// fp32 screening + fused second stage: warp kernel (n = 2048)
 cudaError_t launch_screen_warp(const ScreenParams &p, int sm_count, cudaStream_t st);
-cudaError_t launch_screen_block(int log2m, const ScreenParams &p, int sm_count, cudaStream_t st);
 // n = 128 .. 1024: sixteen .. two series per warp (muse_screen_sub.cuh)
 cudaError_t launch_screen_sub1(const ScreenParams &p, int sm_count, cudaStream_t st);
 cudaError_t launch_screen_sub2(const ScreenParams &p, int sm_count, cudaStream_t st);
@@ -35,10 +32,6 @@ cudaError_t launch_screen_big13_a(int nz, const ScreenParams &p, int sm_count, c
 cudaError_t launch_screen_big13_b(int nz, const ScreenParams &p, int sm_count, cudaStream_t st);
 cudaError_t launch_screen_big13_c(int nz, const ScreenParams &p, int sm_count, cudaStream_t st);
 cudaError_t launch_screen_big13_d(int nz, const ScreenParams &p, int sm_count, cudaStream_t st);
-// n = 16384 at twice the occupancy (muse_screen_wide.cuh); its twiddle tables are fill_wide_twiddles'
-cudaError_t launch_screen_wide(const ScreenParams &p, int sm_count, cudaStream_t st);
-// the same pass for up to ScreenMultiCfg::QC reference queries at once (n = 2048)
-cudaError_t launch_screen_multi(const ScreenParams &p, const MultiQuery *d_queries, int nq, int sm_count, cudaStream_t st);
 
 // the second stage for up to RefineMultiCfg::QMAX queries with precomputed bounds (n = 2048)
 cudaError_t launch_refine_multi(const ScreenParams &p, const MultiQuery *d_queries, int nq, int sm_count, unsigned *d_next, cudaStream_t st);

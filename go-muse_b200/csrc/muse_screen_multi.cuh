@@ -1,24 +1,10 @@
-// muse_screen_multi.cuh -- the fused fp32 screening pass of muse_screen.cuh for SEVERAL reference queries
-// in ONE pass over the slab (SURVEY 8f rank 2 / BASELINE.json configs[4]: many references, one store).
+// muse_screen_multi.cuh -- many reference queries in ONE pass over the slab (SURVEY 8f rank 2 / BASELINE.json configs[4]:
+// many references, one store).
 //
-// go-muse builds one Batch per reference (muse_batch.go:23-52), so Q queries stream the store Q times and
-// transform every series Q times.  Nothing about a series' spectrum depends on the reference: here a warp
-// loads its row and runs the forward FFT_1024 ONCE, keeps the 1024 magnitudes |2Y_k| in registers (as the 16
-// mirror pairs + the middle bin of muse_screen.cuh) and the spectrum itself in shared memory (the warp's row buffer),
-// and then walks the queries of the launch:
-//     U_q = (1/n) sum_f |Y_f| |X_q,f| / std * (1 + 1e-5) + slack      (16 packed FMAs against the query's weights,
-//                                                                       which sit in shared memory for the whole launch)
-// and, when U_q reaches query q's RUNNING top-N cut-off, the second stage of muse_screen.cuh for that query
-// (spectrum reloaded from the stash, conj(Y)*X_q, inverse FFT_1024, maxima inside / outside the lag window).
-// Every query has its own cut-off state (muse_batch::d_cut) and its own bound array (muse_batch::d_U): after the
-// launch each query's batch is exactly where a single-query run is after ITS screening kernel, and the
-// unchanged tail (survivors -> exact fp64 kernel -> filter -> top-N) finishes it.  The error budget of the
-// bounds is that of muse_screen.cuh (the same operations on the same values; only the order of the 33-term
-// accumulation differs, which the 1e-5 relative slack covers 30 times over).
-//
-// Cost per (series, query): 8 LDS.128 + 16 FFMA2 + a 5-step butterfly ~ 50 warp instructions (four queries at a
-// time, so that their dependency chains overlap), against ~1000 for the row's load + transform, which is paid
-// once per launch instead of once per query.
+// go-muse builds one Batch per reference (muse_batch.go:23-52), so Q queries stream the store Q times and transform
+// every series Q times.  Nothing about a series' spectrum depends on the reference: the bounds of all queries come from
+// one bf16 contraction on the tensor cores (muse_bounds_tc.cuh), and refine_multi_kernel below transforms each row ONCE
+// and runs the second stage for every query whose bound needs it.
 #pragma once
 
 #include "muse_screen.cuh"
@@ -26,35 +12,13 @@
 namespace muse {
 
 struct MultiQuery {
-    const float4 *sw;     // the query's (w_k, A[k], A[M-k]) table (only the weights are read here)
+    const float4 *sw;     // the query's (w_k, A[k], A[M-k]) table (refine_multi_kernel does not read it)
     const float4 *sx;     // (Xt[k], Xt[M-k]) in fp32, k < M/2
     cf x_mid;             // Xt[M/2]
     float a_mid;          // A[M/2]
     int pad;
     unsigned *cut;        // the query's cut-off state: [0] running cut-off bits, [2..3] refined count, [4..] histogram
     float *out_U;         // [count] upper bound on the score for this query
-};
-
-#ifndef MUSE_MULTI_WARPS
-#define MUSE_MULTI_WARPS 10   // measured (16 queries x 1 M series): 7 warps + separate stash 8.04 ms, 12 warps 7.93 ms, 10 warps 7.32 ms
-#endif
-struct ScreenMultiCfg {
-    using G = Geo<10, 5>;
-    static constexpr int MAX_WARPS = MUSE_MULTI_WARPS;   // 168 registers per thread, no spills
-    static constexpr int QC = 16;               // queries per launch (their weights: 64 KB of shared memory)
-    static constexpr int NREF = ScreenWarpCfg::NREF;
-    static constexpr size_t SMEM_BUDGET = 227 * 1024;
-    static constexpr size_t EX_BYTES = ScreenWarpCfg::EX_BYTES;
-    static constexpr size_t STASH_BYTES = (size_t)G::M * sizeof(cf);
-    static constexpr size_t W_BYTES = (size_t)QC * (G::M / 2) * sizeof(cf) + 128;      // weights + A[M/2] per query
-    // one buffer per warp, three uses in turn: the row (bulk copy), the forward FFT exchange, the spectrum stash
-    static size_t row_bytes(int N) { const size_t r = ScreenWarpCfg::row_bytes(N); return r > STASH_BYTES ? r : STASH_BYTES; }
-    static size_t warp_bytes(int N) { return row_bytes(N); }
-    static int warps(int N) {
-        const size_t w = (SMEM_BUDGET - NREF * EX_BYTES - W_BYTES) / warp_bytes(N);
-        return (int)(w > MAX_WARPS ? MAX_WARPS : w);
-    }
-    static size_t smem_bytes(int N) { return (size_t)warps(N) * warp_bytes(N) + NREF * EX_BYTES + W_BYTES; }
 };
 
 #if defined(__CUDACC__)
@@ -67,259 +31,6 @@ __device__ __forceinline__ void cut_count_and_raise_at(unsigned *cut, int top_n,
     q.top_n = top_n;
     cut_count_and_raise(q, L, t);
 }
-
-template <int NZ>
-__global__ void __launch_bounds__(ScreenMultiCfg::MAX_WARPS * 32, 1)
-score_screen_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queries, const int nq, const unsigned warp_bytes,
-                          const unsigned row_bytes) {
-    using C = ScreenMultiCfg;
-    using G = typename C::G;
-    constexpr int P = 32, M = G::M;
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    __shared__ __align__(8) unsigned long long bars[C::MAX_WARPS];
-    __shared__ unsigned ex_locks[C::NREF];
-
-    const int w = threadIdx.x >> 5;
-    const int t = threadIdx.x & 31;
-    const int nwarps = (int)(blockDim.x >> 5);
-    const int count = (int)prm.count;
-    const int stride = (int)(gridDim.x * nwarps);
-    const int pos0 = (int)(blockIdx.x * nwarps) + w;
-    unsigned char *buf = smem_raw + (size_t)w * warp_bytes;
-    const cd *rowc = reinterpret_cast<const cd *>(buf);
-    cf *sm = reinterpret_cast<cf *>(buf);                       // forward exchange: the row buffer itself
-    cf *stash = reinterpret_cast<cf *>(buf);                    // ... and then the series' spectrum, slot j of lane t at [32 j + t]
-    unsigned char *refbase = smem_raw + (size_t)nwarps * warp_bytes;
-    cf *sA = reinterpret_cast<cf *>(refbase + (size_t)C::NREF * C::EX_BYTES);     // [nq][512] (A[k], A[M-k])
-    float *sAmid = reinterpret_cast<float *>(sA + (size_t)C::QC * (M / 2));       // [nq] A[M/2]
-    const int N = prm.N;
-    const int Nh = (N + 1) >> 1;      // complex slots holding samples (odd N: the pad column of the last one holds the row's mean, RowStat)
-    const unsigned bar = smem_u32(&bars[w]);
-    const int partner = (P - t) & (P - 1);
-    const bool lane0 = (t == 0);
-    const bool last_in = t + (NZ - 1) * 32 < Nh;
-
-    if (threadIdx.x < C::NREF) ex_locks[threadIdx.x] = 0u;
-    if (t == 0) {
-        mbar_init(bar, 1);
-        if (pos0 < count) bulk_load(smem_u32(buf), prm.slab + (int64_t)pos0 * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
-    }
-    // weights of query q for the mirror pairs k = t + 32 j: the pairs of slots j = 2 j2 and 2 j2 + 1 share one 16-byte
-    // entry [q][j2][t] (one LDS.128 per two packed FMAs)
-    for (int i = threadIdx.x; i < nq * (M / 2); i += blockDim.x) {
-        const int q = i >> 9, k = i & (M / 2 - 1), j = k >> 5, tt = k & 31;
-        const float4 s = queries[q].sw[k];
-        sA[((q * (P / 4) + (j >> 1)) * 32 + tt) * 2 + (j & 1)] = cf{s.z, s.w};
-    }
-    if ((int)threadIdx.x < nq) sAmid[threadIdx.x] = queries[threadIdx.x].a_mid;
-    // lane q looks after query q: its cut-off word and its row of bounds
-    unsigned *my_cut = t < nq ? queries[t].cut : nullptr;
-    float *my_out = t < nq ? queries[t].out_U : nullptr;
-    __syncthreads();
-
-    for (unsigned pp = (unsigned)pos0; (int)(pp & 0x7fffffffu) < count; pp = ((pp & 0x7fffffffu) + (unsigned)stride) | (~pp & 0x80000000u)) {
-        const int pos = (int)(pp & 0x7fffffffu);
-        const unsigned phase = pp >> 31;
-        // the running cut-offs of all queries, read at the top of the iteration and consumed after the transform
-        unsigned cut_raw = 0x7f800000u;     // +inf: no such query
-        if (my_cut) cut_raw = ld_relaxed_u32(my_cut);
-        const RowStat rs = prm.row_stat[pos];
-        const double mu = rs.mean;
-        mbar_wait(bar, phase);
-
-        cf v[P];
-#pragma unroll
-        for (int r = 0; r < P; r++) {
-            if (r < NZ) {
-                const cd x = (r == NZ - 1 && !last_in) ? cd{mu, mu} : rowc[t + r * 32];
-                v[r] = cf{(float)(x.x - mu), (float)(x.y - mu)};
-            } else {
-                v[r] = cf{0.f, 0.f};
-            }
-        }
-        __syncwarp();
-        const int next = pos + stride;
-
-        // ---- forward FFT_1024 (as score_screen_warp_kernel) ----
-        Dft32Lead<NZ, float>::run(v);
-#pragma unroll
-        for (int j = 0; j < P; j++) {
-            cf val = v[Perm<P>::at(j)];
-            if (j > 0) val = cmul(val, prm.twp[(j - 1) * 32 + t]);
-            sm[G::pad(32 * t + j)] = val;
-        }
-        __syncwarp();
-        fft_pass_load<10, 5, 1, float>(v, sm, t);
-        __syncwarp();
-        Dft<P, float>::run(v);                          // v[Perm(j)] = Z[t + 32*j]
-
-        // ---- the spectrum goes to the stash: the same buffer once more (the exchange has been read, __syncwarp above;
-        //      every lane reads back only what it wrote) ----
-#pragma unroll
-        for (int j = 0; j < P; j++) stash[32 * j + t] = v[Perm<P>::at(j)];
-
-        // ---- magnitudes (|2Y_k|, |2Y_(M-k)|), k = t + 32*j, j < 16, and |Z_512| ----
-        cf mg[P / 2];
-#pragma unroll
-        for (int j = 0; j < P / 2; j++) {
-            const cf zk = v[Perm<P>::at(j)];
-            const cf zp = v[Perm<P>::at(P - 1 - j)];
-            const cf zs = v[Perm<P>::at((P - j) & (P - 1))];
-            cf src, zm;
-            src.x = lane0 ? zs.x : zp.x;
-            src.y = lane0 ? zs.y : zp.y;
-            zm.x = __shfl_sync(0xffffffffu, src.x, partner);
-            zm.y = __shfl_sync(0xffffffffu, src.y, partner);
-            const float4 s = prm.sw[t + 32 * j];
-            const cf zmc = cconj(zm);
-            const cf e = cadd(zk, zmc);
-            const cf o = cmul_negi(csub(zk, zmc));
-            const cf wo = cmul(o, cf{s.x, s.y});
-            const cf y1 = cadd(e, wo);
-            const cf y2 = csub(e, wo);
-            const cf q1 = pmul(y1, y1), q2 = pmul(y2, y2);
-            mg[j] = cf{sqrt_approx(q1.x + q1.y), sqrt_approx(q2.x + q2.y)};
-        }
-        float mg_mid;
-        {
-            const cf z = v[Perm<P>::at(P / 2)];
-            const cf q = pmul(z, z);
-            mg_mid = lane0 ? 2.f * sqrt_approx(q.x + q.y) : 0.f;      // k = 512: lane 0, slot 16
-        }
-
-        // ---- all bounds first (lane q keeps query q's), four queries per step: their 8 accumulation chains and 4
-        //      butterfly reductions overlap (one at a time leaves a warp waiting on 8 FFMA2 and 5 dependent shuffles) ----
-        float my_U = 2.f;
-        for (int q = 0; q < nq; q += 4) {
-            float acc4[4];
-#pragma unroll
-            for (int i = 0; i < 4; i++) {
-                const int qi = q + i < nq ? q + i : nq - 1;
-                const float4 *Aq = reinterpret_cast<const float4 *>(sA) + (size_t)qi * (M / 4) + t;
-                cf a0{0.f, 0.f}, a1{0.f, 0.f};
-#pragma unroll
-                for (int j2 = 0; j2 < P / 4; j2++) {
-                    const float4 wq = Aq[32 * j2];
-                    a0 = pfma(mg[2 * j2], cf{wq.x, wq.y}, a0);
-                    a1 = pfma(mg[2 * j2 + 1], cf{wq.z, wq.w}, a1);
-                }
-                acc4[i] = fmaf(mg_mid, sAmid[qi], (a0.x + a0.y) + (a1.x + a1.y));
-            }
-#pragma unroll
-            for (int off = 16; off > 0; off >>= 1) {
-#pragma unroll
-                for (int i = 0; i < 4; i++) acc4[i] += __shfl_xor_sync(0xffffffffu, acc4[i], off);
-            }
-#pragma unroll
-            for (int i = 0; i < 4; i++) {
-                float U = acc4[i] * rs.rstd * 1.00001f + MUSE_SCREEN_SLACK;
-                if (!(U == U)) U = 2.f;
-                if (t == q + i) my_U = U;      // q + i >= nq: a duplicate of the last query on a lane without one
-            }
-        }
-        // ---- then the second stage for every query whose bound reaches ITS running cut-off (the magnitudes are dead
-        //      by now; consecutive refinements of one series run the same code back to back) ----
-        unsigned todo = __ballot_sync(0xffffffffu, t < nq && my_U >= __uint_as_float(cut_raw) && my_U < 1.5f);
-        while (todo) {
-            const int q = __ffs(todo) - 1;
-            todo &= todo - 1;
-            float U = __shfl_sync(0xffffffffu, my_U, q);
-            const float cut_now = __uint_as_float(__shfl_sync(0xffffffffu, cut_raw, q));
-            {
-                // ---- second stage for query q: spectrum back from the stash, conj(Y)*X_q, inverse FFT, window maxima ----
-                const MultiQuery mq = queries[q];
-                cf z[P];
-#pragma unroll
-                for (int j = 0; j < P; j++) z[Perm<P>::at(j)] = stash[32 * j + t];
-#pragma unroll
-                for (int j = 0; j < P / 2; j++) {
-                    const cf zk = z[Perm<P>::at(j)];
-                    const cf zp = z[Perm<P>::at(P - 1 - j)];
-                    const cf zs = z[Perm<P>::at((P - j) & (P - 1))];
-                    cf src, zm;
-                    src.x = lane0 ? zs.x : zp.x;
-                    src.y = lane0 ? zs.y : zp.y;
-                    zm.x = __shfl_sync(0xffffffffu, src.x, partner);
-                    zm.y = __shfl_sync(0xffffffffu, src.y, partner);
-                    const float4 s = prm.sw[t + 32 * j];
-                    const float4 x = mq.sx[t + 32 * j];
-                    cf ok, om;
-                    pointwise_pair(zk, zm, cf{s.x, s.y}, cf{x.x, x.y}, cf{x.z, x.w}, ok, om);
-                    cf rcv;
-                    rcv.x = __shfl_sync(0xffffffffu, om.x, partner);
-                    rcv.y = __shfl_sync(0xffffffffu, om.y, partner);
-                    z[Perm<P>::at(j)] = ok;
-                    cf &hi = z[Perm<P>::at(P - 1 - j)];
-                    hi.x = lane0 ? hi.x : rcv.x;
-                    hi.y = lane0 ? hi.y : rcv.y;
-                    if (j > 0) {
-                        cf &own = z[Perm<P>::at(P - j)];
-                        own.x = lane0 ? om.x : own.x;
-                        own.y = lane0 ? om.y : own.y;
-                    }
-                }
-                {
-                    cf &mid = z[Perm<P>::at(P / 2)];
-                    cf ok, om;
-                    pointwise_pair(mid, mid, cf{0.f, -1.f}, mq.x_mid, mq.x_mid, ok, om);
-                    mid.x = lane0 ? ok.x : mid.x;
-                    mid.y = lane0 ? ok.y : mid.y;
-                }
-                cf u[P];
-#pragma unroll
-                for (int j = 0; j < P; j++) u[j] = z[Perm<P>::at(j)];
-                Dft<P, float>::run(u);
-                {
-                    const int slot = ex_acquire(ex_locks, t, w);
-                    cf *smr = reinterpret_cast<cf *>(refbase + (size_t)slot * C::EX_BYTES);
-#pragma unroll
-                    for (int j = 0; j < P; j++) {
-                        cf val = u[Perm<P>::at(j)];
-                        if (j > 0) val = cmul(val, prm.twp[(j - 1) * 32 + t]);
-                        smr[G::pad(32 * t + j)] = val;
-                    }
-                    __syncwarp();
-                    fft_pass_load<10, 5, 1, float>(u, smr, t);
-                    ex_release(ex_locks, t, slot);
-                }
-                Dft<P, float>::run(u);
-                float m_in = 0.f, m_out = 0.f;
-                const int base = 2 * t - prm.win_lo;
-#pragma unroll
-                for (int j = 0; j < P; j++) {
-                    const cf r = u[Perm<P>::at(j)];
-                    const bool in0 = ((base + 64 * j) & (2 * M - 1)) <= prm.win_len;
-                    const bool in1 = ((base + 64 * j + 1) & (2 * M - 1)) <= prm.win_len;
-                    const float b0 = fabsf(r.y), b1 = fabsf(r.x);
-                    m_in = fmaxf(m_in, in0 ? b0 : 0.f);
-                    m_out = fmaxf(m_out, in0 ? 0.f : b0);
-                    m_in = fmaxf(m_in, in1 ? b1 : 0.f);
-                    m_out = fmaxf(m_out, in1 ? 0.f : b1);
-                }
-#pragma unroll
-                for (int off = 16; off > 0; off >>= 1) {
-                    m_in = fmaxf(m_in, __shfl_xor_sync(0xffffffffu, m_in, off));
-                    m_out = fmaxf(m_out, __shfl_xor_sync(0xffffffffu, m_out, off));
-                }
-                float L = -1.f;
-                U = refine_decide(U, m_in * rs.rstd, m_out * rs.rstd, L, 0);
-                if (t == 0) atomicAdd(reinterpret_cast<unsigned long long *>(mq.cut + 2), 1ull);
-                if (L >= prm.thr && L >= cut_now) cut_count_and_raise_at(mq.cut, prm.top_n, L, t);
-            }
-            if (t == q) my_U = U;
-        }
-        if (my_out) my_out[pos] = my_U;
-        // the stash is no longer needed: hand the buffer to the copy engine for the warp's next row.  (No prefetch under
-        // the transform as in 5.2: a separate stash costs 8 KB per warp, i.e. 7 warps per SM instead of 10 - 12, and this
-        // kernel is bound by latency hiding, not by DRAM.)
-        __syncwarp();
-        if (t == 0 && next < count) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            bulk_load(smem_u32(buf), prm.slab + (int64_t)next * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
-        }
-    }
-}
-
 
 // ---- second stage for up to 256 queries whose bounds were computed elsewhere (muse_bounds_tc.cuh) -------------------
 // One pass over the store: a warp loads its row, runs the forward FFT_1024 once, stashes the spectrum in shared memory

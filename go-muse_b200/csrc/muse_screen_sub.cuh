@@ -21,8 +21,6 @@
 // run bit-identical to the all-exact run (tests/test_gpu_screen.py).
 #pragma once
 
-#include <stdlib.h>
-
 #include "muse_screen.cuh"
 
 namespace muse {
@@ -41,7 +39,7 @@ struct ScreenSubCfg {
     // buffers of a warp's series sit a multiple of 128 bytes plus SKEW apart, which spreads the series over the
     // shared-memory banks: without it the 16 series of a warp at T = 2 (2 lanes x 16 bytes each) hit the same 8 banks on
     // every row read and every exchange.  Measured (kernel, 11.5 GB stores, skew 0 -> 8 T): n = 128 5.17 -> 2.48 ms,
-    // n = 256 3.08 -> 2.29 ms, n = 512 2.08 -> 1.92 ms, n = 1024 unchanged (MUSE_SUB_SKEW overrides, for such sweeps)
+    // n = 256 3.08 -> 2.29 ms, n = 512 2.08 -> 1.92 ms, n = 1024 unchanged
     static constexpr int SKEW = (8 * T) % 128;
     // The cheaper pair bound (muse_screen.cuh) pays where the kernel is bound by instruction issue and costs where it is
     // bound by HBM (it doubles the second stages).  Measured, bin-by-bin sum -> pair bound: n = 128 2.41 -> 2.21 ms,
@@ -49,13 +47,9 @@ struct ScreenSubCfg {
     static constexpr bool PAIR_BOUND = LOG2T <= 2;
     static constexpr size_t EX_STRIDE = EX_SERIES + SKEW;
     static constexpr size_t EX_BYTES = (size_t)GS * EX_STRIDE;
-    static size_t row_skew() {
-        static const long env = getenv("MUSE_SUB_SKEW") ? atol(getenv("MUSE_SUB_SKEW")) : -1;
-        return env >= 0 ? (size_t)env / 16 * 16 : (size_t)SKEW;
-    }
     static size_t row_bytes(int N) {
         const size_t r = ((size_t)N * 8 + 127) / 128 * 128;
-        return (r > EX_SERIES ? r : EX_SERIES) + row_skew();
+        return (r > EX_SERIES ? r : EX_SERIES) + SKEW;
     }
     static size_t warp_bytes(int N) { return (size_t)GS * row_bytes(N); }
     static int warps(int N) {

@@ -45,8 +45,7 @@ DefaultLabel = "uid"  # labels.go:7
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 # translation units of libmuse_b200.so: the C ABI and one file per family of kernel instantiations
-SOURCES = ["muse_api.cu", "kernels_exact.cu", "kernels_screen_warp.cu", "kernels_screen_block.cu",
-           "kernels_screen_big.cu", "kernels_screen_big13_a.cu", "kernels_screen_big13_b.cu", "kernels_screen_big13_c.cu",
+SOURCES = ["muse_api.cu", "kernels_exact.cu", "kernels_screen_warp.cu", "kernels_screen_big.cu", "kernels_screen_big13_a.cu", "kernels_screen_big13_b.cu", "kernels_screen_big13_c.cu",
            "kernels_screen_big13_d.cu", "kernels_screen_multi.cu", "kernels_bounds_tc.cu", "kernels_long.cu",
            "kernels_screen_sub1.cu", "kernels_screen_sub2.cu", "kernels_screen_sub3.cu", "kernels_screen_sub4.cu"]
 

@@ -209,16 +209,15 @@ int  muse_batch_xcorr(muse_batch *b, int64_t local_index, double *cc, int32_t *s
  * reference, top_n <= series / 4)
  * the screening bounds of up to 256 references at a time are ONE bf16 contraction on the tensor cores (tcgen05.mma,
  * muse_multi_bounds_tc), the second stages of all of them one launch over the store, and each query then finishes
- * on the exact fp64 kernel like a single run -- results identical to the separate runs.  MUSE_MULTI_TC=0 takes the
- * fp32 multi-query kernel instead (16 references per pass over the store).  Other shapes are served as separate
- * batches on the resident store. */
+ * on the exact fp64 kernel like a single run -- results identical to the separate runs.  Other shapes are served as
+ * separate batches on the resident store. */
 int  muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, int64_t n_refs, int64_t ref_len,
                     const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n, double threshold,
                     int32_t sign_filter, int32_t mode,
                     double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out);
 
 /* Totals of the context's last muse_multi_run over all its queries: (series, query) pairs that took the fp32 second stage and
- * pairs re-scored by the fp64 kernel (one-pass paths only; 0 otherwise). */
+ * pairs re-scored by the fp64 kernel (tensor-core path only; 0 otherwise). */
 int  muse_multi_last_stats(const muse_ctx *ctx, int64_t *n_refined, int64_t *n_rescored);
 
 /* Device times (ms) of the last launch group of the tensor-core multi-query path: [0] magnitudes of the store, [1] the bounds

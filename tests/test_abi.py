@@ -119,19 +119,6 @@ def test_big_kernel_phases_on_cpu(tmp_path):
     assert out.stdout.count(" ok") == 10 and "FAIL" not in out.stdout
 
 
-def test_wide_kernel_phases_on_cpu(tmp_path):
-    """score_screen_wide_kernel's phases (n = 16384 on 512 threads: radix 16, 16, 16 and a mirror-paired radix-2 pass,
-    split and conj(Y)*X in registers, transposed inverse 2, 16, 16, 16) thread by thread on the CPU against a
-    double-precision FFT."""
-    import subprocess
-    exe = str(tmp_path / "muse_emulate_wide")
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-I", os.path.join(ROOT, "go-muse_b200", "csrc"),
-                           "-I", "/usr/local/cuda/include", os.path.join(ROOT, "tests", "cpp", "emulate_wide.cpp"), "-o", exe])
-    out = subprocess.run([exe], capture_output=True, text=True)
-    assert out.returncode == 0, out.stdout
-    assert out.stdout.count(" ok") == 5 and "FAIL" not in out.stdout
-
-
 def test_merge_partials_against_a_model():
     """muse_merge_partials against a direct Python model on random shard outputs: group max across shards
     BEFORE the filter (muse_batch.go:87-89, SURVEY F2), ties by lowest global series index, filter

@@ -80,10 +80,9 @@ def test_screened_run_equals_exact_run(ctx, N):
 
 
 @pytest.mark.parametrize("N", [10080, 16384, 8195])
-def test_wide_kernel_variant_equals_exact_run(ctx, N, monkeypatch):
-    """The 512-thread variant of the n = 16384 screening kernel (MUSE_WIDE13=1; off by default because it measured slower):
-    ungrouped and grouped screened runs must still be the all-exact run, bit for bit."""
-    monkeypatch.setenv("MUSE_WIDE13", "1")
+def test_n16384_screened_runs_equal_exact_runs(ctx, N):
+    """The n = 16384 screening kernel on short, full and odd rows: ungrouped and grouped screened runs must be the
+    all-exact run, bit for bit, and the refined bounds must dominate the exact scores."""
     rng = np.random.default_rng(13 * N)
     S = 5000
     Y = _adversarial(rng, S, N)
@@ -366,9 +365,9 @@ def test_scratch_pool_survives_batch_churn(ctx):
 
 @pytest.mark.parametrize("N", [1440, 1030, 2048])
 def test_one_pass_multi_query_run_equals_exact_runs(ctx, N):
-    # muse_multi_run at FFT length 2048: score_screen_multi_kernel bounds ALL queries of a launch in one pass over
-    # the slab (16 per launch: 21 queries = 16 + 5), each query then finishes on its own tail.  Every query must
-    # return exactly what its own all-exact Batch.Run returns; a constant reference fails for itself only.
+    # muse_multi_run at FFT length 2048: the tensor-core path bounds ALL queries of a launch group (up to 256) in one bf16
+    # contraction and refines them in one pass over the slab, then finishes their tails with one launch per stage.
+    # Every query must return exactly what its own all-exact Batch.Run returns; a constant reference fails for itself only.
     rng = np.random.default_rng(N + 7)
     S, Q = 30000, 21
     Y = _adversarial(rng, S, N)
@@ -401,9 +400,9 @@ def test_one_pass_multi_query_run_equals_exact_runs(ctx, N):
 
 
 def test_multi_query_randomised_against_separate_runs(ctx):
-    # random shapes around the one-pass path's edges: query counts 2 .. 35 (chunks of 16 with remainders of 0, 1, 2),
-    # store sizes that do not divide by the warps of a block, top_n from 1 to a quarter of the store, thresholds from
-    # 0 to beyond every score, windows from 0 to all lags.  Reference: the same queries as separate screened batches
+    # random shapes around the tensor-core path's edges: query counts 2 .. 35 (one launch group each), store sizes that
+    # do not divide by the warps of a block, top_n from 1 to a quarter of the store, thresholds from 0 to beyond every
+    # score, windows from 0 to all lags.  Reference: the same queries as separate screened batches
     # (themselves pinned to the all-exact run by the tests above).
     rng = np.random.default_rng(2026)
     for case in range(8):
