@@ -37,14 +37,17 @@ static int fail(int code, const char *fmt, ...) {
     return code;
 }
 
-#define CU(call)                                                                                   \
-    do {                                                                                           \
-        cudaError_t e_ = (call);                                                                   \
-        if (e_ != cudaSuccess) {                                                                   \
-            (void)cudaGetLastError(); /* reported here: must not resurface in a later cudaGetLastError() check */ \
-            return fail(e_ == cudaErrorMemoryAllocation ? MUSE_ERR_OUT_OF_MEMORY : MUSE_ERR_CUDA,  \
-                        "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
-        }                                                                                          \
+// A failed runtime call: its error is reported here, so it must not resurface in a later cudaGetLastError() check.
+static int cuda_fail(cudaError_t e, const char *call, const char *file, int line) {
+    (void)cudaGetLastError();
+    return fail(e == cudaErrorMemoryAllocation ? MUSE_ERR_OUT_OF_MEMORY : MUSE_ERR_CUDA, "%s failed: %s (%s:%d)", call,
+                cudaGetErrorString(e), file, line);
+}
+
+#define CU(call)                                                                 \
+    do {                                                                         \
+        cudaError_t e_ = (call);                                                 \
+        if (e_ != cudaSuccess) return cuda_fail(e_, #call, __FILE__, __LINE__); \
     } while (0)
 
 extern "C" const char *muse_last_error(void) { return g_err; }
@@ -164,16 +167,6 @@ struct muse_batch : RunScratch {
 
 static inline cudaStream_t bstream(const muse_batch *b) { return b->ctx->stream; }
 
-struct DeviceGuard {
-    int prev;
-    bool ok;
-    explicit DeviceGuard(int dev) : prev(-1), ok(true) {
-        if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
-        if (prev != dev) ok = (cudaSetDevice(dev) == cudaSuccess);
-    }
-    ~DeviceGuard() {}
-};
-
 // ------------------------------------------------------------------------------------
 // context
 // ------------------------------------------------------------------------------------
@@ -195,11 +188,22 @@ extern "C" int muse_ctx_create(int device, muse_ctx **out) {
     return MUSE_OK;
 }
 
-static void scratch_free(RunScratch &r) {
+// the arrays of scratch_cap entries (ensure_scratch)
+static void free_scratch(RunScratch &r) {
     cudaFree(r.d_score); cudaFree(r.d_lag); cudaFree(r.d_slot);
     cudaFree(r.d_ckey); cudaFree(r.d_skey); cudaFree(r.d_cidx); cudaFree(r.d_sidx);
     cudaFree(r.d_clag); cudaFree(r.d_slag);
-    cudaFree(r.d_U); cudaFree(r.d_list); cudaFree(r.d_L); cudaFree(r.d_W);
+    r.d_clag = r.d_slag = nullptr;
+    cudaFree(r.d_U); cudaFree(r.d_list);
+    r.d_U = nullptr; r.d_list = nullptr;
+    r.d_score = nullptr; r.d_lag = nullptr; r.d_slot = nullptr;
+    r.d_ckey = r.d_skey = nullptr; r.d_cidx = r.d_sidx = nullptr;
+    r.scratch_cap = 0;
+}
+
+static void scratch_free(RunScratch &r) {
+    free_scratch(r);
+    cudaFree(r.d_L); cudaFree(r.d_W);
     cudaFree(r.d_gmax); cudaFree(r.d_hkeys); cudaFree(r.d_gidx);
     cudaFree(r.d_flag); cudaFree(r.d_counters); cudaFree(r.d_sel); cudaFree(r.d_cut);
     cudaFree(r.d_ref); cudaFree(r.Xt); cudaFree(r.twM); cudaFree(r.twn);
@@ -694,7 +698,6 @@ static int64_t next_pow2(int64_t v) {   // == nextPowOf2 (xcorr.go:19-24) for 1 
 // one block per series above)
 static int screen_is_fused(int log2m) { return log2m >= 6 && log2m <= 13; }
 static int screen_is_big(int log2m) { return log2m >= 11 && log2m <= 13; }      // muse_screen_big.cuh
-static int screen_log2m_supported(int log2m) { return screen_is_fused(log2m); }
 
 // The per-reference tables of the fp32 kernels, from Xt on the device: weights of the bound
 // A[k] = |Xt[k]| * (1 at DC and Nyquist, else 2) rounded UP (the bound must not shrink), one 16-byte entry per
@@ -732,7 +735,7 @@ static int ensure_ref_tables(muse_batch *b, int64_t ld) {
         b->d_ref_cap = ld;
     }
     if (!b->d_mid) CU(cudaMalloc(&b->d_mid, sizeof(float) * 4));
-    const bool want_screen = screen_log2m_supported(b->log2m);
+    const bool want_screen = screen_is_fused(b->log2m);
     if (b->tab_n == n && (b->tab_screen || !want_screen)) return MUSE_OK;
     if (b->is_long) {      // the reference's transform has n entries, the twiddles are generated on the device
         cudaFree(b->Xt); cudaFree(b->twM); cudaFree(b->twn); cudaFree(b->twp_f); cudaFree(b->twi_f); cudaFree(b->swtw); cudaFree(b->sw_f); cudaFree(b->sx_f); cudaFree(b->sb_f);
@@ -806,15 +809,14 @@ static int ensure_long_work(muse_batch *b, int64_t count);
 static LongParams long_params(const muse_batch *b, const double *slab, int64_t count, const int32_t *idx, int signed_scores);
 
 // as CU, for code that owns a half-built batch `b`: it goes back to the pool before the error is returned
-#define CUB(call)                                                                                  \
-    do {                                                                                           \
-        cudaError_t e_ = (call);                                                                   \
-        if (e_ != cudaSuccess) {                                                                   \
-            (void)cudaGetLastError();                                                              \
-            muse_batch_destroy(b);                                                                 \
-            return fail(e_ == cudaErrorMemoryAllocation ? MUSE_ERR_OUT_OF_MEMORY : MUSE_ERR_CUDA,  \
-                        "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
-        }                                                                                          \
+#define CUB(call)                                                          \
+    do {                                                                   \
+        cudaError_t e_ = (call);                                           \
+        if (e_ != cudaSuccess) {                                           \
+            const int rc_ = cuda_fail(e_, #call, __FILE__, __LINE__);      \
+            muse_batch_destroy(b);                                         \
+            return rc_;                                                    \
+        }                                                                  \
     } while (0)
 
 // The batch object with its pooled scratch, the tables of its FFT length and its small allocations: nothing is launched.
@@ -961,18 +963,6 @@ extern "C" int muse_batch_create(muse_ctx *ctx, muse_group *g, const double *ref
     return MUSE_OK;
 }
 
-static void free_scratch(muse_batch *b) {
-    cudaFree(b->d_score); cudaFree(b->d_lag); cudaFree(b->d_slot);
-    cudaFree(b->d_ckey); cudaFree(b->d_skey); cudaFree(b->d_cidx); cudaFree(b->d_sidx);
-    cudaFree(b->d_clag); cudaFree(b->d_slag);
-    b->d_clag = b->d_slag = nullptr;
-    cudaFree(b->d_U); cudaFree(b->d_list);
-    b->d_U = nullptr; b->d_list = nullptr;
-    b->d_score = nullptr; b->d_lag = nullptr; b->d_slot = nullptr;
-    b->d_ckey = b->d_skey = nullptr; b->d_cidx = b->d_sidx = nullptr;
-    b->scratch_cap = 0;
-}
-
 extern "C" void muse_batch_destroy(muse_batch *b) {
     if (!b) return;
     cudaSetDevice(b->ctx->device);
@@ -995,7 +985,7 @@ extern "C" int64_t muse_batch_fft_len(const muse_batch *b) { return b ? b->n : 0
 static int ensure_scratch(muse_batch *b) {
     const int64_t S = b->g->size;
     if (S <= b->scratch_cap) return MUSE_OK;
-    free_scratch(b);
+    free_scratch(*b);
     const int64_t cap = std::max<int64_t>(S, 1024);
     CU(cudaMalloc(&b->d_score, sizeof(double) * (size_t)cap));
     CU(cudaMalloc(&b->d_lag, sizeof(int32_t) * (size_t)cap));
@@ -1170,8 +1160,9 @@ struct Rec {
 
 // Key bits per group-by column.  64 / ncols each when every column's cardinality fits: that packing does not depend on the
 // store, so the shards of a multi-GPU run merge on it.  Otherwise ceil(log2(cardinality)) of THIS store's columns, which
-// any number of keys up to MUSE_MAX_KEY_COLS can use as long as the widths sum to at most 64 bits (*rank_independent = 0).
-static int key_bits(const muse_group *g, const int32_t *key_cols, int n_key_cols, int *bits, int *rank_independent) {
+// any number of keys up to MUSE_MAX_KEY_COLS can use as long as the widths sum to at most 64 bits.  A shard (shard = true)
+// cannot: the shards merge on the keys, so they must not depend on the store.
+static int key_bits(const muse_group *g, const int32_t *key_cols, int n_key_cols, int *bits, bool shard) {
     if (n_key_cols > MUSE_MAX_KEY_COLS) return fail(MUSE_ERR_UNSUPPORTED, "grouping by more than %d label keys", MUSE_MAX_KEY_COLS);
     const int fixed = 64 / n_key_cols;
     bool fits = true;
@@ -1188,18 +1179,18 @@ static int key_bits(const muse_group *g, const int32_t *key_cols, int n_key_cols
     }
     if (fits) {
         for (int c = 0; c < n_key_cols; c++) bits[c] = fixed;
-        if (rank_independent) *rank_independent = 1;
         return MUSE_OK;
     }
     if (total > 64)
         return fail(MUSE_ERR_UNSUPPORTED, "the label cardinalities of the %d group-by keys need %d key bits (at most 64)", n_key_cols, total);
-    if (rank_independent) *rank_independent = 0;
+    if (shard)
+        return fail(MUSE_ERR_UNSUPPORTED, "shards merge on group keys of at most %d bits per column (64 / %d keys)", fixed, n_key_cols);
     return MUSE_OK;
 }
 
-static int setup_group_table(muse_batch *b, const RunArgs &a, KeyCols &kc, GroupTable &gt) {
+static int setup_group_table(muse_batch *b, const RunArgs &a, bool shard, KeyCols &kc, GroupTable &gt) {
     muse_group *g = b->g;
-    int rc = key_bits(g, a.key_cols, a.n_key_cols, kc.bits, nullptr);
+    int rc = key_bits(g, a.key_cols, a.n_key_cols, kc.bits, shard);
     if (rc) return rc;
     kc.ncols = a.n_key_cols;
     long double prod = 1;
@@ -1240,10 +1231,38 @@ static int setup_group_table(muse_batch *b, const RunArgs &a, KeyCols &kc, Group
     return MUSE_OK;
 }
 
+// Group max and representative of every series on its exact score (group_max_kernel, group_rep_kernel): d_slot and the
+// group table `gt` hold them when the work queued on the stream has run.
+static int queue_group_reps(muse_batch *b, const RunArgs &a, bool shard, KeyCols &kc, GroupTable &gt) {
+    memset(&gt, 0, sizeof(gt));
+    memset(&kc, 0, sizeof(kc));
+    int rc = setup_group_table(b, a, shard, kc, gt);
+    if (rc) return rc;
+    const int64_t S = b->g->size;
+    if (S > 0) {
+        const unsigned blocks = (unsigned)((S + 255) / 256);
+        group_max_kernel<<<blocks, 256, 0, bstream(b)>>>(gt, kc, b->d_score, S, b->d_slot);
+        group_rep_kernel<<<blocks, 256, 0, bstream(b)>>>(gt, b->d_score, S, b->d_slot);
+    }
+    b->timing.n_launches += 2;
+    return MUSE_OK;
+}
+
 // fused screened runs launch the exact kernel over at most this many listed series without knowing
 // the list length on the host; run_fused_overflow finishes a longer list after the fact
 #define MUSE_EXACT_UB 32768
 static int run_fused_overflow(muse_batch *b, int64_t n_exact, bool refill);
+
+// The run's statistics from its counters (d_counters, read back to the host): a fused run's [2] is its exact list and [3]
+// its refined count; any other run re-scores [2] + [3] (screened runs: pilot + second round).
+static void settle_counters(muse_batch *b, const unsigned long long *h_n) {
+    if (b->fused_run) {
+        b->timing.n_rescored = (int64_t)h_n[2];
+        b->timing.n_refined = (int64_t)h_n[3];
+    } else {
+        b->timing.n_rescored = (int64_t)(h_n[2] + h_n[3]);
+    }
+}
 
 // Produces the selected records on the host (unsorted).  apply_filter == 0 keeps every
 // representative (grouped multi-GPU partials, SURVEY F2).
@@ -1256,15 +1275,11 @@ static int run_select(muse_batch *b, const RunArgs &a, int apply_filter, int64_t
     const unsigned blocks = (unsigned)((S + 255) / 256);
     GroupTable gt;
     memset(&gt, 0, sizeof(gt));
-    KeyCols kc;
-    memset(&kc, 0, sizeof(kc));
     const bool grouped = a.n_key_cols > 0;
     if (grouped) {
-        int rc = setup_group_table(b, a, kc, gt);
+        KeyCols kc;
+        int rc = queue_group_reps(b, a, false, kc, gt);
         if (rc) return rc;
-        group_max_kernel<<<blocks, 256, 0, st>>>(gt, kc, b->d_score, S, b->d_slot);
-        group_rep_kernel<<<blocks, 256, 0, st>>>(gt, b->d_score, S, b->d_slot);
-        b->timing.n_launches += 2;
     }
     CU(cudaMemsetAsync(b->d_counters, 0, sizeof(unsigned long long) * 2, st));
     FilterArgs f{a.max_lag, a.threshold, a.sign_filter, apply_filter};
@@ -1284,21 +1299,16 @@ static int run_select(muse_batch *b, const RunArgs &a, int apply_filter, int64_t
     CU(cudaMemcpyAsync(h_lag, b->d_clag, sizeof(int32_t) * CH, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     unsigned long long ncand = h_n[0];
-    if (b->fused_run) {
-        b->timing.n_rescored = (int64_t)h_n[2];
-        b->timing.n_refined = (int64_t)h_n[3];
-        if (b->fused_run == 1 && (int64_t)h_n[2] > std::min<int64_t>(S, MUSE_EXACT_UB)) {
-            // rare: more exact candidates than the fixed launch covered -> finish them and select again
-            const int64_t n_exact = (int64_t)h_n[2];
-            int rc = run_fused_overflow(b, n_exact, false);
-            if (rc) return rc;
-            b->fused_run = 0;
-            rc = run_select(b, a, apply_filter, limit, recs);
-            b->timing.n_rescored = n_exact;
-            return rc;
-        }
-    } else {
-        b->timing.n_rescored = (int64_t)(h_n[2] + h_n[3]);     // screened runs: pilot + second round
+    settle_counters(b, h_n);
+    if (b->fused_run == 1 && (int64_t)h_n[2] > std::min<int64_t>(S, MUSE_EXACT_UB)) {
+        // rare: more exact candidates than the fixed launch covered -> finish them and select again
+        const int64_t n_exact = (int64_t)h_n[2];
+        int rc = run_fused_overflow(b, n_exact, false);
+        if (rc) return rc;
+        b->fused_run = 0;
+        rc = run_select(b, a, apply_filter, limit, recs);
+        b->timing.n_rescored = n_exact;
+        return rc;
     }
     if (ncand == 0) return MUSE_OK;
     auto better = [](const Rec &x, const Rec &y) { return x.key != y.key ? x.key > y.key : x.idx < y.idx; };
@@ -1405,17 +1415,14 @@ static ScreenParams screen_params(muse_batch *b) {
 
 // Arms the fused refinement of the warp kernel: running cut-off = cut0 (+inf: bounds only),
 // counters and histogram cleared, lag window in the kernel's rotated cc index.
-__global__ void init_cut_kernel(unsigned *state, float cut0) {
+__device__ __forceinline__ void init_cut_body(unsigned *state, float cut0) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < 4 + MUSE_CUT_WORDS) state[i] = (i == 0) ? __float_as_uint(cut0) : 0u;
 }
+__global__ void init_cut_kernel(unsigned *state, float cut0) { init_cut_body(state, cut0); }
 
 // the same for the queries of a multi-query launch: blockIdx.y = query
-__global__ void init_cut_batch_kernel(unsigned *const *__restrict__ states, float cut0) {
-    unsigned *state = states[blockIdx.y];
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < 4 + MUSE_CUT_WORDS) state[i] = (i == 0) ? __float_as_uint(cut0) : 0u;
-}
+__global__ void init_cut_batch_kernel(unsigned *const *__restrict__ states, float cut0) { init_cut_body(states[blockIdx.y], cut0); }
 
 // skip_init: the cut-off state is armed by init_cut_batch_kernel for all the queries of a launch at once
 static int arm_refinement(muse_batch *b, ScreenParams &sp, float cut0, int64_t max_lag, int64_t top_n, double threshold, bool skip_init = false) {
@@ -1444,10 +1451,11 @@ static int arm_refinement(muse_batch *b, ScreenParams &sp, float cut0, int64_t m
 }
 
 // idx list of every series whose (refined) bound reaches the final cut-off, read from device memory
-__global__ void survivors_cut_kernel(const float *__restrict__ U, int64_t S, const unsigned *__restrict__ cut_bits,
-                                     int32_t *__restrict__ out, unsigned long long *n) {
+// (n = counters + 2: the list length, then the refined count, which rides along)
+__device__ __forceinline__ void survivors_cut_body(const float *__restrict__ U, int64_t S, const unsigned *__restrict__ cut_bits,
+                                                   int32_t *__restrict__ out, unsigned long long *n) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i == 0) n[1] = *reinterpret_cast<const unsigned long long *>(cut_bits + 2);      // the refined count rides along (counters[3])
+    if (i == 0) n[1] = *reinterpret_cast<const unsigned long long *>(cut_bits + 2);
     const float lo = __uint_as_float(*cut_bits);
     const bool take = i < S && U[i] >= lo;
     const unsigned mask = __ballot_sync(0xffffffffu, take);
@@ -1458,6 +1466,10 @@ __global__ void survivors_cut_kernel(const float *__restrict__ U, int64_t S, con
     base = __shfl_sync(0xffffffffu, base, leader);
     if (take) out[base + __popc(mask & ((1u << lane) - 1u))] = (int32_t)i;
 }
+__global__ void survivors_cut_kernel(const float *__restrict__ U, int64_t S, const unsigned *__restrict__ cut_bits,
+                                     int32_t *__restrict__ out, unsigned long long *n) {
+    survivors_cut_body(U, S, cut_bits, out, n);
+}
 
 // the batched tails of muse_multi_run: blockIdx.y = query (MultiTail, muse_select.cuh)
 __global__ void tail_reset_kernel(const MultiTail *__restrict__ tails, int nq) {
@@ -1467,17 +1479,7 @@ __global__ void tail_reset_kernel(const MultiTail *__restrict__ tails, int nq) {
 }
 __global__ void survivors_cut_batch_kernel(const MultiTail *__restrict__ tails, int64_t S) {
     const MultiTail t = tails[blockIdx.y];
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i == 0) t.counters[3] = *reinterpret_cast<const unsigned long long *>(t.cut + 2);
-    const float lo = __uint_as_float(*t.cut);
-    const bool take = i < S && t.U[i] >= lo;
-    const unsigned mask = __ballot_sync(0xffffffffu, take);
-    if (mask == 0u) return;
-    const int lane = threadIdx.x & 31, leader = __ffs(mask) - 1;
-    unsigned long long base = 0;
-    if (lane == leader) base = atomicAdd(t.counters + 2, (unsigned long long)__popc(mask));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (take) t.list[base + __popc(mask & ((1u << lane) - 1u))] = (int32_t)i;
+    survivors_cut_body(t.U, S, t.cut, t.list, t.counters + 2);
 }
 // reference preparation of a launch's queries: screen_tables_kernel with blockIdx.y = query; the 4 floats of every query
 // (std-zero flag, A[M/2], Xt[M/2]) land in ONE array for one copy to the host
@@ -1587,7 +1589,7 @@ static int score_fused_grouped(muse_batch *b, const RunArgs &a) {
     memset(&gt, 0, sizeof(gt));
     KeyCols kc;
     memset(&kc, 0, sizeof(kc));
-    rc = setup_group_table(b, a, kc, gt);
+    rc = setup_group_table(b, a, false, kc, gt);
     if (rc) return rc;
     const unsigned blocks = (unsigned)((S + 255) / 256);
     const bool running = screen_is_big(b->log2m);      // the kernel itself keeps each group's best lower bound
@@ -1702,6 +1704,36 @@ static int finish_timing(muse_batch *b) {
     return MUSE_OK;
 }
 
+// A run queued without a final synchronisation (timing_pending): its times and counters once its end-of-run event is complete.
+static int finish_pending_timing(muse_batch *b) {
+    CU(cudaEventSynchronize(b->ev[3]));
+    read_timing_events(b);
+    settle_counters(b, reinterpret_cast<const unsigned long long *>(b->h_pin));
+    b->timing_pending = 0;
+    return MUSE_OK;
+}
+
+// The records of a padded list up to its first padding record (flags != 0), at most top_n, into the caller's arrays: their count.
+static int64_t records_out(const muse_partial *r, int64_t top_n, double *scores, int64_t *lags, int64_t *series_idx) {
+    int64_t k = 0;
+    for (; k < top_n && r[k].flags == 0; k++) {
+        scores[k] = r[k].score;
+        lags[k] = r[k].lag;
+        series_idx[k] = r[k].series_idx;
+    }
+    return k;
+}
+
+// The same for the host path's sorted records, whose series indices are local to the store.
+static int64_t records_out(const muse_batch *b, const std::vector<Rec> &recs, double *scores, int64_t *lags, int64_t *series_idx) {
+    for (size_t i = 0; i < recs.size(); i++) {
+        scores[i] = recs[i].score();
+        lags[i] = recs[i].lag();
+        series_idx[i] = b->g->global_offset + recs[i].idx;
+    }
+    return (int64_t)recs.size();
+}
+
 static int queue_topn_records(muse_batch *b, const RunArgs &a, muse_partial *d_out, int64_t capacity);
 
 // Ungrouped runs with a device-side top-N, in two halves: queue = scores, filter, rank, copy of the top_n records into
@@ -1726,15 +1758,8 @@ static int device_topn_finish(muse_batch *b, const RunArgs &a, double *scores, i
     const int64_t top_n = a.top_n;
     const muse_partial *h_rec = reinterpret_cast<const muse_partial *>(b->h_pin + 64);
     if (h_rec[0].flags != 2) {
-        int64_t k = 0;
-        for (; k < top_n && h_rec[k].flags == 0; k++) {
-            scores[k] = h_rec[k].score;
-            lags[k] = h_rec[k].lag;
-            series_idx[k] = h_rec[k].series_idx;
-        }
-        *n_out = k;
-        muse_timing t;
-        return muse_batch_last_timing(b, &t);      // settles timing_pending (events are complete)
+        *n_out = records_out(h_rec, top_n, scores, lags, series_idx);
+        return finish_pending_timing(b);
     }
     b->timing_pending = 0;
     const unsigned long long *h_n = reinterpret_cast<const unsigned long long *>(b->h_pin);
@@ -1744,15 +1769,10 @@ static int device_topn_finish(muse_batch *b, const RunArgs &a, double *scores, i
         if (rc) return rc;
         b->fused_run = 0;
     }
-    std::vector<Rec> recs2;
-    rc = run_select(b, a, 1, top_n, recs2);
+    std::vector<Rec> recs;
+    rc = run_select(b, a, 1, top_n, recs);
     if (rc) return rc;
-    for (size_t i = 0; i < recs2.size(); i++) {
-        scores[i] = recs2[i].score();
-        lags[i] = recs2[i].lag();
-        series_idx[i] = b->g->global_offset + recs2[i].idx;
-    }
-    *n_out = (int64_t)recs2.size();
+    *n_out = records_out(b, recs, scores, lags, series_idx);
     return finish_timing(b);
 }
 
@@ -1784,12 +1804,7 @@ extern "C" int muse_batch_run_ex(muse_batch *b, const int32_t *key_cols, int32_t
     std::vector<Rec> recs;
     rc = run_select(b, a, 1, top_n, recs);
     if (rc) return rc;
-    for (size_t i = 0; i < recs.size(); i++) {
-        scores[i] = recs[i].score();
-        lags[i] = recs[i].lag();
-        series_idx[i] = b->g->global_offset + recs[i].idx;
-    }
-    *n_out = (int64_t)recs.size();
+    *n_out = records_out(b, recs, scores, lags, series_idx);
     return finish_timing(b);
 }
 
@@ -1810,6 +1825,37 @@ extern "C" int64_t muse_batch_partial_capacity(muse_batch *b, const int32_t *key
     return b->g->size;   // at most one representative per series
 }
 
+// The launch of a device-side top-N (partial_topn_kernel, partial_topn_push_kernel) behind queue_candidates.
+struct TopnLaunch {
+    long long exact_bound;   // the fused path's exact launch bound (its list must not be longer), else -1
+    unsigned blocks;
+};
+
+// Queues the filter of an ungrouped run's exact scores into the candidate list (counters[0]).  counters[0..1] (candidates,
+// selected) are still zero: run_scores cleared all four and ungrouped scoring writes only [2..3].
+static TopnLaunch queue_candidates(muse_batch *b, const RunArgs &a) {
+    const int64_t S = b->g->size;
+    cudaStream_t st = bstream(b);
+    if (S > 0) {
+        FilterArgs f{a.max_lag, a.threshold, a.sign_filter, 1};
+        Cand cand{b->d_ckey, b->d_cidx, b->d_clag, b->d_counters};
+        if (b->fused_run == 1) {
+            // only the listed series have scores: filter those (the list's length stays on the device)
+            const int64_t lim = std::min<int64_t>(S, MUSE_EXACT_UB);
+            emit_listed_kernel<<<(unsigned)((lim + 255) / 256), 256, 0, st>>>(b->d_list, b->d_counters + 2, lim, b->d_score, b->d_lag, f, cand);
+        } else {
+            GroupTable gt;
+            memset(&gt, 0, sizeof(gt));
+            emit_candidates_kernel<<<(unsigned)((S + 255) / 256), 256, 0, st>>>(gt, nullptr, b->d_score, b->d_lag, S, f, cand);
+        }
+        b->timing.n_launches++;
+    }
+    // the grid covers MUSE_PARTIAL_RANK_CAP candidates; blocks past the real count (device side) leave at once
+    const long long exact_bound = b->fused_run == 1 ? (long long)std::min<int64_t>(S, MUSE_EXACT_UB) : -1;
+    const unsigned pblocks = (unsigned)std::min<int64_t>((std::max<int64_t>(S, 1) + 7) / 8, (int64_t)b->ctx->sm_count * 8);   // 8 warps per block, one warp per candidate
+    return TopnLaunch{exact_bound, pblocks};
+}
+
 // Ungrouped shard partials without a host round trip: scores, filter and the shard's top_n stay on
 // the device; `d_out` (DEVICE memory, `capacity` >= top_n records) is complete when the work queued
 // on the context's stream has run.  Nothing is synchronised here, so a collective enqueued on the
@@ -1820,32 +1866,13 @@ static int queue_topn_records(muse_batch *b, const RunArgs &a_in, muse_partial *
     static_assert(sizeof(PartialRec) == sizeof(muse_partial), "PartialRec mirrors muse_partial");
     RunArgs a = a_in;
     a.list_only = 1;
-    const int64_t top_n = a.top_n;
     int rc = run_scores(b, a);
     if (rc) return rc;
-    const int64_t S = b->g->size;
     cudaStream_t st = bstream(b);
-    // counters[0..1] (candidates, selected) are still zero: run_scores cleared all four and ungrouped scoring writes only [2..3]
-    if (S > 0) {
-        FilterArgs f{a.max_lag, a.threshold, a.sign_filter, 1};
-        Cand cand{b->d_ckey, b->d_cidx, b->d_clag, b->d_counters};
-        GroupTable gt;
-        memset(&gt, 0, sizeof(gt));
-        if (b->fused_run == 1) {
-            // only the listed series have scores: filter those (the list's length stays on the device)
-            const int64_t lim = std::min<int64_t>(S, MUSE_EXACT_UB);
-            emit_listed_kernel<<<(unsigned)((lim + 255) / 256), 256, 0, st>>>(b->d_list, b->d_counters + 2, lim, b->d_score, b->d_lag, f, cand);
-        } else {
-            emit_candidates_kernel<<<(unsigned)((S + 255) / 256), 256, 0, st>>>(gt, nullptr, b->d_score, b->d_lag, S, f, cand);
-        }
-        b->timing.n_launches++;
-    }
-    // the grid covers MUSE_PARTIAL_RANK_CAP candidates; blocks past the real count (device side) leave at once
-    const long long exact_bound = b->fused_run == 1 ? (long long)std::min<int64_t>(S, MUSE_EXACT_UB) : -1;
-    const unsigned pblocks = (unsigned)std::min<int64_t>((std::max<int64_t>(S, 1) + 7) / 8, (int64_t)b->ctx->sm_count * 8);   // 8 warps per block, one warp per candidate
-    partial_topn_kernel<<<pblocks, 256, 0, st>>>(b->d_ckey, b->d_cidx, b->d_clag, b->d_counters, (long long)top_n,
-                                                 (long long)b->g->global_offset, exact_bound, reinterpret_cast<PartialRec *>(d_out),
-                                                 (long long)capacity);
+    const TopnLaunch tl = queue_candidates(b, a);
+    partial_topn_kernel<<<tl.blocks, 256, 0, st>>>(b->d_ckey, b->d_cidx, b->d_clag, b->d_counters, (long long)a.top_n,
+                                                   (long long)b->g->global_offset, tl.exact_bound, reinterpret_cast<PartialRec *>(d_out),
+                                                   (long long)capacity);
     b->timing.n_launches++;
     CU(cudaGetLastError());
     // statistics and the end-of-run event are picked up by muse_batch_last_timing
@@ -1871,11 +1898,9 @@ static int host_keys(muse_batch *b, const RunArgs &a, const std::vector<Rec> &re
     // canonical group key of each record's series (labels fetched per record)
     keys.resize(recs.size());
     muse_group *g = b->g;
-    int bits[MUSE_MAX_KEY_COLS], rank_independent = 0;
-    int rc = key_bits(g, a.key_cols, a.n_key_cols, bits, &rank_independent);
+    int bits[MUSE_MAX_KEY_COLS];
+    int rc = key_bits(g, a.key_cols, a.n_key_cols, bits, true);
     if (rc) return rc;
-    if (!rank_independent)
-        return fail(MUSE_ERR_UNSUPPORTED, "shard partials need group keys of at most %d bits per column (64 / %d keys)", 64 / a.n_key_cols, a.n_key_cols);
     cudaStream_t st = bstream(b);
     std::vector<int32_t> ids(recs.size() * (size_t)a.n_key_cols);
     if (recs.size() > 4096) {
@@ -2048,6 +2073,19 @@ static int tc_bounds_queue(muse_ctx *ctx, muse_group *g, muse_batch **bs, int nq
     return MUSE_OK;
 }
 
+// ctx->d_multi_refs for rows of the store's length and pitch: MUSE_MULTI_GROUP reference rows, pad columns zero
+static int ensure_multi_refs(muse_ctx *ctx, const muse_group *g) {
+    if (ctx->d_multi_ld == g->ld && ctx->d_multi_n == g->N) return MUSE_OK;
+    cudaFree(ctx->d_multi_refs);
+    ctx->d_multi_refs = nullptr;
+    ctx->d_multi_ld = ctx->d_multi_n = 0;
+    CU(cudaMalloc(&ctx->d_multi_refs, sizeof(double) * (size_t)MUSE_MULTI_GROUP * (size_t)g->ld));
+    CU(cudaMemsetAsync(ctx->d_multi_refs, 0, sizeof(double) * (size_t)MUSE_MULTI_GROUP * (size_t)g->ld, ctx->stream));
+    ctx->d_multi_ld = g->ld;
+    ctx->d_multi_n = g->N;
+    return MUSE_OK;
+}
+
 static bool tc_shape_ok(const muse_group *g, int64_t ref_len) {
     return ref_len == g->N && next_pow2(ref_len) == 2048;
 }
@@ -2087,33 +2125,21 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
         ctx->mt_top_n = top_n;
     }
     unsigned char *d = ctx->d_mt, *h = ctx->h_mt;
-    if (ctx->d_multi_ld != g->ld || ctx->d_multi_n != g->N) {
-        cudaFree(ctx->d_multi_refs);
-        ctx->d_multi_refs = nullptr;
-        ctx->d_multi_ld = ctx->d_multi_n = 0;
-        CU(cudaMalloc(&ctx->d_multi_refs, sizeof(double) * (size_t)MUSE_MULTI_GROUP * (size_t)g->ld));
-        CU(cudaMemsetAsync(ctx->d_multi_refs, 0, sizeof(double) * (size_t)MUSE_MULTI_GROUP * (size_t)g->ld, st));
-        ctx->d_multi_ld = g->ld;
-        ctx->d_multi_n = g->N;
-    }
+    int rc = ensure_multi_refs(ctx, g);
+    if (rc) return rc;
     CU(cudaMemcpy2DAsync(ctx->d_multi_refs, sizeof(double) * (size_t)g->ld, refs, sizeof(double) * (size_t)ref_len,
                          sizeof(double) * (size_t)ref_len, (size_t)nq, cudaMemcpyHostToDevice, st));
     std::vector<muse_batch *> bs((size_t)nq, nullptr);
-    int rc = MUSE_OK;
     auto cleanup = [&](int code) {
         cudaStreamSynchronize(st);
         for (muse_batch *b : bs)
             if (b) muse_batch_destroy(b);
         return code;
     };
-#define CUM(call)                                                                                                        \
-    do {                                                                                                                 \
-        cudaError_t e_ = (call);                                                                                         \
-        if (e_ != cudaSuccess) {                                                                                         \
-            (void)cudaGetLastError();                                                                                    \
-            return cleanup(fail(e_ == cudaErrorMemoryAllocation ? MUSE_ERR_OUT_OF_MEMORY : MUSE_ERR_CUDA, "%s failed: %s (%s:%d)", \
-                                #call, cudaGetErrorString(e_), __FILE__, __LINE__));                                      \
-        }                                                                                                                \
+#define CUM(call)                                                                         \
+    do {                                                                                  \
+        cudaError_t e_ = (call);                                                          \
+        if (e_ != cudaSuccess) return cleanup(cuda_fail(e_, #call, __FILE__, __LINE__)); \
     } while (0)
 
     // ---- reference preparation: one launch per stage ----
@@ -2258,13 +2284,7 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
             if (rc) return cleanup(rc);
             continue;
         }
-        int64_t c = 0;
-        for (; c < top_n && r[c].flags == 0; c++) {
-            sc[c] = r[c].score;
-            lg[c] = r[c].lag;
-            ix[c] = r[c].series_idx;
-        }
-        n_out[i] = c;
+        n_out[i] = records_out(r, top_n, sc, lg, ix);
     }
 #undef CUM
     return cleanup(MUSE_OK);
@@ -2349,20 +2369,14 @@ extern "C" int muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, 
         int n_made = 0;
         // the references of the group: ONE upload (rows at the slab's pitch, pad columns zero), then queued back to
         // back, ONE round trip
-        if (ref_len == g->N && (ctx->d_multi_ld != g->ld || ctx->d_multi_n != g->N)) {
-            cudaFree(ctx->d_multi_refs);
-            ctx->d_multi_refs = nullptr;
-            ctx->d_multi_ld = ctx->d_multi_n = 0;
-            CU(cudaMalloc(&ctx->d_multi_refs, sizeof(double) * (size_t)MUSE_MULTI_GROUP * (size_t)g->ld));
-            CU(cudaMemsetAsync(ctx->d_multi_refs, 0, sizeof(double) * (size_t)MUSE_MULTI_GROUP * (size_t)g->ld, ctx->stream));
-            ctx->d_multi_ld = g->ld;
-            ctx->d_multi_n = g->N;
-        }
         const bool rows_on_device = ref_len == g->N;
-        if (rows_on_device)
+        if (rows_on_device) {
+            rc = ensure_multi_refs(ctx, g);
+            if (rc) return rc;
             CU(cudaMemcpy2DAsync(ctx->d_multi_refs, sizeof(double) * (size_t)g->ld, refs + (size_t)q0 * (size_t)ref_len,
                                  sizeof(double) * (size_t)ref_len, sizeof(double) * (size_t)ref_len, (size_t)nq,
                                  cudaMemcpyHostToDevice, ctx->stream));
+        }
         for (int i = 0; i < nq && rc == MUSE_OK; i++) {
             rc = batch_create_queue(ctx, g, refs + (size_t)(q0 + i) * (size_t)ref_len, ref_len, &made[n_made],
                                     rows_on_device ? ctx->d_multi_refs + (size_t)i * (size_t)g->ld : nullptr);
@@ -2485,6 +2499,27 @@ struct muse_exchange {
     // ([capacity] records, [MUSE_MULTI_GROUP] counts; the host copy then receives the [world] flag words of the step)
     unsigned char *d_send, *h_send;
 };
+
+// Opens the next step of the exchange: a new epoch, and every rank's receive records and flags of the epoch's parity.
+static ExchangePeers exchange_step(muse_exchange *x) {
+    x->epoch++;
+    const int par = (int)(x->epoch & 1ull);
+    ExchangePeers ex;
+    memset(&ex, 0, sizeof(ex));
+    for (int r = 0; r < x->world; r++) {
+        ex.recs[r] = reinterpret_cast<PartialRec *>(x->peer_base[r] + (size_t)par * x->recs_bytes);
+        ex.flags[r] = reinterpret_cast<unsigned long long *>(x->peer_base[r] + 2 * x->recs_bytes) + (size_t)par * x->world;
+    }
+    ex.world = x->world;
+    ex.rank = x->rank;
+    ex.epoch = x->epoch;
+    ex.done_blocks = x->d_done;
+    return ex;
+}
+
+// exchange_wait_kernel's limit, ~10 s at ~2 GHz: ranks may be a whole host->device upload apart, but a peer that never
+// arrives must not hang the box
+#define MUSE_EXCHANGE_TIMEOUT_CYCLES 20000000000ll
 
 static size_t exchange_bytes(int world, int64_t capacity) {
     return 2 * (size_t)world * (size_t)capacity * sizeof(muse_partial) + 2 * (size_t)world * sizeof(unsigned long long);
@@ -2610,62 +2645,24 @@ extern "C" int muse_batch_run_exchange_ex(muse_batch *b, muse_exchange *x, const
     if (rc) return rc;
     const int64_t S = b->g->size;
     cudaStream_t st = bstream(b);
-    x->epoch++;
-    const int par = (int)(x->epoch & 1ull);
-    ExchangePeers ex;
-    memset(&ex, 0, sizeof(ex));
-    for (int r = 0; r < x->world; r++) {
-        ex.recs[r] = reinterpret_cast<PartialRec *>(x->peer_base[r] + (size_t)par * x->recs_bytes);
-        ex.flags[r] = reinterpret_cast<unsigned long long *>(x->peer_base[r] + 2 * x->recs_bytes) + (size_t)par * x->world;
-    }
-    ex.world = x->world;
-    ex.rank = x->rank;
-    ex.epoch = x->epoch;
-    ex.done_blocks = x->d_done;
+    const ExchangePeers ex = exchange_step(x);
     if (grouped) {
         // group max and representative of THIS shard on the exact scores (as run_select does), then the push
         GroupTable gt;
-        memset(&gt, 0, sizeof(gt));
         KeyCols kc;
-        memset(&kc, 0, sizeof(kc));
-        int rank_independent = 0;
-        rc = key_bits(b->g, key_cols, n_key_cols, kc.bits, &rank_independent);
+        rc = queue_group_reps(b, a, true, kc, gt);
         if (rc) return rc;
-        if (!rank_independent)
-            return fail(MUSE_ERR_UNSUPPORTED, "shards merge on group keys of at most %d bits per column (64 / %d keys)", 64 / n_key_cols, n_key_cols);
-        rc = setup_group_table(b, a, kc, gt);
-        if (rc) return rc;
+        // one block even for an empty shard: its last block releases the shard's flag, which the peers wait for
         const unsigned blocks = (unsigned)((std::max<int64_t>(S, 1) + 255) / 256);
-        if (S > 0) {
-            group_max_kernel<<<blocks, 256, 0, st>>>(gt, kc, b->d_score, S, b->d_slot);
-            group_rep_kernel<<<blocks, 256, 0, st>>>(gt, b->d_score, S, b->d_slot);
-        }
         group_records_push_kernel<<<blocks, 256, 0, st>>>(gt, kc, b->d_slot, b->d_score, b->d_lag, (long long)S, (long long)b->g->global_offset,
                                                           (long long)x->capacity, x->d_nlocal, ex);
-        b->timing.n_launches += 3;
     } else {
-        // counters[0..1] (candidates, selected) are still zero: run_scores cleared all four and ungrouped scoring writes only [2..3]
-        if (S > 0) {
-            FilterArgs f{a.max_lag, a.threshold, a.sign_filter, 1};
-            Cand cand{b->d_ckey, b->d_cidx, b->d_clag, b->d_counters};
-            if (b->fused_run == 1) {
-                const int64_t lim = std::min<int64_t>(S, MUSE_EXACT_UB);
-                emit_listed_kernel<<<(unsigned)((lim + 255) / 256), 256, 0, st>>>(b->d_list, b->d_counters + 2, lim, b->d_score, b->d_lag, f, cand);
-            } else {
-                GroupTable gt;
-                memset(&gt, 0, sizeof(gt));
-                emit_candidates_kernel<<<(unsigned)((S + 255) / 256), 256, 0, st>>>(gt, nullptr, b->d_score, b->d_lag, S, f, cand);
-            }
-            b->timing.n_launches++;
-        }
-        const long long exact_bound = b->fused_run == 1 ? (long long)std::min<int64_t>(S, MUSE_EXACT_UB) : -1;
-        const unsigned pblocks = (unsigned)std::min<int64_t>((std::max<int64_t>(S, 1) + 7) / 8, (int64_t)b->ctx->sm_count * 8);
-        partial_topn_push_kernel<<<pblocks, 256, 0, st>>>(b->d_ckey, b->d_cidx, b->d_clag, b->d_counters, (long long)top_n,
-                                                          (long long)b->g->global_offset, exact_bound, (long long)x->capacity, ex);
-        b->timing.n_launches++;
+        const TopnLaunch tl = queue_candidates(b, a);
+        partial_topn_push_kernel<<<tl.blocks, 256, 0, st>>>(b->d_ckey, b->d_cidx, b->d_clag, b->d_counters, (long long)top_n,
+                                                            (long long)b->g->global_offset, tl.exact_bound, (long long)x->capacity, ex);
     }
-    // ~10 s at ~2 GHz: ranks may be a whole host->device upload apart, but a peer that never arrives must not hang the box
-    exchange_wait_kernel<<<1, 32, 0, st>>>(ex.flags[x->rank], x->world, x->epoch, 20000000000ll, x->d_status);
+    b->timing.n_launches++;
+    exchange_wait_kernel<<<1, 32, 0, st>>>(ex.flags[x->rank], x->world, x->epoch, MUSE_EXCHANGE_TIMEOUT_CYCLES, x->d_status);
     // merge on the device: the hash table, candidate counter and status start from zero
     CU(cudaMemsetAsync(x->merge.hkeys, 0, x->merge_bytes / 3 * 2, st));                       // keys and maxima
     CU(cudaMemsetAsync(x->merge.gidx, 0xff, x->merge_bytes / 3, st));                         // representatives: +inf
@@ -2694,13 +2691,7 @@ extern "C" int muse_batch_run_exchange_ex(muse_batch *b, muse_exchange *x, const
     const muse_partial *recs = reinterpret_cast<const muse_partial *>(x->h_recs);
     if (top_n > 0 && recs[0].flags == 2)
         return fail(MUSE_ERR_UNSUPPORTED, "host path needed: a shard's record list was too long for the device-side select or merge");
-    int64_t k = 0;
-    for (; k < top_n && recs[k].flags == 0; k++) {
-        scores[k] = recs[k].score;
-        lags[k] = recs[k].lag;
-        series_idx[k] = recs[k].series_idx;
-    }
-    *n_out = k;
+    *n_out = records_out(recs, top_n, scores, lags, series_idx);
     return MUSE_OK;
 }
 
@@ -2773,26 +2764,14 @@ extern "C" int muse_multi_run_exchange(muse_group *g, muse_exchange *x, const do
                 local_rc = fail(MUSE_ERR_CUDA, "muse_multi_run_exchange: send table: %s", cudaGetErrorString(e));
             }
         }
-        x->epoch++;
-        const int par = (int)(x->epoch & 1ull);
-        ExchangePeers ex;
-        memset(&ex, 0, sizeof(ex));
-        for (int r = 0; r < x->world; r++) {
-            ex.recs[r] = reinterpret_cast<PartialRec *>(x->peer_base[r] + (size_t)par * x->recs_bytes);
-            ex.flags[r] = reinterpret_cast<unsigned long long *>(x->peer_base[r] + 2 * x->recs_bytes) + (size_t)par * x->world;
-        }
-        ex.world = x->world;
-        ex.rank = x->rank;
-        ex.epoch = x->epoch;
-        ex.done_blocks = x->d_done;
+        const ExchangePeers ex = exchange_step(x);
         const long long total = (long long)nq * top_n;
         const unsigned pblocks = (unsigned)std::max<long long>(1, std::min<long long>((total + 255) / 256, (long long)ctx->sm_count * 4));
         const long long *d_cnt = reinterpret_cast<const long long *>(x->d_send);
         const PartialRec *d_tab = reinterpret_cast<const PartialRec *>(x->d_send + (size_t)MUSE_MULTI_GROUP * sizeof(long long));
         multi_records_push_kernel<<<pblocks, 256, 0, st>>>(d_tab, d_cnt, nq, (long long)top_n, (long long)x->capacity,
                                                            local_rc != MUSE_OK ? 1 : 0, ex);
-        // ~10 s at ~2 GHz, as muse_batch_run_exchange_ex
-        exchange_wait_kernel<<<1, 32, 0, st>>>(ex.flags[x->rank], x->world, x->epoch, 20000000000ll, x->d_status);
+        exchange_wait_kernel<<<1, 32, 0, st>>>(ex.flags[x->rank], x->world, x->epoch, MUSE_EXCHANGE_TIMEOUT_CYCLES, x->d_status);
         multi_merge_kernel<<<(unsigned)nq, 256, 0, st>>>(ex.recs[x->rank], x->world, (long long)x->capacity, (long long)top_n, x->d_out, nullptr);
         CU(cudaGetLastError());
         int *h_status = reinterpret_cast<int *>(x->h_recs + (size_t)x->capacity * sizeof(muse_partial));
@@ -2813,13 +2792,7 @@ extern "C" int muse_multi_run_exchange(muse_group *g, muse_exchange *x, const do
         for (int q = 0; q < nq; q++) {
             if (no[q] < 0) continue;      // std(ref) == 0 on every rank (muse_batch.go:38-41)
             const size_t row = (size_t)q * (size_t)top_n;
-            int64_t k = 0;
-            for (; k < top_n && recs[row + k].flags == 0; k++) {
-                sc[row + k] = recs[row + k].score;
-                lg[row + k] = recs[row + k].lag;
-                ix[row + k] = recs[row + k].series_idx;
-            }
-            no[q] = k;
+            no[q] = records_out(recs + row, top_n, sc + row, lg + row, ix + row);
         }
     }
     return MUSE_OK;
@@ -2869,16 +2842,8 @@ extern "C" int muse_batch_last_timing(const muse_batch *cb, muse_timing *out) {
     muse_batch *b = const_cast<muse_batch *>(cb);
     if (b->timing_pending) {     // a device-side run (muse_batch_run_partial_device): finish its bookkeeping now
         CU(cudaSetDevice(b->ctx->device));
-        CU(cudaEventSynchronize(b->ev[3]));
-        read_timing_events(b);
-        const unsigned long long *h_n = reinterpret_cast<const unsigned long long *>(b->h_pin);
-        if (b->fused_run) {
-            b->timing.n_rescored = (int64_t)h_n[2];
-            b->timing.n_refined = (int64_t)h_n[3];
-        } else {
-            b->timing.n_rescored = (int64_t)(h_n[2] + h_n[3]);
-        }
-        b->timing_pending = 0;
+        const int rc = finish_pending_timing(b);
+        if (rc) return rc;
     }
     *out = b->timing;
     return MUSE_OK;

@@ -315,6 +315,30 @@ struct PartialRec {           // == muse_partial (include/muse_b200.h)
     int flags;
 };
 
+// Position of candidate (k, ix) in the (|score| desc, index asc) order: the number of the n candidates that come before it,
+// counted by the calling warp.  Its lanes stride over the list, four independent loads in flight per lane (the list is 48 KB
+// at C3: L1/L2 resident, but one dependent load per step made this kernel 31 us).
+__device__ __forceinline__ unsigned rank_of(const unsigned long long *__restrict__ ckey, const int32_t *__restrict__ cidx, unsigned long long n,
+                                            unsigned long long k, unsigned ix, int lane) {
+    unsigned before = 0;
+    unsigned long long j = lane;
+    for (; j + 96 < n; j += 128) {
+        const unsigned long long k0 = ckey[j], k1 = ckey[j + 32], k2 = ckey[j + 64], k3 = ckey[j + 96];
+        const unsigned i0 = (unsigned)cidx[j], i1 = (unsigned)cidx[j + 32], i2 = (unsigned)cidx[j + 64], i3 = (unsigned)cidx[j + 96];
+        before += (k0 > k || (k0 == k && i0 < ix)) ? 1u : 0u;
+        before += (k1 > k || (k1 == k && i1 < ix)) ? 1u : 0u;
+        before += (k2 > k || (k2 == k && i2 < ix)) ? 1u : 0u;
+        before += (k3 > k || (k3 == k && i3 < ix)) ? 1u : 0u;
+    }
+    for (; j < n; j += 32) {
+        const unsigned long long kj = ckey[j];
+        before += (kj > k || (kj == k && (unsigned)cidx[j] < ix)) ? 1u : 0u;
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) before += __shfl_xor_sync(0xffffffffu, before, off);
+    return before;
+}
+
 __device__ __forceinline__ void partial_topn_body(const unsigned long long *__restrict__ ckey, const int32_t *__restrict__ cidx,
                                                   const int32_t *__restrict__ clag, const unsigned long long *__restrict__ counters, long long top_n,
                                                   long long global_offset, long long exact_list_bound, PartialRec *__restrict__ out, long long capacity) {
@@ -326,29 +350,13 @@ __device__ __forceinline__ void partial_topn_body(const unsigned long long *__re
     for (long long r = take + gtid; r < capacity; r += (long long)gridDim.x * blockDim.x)
         out[r] = PartialRec{0ull, 0.0, 0ll, 0, (overflow && r == 0) ? 2 : 1};
     if (overflow) return;
-    // one warp per candidate; its lanes stride over the list, four independent loads in flight per lane
-    // (the list is 48 KB at C3: L1/L2 resident, but one dependent load per step made this kernel 31 us)
+    // one warp per candidate
     const int lane = threadIdx.x & 31;
     const unsigned long long nwarps = ((unsigned long long)gridDim.x * blockDim.x) >> 5;
     for (unsigned long long i = (unsigned long long)gtid >> 5; i < n; i += nwarps) {
         const unsigned long long k = ckey[i];
         const unsigned ix = (unsigned)cidx[i];
-        unsigned before = 0;
-        unsigned long long j = lane;
-        for (; j + 96 < n; j += 128) {
-            const unsigned long long k0 = ckey[j], k1 = ckey[j + 32], k2 = ckey[j + 64], k3 = ckey[j + 96];
-            const unsigned i0 = (unsigned)cidx[j], i1 = (unsigned)cidx[j + 32], i2 = (unsigned)cidx[j + 64], i3 = (unsigned)cidx[j + 96];
-            before += (k0 > k || (k0 == k && i0 < ix)) ? 1u : 0u;
-            before += (k1 > k || (k1 == k && i1 < ix)) ? 1u : 0u;
-            before += (k2 > k || (k2 == k && i2 < ix)) ? 1u : 0u;
-            before += (k3 > k || (k3 == k && i3 < ix)) ? 1u : 0u;
-        }
-        for (; j < n; j += 32) {
-            const unsigned long long kj = ckey[j];
-            before += (kj > k || (kj == k && (unsigned)cidx[j] < ix)) ? 1u : 0u;
-        }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) before += __shfl_xor_sync(0xffffffffu, before, off);
+        const unsigned before = rank_of(ckey, cidx, n, k, ix, lane);
         if (lane == 0 && (long long)before < top_n) {
             const int ls = clag[i];
             const double a = __longlong_as_double((long long)k);
@@ -394,6 +402,24 @@ __device__ __forceinline__ unsigned long long ld_acquire_sys_u64(const unsigned 
     return v;
 }
 
+// true in the last block of the grid to finish, once everything this GPU stored is ordered (system scope) before the flags
+// that block releases
+__device__ __forceinline__ bool last_block_fenced(unsigned *done_blocks) {
+    __shared__ bool last;
+    __threadfence_system();
+    __syncthreads();
+    if (threadIdx.x == 0) last = (atomicAdd(done_blocks, 1u) == gridDim.x - 1);
+    __syncthreads();
+    if (!last) return false;
+    __threadfence_system();
+    return true;
+}
+// by the last block: flag [rank] of every rank = word, and the block counter ready for the next launch
+__device__ __forceinline__ void release_flags(const ExchangePeers &ex, unsigned long long word) {
+    if (threadIdx.x < ex.world) st_release_sys_u64(&ex.flags[threadIdx.x][ex.rank], word);
+    if (threadIdx.x == 0) *ex.done_blocks = 0u;
+}
+
 __global__ void __launch_bounds__(256)
 partial_topn_push_kernel(const unsigned long long *__restrict__ ckey, const int32_t *__restrict__ cidx,
                          const int32_t *__restrict__ clag, const unsigned long long *__restrict__ counters, long long top_n,
@@ -413,22 +439,7 @@ partial_topn_push_kernel(const unsigned long long *__restrict__ ckey, const int3
         for (unsigned long long i = (unsigned long long)gtid >> 5; i < n; i += nwarps) {
             const unsigned long long k = ckey[i];
             const unsigned ix = (unsigned)cidx[i];
-            unsigned before = 0;
-            unsigned long long j = lane;
-            for (; j + 96 < n; j += 128) {
-                const unsigned long long k0 = ckey[j], k1 = ckey[j + 32], k2 = ckey[j + 64], k3 = ckey[j + 96];
-                const unsigned i0 = (unsigned)cidx[j], i1 = (unsigned)cidx[j + 32], i2 = (unsigned)cidx[j + 64], i3 = (unsigned)cidx[j + 96];
-                before += (k0 > k || (k0 == k && i0 < ix)) ? 1u : 0u;
-                before += (k1 > k || (k1 == k && i1 < ix)) ? 1u : 0u;
-                before += (k2 > k || (k2 == k && i2 < ix)) ? 1u : 0u;
-                before += (k3 > k || (k3 == k && i3 < ix)) ? 1u : 0u;
-            }
-            for (; j < n; j += 32) {
-                const unsigned long long kj = ckey[j];
-                before += (kj > k || (kj == k && (unsigned)cidx[j] < ix)) ? 1u : 0u;
-            }
-#pragma unroll
-            for (int off = 16; off > 0; off >>= 1) before += __shfl_xor_sync(0xffffffffu, before, off);
+            const unsigned before = rank_of(ckey, cidx, n, k, ix, lane);
             if ((long long)before < top_n) {
                 const int ls = clag[i];
                 const double a = __longlong_as_double((long long)k);
@@ -438,18 +449,9 @@ partial_topn_push_kernel(const unsigned long long *__restrict__ ckey, const int3
             }
         }
     }
-    // last block of the grid: everything this GPU stored is ordered before the flags it releases
-    __shared__ bool last;
-    __threadfence_system();
-    __syncthreads();
-    if (threadIdx.x == 0) last = (atomicAdd(ex.done_blocks, 1u) == gridDim.x - 1);
-    __syncthreads();
-    if (!last) return;
-    __threadfence_system();
+    if (!last_block_fenced(ex.done_blocks)) return;
     // flag word: (epoch << 32) | records in the slot (the whole slot: it is padded), 0xffffffff = take the host path
-    const unsigned long long word = (ex.epoch << 32) | (overflow ? 0xffffffffull : (unsigned long long)capacity);
-    if (threadIdx.x < ex.world) st_release_sys_u64(&ex.flags[threadIdx.x][ex.rank], word);
-    if (threadIdx.x == 0) *ex.done_blocks = 0u;
+    release_flags(ex, (ex.epoch << 32) | (overflow ? 0xffffffffull : (unsigned long long)capacity));
 }
 
 // Lane r waits until rank r's flag in the LOCAL buffer has reached `epoch` (bounded spin); status != 0: timed out.
@@ -490,17 +492,8 @@ multi_records_push_kernel(const PartialRec *__restrict__ table, const long long 
             for (int d = 0; d < ex.world; d++) ex.recs[d][slot0 + g] = rec;
         }
     }
-    // last block of the grid: everything this GPU stored is ordered before the flags it releases
-    __shared__ bool last;
-    __threadfence_system();
-    __syncthreads();
-    if (threadIdx.x == 0) last = (atomicAdd(ex.done_blocks, 1u) == gridDim.x - 1);
-    __syncthreads();
-    if (!last) return;
-    __threadfence_system();
-    const unsigned long long word = (ex.epoch << 32) | (failed ? MUSE_EXCHANGE_RANK_FAILED : (unsigned long long)total);
-    if (threadIdx.x < ex.world) st_release_sys_u64(&ex.flags[threadIdx.x][ex.rank], word);
-    if (threadIdx.x == 0) *ex.done_blocks = 0u;
+    if (!last_block_fenced(ex.done_blocks)) return;
+    release_flags(ex, (ex.epoch << 32) | (failed ? MUSE_EXCHANGE_RANK_FAILED : (unsigned long long)total));
 }
 
 // a precedes b in (|score| desc, global series index asc), the order of results.go:81-85 with ties by index
@@ -585,20 +578,10 @@ group_records_push_kernel(GroupTable gt, KeyCols kc, const int64_t *__restrict__
             }
         }
     }
-    __shared__ bool last;
-    __threadfence_system();
-    __syncthreads();
-    if (threadIdx.x == 0) last = (atomicAdd(ex.done_blocks, 1u) == gridDim.x - 1);
-    __syncthreads();
-    if (!last) return;
-    __threadfence_system();
+    if (!last_block_fenced(ex.done_blocks)) return;
     const unsigned long long n = *n_local;
-    const unsigned long long word = (ex.epoch << 32) | (n > (unsigned long long)capacity ? 0xffffffffull : n);
-    if (threadIdx.x < ex.world) st_release_sys_u64(&ex.flags[threadIdx.x][ex.rank], word);
-    if (threadIdx.x == 0) {
-        *ex.done_blocks = 0u;
-        *n_local = 0ull;
-    }
+    release_flags(ex, (ex.epoch << 32) | (n > (unsigned long long)capacity ? 0xffffffffull : n));
+    if (threadIdx.x == 0) *n_local = 0ull;
 }
 
 // ---- merge of all shards' records on the device: group max across shards BEFORE the filter (muse_batch.go:87-89, ties ->
