@@ -83,7 +83,8 @@ struct RunScratch {
     unsigned long long *d_counters;   // [0] ncand, [1] nselected, [2] exact list length, [3] refined
     SelectState *d_sel;
     int32_t *d_flag;
-    unsigned *d_cut;                  // fused refinement state: [0] cut bits, [2..3] n_refined (u64), [4..] coarse + fine histogram
+    unsigned *d_cut;                  // fused refinement state: [0] cut bits, [1] series claims of the warp kernel, [2..3] n_refined (u64),
+                                      // [4..] coarse + fine histogram
     // group table
     int64_t table_cap;
     unsigned long long *d_gmax, *d_hkeys;
@@ -1408,13 +1409,14 @@ static ScreenParams screen_params(muse_batch *b) {
     sp.row_stat = b->g->row_stat;
     sp.cut_bits = b->d_cut;
     sp.n_refined = reinterpret_cast<unsigned long long *>(b->d_cut + 2);
+    sp.next_claim = b->d_cut + 1;
     sp.cut_hist = b->d_cut + 4;
     sp.top_n = 1;
     return sp;
 }
 
 // Arms the fused refinement of the warp kernel: running cut-off = cut0 (+inf: bounds only),
-// counters and histogram cleared, lag window in the kernel's rotated cc index.
+// counters (series claims, n_refined) and histogram cleared, lag window in the kernel's rotated cc index.
 __device__ __forceinline__ void init_cut_body(unsigned *state, float cut0) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < 4 + MUSE_CUT_WORDS) state[i] = (i == 0) ? __float_as_uint(cut0) : 0u;

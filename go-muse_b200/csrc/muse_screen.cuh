@@ -87,6 +87,7 @@ struct ScreenParams {
     unsigned *cut_bits;   // running lower bound on the final top-N cut-off (float bits, only ever raised)
     unsigned *cut_hist;   // [MUSE_CUT_WORDS] 64 coarse, 64*64 middle, 64^3 fine counts of lower bounds
     unsigned long long *n_refined;
+    unsigned *next_claim; // warp kernel: counter of the claims of series handed out so far (cleared with the cut-off state)
     int top_n;            // series needed above the cut before it may rise
     int win_lo, win_len;  // lag window in the kernel's rotated cc index: (idx - win_lo) mod n <= win_len
     float thr;            // threshold rounded up to fp32 (a lower bound must reach it to count)
@@ -301,6 +302,7 @@ struct ScreenWarpCfg {
     using G = Geo<10, 5>;                       // M = 1024 = 32 x 32: one warp per series
     static constexpr int MAX_WARPS = 12;        // 3 warps per scheduler at up to 168 registers per thread (16 at 128 measured equal)
     static constexpr int NREF = 2;              // exchange buffers for the (rare) second stage, shared under a lock
+    static constexpr int CLAIM = 2;             // consecutive series per claim from the hand-out counter (a power of two)
     static constexpr size_t SMEM_BUDGET = 227 * 1024;
     static constexpr size_t EX_BYTES = ((size_t)(G::MP + 1) * sizeof(cf) + 127) / 128 * 128;   // padded FFT exchange buffer
     static size_t row_bytes(int N) { const size_t r = ((size_t)N * 8 + 127) / 128 * 128; return r > EX_BYTES ? r : EX_BYTES; }
@@ -331,11 +333,20 @@ __device__ __forceinline__ void ex_release(unsigned *locks, int t, int slot) {
     }
 }
 
-// Persistent kernel, one block per SM, every warp an independent pipeline over its own series
-// (pos = first, first + stride, ...): its row buffer is refilled by the next cp.async.bulk as
-// soon as the 23 x 16 bytes per lane are in registers, so the DRAM latency of row i+1 hides
-// behind the FFT of row i and ~10 rows per SM are in flight at any time.  The FFT exchange
-// goes through a separate per-warp buffer.
+// Persistent kernel, one block per SM, every warp an independent pipeline over its own series:
+// its row buffer is refilled by the next cp.async.bulk as soon as the 23 x 16 bytes per lane
+// are in registers, so the DRAM latency of row i+1 hides behind the FFT of row i and ~10 rows
+// per SM are in flight at any time.  The FFT exchange goes through a separate per-warp buffer.
+//
+// Work hand-out: a warp takes CLAIM consecutive series at a time.  Claim r < W (the warps of the
+// grid) is warp r's own; later claims come from a device counter (prm.next_claim, cleared with the
+// cut-off state), claim W + c to the warp whose increment of it returned c.  A fixed stride of W series
+// aliases with any store whose rows repeat with a period dividing W (W = 1776 on 148 SMs; the
+// benchmark's rows repeat rect, line, noise, and only rect rows take the second stage): some warps
+// got every expensive row and the rest of the SM idled behind them.  The claim is issued at the
+// top of the last iteration of a claim and consumed at the re-arm, behind the first FFT pass, so
+// its L2 round trip stays off the critical path; the index then waits in shared memory (next_of),
+// not in a register across the rest of the FFT.
 //
 // NZ = ceil(N/64) (17..32 for n = 2048) is a template parameter so that the loads, the
 // conversions and the first radix-4 stage of the zero rows disappear at compile time.  The
@@ -367,13 +378,14 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) unsigned long long bars[C::MAX_WARPS];
     __shared__ unsigned ex_locks[C::NREF];
+    __shared__ int next_of[C::MAX_WARPS];      // the warp's next series: written at the re-arm, read at the end of the iteration
 
     const int w = threadIdx.x >> 5;
     const int t = threadIdx.x & 31;
     // 32-bit series indices (a store holds < 2^31 series): the kernel sits on a register cliff at 168
     const int count = (int)prm.count;
-    const int stride = (int)(gridDim.x * (blockDim.x >> 5));
-    const int pos0 = (int)(blockIdx.x * (blockDim.x >> 5)) + w;
+    const int grid_warps = (int)(gridDim.x * (blockDim.x >> 5));
+    const int pos0 = ((int)(blockIdx.x * (blockDim.x >> 5)) + w) * C::CLAIM;
     unsigned char *buf = smem_raw + (size_t)w * warp_bytes;
     const cd *rowc = reinterpret_cast<const cd *>(buf);
     cf *sm = reinterpret_cast<cf *>(buf);                       // forward exchange: the row buffer itself
@@ -394,14 +406,23 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
 
     // mbarrier phase parity = iteration parity; it rides in bit 31 of the loop counter (count < 2^31):
     // a separate loop-carried register is one too many for the allocator at 168 and gets spilled
-    for (unsigned pp = (unsigned)pos0; (int)(pp & 0x7fffffffu) < count; pp = ((pp & 0x7fffffffu) + (unsigned)stride) | (~pp & 0x80000000u)) {
+    unsigned pp = (unsigned)pos0;
+    while ((int)(pp & 0x7fffffffu) < count) {
         const int pos = (int)(pp & 0x7fffffffu);
         const unsigned phase = pp >> 31;
+        const bool claim_ends = (pos & (C::CLAIM - 1)) == C::CLAIM - 1;
         // running cut-off: one lane reads it (so that the whole warp takes the same branch below) at
         // the top of the iteration; the value is consumed only after U is known, a thousand
         // instructions later, so the L2 round trip stays off the critical path.  +inf = no refinement
-        unsigned cut_raw = 0u;
-        if (t == 0) cut_raw = ld_relaxed_u32(prm.cut_bits);
+        unsigned cut_raw = 0u, claim = 0u;
+        if (t == 0) {
+            cut_raw = ld_relaxed_u32(prm.cut_bits);
+            // consumed at the re-arm.  An increment, not atomicAdd(.., 1): ptxas turns that (and atomicInc with a constant
+            // limit) into a warp-aggregated atomic whose shuffle of the result waits for the L2 round trip right here.  The
+            // limit never wraps the counter: a claim is made only after a series < count that ends a claim, at most
+            // count / CLAIM times.
+            if (claim_ends) claim = atomicInc(prm.next_claim, (unsigned)count);
+        }
         const RowStat rs = prm.row_stat[pos];   // fp64 mean and 1/std from the ingest pass (xcorr.go:84-95); in flight with the row
         const double mu = rs.mean;
         mbar_wait(bar, phase);      // every lane waits itself (one polling lane + __syncwarp measured 3x slower)
@@ -418,7 +439,6 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
             }
         }
         __syncwarp();                       // the row is consumed: the buffer becomes the exchange buffer
-        const int next = pos + stride;      // < 2^31: the launcher keeps count + stride below it
 
         // ---- forward FFT_1024: pruned radix-32, twiddle, exchange through smem, radix-32 ----
         Dft32Lead<NZ, float>::run(v);
@@ -431,11 +451,16 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
         __syncwarp();
         fft_pass_load<10, 5, 1, float>(v, sm, t);
         __syncwarp();
-        if (t == 0 && next < count) {       // the exchange is over: hand the buffer to the copy engine for the next row
-            asm volatile("" ::"r"(__float_as_uint(v[P - 1].y)) : "memory");
-            // the generic-proxy reads and writes of the exchange are ordered before the async-proxy write of the copy
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            bulk_load(smem_u32(buf), prm.slab + (int64_t)next * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
+        if (t == 0) {                       // the exchange is over: hand the buffer to the copy engine for the next row
+            // next < grid_warps * CLAIM + count < 2^31: the counter stays below count / CLAIM
+            const int next = claim_ends ? (grid_warps + (int)claim) * C::CLAIM : pos + 1;
+            next_of[w] = next;
+            if (next < count) {
+                asm volatile("" ::"r"(__float_as_uint(v[P - 1].y)) : "memory");
+                // the generic-proxy reads and writes of the exchange are ordered before the async-proxy write of the copy
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                bulk_load(smem_u32(buf), prm.slab + (int64_t)next * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
+            }
         }
         Dft<P, float>::run(v);                          // v[Perm(j)] = Z[t + 32*j]
 
@@ -566,6 +591,8 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
             prm.out_U[pos] = U;
             if (prm.out_L) prm.out_L[pos] = L;
         }
+        __syncwarp();                       // next_of[w] of lane 0's re-arm
+        pp = (unsigned)next_of[w] | (~pp & 0x80000000u);
     }
 }
 
