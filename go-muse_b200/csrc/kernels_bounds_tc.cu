@@ -4,30 +4,14 @@
 
 namespace muse {
 
-template <int NZ>
-static cudaError_t launch_mag_tiles_nz(const ScreenParams &p, unsigned char *a_tiles, float *mid, int sm_count, cudaStream_t st) {
+cudaError_t launch_mag_tiles(const ScreenParams &p, unsigned char *a_tiles, float *mid, int sm_count, cudaStream_t st) {
     using C = ScreenWarpCfg;
-    auto kern = mag_tiles_kernel<NZ>;
     const int warps = C::warps(p.N);
     const size_t wb = C::warp_bytes(p.N);
-    const size_t smem = (size_t)warps * wb;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    int64_t blocks = (p.count + warps - 1) / warps;      // persistent: one block per SM
-    if (blocks > sm_count) blocks = sm_count;
-    kern<<<(unsigned)blocks, warps * 32, smem, st>>>(p, a_tiles, mid, (unsigned)wb);
-    return cudaGetLastError();
-}
-
-cudaError_t launch_mag_tiles(const ScreenParams &p, unsigned char *a_tiles, float *mid, int sm_count, cudaStream_t st) {
-    switch (ScreenWarpCfg::nz(p.N)) {
-#define MUSE_NZ_CASE(z) case z: return launch_mag_tiles_nz<z>(p, a_tiles, mid, sm_count, st);
-        MUSE_NZ_CASE(17) MUSE_NZ_CASE(18) MUSE_NZ_CASE(19) MUSE_NZ_CASE(20) MUSE_NZ_CASE(21) MUSE_NZ_CASE(22)
-        MUSE_NZ_CASE(23) MUSE_NZ_CASE(24) MUSE_NZ_CASE(25) MUSE_NZ_CASE(26) MUSE_NZ_CASE(27) MUSE_NZ_CASE(28)
-        MUSE_NZ_CASE(29) MUSE_NZ_CASE(30) MUSE_NZ_CASE(31) MUSE_NZ_CASE(32)
-#undef MUSE_NZ_CASE
-    }
-    return cudaErrorInvalidValue;
+    return dispatch_nz(C::nz(p.N), [&](auto nz) {
+        return launch_persistent(mag_tiles_kernel<decltype(nz)::value>, p.count, warps, (size_t)warps * wb, sm_count, st, p, a_tiles, mid,
+                                 (unsigned)wb);
+    });
 }
 
 cudaError_t launch_weight_tiles(const float4 *const *d_sw, int nq, unsigned char *b_tiles, cudaStream_t st) {

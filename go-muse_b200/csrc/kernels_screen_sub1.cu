@@ -3,31 +3,6 @@
 
 namespace muse {
 
-template <int NZ>
-static cudaError_t launch_screen_sub1_nz(const ScreenParams &p, int sm_count, cudaStream_t st) {
-    using C = ScreenSubCfg<1>;
-    auto kern = score_screen_sub_kernel<1, NZ>;
-    const int warps = C::warps(p.N);
-    const size_t smem = C::smem_bytes(p.N);
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    const int64_t units = (p.count + C::GS - 1) / C::GS;
-    int64_t blocks = (units + warps - 1) / warps;         // persistent: one block per SM
-    if (blocks > sm_count) blocks = sm_count;
-    kern<<<(unsigned)blocks, warps * 32, smem, st>>>(p, (unsigned)C::warp_bytes(p.N), (unsigned)C::row_bytes(p.N));
-    return cudaGetLastError();
-}
-
-// one instantiation per number of rows of T complex slots that hold samples
-cudaError_t launch_screen_sub1(const ScreenParams &p, int sm_count, cudaStream_t st) {
-    switch (ScreenSubCfg<1>::nz(p.N)) {
-#define MUSE_NZ_CASE(z) case z: return launch_screen_sub1_nz<z>(p, sm_count, st);
-        MUSE_NZ_CASE(17) MUSE_NZ_CASE(18) MUSE_NZ_CASE(19) MUSE_NZ_CASE(20) MUSE_NZ_CASE(21) MUSE_NZ_CASE(22)
-        MUSE_NZ_CASE(23) MUSE_NZ_CASE(24) MUSE_NZ_CASE(25) MUSE_NZ_CASE(26) MUSE_NZ_CASE(27) MUSE_NZ_CASE(28)
-        MUSE_NZ_CASE(29) MUSE_NZ_CASE(30) MUSE_NZ_CASE(31) MUSE_NZ_CASE(32)
-#undef MUSE_NZ_CASE
-    }
-    return cudaErrorInvalidValue;
-}
+template cudaError_t launch_screen_sub<1>(const ScreenParams &, int, cudaStream_t);
 
 }  // namespace muse

@@ -3,31 +3,13 @@
 
 namespace muse {
 
-template <int NZ>
-static cudaError_t launch_screen_warp_nz(const ScreenParams &p, int sm_count, cudaStream_t st) {
-    using C = ScreenWarpCfg;
-    auto kern = score_screen_warp_kernel<NZ>;
-    const int warps = C::warps(p.N);
-    const size_t wb = C::warp_bytes(p.N);
-    const size_t smem = C::smem_bytes(p.N);
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    int64_t blocks = (p.count + warps - 1) / warps;      // persistent: one block per SM
-    if (blocks > sm_count) blocks = sm_count;
-    kern<<<(unsigned)blocks, warps * 32, smem, st>>>(p, (unsigned)wb, (unsigned)C::row_bytes(p.N));
-    return cudaGetLastError();
-}
-
 // one instantiation per number of non-zero rows of 32 complex slots (N = 1026 .. 2048)
 cudaError_t launch_screen_warp(const ScreenParams &p, int sm_count, cudaStream_t st) {
-    switch (ScreenWarpCfg::nz(p.N)) {
-#define MUSE_NZ_CASE(z) case z: return launch_screen_warp_nz<z>(p, sm_count, st);
-        MUSE_NZ_CASE(17) MUSE_NZ_CASE(18) MUSE_NZ_CASE(19) MUSE_NZ_CASE(20) MUSE_NZ_CASE(21) MUSE_NZ_CASE(22)
-        MUSE_NZ_CASE(23) MUSE_NZ_CASE(24) MUSE_NZ_CASE(25) MUSE_NZ_CASE(26) MUSE_NZ_CASE(27) MUSE_NZ_CASE(28)
-        MUSE_NZ_CASE(29) MUSE_NZ_CASE(30) MUSE_NZ_CASE(31) MUSE_NZ_CASE(32)
-#undef MUSE_NZ_CASE
-    }
-    return cudaErrorInvalidValue;
+    using C = ScreenWarpCfg;
+    return dispatch_nz(C::nz(p.N), [&](auto nz) {
+        return launch_persistent(score_screen_warp_kernel<decltype(nz)::value>, p.count, C::warps(p.N), C::smem_bytes(p.N), sm_count, st, p,
+                                 (unsigned)C::warp_bytes(p.N), (unsigned)C::row_bytes(p.N));
+    });
 }
 
 }  // namespace muse

@@ -1358,10 +1358,9 @@ static int run_select(muse_batch *b, const RunArgs &a, int apply_filter, int64_t
 static cudaError_t launch_screen(const muse_batch *b, const ScreenParams &p, cudaStream_t st) {
     if (b->log2m == 10) return launch_screen_warp(p, b->ctx->sm_count, st);
     if (screen_is_big(b->log2m)) return launch_screen_big(b->log2m, p, b->ctx->sm_count, st);
-    if (b->log2m == 6) return launch_screen_sub1(p, b->ctx->sm_count, st);
-    if (b->log2m == 7) return launch_screen_sub2(p, b->ctx->sm_count, st);
-    if (b->log2m == 8) return launch_screen_sub3(p, b->ctx->sm_count, st);
-    if (b->log2m == 9) return launch_screen_sub4(p, b->ctx->sm_count, st);
+    static cudaError_t (*const sub[])(const ScreenParams &, int, cudaStream_t) = {launch_screen_sub<1>, launch_screen_sub<2>,
+                                                                                 launch_screen_sub<3>, launch_screen_sub<4>};
+    if (b->log2m >= 6 && b->log2m <= 9) return sub[b->log2m - 6](p, b->ctx->sm_count, st);
     return cudaErrorInvalidValue;
 }
 

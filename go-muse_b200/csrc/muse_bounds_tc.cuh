@@ -86,7 +86,6 @@ template <int NZ>
 __global__ void __launch_bounds__(ScreenWarpCfg::MAX_WARPS * 32, 1)
 mag_tiles_kernel(const ScreenParams prm, unsigned char *__restrict__ a_tiles, float *__restrict__ mid, const unsigned warp_bytes) {
     using C = ScreenWarpCfg;
-    using G = typename C::G;
     constexpr int P = 32;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) unsigned long long bars[C::MAX_WARPS];
@@ -108,6 +107,7 @@ mag_tiles_kernel(const ScreenParams prm, unsigned char *__restrict__ a_tiles, fl
 
     if (t == 0) {
         mbar_init(bar, 1);
+        mbar_init_fence();
         if (pos0 < count) bulk_load(smem_u32(buf), prm.slab + (int64_t)pos0 * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
     }
     __syncthreads();
@@ -117,56 +117,31 @@ mag_tiles_kernel(const ScreenParams prm, unsigned char *__restrict__ a_tiles, fl
         const double mu = prm.row_stat[pos].mean;
         mbar_wait(bar, phase);
         cf v[P];
-#pragma unroll
-        for (int r = 0; r < P; r++) {
-            if (r < NZ) {
-                const cd x = (r == NZ - 1 && !last_in) ? cd{mu, mu} : rowc[t + r * 32];
-                v[r] = cf{(float)(x.x - mu), (float)(x.y - mu)};
-            } else {
-                v[r] = cf{0.f, 0.f};
-            }
-        }
+        load_centred<NZ, 32>(v, rowc, t, mu, last_in);
         __syncwarp();
         const int next = pos + stride;
         Dft32Lead<NZ, float>::run(v);
-#pragma unroll
-        for (int j = 0; j < P; j++) {
-            cf val = v[Perm<P>::at(j)];
-            if (j > 0) val = cmul(val, prm.twp[(j - 1) * 32 + t]);
-            sm[G::pad(32 * t + j)] = val;
-        }
-        __syncwarp();
-        fft_pass_load<10, 5, 1, float>(v, sm, t);
+        screen_pass0<32>(v, sm, prm.twp, t);
         __syncwarp();
         if (t == 0 && next < count) {       // the exchange is over: the buffer goes back to the copy engine
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             bulk_load(smem_u32(buf), prm.slab + (int64_t)next * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
         }
-        Dft<P, float>::run(v);                          // v[Perm(j)] = Z[t + 32*j]
+        screen_pass1<32>(v);                            // v[Perm(j)] = Z[t + 32*j]
 
         unsigned pk[16], pl[16];                        // bf16 (hi | lo) pairs (|2Y_k|, |2Y_(M-k)|), kk = 32 t + 2 j + side
 #pragma unroll
         for (int j = 0; j < P / 2; j++) {
             const cf zk = v[Perm<P>::at(j)];
-            const cf zp = v[Perm<P>::at(P - 1 - j)];
-            const cf zs = v[Perm<P>::at((P - j) & (P - 1))];
-            cf src, zm;
-            src.x = lane0 ? zs.x : zp.x;
-            src.y = lane0 ? zs.y : zp.y;
-            zm.x = __shfl_sync(0xffffffffu, src.x, partner);
-            zm.y = __shfl_sync(0xffffffffu, src.y, partner);
+            const cf zm = mirror_of<32>(v, j, lane0, partner);
             const float4 s = prm.sw[t + 32 * j];            // only the split twiddle is used here
             const cf zmc = cconj(zm);
-            const cf e = cadd(zk, zmc);
-            const cf o = cmul_negi(csub(zk, zmc));
-            const cf wo = cmul(o, cf{s.x, s.y});
-            const cf y1 = cadd(e, wo);
-            const cf y2 = csub(e, wo);
-            const cf q1 = pmul(y1, y1), q2 = pmul(y2, y2);
+            cf qk, qm;
+            split_sq(cadd(zk, zmc), csub(zk, zmc), cf{s.x, s.y}, qk, qm);
             // sqrt.approx is within 2 ulp either way: the epilogue's factor covers it
             unsigned h0, l0, h1, l1;
-            bf16_split(sqrt_approx(q1.x + q1.y), h0, l0);
-            bf16_split(sqrt_approx(q2.x + q2.y), h1, l1);
+            bf16_split(sqrt_approx(qk.x + qk.y), h0, l0);
+            bf16_split(sqrt_approx(qm.x + qm.y), h1, l1);
             pk[j] = h0 | (h1 << 16);
             pl[j] = l0 | (l1 << 16);
         }
@@ -216,14 +191,6 @@ __global__ void weight_tiles_kernel(const float4 *const *__restrict__ sw, int nq
 }
 
 // ---- 3. the contraction on the tensor cores -------------------------------------------------------------------------
-__device__ __forceinline__ void mbar_expect_tx(unsigned bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_copy_g2s(unsigned dst, const void *src, unsigned bytes, unsigned bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
-                 "r"(bytes), "r"(bar)
-                 : "memory");
-}
 // UMMA shared-memory descriptor, K-major, no swizzle (cute::UMMA::SmemDescriptor: start address, LBO and SBO in units of
 // 16 bytes at bits [0,14), [16,30), [32,46); version 1 at [46,48); layout type 0 at [61,64))
 __device__ __forceinline__ unsigned long long umma_desc(unsigned smem_addr, unsigned lbo_bytes, unsigned sbo_bytes) {
@@ -276,11 +243,11 @@ bounds_tc_kernel(const TcBoundsParams prm) {
 
     if (threadIdx.x == 0) {
         for (int i = 0; i < C::STAGES; i++) {
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&full_bar[i])) : "memory");
-            asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&empty_bar[i])) : "memory");
+            mbar_init(smem_u32(&full_bar[i]), 1);
+            mbar_init(smem_u32(&empty_bar[i]), 1);
         }
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&done_bar)) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(smem_u32(&done_bar), 1);
+        mbar_init_fence();
     }
     for (int i = threadIdx.x; i < C::TN; i += blockDim.x) s_amid[i] = i < prm.nq ? prm.amid[i] : 0.f;
     if (warp == 1) {      // all 512 TMEM columns: two 128 x 256 fp32 accumulators
@@ -301,9 +268,9 @@ bounds_tc_kernel(const TcBoundsParams prm) {
                 if (kt >= C::STAGES) mbar_wait(smem_u32(&empty_bar[s]), (unsigned)((kt / C::STAGES - 1) & 1));
                 const unsigned fb = smem_u32(&full_bar[s]);
                 const unsigned dst = stage_u32 + (unsigned)s * C::STAGE_BYTES;
-                mbar_expect_tx(fb, (unsigned)C::STAGE_BYTES);
-                bulk_copy_g2s(dst, a_src + (size_t)kt * C::A_TILE_BYTES, (unsigned)C::A_TILE_BYTES, fb);
-                bulk_copy_g2s(dst + C::A_TILE_BYTES, prm.b_tiles + (size_t)kt * C::B_TILE_BYTES, (unsigned)C::B_TILE_BYTES, fb);
+                mbar_expect(fb, (unsigned)C::STAGE_BYTES);
+                bulk_copy(dst, a_src + (size_t)kt * C::A_TILE_BYTES, (unsigned)C::A_TILE_BYTES, fb);
+                bulk_copy(dst + C::A_TILE_BYTES, prm.b_tiles + (size_t)kt * C::B_TILE_BYTES, (unsigned)C::B_TILE_BYTES, fb);
             }
         }
     } else if (warp == 1) {

@@ -4,6 +4,8 @@
 
 #include <cuda_runtime.h>
 
+#include <type_traits>
+
 #include "muse_exact.cuh"
 #include "muse_screen_big.cuh"
 #include "muse_screen_sub.cuh"
@@ -18,13 +20,49 @@ cudaError_t launch_exact_batch(int mode, const ExactParams *d_table, int nq, int
 // points per thread of the exact kernel for each FFT size (fixes the twiddle layout of ExactParams::twM)
 inline int exact_log2p(int log2m) { return log2m < 4 ? log2m : 4; }
 
+// f(std::integral_constant<int, NZ>()) for nz = NZ in 17 .. 32: the rows of complex slots that hold samples, one
+// instantiation of the n <= 2048 kernels per value
+template <typename F>
+cudaError_t dispatch_nz(int nz, F &&f) {
+    switch (nz) {
+#define MUSE_NZ_CASE(z) case z: return f(std::integral_constant<int, z>());
+        MUSE_NZ_CASE(17) MUSE_NZ_CASE(18) MUSE_NZ_CASE(19) MUSE_NZ_CASE(20) MUSE_NZ_CASE(21) MUSE_NZ_CASE(22)
+        MUSE_NZ_CASE(23) MUSE_NZ_CASE(24) MUSE_NZ_CASE(25) MUSE_NZ_CASE(26) MUSE_NZ_CASE(27) MUSE_NZ_CASE(28)
+        MUSE_NZ_CASE(29) MUSE_NZ_CASE(30) MUSE_NZ_CASE(31) MUSE_NZ_CASE(32)
+#undef MUSE_NZ_CASE
+    }
+    return cudaErrorInvalidValue;
+}
+
+// persistent grid of blocks of `warps` warps: one per SM, fewer when `units` (one per warp) fill fewer
+inline int64_t persistent_blocks(int64_t units, int warps, int sm_count) {
+    const int64_t blocks = (units + warps - 1) / warps;
+    return blocks > sm_count ? sm_count : blocks;
+}
+template <typename... P, typename... A>
+cudaError_t launch_persistent(void (*kern)(P...), int64_t units, int warps, size_t smem, int sm_count, cudaStream_t st, A... args) {
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    kern<<<(unsigned)persistent_blocks(units, warps, sm_count), warps * 32, smem, st>>>(args...);
+    return cudaGetLastError();
+}
+
 // fp32 screening + fused second stage: warp kernel (n = 2048)
 cudaError_t launch_screen_warp(const ScreenParams &p, int sm_count, cudaStream_t st);
-// n = 128 .. 1024: sixteen .. two series per warp (muse_screen_sub.cuh)
-cudaError_t launch_screen_sub1(const ScreenParams &p, int sm_count, cudaStream_t st);
-cudaError_t launch_screen_sub2(const ScreenParams &p, int sm_count, cudaStream_t st);
-cudaError_t launch_screen_sub3(const ScreenParams &p, int sm_count, cudaStream_t st);
-cudaError_t launch_screen_sub4(const ScreenParams &p, int sm_count, cudaStream_t st);
+// n = 128 .. 1024: sixteen .. two series per warp (muse_screen_sub.cuh); LOG2T = log2m - 5 = 1 .. 4, one per translation
+// unit (kernels_screen_sub<LOG2T>.cu)
+template <int LOG2T>
+cudaError_t launch_screen_sub(const ScreenParams &p, int sm_count, cudaStream_t st) {
+    using C = ScreenSubCfg<LOG2T>;
+    return dispatch_nz(C::nz(p.N), [&](auto nz) {
+        return launch_persistent(score_screen_sub_kernel<LOG2T, decltype(nz)::value>, (p.count + C::GS - 1) / C::GS, C::warps(p.N), C::smem_bytes(p.N),
+                                 sm_count, st, p, (unsigned)C::warp_bytes(p.N), (unsigned)C::row_bytes(p.N));
+    });
+}
+extern template cudaError_t launch_screen_sub<1>(const ScreenParams &, int, cudaStream_t);
+extern template cudaError_t launch_screen_sub<2>(const ScreenParams &, int, cudaStream_t);
+extern template cudaError_t launch_screen_sub<3>(const ScreenParams &, int, cudaStream_t);
+extern template cudaError_t launch_screen_sub<4>(const ScreenParams &, int, cudaStream_t);
 // n = 4096 .. 16384 (muse_screen_big.cuh)
 cudaError_t launch_screen_big(int log2m, const ScreenParams &p, int sm_count, cudaStream_t st);
 // n = 16384: nz = rows of 256 complex slots that hold samples, 17 .. 32, four per translation unit

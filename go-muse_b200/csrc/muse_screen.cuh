@@ -132,18 +132,26 @@ __device__ __forceinline__ float group_sum_f(float x) {
     return x;
 }
 
-// ---- cp.async.bulk / mbarrier plumbing of the warp kernel (SASS UBLKCP, SYNCS) ----
+// ---- cp.async.bulk / mbarrier plumbing of the screening kernels and the tensor-core bounds (SASS UBLKCP, SYNCS) ----
 __device__ __forceinline__ unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
 
+// a block's barriers are initialised, then published by one mbar_init_fence before the first copy or wait
 __device__ __forceinline__ void mbar_init(unsigned bar, unsigned count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
-__device__ __forceinline__ void bulk_load(unsigned dst, const void *src, unsigned bytes, unsigned bar) {
+__device__ __forceinline__ void mbar_init_fence() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+__device__ __forceinline__ void mbar_expect(unsigned bar, unsigned bytes) {
     asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void bulk_copy(unsigned dst, const void *src, unsigned bytes, unsigned bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
                  "r"(bytes), "r"(bar)
                  : "memory");
+}
+// one copy that completes the barrier's current phase
+__device__ __forceinline__ void bulk_load(unsigned dst, const void *src, unsigned bytes, unsigned bar) {
+    mbar_expect(bar, bytes);
+    bulk_copy(dst, src, bytes, bar);
 }
 __device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
     unsigned done;
@@ -211,24 +219,26 @@ __device__ __forceinline__ int cut_level(const unsigned *cnt, int t, unsigned &n
     return __shfl_sync(0xffffffffu, idx, leader);
 }
 
-__device__ __forceinline__ void cut_count_and_raise(const ScreenParams &prm, float L, int t) {
+// cut_bits / cut_hist / top_n: the cut-off state of ScreenParams, or of one query of a multi-query run.  Arguments that
+// are kernel parameters are taken by reference here and in the blocks below, so that they are read where they are used.
+__device__ __forceinline__ void cut_count_and_raise(unsigned *const &cut_bits, unsigned *const &cut_hist, const int &top_n, float L, int t) {
     int bin = (int)(L * (float)MUSE_CUT_BINS);
     bin = bin < 0 ? 0 : (bin >= MUSE_CUT_BINS ? MUSE_CUT_BINS - 1 : bin);
-    unsigned *coarse = prm.cut_hist, *mid = coarse + 64, *fine = mid + 64 * 64;
+    unsigned *coarse = cut_hist, *mid = coarse + 64, *fine = mid + 64 * 64;
     if (t == 0) {
         atomicAdd(&fine[bin], 1u);
         atomicAdd(&mid[bin >> 6], 1u);
         atomicAdd(&coarse[bin >> 12], 1u);
     }
     __syncwarp();
-    unsigned need = (unsigned)prm.top_n;
+    unsigned need = (unsigned)top_n;
     const int c = cut_level(coarse, t, need);
     if (c < 0) return;
     const int m = cut_level(mid + c * 64, t, need);
     if (m < 0) return;                  // the three levels are incremented separately: a reader may see them out of step
     const int f = cut_level(fine + (c * 64 + m) * 64, t, need);
     if (f < 0) return;
-    if (t == 0) atomicMax(prm.cut_bits, __float_as_uint((float)((c * 64 + m) * 64 + f) / (float)MUSE_CUT_BINS));
+    if (t == 0) atomicMax(cut_bits, __float_as_uint((float)((c * 64 + m) * 64 + f) / (float)MUSE_CUT_BINS));
 }
 
 // Refined decision for one series from the fp32 maxima of |cc| inside / outside the lag window
@@ -249,6 +259,183 @@ __device__ __forceinline__ float refine_decide(float U, float s_in, float s_out,
     if (s_in * 0.99999f - MUSE_SCREEN_SLACK > s_out * 1.00001f + MUSE_SCREEN_SLACK)
         L = fminf(s_in * 0.99999f, 1.f) - MUSE_SCREEN_SLACK;      // certainly inside
     return fminf(U, u32);
+}
+
+// ---- the register-resident half-length transform of the n <= 2048 kernels, T = 2 .. 32 lanes per series ----
+// M = 32 T complex points, 32 per lane.  Pass 0 is one radix-32 DFT per lane over the inputs z[t + T r]; pass 1 is
+// GS = 32 / T radix-T DFTs per lane.  Output k = t + T m (m = slot) then sits in register screen_reg<T>(m), and its
+// mirror M - k in lane (T - t) % T, slot 31 - m (lane 0: its own slot (32 - m) % 32; k = 0 pairs with itself and yields
+// the DC and Nyquist terms, k = M/2 is lane 0's slot 16).  Every shuffle below has width T.  At T = 32 this is the
+// n = 2048 layout: GS = 1 and screen_reg<32>(m) = Perm<32>::at(m).
+
+// register of slot m after the last pass: butterfly m % GS, its output m / GS
+template <int T>
+MUSE_HD constexpr int screen_reg(int m) {
+    return (m % (32 / T)) * T + Perm<T>::at(m / (32 / T));
+}
+
+// Centred samples in fp32 straight from the row buffer: v[r] = row[t + T r] - mean for the NZ rows of T complex slots that
+// hold samples, 0 beyond.  last_in: this lane's slot of the last row holds samples (odd N: the slot past them holds the
+// row's mean, RowStat; it and the slots beyond the row are read as mu, i.e. as 0).
+template <int NZ, int T>
+__device__ __forceinline__ void load_centred(cf (&v)[32], const cd *rowc, int t, double mu, bool last_in) {
+#pragma unroll
+    for (int r = 0; r < 32; r++) {
+        if (r < NZ) {
+            const cd x = (r == NZ - 1 && !last_in) ? cd{mu, mu} : rowc[t + r * T];
+            v[r] = cf{(float)(x.x - mu), (float)(x.y - mu)};
+        } else {
+            v[r] = cf{0.f, 0.f};
+        }
+    }
+}
+
+// Pass 0 after its radix-32 DFT, which the caller runs (Dft32Lead<NZ> on the zero-padded forward input, Dft<32> on the
+// inverse's, ahead of taking a locked exchange buffer): twiddle W_M^(j t) from tw (the pass twiddles), scatter into the
+// exchange buffer ex, gather the inputs of pass 1.
+template <int T>
+__device__ __forceinline__ void screen_pass0(cf (&v)[32], cf *ex, const cf *const &tw, int t) {
+    constexpr int LOG2M = 5 + (T >= 2) + (T >= 4) + (T >= 8) + (T >= 16) + (T >= 32);
+    using G = Geo<LOG2M, 5>;
+#pragma unroll
+    for (int j = 0; j < 32; j++) {
+        cf val = v[Perm<32>::at(j)];
+        if (j > 0) val = cmul(val, tw[(j - 1) * T + t]);
+        ex[G::pad(32 * t + j)] = val;
+    }
+    __syncwarp();
+    fft_pass_load<LOG2M, 5, 1, float>(v, ex, t);
+}
+
+// pass 1: v[screen_reg<T>(m)] = Z[t + T m]
+template <int T>
+__device__ __forceinline__ void screen_pass1(cf *v) {
+#pragma unroll
+    for (int c = 0; c < 32 / T; c++) Dft<T, float>::run(v + c * T);
+}
+
+// Z[M - k] for k = t + T m, m < 16 (the layout above)
+template <int T>
+__device__ __forceinline__ cf mirror_of(const cf (&v)[32], int m, bool lane0, int partner) {
+    const cf zp = v[screen_reg<T>(31 - m)];
+    const cf zs = v[screen_reg<T>((32 - m) & 31)];
+    cf src, zm;
+    src.x = lane0 ? zs.x : zp.x;
+    src.y = lane0 ? zs.y : zp.y;
+    zm.x = __shfl_sync(0xffffffffu, src.x, partner, T);
+    zm.y = __shfl_sync(0xffffffffu, src.y, partner, T);
+    return zm;
+}
+
+// The real split of a mirror pair from e = Z_k + conj(Z_(M-k)), d = Z_k - conj(Z_(M-k)) and the split twiddle
+// w = exp(-2 pi i k / n): the squared parts of 2Y_k (qk) and 2conj(Y_(M-k)) (qm), |2Y_k|^2 = qk.x + qk.y.  The caller
+// adds them where it takes the square root: that keeps its order of the additions and square roots.
+__device__ __forceinline__ void split_sq(cf e, cf d, cf w, cf &qk, cf &qm) {
+    const cf wo = cmul(cmul_negi(d), w);
+    const cf y1 = cadd(e, wo);                      // 2*Y_k
+    const cf y2 = csub(e, wo);                      // 2*conj(Y_(M-k))
+    qk = pmul(y1, y1);
+    qm = pmul(y2, y2);
+}
+
+// This lane's series' sum_k |2Y_k| A[k] (the bound U before 1/std and the slack), summed over its T lanes.  PAIR: the
+// pair bound: 2Y_k = e + w o and 2conj(Y_(M-k)) = e - w o with |w| = 1 give |2Y_k|^2 + |2Y_(M-k)|^2 = 2 (|e|^2 + |d|^2),
+// d = Z_k - conj(Z_(M-k)) (|d| = |o|), so by Cauchy-Schwarz
+//   |2Y_k| A[k] + |2Y_(M-k)| A[M-k] <= sqrt(|e|^2 + |d|^2) * B[k]:
+// no twiddle, one square root per pair.  It passes 5.5 % of the benchmark's series on to the second stage where the
+// bin-by-bin sum (!PAIR) passed 3.6 %, for a third fewer instructions in this loop on every series.
+template <int T, bool PAIR>
+__device__ __forceinline__ float screen_bound(const cf (&v)[32], const ScreenParams &prm, int t, bool lane0, int partner) {
+    float acc = 0.f;
+#pragma unroll
+    for (int m = 0; m < 16; m++) {
+        const cf zk = v[screen_reg<T>(m)];
+        const cf zm = mirror_of<T>(v, m, lane0, partner);
+        const cf zmc = cconj(zm);
+        const cf e = cadd(zk, zmc);
+        if constexpr (PAIR) {
+            const cf d = csub(zk, zmc);
+            const cf q = pfma(d, d, pmul(e, e));
+            acc = fmaf(sqrt_approx(q.x + q.y), prm.sb[t + T * m], acc);
+        } else {
+            const float4 sv = prm.sw[t + T * m];            // (w_k.x, w_k.y, A[k], A[M-k])
+            cf qk, qm;
+            split_sq(e, csub(zk, zmc), cf{sv.x, sv.y}, qk, qm);
+            acc = fmaf(sqrt_approx(qk.x + qk.y), sv.z, fmaf(sqrt_approx(qm.x + qm.y), sv.w, acc));
+        }
+    }
+    {   // k = M/2: lane 0, slot 16 (weight 0 on the other lanes)
+        const cf z = v[screen_reg<T>(16)];
+        const cf q = pmul(z, z);
+        acc = fmaf(sqrt_approx(q.x + q.y), lane0 ? 2.f * prm.a_mid : 0.f, acc);
+    }
+    return group_sum_f<T>(acc);
+}
+
+__device__ __forceinline__ cf split_twiddle(float4 s) { return cf{s.x, s.y}; }      // (w_k, A[k], A[M-k]) of ScreenParams::sw
+__device__ __forceinline__ cf split_twiddle(cf s) { return s; }
+
+// conj(Y)*X on the mirror pairs of the split (pointwise_pair), in place: Z'[k] -> own slot m; Z'[M-k] -> the partner's
+// slot 31 - m (lane 0: its own slot 32 - m); k = M/2 pairs with itself (w = -i).  sw: split twiddles, k < M/2 (float4 or
+// cf); sx, x_mid: the reference's Xt.  Leaves the swapped values the inverse, swap(FFT(swap(.))), starts from.
+template <int T, typename SW>
+__device__ __forceinline__ void conj_mul_pairs(cf (&v)[32], const SW *const &sw, const float4 *const &sx, const cf &x_mid, int t, bool lane0,
+                                               int partner) {
+#pragma unroll
+    for (int m = 0; m < 16; m++) {
+        const cf zk = v[screen_reg<T>(m)];
+        const cf zm = mirror_of<T>(v, m, lane0, partner);
+        const cf w = split_twiddle(sw[t + T * m]);
+        const float4 x = sx[t + T * m];
+        cf ok, om;
+        pointwise_pair(zk, zm, w, cf{x.x, x.y}, cf{x.z, x.w}, ok, om);
+        cf rcv;
+        rcv.x = __shfl_sync(0xffffffffu, om.x, partner, T);
+        rcv.y = __shfl_sync(0xffffffffu, om.y, partner, T);
+        v[screen_reg<T>(m)] = ok;
+        cf &hi = v[screen_reg<T>(31 - m)];
+        hi.x = lane0 ? hi.x : rcv.x;
+        hi.y = lane0 ? hi.y : rcv.y;
+        if (m > 0) {
+            cf &own = v[screen_reg<T>(32 - m)];
+            own.x = lane0 ? om.x : own.x;
+            own.y = lane0 ? om.y : own.y;
+        }
+    }
+    cf &mid = v[screen_reg<T>(16)];
+    cf ok, om;
+    pointwise_pair(mid, mid, cf{0.f, -1.f}, x_mid, x_mid, ok, om);
+    mid.x = lane0 ? ok.x : mid.x;
+    mid.y = lane0 ? ok.y : mid.y;
+}
+
+// Maxima of |cc'| inside and outside the lag window over the series' T lanes, from the inverse's output in u
+// (u[c T + Perm<T>(jj)] = (cc'[2i+1], cc'[2i]), i = t + c T + 32 jj; cc' = std * cc rotated by pad).
+template <int T>
+__device__ __forceinline__ void window_maxima(const cf (&u)[32], int t, const int &win_lo, const int &win_len, float &m_in, float &m_out) {
+    m_in = 0.f;
+    m_out = 0.f;
+    const int base = 2 * t - win_lo;
+#pragma unroll
+    for (int c = 0; c < 32 / T; c++) {
+#pragma unroll
+        for (int jj = 0; jj < T; jj++) {
+            const cf r = u[c * T + Perm<T>::at(jj)];
+            const int i2 = base + 2 * (c * T + 32 * jj);
+            const bool in0 = (i2 & (64 * T - 1)) <= win_len;      // n = 2 M = 64 T
+            const bool in1 = ((i2 + 1) & (64 * T - 1)) <= win_len;
+            const float a0 = fabsf(r.y), a1 = fabsf(r.x);
+            m_in = fmaxf(m_in, in0 ? a0 : 0.f);
+            m_out = fmaxf(m_out, in0 ? 0.f : a0);
+            m_in = fmaxf(m_in, in1 ? a1 : 0.f);
+            m_out = fmaxf(m_out, in1 ? 0.f : a1);
+        }
+    }
+#pragma unroll
+    for (int off = T / 2; off > 0; off >>= 1) {
+        m_in = fmaxf(m_in, __shfl_xor_sync(0xffffffffu, m_in, off));
+        m_out = fmaxf(m_out, __shfl_xor_sync(0xffffffffu, m_out, off));
+    }
 }
 
 #if defined(__CUDACC__)
@@ -352,11 +539,10 @@ __device__ __forceinline__ void ex_release(unsigned *locks, int t, int slot) {
 // conversions and the first radix-4 stage of the zero rows disappear at compile time.  The
 // |Y_f| bound is invariant under rotation of the padded series, so the zeros trail.
 //
-// Split: lane t holds Z[t + 32j] in slot j.  Bins k and M-k share e = Z[k] + conj(Z[M-k]) and
-// w*o, 2Y[k] = e + w*o, 2conj(Y[M-k]) = e - w*o, so each lane walks only j < 16 (k < 512) and
-// gets both magnitudes from one mirror exchange: Z[M-k] sits in lane (32-t)%32, slot 31-j
-// (lane 0: its own slot (32-j)%32; k = 0 pairs with itself and yields the DC and Nyquist
-// terms).  Only k = 512 (lane 0, slot 16, its own mirror) is left over: |2Y[512]| = 2|Z[512]|.
+// Split: lane t holds Z[t + 32j] in slot j (the transform's layout at T = 32).  Bins k and M-k share
+// e = Z[k] + conj(Z[M-k]) and w*o, 2Y[k] = e + w*o, 2conj(Y[M-k]) = e - w*o, so each lane walks only
+// j < 16 (k < 512) and gets both magnitudes from one mirror exchange.  Only k = 512 (lane 0, slot 16,
+// its own mirror) is left over: |2Y[512]| = 2|Z[512]|.
 //
 // Fused second stage: U is loose (it ignores every phase), and on the benchmark's data
 // a few percent of the series have U above the top-N cut-off.  A warp whose U reaches the
@@ -373,8 +559,7 @@ template <int NZ>
 __global__ void __launch_bounds__(ScreenWarpCfg::MAX_WARPS * 32, 1)
 score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, const unsigned row_bytes) {
     using C = ScreenWarpCfg;
-    using G = typename C::G;
-    constexpr int P = 32, M = G::M;
+    constexpr int P = 32;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) unsigned long long bars[C::MAX_WARPS];
     __shared__ unsigned ex_locks[C::NREF];
@@ -400,6 +585,7 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
     if (threadIdx.x < C::NREF) ex_locks[threadIdx.x] = 0u;
     if (t == 0) {
         mbar_init(bar, 1);
+        mbar_init_fence();
         if (pos0 < count) bulk_load(smem_u32(buf), prm.slab + (int64_t)pos0 * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
     }
     __syncthreads();
@@ -427,29 +613,13 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
         const double mu = rs.mean;
         mbar_wait(bar, phase);      // every lane waits itself (one polling lane + __syncwarp measured 3x slower)
 
-        // ---- centred samples in fp32 straight from the row buffer ----
         cf v[P];
-#pragma unroll
-        for (int r = 0; r < P; r++) {
-            if (r < NZ) {
-                const cd x = (r == NZ - 1 && !last_in) ? cd{mu, mu} : rowc[t + r * 32];
-                v[r] = cf{(float)(x.x - mu), (float)(x.y - mu)};
-            } else {
-                v[r] = cf{0.f, 0.f};
-            }
-        }
+        load_centred<NZ, 32>(v, rowc, t, mu, last_in);
         __syncwarp();                       // the row is consumed: the buffer becomes the exchange buffer
 
         // ---- forward FFT_1024: pruned radix-32, twiddle, exchange through smem, radix-32 ----
         Dft32Lead<NZ, float>::run(v);
-#pragma unroll
-        for (int j = 0; j < P; j++) {
-            cf val = v[Perm<P>::at(j)];
-            if (j > 0) val = cmul(val, prm.twp[(j - 1) * 32 + t]);          // W_1024^(j*t)
-            sm[G::pad(32 * t + j)] = val;
-        }
-        __syncwarp();
-        fft_pass_load<10, 5, 1, float>(v, sm, t);
+        screen_pass0<32>(v, sm, prm.twp, t);
         __syncwarp();
         if (t == 0) {                       // the exchange is over: hand the buffer to the copy engine for the next row
             // next < grid_warps * CLAIM + count < 2^31: the counter stays below count / CLAIM
@@ -462,37 +632,8 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
                 bulk_load(smem_u32(buf), prm.slab + (int64_t)next * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
             }
         }
-        Dft<P, float>::run(v);                          // v[Perm(j)] = Z[t + 32*j]
-
-        // ---- the bound over the mirror pairs (k, M-k), k = t + 32*j, j < 16 ----
-        float acc = 0.f;
-#pragma unroll
-        for (int j = 0; j < P / 2; j++) {
-            const cf zk = v[Perm<P>::at(j)];
-            const cf zp = v[Perm<P>::at(P - 1 - j)];
-            const cf zs = v[Perm<P>::at((P - j) & (P - 1))];
-            cf src, zm;
-            src.x = lane0 ? zs.x : zp.x;
-            src.y = lane0 ? zs.y : zp.y;
-            zm.x = __shfl_sync(0xffffffffu, src.x, partner);
-            zm.y = __shfl_sync(0xffffffffu, src.y, partner);
-            // pair bound: 2Y_k = e + w o and 2conj(Y_(M-k)) = e - w o with |w| = 1 give |2Y_k|^2 + |2Y_(M-k)|^2 = 2 (|e|^2 + |d|^2),
-            // d = Z_k - conj(Z_(M-k)) (|d| = |o|), so by Cauchy-Schwarz
-            //   |2Y_k| A[k] + |2Y_(M-k)| A[M-k] <= sqrt(|e|^2 + |d|^2) * B[k]:
-            // no twiddle, one square root per pair.  It passes 5.5 % of the benchmark's series on to the second stage where
-            // the bin-by-bin sum passed 3.6 %, for a third fewer instructions in this loop on every series.
-            const cf zmc = cconj(zm);
-            const cf e = cadd(zk, zmc);
-            const cf d = csub(zk, zmc);
-            const cf q = pfma(d, d, pmul(e, e));
-            acc = fmaf(sqrt_approx(q.x + q.y), prm.sb[t + 32 * j], acc);
-        }
-        {   // k = 512: lane 0, slot 16 (weight 0 on the other lanes)
-            const cf z = v[Perm<P>::at(P / 2)];
-            const cf q = pmul(z, z);
-            acc = fmaf(sqrt_approx(q.x + q.y), lane0 ? 2.f * prm.a_mid : 0.f, acc);
-        }
-        acc = group_sum_f<32>(acc);
+        screen_pass1<32>(v);                            // v[Perm(j)] = Z[t + 32*j]
+        const float acc = screen_bound<32, true>(v, prm, t, lane0, partner);
 
         // rstd is NaN for a row no fp32 statement may be made about (RowStat); NaN/Inf samples make acc NaN:
         // either way the bound is NaN and the exact kernel decides
@@ -506,18 +647,12 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
         const int bsrc = (__float_as_uint(acc) == 0x7fc12345u) ? 1 : 0;
         const float cut_now = __uint_as_float(__shfl_sync(0xffffffffu, cut_raw, bsrc));
         if (U >= cut_now && U < 1.5f) {      // warp-uniform: U comes out of a butterfly reduction
-            // ---- conj(Y)*X on the mirror pairs of the split (pointwise_pair), in place:
-            //      Z'[k] -> own slot j;  Z'[M-k] -> the partner's slot 31-j (lane 0: its own slot 32-j) ----
+            // ---- conj(Y)*X: conj_mul_pairs<32>, written out because with it ptxas swaps the registers of the last row's
+            //      two copies of mu at NZ = 24, 28 and 32 ----
 #pragma unroll
             for (int j = 0; j < P / 2; j++) {
                 const cf zk = v[Perm<P>::at(j)];
-                const cf zp = v[Perm<P>::at(P - 1 - j)];
-                const cf zs = v[Perm<P>::at((P - j) & (P - 1))];
-                cf src, zm;
-                src.x = lane0 ? zs.x : zp.x;
-                src.y = lane0 ? zs.y : zp.y;
-                zm.x = __shfl_sync(0xffffffffu, src.x, partner);
-                zm.y = __shfl_sync(0xffffffffu, src.y, partner);
+                const cf zm = mirror_of<32>(v, j, lane0, partner);
                 const float4 s = prm.sw[t + 32 * j];
                 const float4 x = prm.sx[t + 32 * j];
                 cf ok, om;
@@ -549,43 +684,18 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
             Dft<P, float>::run(u);
             {
                 const int slot = ex_acquire(ex_locks, t, w);
-                cf *smr = reinterpret_cast<cf *>(refbase + (size_t)slot * C::EX_BYTES);
-#pragma unroll
-                for (int j = 0; j < P; j++) {
-                    cf val = u[Perm<P>::at(j)];
-                    if (j > 0) val = cmul(val, prm.twp[(j - 1) * 32 + t]);
-                    smr[G::pad(32 * t + j)] = val;
-                }
-                __syncwarp();
-                fft_pass_load<10, 5, 1, float>(u, smr, t);
+                screen_pass0<32>(u, reinterpret_cast<cf *>(refbase + (size_t)slot * C::EX_BYTES), prm.twp, t);
                 ex_release(ex_locks, t, slot);
             }
-            Dft<P, float>::run(u);      // u[Perm(j)] = (cc'[2i+1], cc'[2i]), i = t + 32*j; cc' = std * cc rotated by pad
-            // ---- max |cc'| inside and outside the lag window ----
-            float m_in = 0.f, m_out = 0.f;
-            const int base = 2 * t - prm.win_lo;
-#pragma unroll
-            for (int j = 0; j < P; j++) {
-                const cf r = u[Perm<P>::at(j)];
-                const bool in0 = ((base + 64 * j) & (2 * M - 1)) <= prm.win_len;
-                const bool in1 = ((base + 64 * j + 1) & (2 * M - 1)) <= prm.win_len;
-                const float a0 = fabsf(r.y), a1 = fabsf(r.x);
-                m_in = fmaxf(m_in, in0 ? a0 : 0.f);
-                m_out = fmaxf(m_out, in0 ? 0.f : a0);
-                m_in = fmaxf(m_in, in1 ? a1 : 0.f);
-                m_out = fmaxf(m_out, in1 ? 0.f : a1);
-            }
-#pragma unroll
-            for (int off = 16; off > 0; off >>= 1) {
-                m_in = fmaxf(m_in, __shfl_xor_sync(0xffffffffu, m_in, off));
-                m_out = fmaxf(m_out, __shfl_xor_sync(0xffffffffu, m_out, off));
-            }
+            screen_pass1<32>(u);        // u[Perm(j)] = (cc'[2i+1], cc'[2i]), i = t + 32*j; cc' = std * cc rotated by pad
+            float m_in, m_out;
+            window_maxima<32>(u, t, prm.win_lo, prm.win_len, m_in, m_out);
             const float rstd = rs.rstd;
             const float s_in = m_in * rstd, s_out = m_out * rstd;
             U = refine_decide(U, s_in, s_out, L, prm.grouped);
             if (t == 0) atomicAdd(prm.n_refined, 1ull);
             // ---- a certain pass at or above the running cut-off: count it and try to raise the cut-off ----
-            if (L >= prm.thr && L >= cut_now) cut_count_and_raise(prm, L, t);
+            if (L >= prm.thr && L >= cut_now) cut_count_and_raise(prm.cut_bits, prm.cut_hist, prm.top_n, L, t);
         }
         if (t == 0) {
             prm.out_U[pos] = U;

@@ -530,7 +530,7 @@ if constexpr (NZ > 0) {
                 atomicAdd(prm.n_refined, 1ull);
                 if (gslot && L > lg_now) atomicMax(gslot, (unsigned long long)__float_as_uint(L));
             }
-            if (!prm.grouped && t < 32 && L >= prm.thr && L >= cut_now) cut_count_and_raise(prm, L, t);
+            if (!prm.grouped && t < 32 && L >= prm.thr && L >= cut_now) cut_count_and_raise(prm.cut_bits, prm.cut_hist, prm.top_n, L, t);
         }
         if (t == 0) {
             prm.out_U[pos] = U;

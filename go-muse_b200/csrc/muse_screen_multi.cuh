@@ -23,15 +23,6 @@ struct MultiQuery {
 
 #if defined(__CUDACC__)
 
-// cut_count_and_raise of muse_screen.cuh on an explicit cut-off state
-__device__ __forceinline__ void cut_count_and_raise_at(unsigned *cut, int top_n, float L, int t) {
-    ScreenParams q;
-    q.cut_bits = cut;
-    q.cut_hist = cut + 4;
-    q.top_n = top_n;
-    cut_count_and_raise(q, L, t);
-}
-
 // ---- second stage for up to 256 queries whose bounds were computed elsewhere (muse_bounds_tc.cuh) -------------------
 // One pass over the store: a warp loads its row, runs the forward FFT_1024 once, stashes the spectrum in shared memory
 // and reads the series' bound against every query of the launch (query q's array out_U[pos], lane l looks after the
@@ -72,8 +63,7 @@ __global__ void __launch_bounds__(RefineMultiCfg::MAX_WARPS * 32, 1)
 refine_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queries, const int nq, const unsigned warp_bytes,
                     unsigned *__restrict__ next_series) {
     using C = RefineMultiCfg;
-    using G = typename C::G;
-    constexpr int P = 32, M = G::M, QI = C::QI;
+    constexpr int P = 32, M = C::G::M, QI = C::QI;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) unsigned long long bars[C::MAX_WARPS];
 
@@ -103,6 +93,7 @@ refine_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queri
 
     if (t == 0) {
         mbar_init(bar, 1);
+        mbar_init_fence();
         if (pos0 < count) bulk_load(smem_u32(buf), prm.slab + (int64_t)pos0 * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
     }
     for (int q = threadIdx.x; q < C::QMAX; q += blockDim.x) {
@@ -136,29 +127,14 @@ refine_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queri
         mbar_wait(bar, phase);
 
         cf v[P];
-#pragma unroll
-        for (int r = 0; r < P; r++) {
-            if (r < NZ) {
-                const cd x = (r == NZ - 1 && !last_in) ? cd{mu, mu} : rowc[t + r * 32];
-                v[r] = cf{(float)(x.x - mu), (float)(x.y - mu)};
-            } else {
-                v[r] = cf{0.f, 0.f};
-            }
-        }
+        load_centred<NZ, 32>(v, rowc, t, mu, last_in);
         __syncwarp();                       // the row is in registers: its buffer becomes exchange + stash
         if (t == 0) next = (int)atomicAdd(next_series, 1u);
         next = __shfl_sync(0xffffffffu, next, 0);
 
         Dft32Lead<NZ, float>::run(v);
-#pragma unroll
-        for (int j = 0; j < P; j++) {
-            cf val = v[Perm<P>::at(j)];
-            if (j > 0) val = cmul(val, s_tw[(j - 1) * 32 + t]);
-            ex[G::pad(32 * t + j)] = val;
-        }
-        __syncwarp();
-        fft_pass_load<10, 5, 1, float>(v, ex, t);
-        Dft<P, float>::run(v);                          // v[Perm(j)] = Z[t + 32*j]
+        screen_pass0<32>(v, ex, s_tw, t);
+        screen_pass1<32>(v);                            // v[Perm(j)] = Z[t + 32*j]
 #pragma unroll
         for (int j = 0; j < P; j++) stash[32 * j + t] = v[Perm<P>::at(j)];      // every lane reads back only what it wrote
 
@@ -199,75 +175,20 @@ refine_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queri
                 cf z[P];
 #pragma unroll
                 for (int j = 0; j < P; j++) z[Perm<P>::at(j)] = stash[32 * j + t];
-#pragma unroll
-                for (int j = 0; j < P / 2; j++) {
-                    const cf zk = z[Perm<P>::at(j)];
-                    const cf zp = z[Perm<P>::at(P - 1 - j)];
-                    const cf zs = z[Perm<P>::at((P - j) & (P - 1))];
-                    cf src, zm;
-                    src.x = lane0 ? zs.x : zp.x;
-                    src.y = lane0 ? zs.y : zp.y;
-                    zm.x = __shfl_sync(0xffffffffu, src.x, partner);
-                    zm.y = __shfl_sync(0xffffffffu, src.y, partner);
-                    const float4 x = mq.sx[t + 32 * j];
-                    cf ok, om;
-                    pointwise_pair(zk, zm, s_sw[t + 32 * j], cf{x.x, x.y}, cf{x.z, x.w}, ok, om);
-                    cf rcv;
-                    rcv.x = __shfl_sync(0xffffffffu, om.x, partner);
-                    rcv.y = __shfl_sync(0xffffffffu, om.y, partner);
-                    z[Perm<P>::at(j)] = ok;
-                    cf &hi = z[Perm<P>::at(P - 1 - j)];
-                    hi.x = lane0 ? hi.x : rcv.x;
-                    hi.y = lane0 ? hi.y : rcv.y;
-                    if (j > 0) {
-                        cf &own = z[Perm<P>::at(P - j)];
-                        own.x = lane0 ? om.x : own.x;
-                        own.y = lane0 ? om.y : own.y;
-                    }
-                }
-                {
-                    cf &midz = z[Perm<P>::at(P / 2)];
-                    cf ok, om;
-                    pointwise_pair(midz, midz, cf{0.f, -1.f}, mq.x_mid, mq.x_mid, ok, om);
-                    midz.x = lane0 ? ok.x : midz.x;
-                    midz.y = lane0 ? ok.y : midz.y;
-                }
+                conj_mul_pairs<32>(z, s_sw, mq.sx, mq.x_mid, t, lane0, partner);
                 cf u[P];
 #pragma unroll
                 for (int j = 0; j < P; j++) u[j] = z[Perm<P>::at(j)];
                 Dft<P, float>::run(u);
                 __syncwarp();                           // the previous use of the exchange buffer has been read
-#pragma unroll
-                for (int j = 0; j < P; j++) {
-                    cf val = u[Perm<P>::at(j)];
-                    if (j > 0) val = cmul(val, s_tw[(j - 1) * 32 + t]);
-                    ex[G::pad(32 * t + j)] = val;
-                }
-                __syncwarp();
-                fft_pass_load<10, 5, 1, float>(u, ex, t);
-                Dft<P, float>::run(u);
-                float m_in = 0.f, m_out = 0.f;
-                const int base = 2 * t - prm.win_lo;
-#pragma unroll
-                for (int j = 0; j < P; j++) {
-                    const cf r = u[Perm<P>::at(j)];
-                    const bool in0 = ((base + 64 * j) & (2 * M - 1)) <= prm.win_len;
-                    const bool in1 = ((base + 64 * j + 1) & (2 * M - 1)) <= prm.win_len;
-                    const float b0 = fabsf(r.y), b1 = fabsf(r.x);
-                    m_in = fmaxf(m_in, in0 ? b0 : 0.f);
-                    m_out = fmaxf(m_out, in0 ? 0.f : b0);
-                    m_in = fmaxf(m_in, in1 ? b1 : 0.f);
-                    m_out = fmaxf(m_out, in1 ? 0.f : b1);
-                }
-#pragma unroll
-                for (int off = 16; off > 0; off >>= 1) {
-                    m_in = fmaxf(m_in, __shfl_xor_sync(0xffffffffu, m_in, off));
-                    m_out = fmaxf(m_out, __shfl_xor_sync(0xffffffffu, m_out, off));
-                }
+                screen_pass0<32>(u, ex, s_tw, t);
+                screen_pass1<32>(u);
+                float m_in, m_out;
+                window_maxima<32>(u, t, prm.win_lo, prm.win_len, m_in, m_out);
                 float L = -1.f;
                 Uq = refine_decide(Uq, m_in * rs.rstd, m_out * rs.rstd, L, 0);
                 if (t == 0) atomicAdd(reinterpret_cast<unsigned long long *>(mq.cut + 2), 1ull);
-                if (L >= prm.thr && L >= cut_now) cut_count_and_raise_at(mq.cut, prm.top_n, L, t);
+                if (L >= prm.thr && L >= cut_now) cut_count_and_raise(mq.cut, mq.cut + 4, prm.top_n, L, t);
 #pragma unroll
                 for (int i = 0; i < QI; i++)
                     if (i == gi && t == ql) {

@@ -3,11 +3,9 @@
 // score_screen_warp_kernel (muse_screen.cuh) with SEVERAL series per warp.
 //
 // M = n/2 = 32 T complex points per series, T = 2, 4, 8, 16 lanes per series (n = 128, 256, 512, 1024), 32 points per
-// lane, so a warp carries GS = 32 / T = 16 .. 2 series side by side in the register layout of the n = 2048 kernel.  Pass 0 is the
-// same pruned radix-32 transform in registers (inputs z[t + T r]), the exchange goes through the series' own row
-// buffer, pass 1 is GS radix-T transforms per lane; its outputs k = t + T m (m = slot) mirror into lane (T - t) % T,
-// slot 31 - m, exactly as in the n = 2048 kernel with 32 replaced by T, so the real split, the magnitudes and (second
-// stage) conj(Y)*X run on mirror exchanges inside each T-lane group (shuffles of width T).
+// lane, so a warp carries GS = 32 / T = 16 .. 2 series side by side.  The transform, the bound and the second stage are
+// the blocks of muse_screen.cuh at this T: the n = 2048 kernel's with 32 replaced by T, the mirror exchanges inside each
+// T-lane group (shuffles of width T).  The forward exchange goes through the series' own row buffer.
 //
 // Rows arrive by cp.async.bulk: one mbarrier per warp, GS copies per iteration, re-armed as soon as the rows are in
 // registers and the exchange is over (SASS UBLKCP, SYNCS), so a warp's next rows are in flight during its transforms.
@@ -58,27 +56,15 @@ struct ScreenSubCfg {
     }
     static size_t smem_bytes(int N) { return (size_t)warps(N) * warp_bytes(N) + NREF * EX_BYTES; }
     static int nz(int N) { return ((N + 1) / 2 + T - 1) / T; }      // rows of T complex slots that hold samples: 17 .. 32
-    // register of slot m (natural index t + T m) after the last pass: butterfly c = m % GS, output m / GS
-    MUSE_HD static constexpr int reg(int m) { return (m % GS) * T + Perm<T>::at(m / GS); }
 };
 
 #if defined(__CUDACC__)
-
-__device__ __forceinline__ void mbar_expect(unsigned bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_copy(unsigned dst, const void *src, unsigned bytes, unsigned bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
-                 "r"(bytes), "r"(bar)
-                 : "memory");
-}
 
 template <int LOG2T, int NZ>
 __global__ void __launch_bounds__(ScreenSubCfg<LOG2T>::MAX_WARPS * 32, 1)
 score_screen_sub_kernel(const ScreenParams prm, const unsigned warp_bytes, const unsigned row_bytes) {
     using C = ScreenSubCfg<LOG2T>;
-    using G = typename C::G;
-    constexpr int P = 32, T = C::T, GS = C::GS, M = G::M, LOG2M = C::LOG2M;
+    constexpr int P = 32, T = C::T, GS = C::GS;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) unsigned long long bars[C::MAX_WARPS];
     __shared__ unsigned ex_locks[C::NREF];
@@ -117,6 +103,7 @@ score_screen_sub_kernel(const ScreenParams prm, const unsigned warp_bytes, const
     if (threadIdx.x < C::NREF) ex_locks[threadIdx.x] = 0u;
     if (lane == 0) {
         mbar_init(bar, 1);
+        mbar_init_fence();
         if (pos0 < units) issue(pos0);
     }
     __syncthreads();
@@ -133,72 +120,21 @@ score_screen_sub_kernel(const ScreenParams prm, const unsigned warp_bytes, const
         mbar_wait(bar, phase);
 
         cf v[P];
-#pragma unroll
-        for (int r = 0; r < P; r++) {
-            if (r < NZ) {
-                const cd x = (r == NZ - 1 && !last_in) ? cd{mu, mu} : rowc[t + r * T];
-                v[r] = cf{(float)(x.x - mu), (float)(x.y - mu)};
-            } else {
-                v[r] = cf{0.f, 0.f};
-            }
-        }
+        load_centred<NZ, T>(v, rowc, t, mu, last_in);
         __syncwarp();
         const int next = pos + stride;
 
         // ---- forward FFT_M: pruned radix-32 over stride T, twiddle, exchange, GS radix-T transforms ----
         Dft32Lead<NZ, float>::run(v);
-#pragma unroll
-        for (int j = 0; j < P; j++) {
-            cf val = v[Perm<P>::at(j)];
-            if (j > 0) val = cmul(val, prm.twp[(j - 1) * T + t]);           // W_M^(j*t)
-            sm[G::pad(32 * t + j)] = val;
-        }
-        __syncwarp();
-        fft_pass_load<LOG2M, 5, 1, float>(v, sm, t);
+        screen_pass0<T>(v, sm, prm.twp, t);
         __syncwarp();
         if (lane == 0 && next < units) {
             asm volatile("" ::"r"(__float_as_uint(v[P - 1].y)) : "memory");
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             issue(next);
         }
-#pragma unroll
-        for (int c = 0; c < GS; c++) Dft<T, float>::run(v + c * T);        // v[reg(m)] = Z[t + T*m]
-
-        // ---- the bound over the mirror pairs (k, M-k), k = t + T*m, m < 16 ----
-        float acc = 0.f;
-#pragma unroll
-        for (int m = 0; m < P / 2; m++) {
-            const cf zk = v[C::reg(m)];
-            const cf zp = v[C::reg(P - 1 - m)];
-            const cf zs = v[C::reg((P - m) & (P - 1))];
-            cf src, zm;
-            src.x = lane0 ? zs.x : zp.x;
-            src.y = lane0 ? zs.y : zp.y;
-            zm.x = __shfl_sync(0xffffffffu, src.x, partner, T);
-            zm.y = __shfl_sync(0xffffffffu, src.y, partner, T);
-            const cf zmc = cconj(zm);
-            const cf e = cadd(zk, zmc);
-            if constexpr (C::PAIR_BOUND) {
-                // the pair bound of score_screen_warp_kernel: |2Y_k| A[k] + |2Y_(M-k)| A[M-k] <= sqrt(|e|^2 + |d|^2) B[k]
-                const cf d = csub(zk, zmc);
-                const cf q = pfma(d, d, pmul(e, e));
-                acc = fmaf(sqrt_approx(q.x + q.y), prm.sb[t + T * m], acc);
-            } else {
-                const float4 sv = prm.sw[t + T * m];            // (w_k.x, w_k.y, A[k], A[M-k])
-                const cf o = cmul_negi(csub(zk, zmc));
-                const cf wo = cmul(o, cf{sv.x, sv.y});
-                const cf y1 = cadd(e, wo);                      // 2*Y_k
-                const cf y2 = csub(e, wo);                      // 2*conj(Y_(M-k))
-                const cf q1 = pmul(y1, y1), q2 = pmul(y2, y2);
-                acc = fmaf(sqrt_approx(q1.x + q1.y), sv.z, fmaf(sqrt_approx(q2.x + q2.y), sv.w, acc));
-            }
-        }
-        {   // k = M/2: lane 0 of the group, slot 16
-            const cf z = v[C::reg(P / 2)];
-            const cf q = pmul(z, z);
-            acc = fmaf(sqrt_approx(q.x + q.y), lane0 ? 2.f * prm.a_mid : 0.f, acc);
-        }
-        acc = group_sum_f<T>(acc);
+        screen_pass1<T>(v);                             // v[screen_reg<T>(m)] = Z[t + T*m]
+        const float acc = screen_bound<T, C::PAIR_BOUND>(v, prm, t, lane0, partner);
 
         float U = acc * rs.rstd * 1.00001f + MUSE_SCREEN_SLACK;
         if (!(U == U)) U = 2.f;
@@ -206,83 +142,20 @@ score_screen_sub_kernel(const ScreenParams prm, const unsigned warp_bytes, const
         const float cut_now = __uint_as_float(__shfl_sync(0xffffffffu, cut_raw, 0));
         const bool need = U >= cut_now && U < 1.5f;                          // uniform over the T lanes of a series
         if (__any_sync(0xffffffffu, need)) {
-            // ---- conj(Y)*X on the mirror pairs, in place ----
-#pragma unroll
-            for (int m = 0; m < P / 2; m++) {
-                const cf zk = v[C::reg(m)];
-                const cf zp = v[C::reg(P - 1 - m)];
-                const cf zs = v[C::reg((P - m) & (P - 1))];
-                cf src, zm;
-                src.x = lane0 ? zs.x : zp.x;
-                src.y = lane0 ? zs.y : zp.y;
-                zm.x = __shfl_sync(0xffffffffu, src.x, partner, T);
-                zm.y = __shfl_sync(0xffffffffu, src.y, partner, T);
-                const float4 sv = prm.sw[t + T * m];
-                const float4 x = prm.sx[t + T * m];
-                cf ok, om;
-                pointwise_pair(zk, zm, cf{sv.x, sv.y}, cf{x.x, x.y}, cf{x.z, x.w}, ok, om);
-                cf rcv;
-                rcv.x = __shfl_sync(0xffffffffu, om.x, partner, T);
-                rcv.y = __shfl_sync(0xffffffffu, om.y, partner, T);
-                v[C::reg(m)] = ok;
-                cf &hi = v[C::reg(P - 1 - m)];
-                hi.x = lane0 ? hi.x : rcv.x;
-                hi.y = lane0 ? hi.y : rcv.y;
-                if (m > 0) {
-                    cf &own = v[C::reg(P - m)];
-                    own.x = lane0 ? om.x : own.x;
-                    own.y = lane0 ? om.y : own.y;
-                }
-            }
-            {   // k = M/2 pairs with itself; w = -i
-                cf &mid = v[C::reg(P / 2)];
-                cf ok, om;
-                pointwise_pair(mid, mid, cf{0.f, -1.f}, prm.x_mid, prm.x_mid, ok, om);
-                mid.x = lane0 ? ok.x : mid.x;
-                mid.y = lane0 ? ok.y : mid.y;
-            }
+            conj_mul_pairs<T>(v, prm.sw, prm.sx, prm.x_mid, t, lane0, partner);
             // ---- inverse FFT_M as swap(FFT(swap(.))) ----
             cf u[P];
 #pragma unroll
-            for (int j = 0; j < P; j++) u[j] = v[C::reg(j)];
+            for (int j = 0; j < P; j++) u[j] = v[screen_reg<T>(j)];
             Dft<P, float>::run(u);
             {
                 const int slot = ex_acquire(ex_locks, lane, w);
-                cf *smr = reinterpret_cast<cf *>(refbase + (size_t)slot * C::EX_BYTES + (size_t)g * C::EX_STRIDE);
-#pragma unroll
-                for (int j = 0; j < P; j++) {
-                    cf val = u[Perm<P>::at(j)];
-                    if (j > 0) val = cmul(val, prm.twp[(j - 1) * T + t]);
-                    smr[G::pad(32 * t + j)] = val;
-                }
-                __syncwarp();
-                fft_pass_load<LOG2M, 5, 1, float>(u, smr, t);
+                screen_pass0<T>(u, reinterpret_cast<cf *>(refbase + (size_t)slot * C::EX_BYTES + (size_t)g * C::EX_STRIDE), prm.twp, t);
                 ex_release(ex_locks, lane, slot);
             }
-#pragma unroll
-            for (int c = 0; c < GS; c++) Dft<T, float>::run(u + c * T);   // u[c*T + Perm(jj)] = (cc'[2i+1], cc'[2i]), i = t + c*T + 32*jj
-            float m_in = 0.f, m_out = 0.f;
-            const int base = 2 * t - prm.win_lo;
-#pragma unroll
-            for (int c = 0; c < GS; c++) {
-#pragma unroll
-                for (int jj = 0; jj < T; jj++) {
-                    const cf r = u[c * T + Perm<T>::at(jj)];
-                    const int i2 = base + 2 * (c * T + 32 * jj);
-                    const bool in0 = (i2 & (2 * M - 1)) <= prm.win_len;
-                    const bool in1 = ((i2 + 1) & (2 * M - 1)) <= prm.win_len;
-                    const float a0 = fabsf(r.y), a1 = fabsf(r.x);
-                    m_in = fmaxf(m_in, in0 ? a0 : 0.f);
-                    m_out = fmaxf(m_out, in0 ? 0.f : a0);
-                    m_in = fmaxf(m_in, in1 ? a1 : 0.f);
-                    m_out = fmaxf(m_out, in1 ? 0.f : a1);
-                }
-            }
-#pragma unroll
-            for (int off = T / 2; off > 0; off >>= 1) {
-                m_in = fmaxf(m_in, __shfl_xor_sync(0xffffffffu, m_in, off));
-                m_out = fmaxf(m_out, __shfl_xor_sync(0xffffffffu, m_out, off));
-            }
+            screen_pass1<T>(u);         // u[c*T + Perm(jj)] = (cc'[2i+1], cc'[2i]), i = t + c*T + 32*jj
+            float m_in, m_out;
+            window_maxima<T>(u, t, prm.win_lo, prm.win_len, m_in, m_out);
             if (need) {
                 const float rstd = rs.rstd;
                 U = refine_decide(U, m_in * rstd, m_out * rstd, L, prm.grouped);
@@ -293,7 +166,7 @@ score_screen_sub_kernel(const ScreenParams prm, const unsigned warp_bytes, const
 #pragma unroll
             for (int gg = 0; gg < GS; gg++) {
                 const float Lg = __shfl_sync(0xffffffffu, Lc, gg * T);
-                if (Lg >= prm.thr && Lg >= cut_now) cut_count_and_raise(prm, Lg, lane);
+                if (Lg >= prm.thr && Lg >= cut_now) cut_count_and_raise(prm.cut_bits, prm.cut_hist, prm.top_n, Lg, lane);
             }
         }
         if (lane0 && valid) {
