@@ -113,8 +113,10 @@ struct muse_ctx {
     cudaStream_t own_stream;   // created with the context
     std::mutex mu;
     std::vector<RunScratch> pool;   // scratch sets of destroyed batches, reused by the next muse_batch_create
-    unsigned char *h_stage[3];      // pinned staging ring for rows that arrive in pageable host memory (muse_group_append)
+    unsigned char *h_stage[3];      // pinned staging ring for rows that arrive in pageable host memory (muse_group_append, muse_group_roll)
     cudaEvent_t stage_ev[3];
+    double *d_roll;                 // device buffer of the new samples of muse_group_roll: at most MUSE_STAGE_BYTES
+    size_t d_roll_bytes;
     // multi-query bounds on the tensor cores (muse_bounds_tc.cuh): magnitudes of the store and weights of a launch's queries
     unsigned char *tc_a, *tc_b;     // bf16 tiles: [S/128][16][16 KB] and [16][32 KB]
     size_t tc_a_bytes;
@@ -230,6 +232,7 @@ extern "C" void muse_ctx_destroy(muse_ctx *c) {
     cudaFree(c->d_mt);
     if (c->h_mt) cudaFreeHost(c->h_mt);
     cudaFree(c->d_multi_refs);
+    cudaFree(c->d_roll);
     cudaStreamDestroy(c->own_stream);
     delete c;
 }
@@ -347,26 +350,29 @@ extern "C" void muse_group_destroy(muse_group *g) {
     delete g;
 }
 
-// Pageable host rows -> slab through a ring of three pinned buffers: MUSE_STAGE_THREADS host threads copy chunk c into
-// buffer c % 3 while chunk c - 1 is on the wire (at most two DMA copies outstanding, so a buffer is free again when its
-// turn comes).  The chunk size is a whole number of rows.
+// Pageable host rows of `width` doubles -> the device through a ring of three pinned buffers: MUSE_STAGE_THREADS host threads
+// copy chunk c into buffer c % 3 while chunk c - 1 is on the wire (at most two DMA copies outstanding, so a buffer is free
+// again when its turn comes).  A chunk is a whole number of rows, at most MUSE_STAGE_BYTES; queue(r0, nr, pinned) enqueues on
+// the context's stream the copy (and whatever follows it) that takes rows [r0, r0 + nr) out of the pinned buffer.
 #define MUSE_STAGE_BYTES ((size_t)64 << 20)
-static int append_staged(muse_group *g, const double *rows, int64_t n_series) {
-    muse_ctx *c = g->ctx;
-    cudaStream_t st = c->stream;
+static int64_t stage_rows_per_chunk(int64_t width) { return (int64_t)(MUSE_STAGE_BYTES / (sizeof(double) * (size_t)width)); }
+
+template <typename Queue>
+static int stage_rows(muse_ctx *c, const double *rows, int64_t n_rows, int64_t width, Queue &&queue) {
     for (int i = 0; i < 3; i++) {
         if (!c->h_stage[i]) CU(cudaHostAlloc((void **)&c->h_stage[i], MUSE_STAGE_BYTES, cudaHostAllocDefault));
         if (!c->stage_ev[i]) CU(cudaEventCreateWithFlags(&c->stage_ev[i], cudaEventDisableTiming));
     }
-    const size_t row_bytes = sizeof(double) * (size_t)g->N;
+    cudaStream_t st = c->stream;
+    const size_t row_bytes = sizeof(double) * (size_t)width;
     if (row_bytes > MUSE_STAGE_BYTES) return fail(MUSE_ERR_UNSUPPORTED, "a row of %zu bytes exceeds the staging buffer", row_bytes);
-    const int64_t rows_per_chunk = (int64_t)(MUSE_STAGE_BYTES / row_bytes);
-    const int64_t n_chunks = (n_series + rows_per_chunk - 1) / rows_per_chunk;
+    const int64_t rows_per_chunk = stage_rows_per_chunk(width);
+    const int64_t n_chunks = (n_rows + rows_per_chunk - 1) / rows_per_chunk;
     unsigned hw = std::thread::hardware_concurrency();
     const char *env = getenv("MUSE_STAGE_THREADS");
     int n_threads = env ? atoi(env) : (int)std::min<unsigned>(hw ? hw : 4u, 12u);
     if (n_threads < 1) n_threads = 1;
-    if ((size_t)n_series * row_bytes < ((size_t)8 << 20)) n_threads = 1;      // small appends: not worth the threads
+    if ((size_t)n_rows * row_bytes < ((size_t)8 << 20)) n_threads = 1;      // small copies: not worth the threads
     std::vector<std::atomic<int>> done((size_t)n_chunks);
     for (auto &d : done) d.store(0, std::memory_order_relaxed);
     std::atomic<int64_t> writable(std::min<int64_t>(n_chunks, 2));      // chunks whose buffer may be filled
@@ -378,7 +384,7 @@ static int append_staged(muse_group *g, const double *rows, int64_t n_series) {
                 if (abort_flag.load(std::memory_order_relaxed)) return;
                 std::this_thread::yield();
             }
-            const int64_t r0 = ch * rows_per_chunk, nr = std::min<int64_t>(rows_per_chunk, n_series - r0);
+            const int64_t r0 = ch * rows_per_chunk, nr = std::min<int64_t>(rows_per_chunk, n_rows - r0);
             const size_t bytes = (size_t)nr * row_bytes;
             const size_t lo = bytes * (size_t)w / (size_t)n_threads / 64 * 64, hi = (w + 1 == n_threads) ? bytes : bytes * (size_t)(w + 1) / (size_t)n_threads / 64 * 64;
             if (hi > lo) memcpy(c->h_stage[ch % 3] + lo, reinterpret_cast<const unsigned char *>(rows) + (size_t)r0 * row_bytes + lo, hi - lo);
@@ -390,7 +396,7 @@ static int append_staged(muse_group *g, const double *rows, int64_t n_series) {
     cudaError_t e = cudaSuccess;
     // the calling thread is worker 0 and the one that talks to the device
     for (int64_t ch = 0; ch < n_chunks && e == cudaSuccess; ch++) {
-        const int64_t r0 = ch * rows_per_chunk, nr = std::min<int64_t>(rows_per_chunk, n_series - r0);
+        const int64_t r0 = ch * rows_per_chunk, nr = std::min<int64_t>(rows_per_chunk, n_rows - r0);
         {
             const size_t bytes = (size_t)nr * row_bytes;
             const size_t hi = (n_threads == 1) ? bytes : bytes / (size_t)n_threads / 64 * 64;
@@ -398,9 +404,7 @@ static int append_staged(muse_group *g, const double *rows, int64_t n_series) {
             done[(size_t)ch].fetch_add(1, std::memory_order_release);
         }
         while (done[(size_t)ch].load(std::memory_order_acquire) < n_threads) std::this_thread::yield();
-        double *dst = g->slab + (size_t)(g->size + r0) * g->ld;
-        if (g->ld == g->N) e = cudaMemcpyAsync(dst, c->h_stage[ch % 3], (size_t)nr * row_bytes, cudaMemcpyHostToDevice, st);
-        else e = cudaMemcpy2DAsync(dst, sizeof(double) * (size_t)g->ld, c->h_stage[ch % 3], row_bytes, row_bytes, (size_t)nr, cudaMemcpyHostToDevice, st);
+        e = queue(r0, nr, reinterpret_cast<const double *>(c->h_stage[ch % 3]));
         if (e == cudaSuccess) e = cudaEventRecord(c->stage_ev[ch % 3], st);
         if (e == cudaSuccess && ch >= 1) e = cudaEventSynchronize(c->stage_ev[(ch - 1) % 3]);      // buffer (ch + 2) % 3 is free again
         writable.store(ch + 3, std::memory_order_release);
@@ -437,7 +441,12 @@ extern "C" int muse_group_append(muse_group *g, const double *rows, int64_t n_se
         // pageable rows (a Go slice, a numpy array): a direct cudaMemcpyAsync stages them through the driver's single
         // bounce buffer at a fraction of the link rate -> chunks are copied into a pinned ring by several host threads
         // while the previous chunk is on the wire
-        rc = append_staged(g, rows, n_series);
+        const size_t row_bytes = sizeof(double) * (size_t)g->N;
+        rc = stage_rows(g->ctx, rows, n_series, g->N, [&](int64_t r0, int64_t nr, const double *src) {
+            double *dst = g->slab + (size_t)(g->size + r0) * g->ld;
+            if (g->ld == g->N) return cudaMemcpyAsync(dst, src, (size_t)nr * row_bytes, cudaMemcpyHostToDevice, st);
+            return cudaMemcpy2DAsync(dst, sizeof(double) * (size_t)g->ld, src, row_bytes, row_bytes, (size_t)nr, cudaMemcpyHostToDevice, st);
+        });
         if (rc != MUSE_OK) return rc;
     } else if (g->ld == g->N) {   // rows are already at the slab's pitch: one flat copy (a pitched copy of 10^6 rows is not always at DMA rate)
         CU(cudaMemcpyAsync(g->slab + (size_t)g->size * g->ld, rows, sizeof(double) * (size_t)g->N * (size_t)n_series,
@@ -682,6 +691,68 @@ extern "C" int muse_group_read_row(muse_group *g, int64_t local_index, double *o
     CU(cudaMemcpyAsync(out_row, g->slab + (size_t)local_index * g->ld, sizeof(double) * (size_t)g->N, cudaMemcpyDeviceToHost,
                        g->ctx->stream));
     CU(cudaStreamSynchronize(g->ctx->stream));
+    return MUSE_OK;
+}
+
+// muse_group_roll / muse_group_roll_device: argument errors, reported before any device work.
+static int roll_check(const muse_group *g, int64_t first, int64_t n_rows, const double *samples, int64_t k, const char *fn) {
+    if (!g) return fail(MUSE_ERR_INVALID_ARG, "%s: group is NULL", fn);
+    if (k < 0 || k > g->N) return fail(MUSE_ERR_INVALID_ARG, "%s: k = %lld not in [0, %lld]", fn, (long long)k, (long long)g->N);
+    if (first < 0 || n_rows < 0 || first > g->size || n_rows > g->size - first)
+        return fail(MUSE_ERR_INVALID_ARG, "%s: rows [%lld, %lld + %lld) not in the store's %lld", fn, (long long)first, (long long)first,
+                    (long long)n_rows, (long long)g->size);
+    if (!samples && k > 0 && n_rows > 0) return fail(MUSE_ERR_INVALID_ARG, "%s: samples is NULL", fn);
+    return MUSE_OK;
+}
+
+extern "C" int muse_group_roll_device(muse_group *g, int64_t first, int64_t n_rows, const double *d_samples, int64_t k) {
+    int rc = roll_check(g, first, n_rows, d_samples, k, "muse_group_roll_device");
+    if (rc != MUSE_OK || k == 0 || n_rows == 0) return rc;
+    CU(cudaSetDevice(g->ctx->device));
+    CU(launch_roll_rows(g->slab, g->ld, (int)g->N, first, n_rows, d_samples, (int)k, g->row_stat, g->ctx->sm_count, g->ctx->stream));
+    CU(cudaStreamSynchronize(g->ctx->stream));
+    return MUSE_OK;
+}
+
+// The new samples reach the device in chunks of whole rows through ctx->d_roll (one buffer: the copy of chunk c + 1 is queued
+// behind the roll of chunk c on the same stream); page-locked samples are copied from where they are, pageable ones through the
+// pinned staging ring.
+extern "C" int muse_group_roll(muse_group *g, int64_t first, int64_t n_rows, const double *samples, int64_t k) {
+    int rc = roll_check(g, first, n_rows, samples, k, "muse_group_roll");
+    if (rc != MUSE_OK || k == 0 || n_rows == 0) return rc;
+    const size_t row_bytes = sizeof(double) * (size_t)k;
+    if (row_bytes > MUSE_STAGE_BYTES) return fail(MUSE_ERR_UNSUPPORTED, "muse_group_roll: %lld new samples per row exceed the %zu-byte staging buffer",
+                                                  (long long)k, MUSE_STAGE_BYTES);
+    muse_ctx *c = g->ctx;
+    CU(cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    const int64_t rows_per_chunk = stage_rows_per_chunk(k);
+    const size_t want = row_bytes * (size_t)std::min<int64_t>(n_rows, rows_per_chunk);
+    if (c->d_roll_bytes < want) {
+        CU(cudaStreamSynchronize(st));
+        cudaFree(c->d_roll);
+        c->d_roll = nullptr;
+        c->d_roll_bytes = 0;
+        CU(cudaMalloc(&c->d_roll, want));
+        c->d_roll_bytes = want;
+    }
+    auto queue = [&](int64_t r0, int64_t nr, const double *src) {
+        cudaError_t e = cudaMemcpyAsync(c->d_roll, src, (size_t)nr * row_bytes, cudaMemcpyHostToDevice, st);
+        if (e == cudaSuccess) e = launch_roll_rows(g->slab, g->ld, (int)g->N, first + r0, nr, c->d_roll, (int)k, g->row_stat, c->sm_count, st);
+        return e;
+    };
+    cudaPointerAttributes attr;
+    const bool pinned = cudaPointerGetAttributes(&attr, samples) == cudaSuccess &&
+                        (attr.type == cudaMemoryTypeHost || attr.type == cudaMemoryTypeManaged);
+    (void)cudaGetLastError();
+    if (pinned) {
+        for (int64_t r0 = 0; r0 < n_rows; r0 += rows_per_chunk)
+            CU(queue(r0, std::min<int64_t>(rows_per_chunk, n_rows - r0), samples + (size_t)r0 * (size_t)k));
+    } else {
+        rc = stage_rows(c, samples, n_rows, k, queue);
+        if (rc != MUSE_OK) return rc;
+    }
+    CU(cudaStreamSynchronize(st));
     return MUSE_OK;
 }
 

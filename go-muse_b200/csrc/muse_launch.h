@@ -78,6 +78,11 @@ cudaError_t launch_mag_tiles(const ScreenParams &p, unsigned char *a_tiles, floa
 cudaError_t launch_weight_tiles(const float4 *const *d_sw, int nq, unsigned char *b_tiles, cudaStream_t st);
 cudaError_t launch_bounds_tc(const TcBoundsParams &p, cudaStream_t st);
 
+// rows [first, first + count) of the slab slide forward by k samples in place, the k new samples of row first + i taken from
+// d_add[i * k ..]; writes their RowStat and, for odd N, the pad column (kernels_roll.cu)
+cudaError_t launch_roll_rows(double *slab, int64_t ld, int N, int64_t first, int64_t count, const double *d_add, int k,
+                             RowStat *stat, int sm_count, cudaStream_t st);
+
 // ---- series above n = 16384 (kernels_long.cu): Stockham passes through global memory, two series per transform ----
 struct LongParams {
     const double *slab;      // [rows][ld] fp64

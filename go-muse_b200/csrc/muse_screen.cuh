@@ -451,6 +451,27 @@ __device__ __forceinline__ RowStat make_row_stat(double pivot, double s1, double
     r.pad = 0u;
     return r;
 }
+
+// The sums of one row for its RowStat, taken by one warp: about the row's first sample (the pivot), lane l adding samples
+// l, l + 32, l + 64, ... in that order, then reduced with xor shuffles.  row_stats_kernel and roll_rows_kernel
+// (kernels_roll.cu) both go through this, so a rolled row's RowStat is bit-identical to the one the same row gets at ingest.
+struct RowSums {
+    double s1 = 0.0, s2 = 0.0;
+    __device__ __forceinline__ void add(double v, double pivot) {
+        const double x = v - pivot;
+        s1 += x;
+        s2 = fma(x, x, s2);
+    }
+    // every lane of the warp calls this; every lane gets the row's RowStat
+    __device__ __forceinline__ RowStat warp_stat(double pivot, int N) {
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) {
+            s1 += __shfl_xor_sync(0xffffffffu, s1, off);
+            s2 += __shfl_xor_sync(0xffffffffu, s2, off);
+        }
+        return make_row_stat(pivot, s1, s2, N);
+    }
+};
 #endif
 
 // RowStat of rows first .. first+count-1; for an odd series length the row's mean is also written into the first pad
@@ -466,19 +487,10 @@ static __global__ void row_stats_kernel(double *__restrict__ slab, int64_t ld, i
     for (int64_t i = warp0; i < count; i += nwarp) {
         const double *row = slab + (first + i) * ld;
         const double pivot = row[0];
-        double s1 = 0.0, s2 = 0.0;
-        for (int k = lane; k < N; k += 32) {
-            const double x = row[k] - pivot;
-            s1 += x;
-            s2 = fma(x, x, s2);
-        }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            s1 += __shfl_xor_sync(0xffffffffu, s1, off);
-            s2 += __shfl_xor_sync(0xffffffffu, s2, off);
-        }
+        RowSums rs;
+        for (int k = lane; k < N; k += 32) rs.add(row[k], pivot);
+        const RowStat r = rs.warp_stat(pivot, N);
         if (lane == 0) {
-            const RowStat r = make_row_stat(pivot, s1, s2, N);
             stat[first + i] = r;
             if (N & 1) slab[(first + i) * ld + N] = r.mean;
         }

@@ -214,6 +214,69 @@ func (g *Group) syncDevice() error {
 	return nil
 }
 
+// rollChunkBytes bounds the new samples handed to muse_group_roll per call: the library copies them (through its pinned
+// staging ring when they sit in pageable Go memory), so nothing larger than one chunk is duplicated on the host.
+const rollChunkBytes = 64 << 20
+
+// Roll slides every series forward by k = len(samples[i]) new samples, y <- y[k:] ++ samples[i] for the i-th series in Add
+// order: on the device store in place (the store is not sent to the device again) and in each Series' values, which a later
+// store rebuild uploads.  Every row holds the same k, 0 <= k <= Length(); the checks come before any device call.  A sharded
+// group (SetShard) rolls its own block of series; nothing is exchanged.  When the device fails part-way the store is dropped
+// and rebuilt from the unchanged values by the next call that needs it, so a failed Roll has no effect.
+func (g *Group) Roll(samples [][]float64) error {
+	if len(samples) != len(g.series) {
+		return fmt.Errorf("Roll: %d rows of samples for %d series", len(samples), len(g.series))
+	}
+	if len(samples) == 0 {
+		return nil
+	}
+	k := len(samples[0])
+	for i, r := range samples {
+		if len(r) != k {
+			return fmt.Errorf("Roll: row %d has %d samples, row 0 has %d", i, len(r), k)
+		}
+	}
+	if k > g.n {
+		return fmt.Errorf("Roll: %d new samples exceed the series length %d", k, g.n)
+	}
+	if k == 0 {
+		return nil
+	}
+	if err := g.syncDevice(); err != nil {
+		return err
+	}
+	per := rollChunkBytes / (8 * k)
+	if per < 1 {
+		per = 1
+	}
+	if per > len(samples) {
+		per = len(samples)
+	}
+	buf := make([]float64, 0, per*k)
+	for first := 0; first < len(samples); first += per {
+		end := first + per
+		if end > len(samples) {
+			end = len(samples)
+		}
+		buf = buf[:0]
+		for _, r := range samples[first:end] {
+			buf = append(buf, r...)
+		}
+		if rc := C.muse_group_roll(g.store, C.int64_t(first), C.int64_t(end-first), (*C.double)(unsafe.Pointer(&buf[0])), C.int64_t(k)); rc != C.MUSE_OK {
+			err := lastError(rc)
+			C.muse_group_destroy(g.store)
+			g.store = nil
+			return err
+		}
+	}
+	for i, s := range g.series {
+		v := make([]float64, 0, g.n)
+		v = append(v, s.vals[k:]...)
+		s.vals = append(v, samples[i]...)
+	}
+	return nil
+}
+
 // keyCols maps label names to device columns; unknown names mean "no series has it", which
 // puts every series in one group (labels.go:61-65 skips absent keys).
 func (g *Group) keyCols(groupByLabels []string) []int32 {

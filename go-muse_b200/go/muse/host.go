@@ -102,7 +102,7 @@ func NewSeries(y []float64, labels *Labels) *Series {
 // Length is the number of samples.
 func (s *Series) Length() int { return len(s.vals) }
 
-// Values exposes the samples; the facade never writes to them.
+// Values exposes the samples; the facade never writes to them (Group.Roll replaces them by a new slice).
 func (s *Series) Values() []float64 { return s.vals }
 
 // Labels returns the label set given at construction.

@@ -47,7 +47,7 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 # translation units of libmuse_b200.so: the C ABI and one file per family of kernel instantiations
 SOURCES = ["muse_api.cu", "kernels_exact.cu", "kernels_screen_warp.cu", "kernels_screen_big.cu", "kernels_screen_big13_a.cu", "kernels_screen_big13_b.cu", "kernels_screen_big13_c.cu",
            "kernels_screen_big13_d.cu", "kernels_screen_multi.cu", "kernels_bounds_tc.cu", "kernels_long.cu",
-           "kernels_screen_sub1.cu", "kernels_screen_sub2.cu", "kernels_screen_sub3.cu", "kernels_screen_sub4.cu"]
+           "kernels_screen_sub1.cu", "kernels_screen_sub2.cu", "kernels_screen_sub3.cu", "kernels_screen_sub4.cu", "kernels_roll.cu"]
 
 
 class MuseError(Exception):
@@ -139,6 +139,8 @@ ABI = {
     "muse_group_clear": (C.c_int, [_vp]),
     "muse_group_read_row": (C.c_int, [_vp, C.c_int64, _dp]),
     "muse_group_read_rows": (C.c_int, [_vp, C.c_int64, C.c_int64, _vp]),
+    "muse_group_roll": (C.c_int, [_vp, C.c_int64, C.c_int64, _vp, C.c_int64]),
+    "muse_group_roll_device": (C.c_int, [_vp, C.c_int64, C.c_int64, _vp, C.c_int64]),
     "muse_batch_create": (C.c_int, [_vp, _vp, _dp, C.c_int64, C.POINTER(_vp)]),
     "muse_batch_destroy": (None, [_vp]),
     "muse_batch_fft_len": (C.c_int64, [_vp]),
@@ -291,6 +293,23 @@ class DeviceStore:
             out = np.empty((n_rows, self.series_len))
         _check(lib().muse_group_read_rows(self.h, first, n_rows, out.ctypes.data_as(_vp)))
         return out
+
+    def roll(self, samples: np.ndarray, first: int = 0):
+        """muse_group_roll: rows [first, first + n_rows) slide forward by k samples in place, row <- row[k:] ++ samples[i],
+        where samples is a host array [n_rows][k] (page-locked memory, e.g. from muse_host_alloc, is copied directly)."""
+        X = np.ascontiguousarray(samples, dtype=np.float64)
+        if X.ndim != 2:
+            raise MuseError(MUSE_ERR_INVALID_ARG, "roll: samples must be [n_rows][k], got shape %r" % (X.shape,))
+        n_rows, k = X.shape
+        if k > self.series_len:
+            raise MuseError(MUSE_ERR_INVALID_ARG, "roll: k = %d new samples exceed the series length %d" % (k, self.series_len))
+        if first < 0:
+            raise MuseError(MUSE_ERR_INVALID_ARG, "roll: first = %d < 0" % first)
+        _check(lib().muse_group_roll(self.h, first, n_rows, X.ctypes.data_as(_vp), k))
+
+    def roll_device(self, ptr: int, first: int, n_rows: int, k: int):
+        """muse_group_roll_device: as roll, the [n_rows][k] samples in DEVICE memory at address ptr."""
+        _check(lib().muse_group_roll_device(self.h, first, n_rows, _vp(ptr), k))
 
     def read_rows_ptr(self, first: int, n_rows: int, ptr: int):
         _check(lib().muse_group_read_rows(self.h, first, n_rows, _vp(ptr)))
@@ -560,7 +579,8 @@ def NewLabels(labels: Dict[str, str]) -> Labels:
 
 
 class Series:
-    """series.go:8-42.  The values are never modified (go-muse z-normalises in place)."""
+    """series.go:8-42.  The values are never modified in place (go-muse z-normalises in place); Group.Roll replaces them by
+    the rolled window."""
 
     def __init__(self, y, labels: Optional[Labels] = None):
         if labels is None or labels.Len() == 0:
@@ -620,6 +640,35 @@ class Group:
                                 % (s.Length(), self.n))
             self.registry[uid] = len(self.series)
             self.series.append(s)
+        return None
+
+    def Roll(self, samples):
+        """Every series slides forward by k new samples, y <- y[k:] ++ samples[i] for the i-th series in Add order, on the
+        device store in place (no re-upload) and in each Series' values (a later store rebuild uploads from those).
+        samples: [len(series)][k], 0 <= k <= Length(); checked before any device call."""
+        rows = [np.asarray(r, dtype=np.float64) for r in samples]
+        if len(rows) != len(self.series):
+            raise MuseError(MUSE_ERR_INVALID_ARG, "Roll: %d rows of samples for %d series" % (len(rows), len(self.series)))
+        if not rows:
+            return None
+        k = rows[0].size
+        for i, r in enumerate(rows):
+            if r.ndim != 1 or r.size != k:
+                raise MuseError(MUSE_ERR_INVALID_ARG, "Roll: row %d has shape %r, row 0 has %d samples" % (i, r.shape, k))
+        if k > self.n:
+            raise MuseError(MUSE_ERR_INVALID_ARG, "Roll: %d new samples exceed the series length %d" % (k, self.n))
+        if k == 0:
+            return None
+        store = self._sync_device()
+        try:
+            store.roll(np.stack(rows), 0)
+        except MuseError:
+            # rows rolled before a device failure: drop the store, the next call rebuilds it from the unchanged values
+            store.close()
+            self._store = None
+            raise
+        for s, r in zip(self.series, rows):
+            s.y = np.concatenate([s.y[k:], r])
         return None
 
     def FilterByLabelValues(self, labels: Labels) -> List[Series]:

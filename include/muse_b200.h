@@ -144,6 +144,20 @@ int  muse_group_clear(muse_group *g);
 int  muse_group_read_row(muse_group *g, int64_t local_index, double *out_row);
 int  muse_group_read_rows(muse_group *g, int64_t first, int64_t n_rows, double *out_rows);
 
+/* Slide rows [first, first + n_rows) of the store forward by k samples, in place (a window of the last N samples of every
+ * series, advanced without sending the store over the link again):
+ *     row_i <- row_i[k .. N) ++ samples[i - first][0 .. k)
+ * samples: dense [n_rows][k] fp64 HOST rows (pageable or page-locked) / DEVICE rows on the context's device.
+ * 0 <= k <= N (k == 0: nothing to do; k == N replaces the rows).  Row statistics (and, for odd N, the pad column) are
+ * recomputed, bit-identical to what muse_group_append computes for the same rows; labels, size and global offset are
+ * unchanged.  Batches created earlier stay valid and see the new rows.  Everything is complete when the call returns (as
+ * muse_group_append).  Argument errors (NULL g; NULL samples with k > 0 and n_rows > 0; k < 0 or k > N; a row range outside
+ * [0, size)) return MUSE_ERR_INVALID_ARG before any device work and leave the store untouched.  Host samples reach the device
+ * in chunks of whole rows of at most 64 MB (page-locked: copied directly; pageable: through the pinned staging ring of
+ * muse_group_append), so k may not exceed 8 M samples there (MUSE_ERR_UNSUPPORTED). */
+int  muse_group_roll(muse_group *g, int64_t first, int64_t n_rows, const double *samples, int64_t k);
+int  muse_group_roll_device(muse_group *g, int64_t first, int64_t n_rows, const double *d_samples, int64_t k);
+
 /* ---- batch -----------------------------------------------------------------
  * NewBatch (muse_batch.go:23-52): checks ref_len against the group
  * (MUSE_ERR_LENGTH_MISMATCH), n = nextPowOf2(ref_len), computes on the device
