@@ -11,9 +11,12 @@
 #include <cstdlib>
 #include <cstring>
 #include <atomic>
+#include <deque>
+#include <memory>
 #include <mutex>
 #include <thread>
 #include <unordered_map>
+#include <utility>
 #include <vector>
 
 #include "../../include/muse_b200.h"
@@ -54,6 +57,95 @@ extern "C" const char *muse_last_error(void) { return g_err; }
 extern "C" const char *muse_version(void) { return "muse_b200 0.1 (sm_100a)"; }
 
 // ------------------------------------------------------------------------------------
+// owners of device and page-locked memory and of events
+// ------------------------------------------------------------------------------------
+// Every device and page-locked allocation of the library is one of these (muse_host_alloc hands its memory to the caller),
+// so whoever holds the owner frees it, on every path.  g_held counts the bytes they hold: [0] device, [1] page-locked.
+static std::atomic<int64_t> g_held[2];
+
+template <typename T, bool Pinned>
+class Buf {
+  public:
+    Buf() = default;
+    Buf(Buf &&o) noexcept { swap(o); }
+    Buf &operator=(Buf &&o) noexcept {      // the old contents go to `o`, which frees them
+        swap(o);
+        return *this;
+    }
+    ~Buf() { release(); }
+    T *get() const { return p_; }
+    operator T *() const { return p_; }
+    int64_t cap() const { return cap_; }
+    // Room for n elements: when n exceeds the capacity, the buffer is freed and reallocated; the contents are not kept.
+    cudaError_t grow(int64_t n) {
+        if (n <= cap_) return cudaSuccess;
+        release();
+        const size_t bytes = sizeof(T) * (size_t)n;
+        cudaError_t e = Pinned ? cudaHostAlloc((void **)&p_, bytes, cudaHostAllocDefault) : cudaMalloc((void **)&p_, bytes);
+        if (e != cudaSuccess) {
+            p_ = nullptr;
+            return e;
+        }
+        cap_ = n;
+        g_held[Pinned] += (int64_t)bytes;
+        return cudaSuccess;
+    }
+
+  private:
+    void swap(Buf &o) {
+        std::swap(p_, o.p_);
+        std::swap(cap_, o.cap_);
+    }
+    void release() {      // cudaFree waits for the device, so work still queued on the buffer is done first
+        if (!p_) return;
+        if (Pinned) cudaFreeHost(p_);
+        else cudaFree(p_);
+        g_held[Pinned] -= (int64_t)(sizeof(T) * (size_t)cap_);
+        p_ = nullptr;
+        cap_ = 0;
+    }
+    T *p_ = nullptr;
+    int64_t cap_ = 0;
+};
+template <typename T>
+using DevBuf = Buf<T, false>;
+using PinnedBuf = Buf<unsigned char, true>;
+
+// K events, created together on first use
+template <int K>
+class Events {
+  public:
+    Events() = default;
+    Events(Events &&o) noexcept { std::swap(e_, o.e_); }
+    Events &operator=(Events &&o) noexcept {
+        std::swap(e_, o.e_);
+        return *this;
+    }
+    ~Events() {
+        for (cudaEvent_t e : e_)
+            if (e) cudaEventDestroy(e);
+    }
+    cudaEvent_t operator[](int i) const { return e_[i]; }
+    cudaError_t create(unsigned flags = cudaEventDefault) {
+        for (cudaEvent_t &e : e_) {
+            const cudaError_t r = e ? cudaSuccess : cudaEventCreateWithFlags(&e, flags);
+            if (r != cudaSuccess) return r;
+        }
+        return cudaSuccess;
+    }
+
+  private:
+    cudaEvent_t e_[K] = {};
+};
+
+extern "C" int muse_held_bytes(int64_t *device_bytes, int64_t *pinned_bytes) {
+    if (!device_bytes || !pinned_bytes) return fail(MUSE_ERR_INVALID_ARG, "muse_held_bytes: NULL argument");
+    *device_bytes = g_held[0].load();
+    *pinned_bytes = g_held[1].load();
+    return MUSE_OK;
+}
+
+// ------------------------------------------------------------------------------------
 // handles
 // ------------------------------------------------------------------------------------
 // Everything a batch needs per run whose size follows the store (not the reference): kept in a small
@@ -66,107 +158,107 @@ extern "C" const char *muse_version(void) { return "muse_b200 0.1 (sm_100a)"; }
 #define MUSE_MULTI_GROUP 256    // queries of one launch of the tensor-core multi-query path (== TcCfg::TN == RefineMultiCfg::QMAX)
 #define MUSE_MULTI_SEPARATE 16  // queries of one group of separate batches in muse_multi_run (one upload, one round trip)
 struct RunScratch {
-    int64_t scratch_cap;
-    double *d_score;
-    int32_t *d_lag;
-    int64_t *d_slot;
-    unsigned long long *d_ckey, *d_skey;
-    int32_t *d_cidx, *d_sidx;
-    int32_t *d_clag, *d_slag;         // 2*lag + sign of the candidates (muse_select.cuh Cand)
-    float *d_U;
-    int32_t *d_list;
-    float *d_L;                       // lower bounds (grouped screened runs, diagnostic entry point)
-    signed char *d_W;                 // grouped screened runs: lag-window verdict of every refined series (ScreenParams::out_W)
-    int64_t d_L_cap;
-    unsigned char *h_pin;             // pinned mailbox for the small device->host results
-    size_t h_pin_bytes;
-    unsigned long long *d_counters;   // [0] ncand, [1] nselected, [2] exact list length, [3] refined
-    SelectState *d_sel;
-    int32_t *d_flag;
-    unsigned *d_cut;                  // fused refinement state: [0] cut bits, [1] series claims of the warp kernel, [2..3] n_refined (u64),
-                                      // [4..] coarse + fine histogram
+    int64_t scratch_cap = 0;                  // entries of the eleven arrays below (ensure_scratch)
+    DevBuf<double> d_score;
+    DevBuf<int32_t> d_lag;
+    DevBuf<int64_t> d_slot;
+    DevBuf<unsigned long long> d_ckey, d_skey;
+    DevBuf<int32_t> d_cidx, d_sidx;
+    DevBuf<int32_t> d_clag, d_slag;           // 2*lag + sign of the candidates (muse_select.cuh Cand)
+    DevBuf<float> d_U;
+    DevBuf<int32_t> d_list;
+    DevBuf<float> d_L;                        // lower bounds (grouped screened runs, diagnostic entry point)
+    DevBuf<signed char> d_W;                  // grouped screened runs: lag-window verdict of every refined series (ScreenParams::out_W)
+    PinnedBuf h_pin;                          // pinned mailbox for the small device->host results
+    DevBuf<unsigned long long> d_counters;    // [0] ncand, [1] nselected, [2] exact list length, [3] refined
+    DevBuf<SelectState> d_sel;
+    DevBuf<int32_t> d_flag;
+    DevBuf<unsigned> d_cut;                   // fused refinement state: [0] cut bits, [1] series claims of the warp kernel, [2..3] n_refined (u64),
+                                              // [4..] coarse + fine histogram
     // group table
-    int64_t table_cap;
-    unsigned long long *d_gmax, *d_hkeys;
-    int32_t *d_gidx;
+    DevBuf<unsigned long long> d_gmax, d_hkeys;
+    DevBuf<int32_t> d_gidx;
     // tables of the reference side.  tab_n: the FFT length the twiddle tables (twM, twn, twp_f, swtw) were filled
     // for -- a set that comes back from the pool with the same n keeps them, only the per-reference ones
     // (d_ref, Xt, sw_f, sx_f, d_mid) are rewritten by muse_batch_create
-    int64_t tab_n, d_ref_cap;
-    int tab_screen;                   // twp_f / swtw / sw_f / sx_f exist for tab_n
-    double *d_ref;                    // padded copy of the reference row
-    cd *Xt, *twM, *twn;
-    cf *twp_f;                        // fp32 screening pass: per-pass twiddles
-    cf *twi_f;                        // n = 4096 .. 16384: twiddle tables of muse_screen_big.cuh
-    float2 *swtw;                     // split twiddles exp(-2*pi*i*k/n), k < M/2, fp32
-    float4 *sw_f;                     // fused kernels: (twn, A[k], A[M-k]) per k < M/2
-    float4 *sx_f;                     // fused refinement: (Xt[k], Xt[M-k]) in fp32 per k < M/2
-    float *sb_f;                      // warp / sub-warp kernels: sqrt(2 (A[k]^2 + A[M-k]^2)) rounded up per k < M/2
-    float *d_mid;                     // [0] std-zero flag of the reference (as float bits), [1] A[M/2], [2..3] Xt[M/2] in fp32
-    cudaEvent_t ev[4];
+    int64_t tab_n = 0;
+    int tab_screen = 0;                       // twp_f / swtw / sw_f / sx_f exist for tab_n
+    DevBuf<double> d_ref;                     // padded copy of the reference row
+    DevBuf<cd> Xt, twM, twn;
+    DevBuf<cf> twp_f;                         // fp32 screening pass: per-pass twiddles
+    DevBuf<cf> twi_f;                         // n = 4096 .. 16384: twiddle tables of muse_screen_big.cuh
+    DevBuf<float2> swtw;                      // split twiddles exp(-2*pi*i*k/n), k < M/2, fp32
+    DevBuf<float4> sw_f;                      // fused kernels: (twn, A[k], A[M-k]) per k < M/2
+    DevBuf<float4> sx_f;                      // fused refinement: (Xt[k], Xt[M-k]) in fp32 per k < M/2
+    DevBuf<float> sb_f;                       // warp / sub-warp kernels: sqrt(2 (A[k]^2 + A[M-k]^2)) rounded up per k < M/2
+    DevBuf<float> d_mid;                      // [0] std-zero flag of the reference (as float bits), [1] A[M/2], [2..3] Xt[M/2] in fp32
+    Events<4> ev;
 };
 
 struct muse_ctx {
-    int device;
-    int sm_count;
-    cudaStream_t stream;       // the stream in use
-    cudaStream_t own_stream;   // created with the context
+    int device = 0;
+    int sm_count = 0;
+    cudaStream_t stream = nullptr;       // the stream in use
+    cudaStream_t own_stream = nullptr;   // created with the context
     std::mutex mu;
-    std::vector<RunScratch> pool;   // scratch sets of destroyed batches, reused by the next muse_batch_create
-    unsigned char *h_stage[3];      // pinned staging ring for rows that arrive in pageable host memory (muse_group_append, muse_group_roll)
-    cudaEvent_t stage_ev[3];
-    double *d_roll;                 // device buffer of the new samples of muse_group_roll: at most MUSE_STAGE_BYTES
-    size_t d_roll_bytes;
+    std::deque<RunScratch> pool;    // scratch sets of destroyed batches, reused by the next muse_batch_create (a deque: taking
+                                    // the front set moves no other set)
+    PinnedBuf h_stage[3];           // pinned staging ring for rows that arrive in pageable host memory (muse_group_append, muse_group_roll)
+    Events<3> stage_ev;
+    DevBuf<double> d_roll;          // device buffer of the new samples of muse_group_roll: at most MUSE_STAGE_BYTES
     // multi-query bounds on the tensor cores (muse_bounds_tc.cuh): magnitudes of the store and weights of a launch's queries
-    unsigned char *tc_a, *tc_b;     // bf16 tiles: [S/128][16][16 KB] and [16][32 KB]
-    size_t tc_a_bytes;
-    float *tc_mid, *tc_amid;        // [S] |2Y_(M/2)| per series, [256] A_q[M/2] per query
-    int64_t tc_mid_cap;
-    void **tc_ptrs;                 // device: [256] sw tables, [256] bound arrays
-    unsigned *d_multi_next;         // work counter of refine_multi_kernel
-    unsigned char *d_mt, *h_mt;     // parameter tables and results of a multi-query launch (MultiTables), device and pinned host
-    int64_t mt_top_n;               // result records per query the two buffers were sized for
-    cudaEvent_t mt_ev[5];           // stage boundaries of the last multi-query launch group: start, magnitudes, bounds, second stages, end
-    int64_t multi_refined, multi_rescored;      // totals of the last muse_multi_run (second stages, fp64 re-scorings)
-    void *d_multi_q;                // query table of refine_multi_kernel (MUSE_MULTI_GROUP entries)
-    double *d_multi_refs;           // [MUSE_MULTI_GROUP][d_multi_ld] reference rows of a muse_multi_run group, pad columns kept zero
-    int64_t d_multi_ld, d_multi_n;
+    DevBuf<unsigned char> tc_a, tc_b;     // bf16 tiles: [S/128][16][16 KB] and [16][32 KB]
+    DevBuf<float> tc_mid, tc_amid;        // [S] |2Y_(M/2)| per series, [256] A_q[M/2] per query
+    DevBuf<void *> tc_ptrs;               // device: [256] sw tables, [256] bound arrays
+    DevBuf<unsigned> d_multi_next;        // work counter of refine_multi_kernel
+    DevBuf<unsigned char> d_mt;           // parameter tables and results of a multi-query launch (MultiTables), device and pinned host
+    PinnedBuf h_mt;
+    Events<5> mt_ev;                // stage boundaries of the last multi-query launch group: start, magnitudes, bounds, second stages, end
+    int64_t multi_refined = 0, multi_rescored = 0;      // totals of the last muse_multi_run (second stages, fp64 re-scorings)
+    DevBuf<MultiQuery> d_multi_q;   // query table of refine_multi_kernel (MUSE_MULTI_GROUP entries)
+    DevBuf<double> d_multi_refs;    // [MUSE_MULTI_GROUP][d_multi_ld] reference rows of a muse_multi_run group, pad columns kept zero
+    int64_t d_multi_ld = 0, d_multi_n = 0;
 };
 
 struct muse_group {
-    muse_ctx *ctx;
-    int64_t N;          // series length
-    int64_t ld;         // row stride in doubles (multiple of 16 -> 128-byte rows)
-    int64_t cap, size;
-    double *slab;       // [cap][ld]
-    int nkeys;
-    int32_t *labels;    // [nkeys][cap]
-    int32_t max_id[MUSE_MAX_LABEL_KEYS];
-    int64_t global_offset;
-    RowStat *row_stat;          // [cap] screening: fp64 mean and fp32 1/std of each row (filled lazily up to stats_upto)
-    int64_t stats_cap, stats_upto;
+    muse_ctx *ctx = nullptr;
+    int64_t N = 0;          // series length
+    int64_t ld = 0;         // row stride in doubles (multiple of 16 -> 128-byte rows)
+    int64_t cap = 0, size = 0;
+    DevBuf<double> slab;    // [cap][ld]
+    int nkeys = 0;
+    DevBuf<int32_t> labels; // [nkeys][cap]
+    int32_t max_id[MUSE_MAX_LABEL_KEYS] = {};
+    int64_t global_offset = 0;
+    DevBuf<RowStat> row_stat;   // [cap] screening: fp64 mean and fp32 1/std of each row (filled lazily up to stats_upto)
+    int64_t stats_upto = 0;
 };
 
 struct muse_batch : RunScratch {
-    muse_ctx *ctx;
-    muse_group *g;
-    int64_t N, n;
-    int log2m;
+    muse_ctx *ctx = nullptr;
+    muse_group *g = nullptr;
+    int64_t N = 0, n = 0;
+    int log2m = 0;
     // fp32 screening pass (n = 128 .. 16384): the tables live in RunScratch
-    int screen_ok;
-    float a_mid;
-    cf x_mid;
-    muse_timing timing;
-    int timing_pending;    // the last run was queued without a final synchronisation (muse_batch_run_partial_device)
-    int fused_run;         // 1: score_fused, 2: score_fused_grouped (d_counters[2] = exact list length, [3] = refined)
-    int prescreened;       // d_U and the cut-off state were filled by the tensor-core multi-query path: the next fused run starts at its tail
-    int signed_run;        // the current run keeps the sign of the scores (muse.go:72-76)
+    int screen_ok = 0;
+    float a_mid = 0.f;
+    cf x_mid = {};
+    muse_timing timing = {};
+    int timing_pending = 0;    // the last run was queued without a final synchronisation (muse_batch_run_partial_device)
+    int fused_run = 0;         // 1: score_fused, 2: score_fused_grouped (d_counters[2] = exact list length, [3] = refined)
+    int prescreened = 0;       // d_U and the cut-off state were filled by the tensor-core multi-query path: the next fused run starts at its tail
+    int signed_run = 0;        // the current run keeps the sign of the scores (muse.go:72-76)
     // n > MUSE_MAX_FUSED_FFT_LEN: Stockham passes through global memory (kernels_long.cu); Xt holds n entries, twM the n twiddles
-    int is_long;
-    void *d_long;          // work buffer of launch_long
-    size_t d_long_bytes;
-    long long long_pairs;  // pairs of series per chunk d_long was sized for
+    int is_long = 0;
+    DevBuf<unsigned char> d_long;   // work buffer of launch_long
+    long long long_pairs = 0;       // pairs of series per chunk d_long was sized for
 };
+
+extern "C" void muse_batch_destroy(muse_batch *b);
+struct BatchDestroy {
+    void operator()(muse_batch *b) const { muse_batch_destroy(b); }
+};
+using BatchPtr = std::unique_ptr<muse_batch, BatchDestroy>;   // a batch that goes back through muse_batch_destroy
 
 static inline cudaStream_t bstream(const muse_batch *b) { return b->ctx->stream; }
 
@@ -182,59 +274,21 @@ extern "C" int muse_ctx_create(int device, muse_ctx **out) {
                     e != cudaSuccess ? cudaGetErrorString(e) : "device count is 0");
     if (device < 0 || device >= count) return fail(MUSE_ERR_INVALID_ARG, "device %d out of range [0,%d)", device, count);
     CU(cudaSetDevice(device));
-    muse_ctx *c = new muse_ctx();
+    std::unique_ptr<muse_ctx> c(new muse_ctx());
     c->device = device;
     CU(cudaDeviceGetAttribute(&c->sm_count, cudaDevAttrMultiProcessorCount, device));
     CU(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
     c->stream = c->own_stream;
-    *out = c;
+    *out = c.release();
     return MUSE_OK;
-}
-
-// the arrays of scratch_cap entries (ensure_scratch)
-static void free_scratch(RunScratch &r) {
-    cudaFree(r.d_score); cudaFree(r.d_lag); cudaFree(r.d_slot);
-    cudaFree(r.d_ckey); cudaFree(r.d_skey); cudaFree(r.d_cidx); cudaFree(r.d_sidx);
-    cudaFree(r.d_clag); cudaFree(r.d_slag);
-    r.d_clag = r.d_slag = nullptr;
-    cudaFree(r.d_U); cudaFree(r.d_list);
-    r.d_U = nullptr; r.d_list = nullptr;
-    r.d_score = nullptr; r.d_lag = nullptr; r.d_slot = nullptr;
-    r.d_ckey = r.d_skey = nullptr; r.d_cidx = r.d_sidx = nullptr;
-    r.scratch_cap = 0;
-}
-
-static void scratch_free(RunScratch &r) {
-    free_scratch(r);
-    cudaFree(r.d_L); cudaFree(r.d_W);
-    cudaFree(r.d_gmax); cudaFree(r.d_hkeys); cudaFree(r.d_gidx);
-    cudaFree(r.d_flag); cudaFree(r.d_counters); cudaFree(r.d_sel); cudaFree(r.d_cut);
-    cudaFree(r.d_ref); cudaFree(r.Xt); cudaFree(r.twM); cudaFree(r.twn);
-    cudaFree(r.twp_f); cudaFree(r.twi_f); cudaFree(r.swtw); cudaFree(r.sw_f); cudaFree(r.sx_f); cudaFree(r.sb_f); cudaFree(r.d_mid);
-    for (int i = 0; i < 4; i++) if (r.ev[i]) cudaEventDestroy(r.ev[i]);
-    if (r.h_pin) cudaFreeHost(r.h_pin);
-    memset(&r, 0, sizeof(r));
 }
 
 extern "C" void muse_ctx_destroy(muse_ctx *c) {
     if (!c) return;
     cudaSetDevice(c->device);
-    for (RunScratch &r : c->pool) scratch_free(r);
-    for (int i = 0; i < 3; i++) {
-        if (c->h_stage[i]) cudaFreeHost(c->h_stage[i]);
-        if (c->stage_ev[i]) cudaEventDestroy(c->stage_ev[i]);
-    }
-    cudaFree(c->tc_a); cudaFree(c->tc_b); cudaFree(c->tc_mid); cudaFree(c->tc_amid); cudaFree(c->tc_ptrs);
-    cudaFree(c->d_multi_q);
-    cudaFree(c->d_multi_next);
-    for (int i = 0; i < 5; i++)
-        if (c->mt_ev[i]) cudaEventDestroy(c->mt_ev[i]);
-    cudaFree(c->d_mt);
-    if (c->h_mt) cudaFreeHost(c->h_mt);
-    cudaFree(c->d_multi_refs);
-    cudaFree(c->d_roll);
-    cudaStreamDestroy(c->own_stream);
-    delete c;
+    const cudaStream_t own = c->own_stream;
+    delete c;      // the pool and every buffer of the context
+    cudaStreamDestroy(own);
 }
 
 extern "C" int muse_ctx_synchronize(muse_ctx *c) {
@@ -269,18 +323,12 @@ static int group_reserve(muse_group *g, int64_t want) {
     if (want <= g->cap) return MUSE_OK;
     int64_t ncap = std::max<int64_t>(want, g->cap + g->cap / 2);
     ncap = std::max<int64_t>(ncap, 16);
-    double *nslab = nullptr;
-    int32_t *nlab = nullptr;
-    RowStat *nstat = nullptr;
-    auto bail = [&](int code) {
-        cudaFree(nslab);
-        cudaFree(nlab);
-        cudaFree(nstat);
-        return code;
-    };
-    cudaError_t e = cudaMalloc(&nslab, sizeof(double) * (size_t)ncap * (size_t)g->ld);
-    if (e == cudaSuccess && g->nkeys > 0) e = cudaMalloc(&nlab, sizeof(int32_t) * (size_t)ncap * (size_t)g->nkeys);
-    if (e == cudaSuccess) e = cudaMalloc(&nstat, sizeof(RowStat) * (size_t)ncap);
+    DevBuf<double> nslab;
+    DevBuf<int32_t> nlab;
+    DevBuf<RowStat> nstat;
+    cudaError_t e = nslab.grow(ncap * g->ld);
+    if (e == cudaSuccess && g->nkeys > 0) e = nlab.grow(ncap * g->nkeys);
+    if (e == cudaSuccess) e = nstat.grow(ncap);
     if (e == cudaSuccess && g->size > 0) {
         e = cudaMemcpyAsync(nslab, g->slab, sizeof(double) * (size_t)g->size * (size_t)g->ld, cudaMemcpyDeviceToDevice, g->ctx->stream);
         for (int k = 0; k < g->nkeys && e == cudaSuccess; k++)
@@ -292,17 +340,13 @@ static int group_reserve(muse_group *g, int64_t want) {
     }
     if (e != cudaSuccess) {
         (void)cudaGetLastError();
-        return bail(fail(e == cudaErrorMemoryAllocation ? MUSE_ERR_OUT_OF_MEMORY : MUSE_ERR_CUDA, "growing the store to %lld series: %s",
-                         (long long)ncap, cudaGetErrorString(e)));
+        return fail(e == cudaErrorMemoryAllocation ? MUSE_ERR_OUT_OF_MEMORY : MUSE_ERR_CUDA, "growing the store to %lld series: %s",
+                    (long long)ncap, cudaGetErrorString(e));
     }
-    if (g->slab) cudaFree(g->slab);
-    if (g->labels) cudaFree(g->labels);
-    if (g->row_stat) cudaFree(g->row_stat);
-    g->slab = nslab;
-    g->labels = nlab;
-    g->row_stat = nstat;
+    std::swap(g->slab, nslab);      // the old arrays are freed on the way out
+    std::swap(g->labels, nlab);
+    std::swap(g->row_stat, nstat);
     g->cap = ncap;
-    g->stats_cap = ncap;
     return MUSE_OK;
 }
 
@@ -325,28 +369,21 @@ extern "C" int muse_group_create(muse_ctx *ctx, int64_t series_len, int32_t n_la
     if (n_label_keys < 0 || n_label_keys > MUSE_MAX_LABEL_KEYS)
         return fail(MUSE_ERR_INVALID_ARG, "n_label_keys %d not in [0,%d]", n_label_keys, MUSE_MAX_LABEL_KEYS);
     CU(cudaSetDevice(ctx->device));
-    muse_group *g = new muse_group();
-    memset(g, 0, sizeof(*g));
+    std::unique_ptr<muse_group> g(new muse_group());
     g->ctx = ctx;
     g->N = series_len;
     g->ld = (series_len + 15) / 16 * 16;
     g->nkeys = n_label_keys;
     for (int k = 0; k < MUSE_MAX_LABEL_KEYS; k++) g->max_id[k] = -1;
-    int rc = group_reserve(g, std::max<int64_t>(capacity_hint, 16));
-    if (rc != MUSE_OK) {
-        delete g;
-        return rc;
-    }
-    *out = g;
+    int rc = group_reserve(g.get(), std::max<int64_t>(capacity_hint, 16));
+    if (rc != MUSE_OK) return rc;
+    *out = g.release();
     return MUSE_OK;
 }
 
 extern "C" void muse_group_destroy(muse_group *g) {
     if (!g) return;
     cudaSetDevice(g->ctx->device);
-    if (g->slab) cudaFree(g->slab);
-    if (g->labels) cudaFree(g->labels);
-    if (g->row_stat) cudaFree(g->row_stat);
     delete g;
 }
 
@@ -359,10 +396,8 @@ static int64_t stage_rows_per_chunk(int64_t width) { return (int64_t)(MUSE_STAGE
 
 template <typename Queue>
 static int stage_rows(muse_ctx *c, const double *rows, int64_t n_rows, int64_t width, Queue &&queue) {
-    for (int i = 0; i < 3; i++) {
-        if (!c->h_stage[i]) CU(cudaHostAlloc((void **)&c->h_stage[i], MUSE_STAGE_BYTES, cudaHostAllocDefault));
-        if (!c->stage_ev[i]) CU(cudaEventCreateWithFlags(&c->stage_ev[i], cudaEventDisableTiming));
-    }
+    for (PinnedBuf &h : c->h_stage) CU(h.grow(MUSE_STAGE_BYTES));
+    CU(c->stage_ev.create(cudaEventDisableTiming));
     cudaStream_t st = c->stream;
     const size_t row_bytes = sizeof(double) * (size_t)width;
     if (row_bytes > MUSE_STAGE_BYTES) return fail(MUSE_ERR_UNSUPPORTED, "a row of %zu bytes exceeds the staging buffer", row_bytes);
@@ -404,7 +439,7 @@ static int stage_rows(muse_ctx *c, const double *rows, int64_t n_rows, int64_t w
             done[(size_t)ch].fetch_add(1, std::memory_order_release);
         }
         while (done[(size_t)ch].load(std::memory_order_acquire) < n_threads) std::this_thread::yield();
-        e = queue(r0, nr, reinterpret_cast<const double *>(c->h_stage[ch % 3]));
+        e = queue(r0, nr, reinterpret_cast<const double *>(c->h_stage[ch % 3].get()));
         if (e == cudaSuccess) e = cudaEventRecord(c->stage_ev[ch % 3], st);
         if (e == cudaSuccess && ch >= 1) e = cudaEventSynchronize(c->stage_ev[(ch - 1) % 3]);      // buffer (ch + 2) % 3 is free again
         writable.store(ch + 3, std::memory_order_release);
@@ -496,15 +531,14 @@ __global__ void transpose_labels_kernel(const int32_t *src, int64_t n, int nkeys
 
 static int refresh_max_ids(muse_group *g, int64_t off, int64_t n) {
     if (g->nkeys == 0 || n == 0) return MUSE_OK;
-    int32_t *d = nullptr;
-    CU(cudaMalloc(&d, sizeof(int32_t) * MUSE_MAX_LABEL_KEYS));
+    DevBuf<int32_t> d;
+    CU(d.grow(MUSE_MAX_LABEL_KEYS));
     CU(cudaMemsetAsync(d, 0xff, sizeof(int32_t) * MUSE_MAX_LABEL_KEYS, g->ctx->stream));
     for (int k = 0; k < g->nkeys; k++)
         max_id_kernel<<<256, 256, 0, g->ctx->stream>>>(g->labels + (size_t)k * g->cap + off, n, d + k);
     int32_t h[MUSE_MAX_LABEL_KEYS];
     CU(cudaMemcpyAsync(h, d, sizeof(h), cudaMemcpyDeviceToHost, g->ctx->stream));
     CU(cudaStreamSynchronize(g->ctx->stream));
-    cudaFree(d);
     for (int k = 0; k < g->nkeys; k++) g->max_id[k] = std::max(g->max_id[k], h[k]);
     return MUSE_OK;
 }
@@ -599,7 +633,7 @@ extern "C" int muse_group_append_synthetic_ex(muse_group *g, int64_t n_series, u
     CU(cudaSetDevice(g->ctx->device));
     int rc = group_reserve(g, g->size + n_series);
     if (rc != MUSE_OK) return rc;
-    int32_t *l0 = g->nkeys >= 1 ? g->labels : nullptr;
+    int32_t *l0 = g->nkeys >= 1 ? g->labels.get() : nullptr;
     int32_t *l1 = g->nkeys >= 2 ? g->labels + (size_t)g->cap : nullptr;
     if (g->nkeys > 2)
         CU(cudaMemsetAsync(g->labels + (size_t)2 * g->cap, 0, sizeof(int32_t) * (size_t)g->cap * (size_t)(g->nkeys - 2), g->ctx->stream));
@@ -727,14 +761,10 @@ extern "C" int muse_group_roll(muse_group *g, int64_t first, int64_t n_rows, con
     CU(cudaSetDevice(c->device));
     cudaStream_t st = c->stream;
     const int64_t rows_per_chunk = stage_rows_per_chunk(k);
-    const size_t want = row_bytes * (size_t)std::min<int64_t>(n_rows, rows_per_chunk);
-    if (c->d_roll_bytes < want) {
+    const int64_t want = k * std::min<int64_t>(n_rows, rows_per_chunk);
+    if (c->d_roll.cap() < want) {
         CU(cudaStreamSynchronize(st));
-        cudaFree(c->d_roll);
-        c->d_roll = nullptr;
-        c->d_roll_bytes = 0;
-        CU(cudaMalloc(&c->d_roll, want));
-        c->d_roll_bytes = want;
+        CU(c->d_roll.grow(want));
     }
     auto queue = [&](int64_t r0, int64_t nr, const double *src) {
         cudaError_t e = cudaMemcpyAsync(c->d_roll, src, (size_t)nr * row_bytes, cudaMemcpyHostToDevice, st);
@@ -800,32 +830,19 @@ __global__ void screen_tables_kernel(const cd *__restrict__ Xt, int M, const flo
 static int ensure_ref_tables(muse_batch *b, int64_t ld) {
     const int64_t n = b->n, M = n / 2;
     cudaStream_t st = bstream(b);
-    if (b->d_ref_cap < ld) {
-        cudaFree(b->d_ref);
-        b->d_ref = nullptr;
-        CU(cudaMalloc(&b->d_ref, sizeof(double) * (size_t)ld));
-        b->d_ref_cap = ld;
-    }
-    if (!b->d_mid) CU(cudaMalloc(&b->d_mid, sizeof(float) * 4));
+    CU(b->d_ref.grow(ld));
+    CU(b->d_mid.grow(4));
     const bool want_screen = screen_is_fused(b->log2m);
     if (b->tab_n == n && (b->tab_screen || !want_screen)) return MUSE_OK;
+    b->tab_n = 0;
+    b->tab_screen = 0;
     if (b->is_long) {      // the reference's transform has n entries, the twiddles are generated on the device
-        cudaFree(b->Xt); cudaFree(b->twM); cudaFree(b->twn); cudaFree(b->twp_f); cudaFree(b->twi_f); cudaFree(b->swtw); cudaFree(b->sw_f); cudaFree(b->sx_f); cudaFree(b->sb_f);
-        b->Xt = b->twM = b->twn = nullptr;
-        b->twp_f = b->twi_f = nullptr; b->swtw = nullptr; b->sw_f = b->sx_f = nullptr; b->sb_f = nullptr;
-        b->tab_n = 0;
-        b->tab_screen = 0;
-        CU(cudaMalloc(&b->Xt, sizeof(cd) * (size_t)n));
-        CU(cudaMalloc(&b->twM, sizeof(cd) * (size_t)n));
+        CU(b->Xt.grow(n));
+        CU(b->twM.grow(n));
         CU(launch_long_twiddles(b->twM, b->log2m + 1, st));
         b->tab_n = n;
         return MUSE_OK;
     }
-    cudaFree(b->Xt); cudaFree(b->twM); cudaFree(b->twn); cudaFree(b->twp_f); cudaFree(b->twi_f); cudaFree(b->swtw); cudaFree(b->sw_f); cudaFree(b->sx_f); cudaFree(b->sb_f);
-    b->Xt = b->twM = b->twn = nullptr;
-    b->twp_f = b->twi_f = nullptr; b->swtw = nullptr; b->sw_f = b->sx_f = nullptr; b->sb_f = nullptr;
-    b->tab_n = 0;
-    b->tab_screen = 0;
     const long double PI2 = 6.283185307179586476925286766559005768L;
     const int log2p = exact_log2p(b->log2m);
     std::vector<cd> twM((size_t)M + 16);
@@ -835,9 +852,9 @@ static int ensure_ref_tables(muse_batch *b, int64_t ld) {
     // twiddle tables, correctly rounded from long double
     std::vector<cd> twn((size_t)(M / 2 + 1));
     for (int64_t k = 0; k <= M / 2; k++) twn[(size_t)k] = cd{(double)cosl(-PI2 * k / n), (double)sinl(-PI2 * k / n)};
-    CU(cudaMalloc(&b->Xt, sizeof(cd) * (size_t)(M + 1)));
-    CU(cudaMalloc(&b->twM, sizeof(cd) * twM.size()));
-    CU(cudaMalloc(&b->twn, sizeof(cd) * (size_t)(M / 2 + 1)));
+    CU(b->Xt.grow(M + 1));
+    CU(b->twM.grow((int64_t)twM.size()));
+    CU(b->twn.grow(M / 2 + 1));
     CU(cudaMemcpyAsync(b->twM, twM.data(), sizeof(cd) * twM.size(), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(b->twn, twn.data(), sizeof(cd) * (size_t)(M / 2 + 1), cudaMemcpyHostToDevice, st));
     std::vector<cf> twp, twi;
@@ -848,7 +865,7 @@ static int ensure_ref_tables(muse_batch *b, int64_t ld) {
             fill_big_twiddles(b->log2m, twi.data(), [&](long long num, long long den) {
                 return cf{(float)cosl(-PI2 * num / den), (float)sinl(-PI2 * num / den)};
             });
-            CU(cudaMalloc(&b->twi_f, sizeof(cf) * twi.size()));
+            CU(b->twi_f.grow((int64_t)twi.size()));
             CU(cudaMemcpyAsync(b->twi_f, twi.data(), sizeof(cf) * twi.size(), cudaMemcpyHostToDevice, st));
         }
         twp.resize((size_t)M + 64);
@@ -857,11 +874,11 @@ static int ensure_ref_tables(muse_batch *b, int64_t ld) {
         });
         swtw.resize((size_t)M / 2);
         for (int64_t k = 0; k < M / 2; k++) swtw[(size_t)k] = make_float2((float)cosl(-PI2 * k / n), (float)sinl(-PI2 * k / n));
-        CU(cudaMalloc(&b->twp_f, sizeof(cf) * twp.size()));
-        CU(cudaMalloc(&b->swtw, sizeof(float2) * swtw.size()));
-        CU(cudaMalloc(&b->sw_f, sizeof(float4) * (size_t)(M / 2)));
-        CU(cudaMalloc(&b->sx_f, sizeof(float4) * (size_t)(M / 2)));
-        CU(cudaMalloc(&b->sb_f, sizeof(float) * (size_t)(M / 2)));
+        CU(b->twp_f.grow((int64_t)twp.size()));
+        CU(b->swtw.grow((int64_t)swtw.size()));
+        CU(b->sw_f.grow(M / 2));
+        CU(b->sx_f.grow(M / 2));
+        CU(b->sb_f.grow(M / 2));
         CU(cudaMemcpyAsync(b->twp_f, twp.data(), sizeof(cf) * twp.size(), cudaMemcpyHostToDevice, st));
         CU(cudaMemcpyAsync(b->swtw, swtw.data(), sizeof(float2) * swtw.size(), cudaMemcpyHostToDevice, st));
     }
@@ -873,27 +890,15 @@ static int ensure_ref_tables(muse_batch *b, int64_t ld) {
 
 // NewBatch in two halves, so that the references of a multi-query launch share ONE round trip: queue = everything
 // up to the copies of the std-zero flag and the middle-bin values into the batch's pinned mailbox; finish (after the
-// stream has been synchronised) = the error of muse_batch.go:38-41 (the batch is destroyed) or the by-value parameters.
+// stream has been synchronised) = the error of muse_batch.go:38-41 (the caller destroys the batch) or the by-value parameters.
 // d_ref_row != NULL: the reference row is already on the device, zero-padded to the slab's row pitch (muse_multi_run
 // uploads the references of a launch with one copy).
-extern "C" void muse_batch_destroy(muse_batch *b);
 static int ensure_long_work(muse_batch *b, int64_t count);
 static LongParams long_params(const muse_batch *b, const double *slab, int64_t count, const int32_t *idx, int signed_scores);
 
-// as CU, for code that owns a half-built batch `b`: it goes back to the pool before the error is returned
-#define CUB(call)                                                          \
-    do {                                                                   \
-        cudaError_t e_ = (call);                                           \
-        if (e_ != cudaSuccess) {                                           \
-            const int rc_ = cuda_fail(e_, #call, __FILE__, __LINE__);      \
-            muse_batch_destroy(b);                                         \
-            return rc_;                                                    \
-        }                                                                  \
-    } while (0)
-
 // The batch object with its pooled scratch, the tables of its FFT length and its small allocations: nothing is launched.
-static int batch_alloc(muse_ctx *ctx, muse_group *g, int64_t ref_len, muse_batch **out) {
-    if (!ctx || !g || !out) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_create: NULL argument");
+static int batch_alloc(muse_ctx *ctx, muse_group *g, int64_t ref_len, BatchPtr &out) {
+    if (!ctx || !g) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_create: NULL argument");
     if (g->ctx != ctx) return fail(MUSE_ERR_INVALID_ARG, "group belongs to another context");
     if (ref_len != g->N)   // muse_batch.go:24-28
         return fail(MUSE_ERR_LENGTH_MISMATCH, "comparison group series (length %lld) does not have the same length as the reference (%lld)",
@@ -901,8 +906,7 @@ static int batch_alloc(muse_ctx *ctx, muse_group *g, int64_t ref_len, muse_batch
     const int64_t n = next_pow2(ref_len);   // muse_batch.go:35
     if (n > MUSE_MAX_FFT_LEN) return fail(MUSE_ERR_UNSUPPORTED, "FFT length %lld > %d", (long long)n, MUSE_MAX_FFT_LEN);
     CU(cudaSetDevice(ctx->device));
-    muse_batch *b = new muse_batch();
-    memset(b, 0, sizeof(*b));
+    BatchPtr b(new muse_batch());
     b->is_long = n > MUSE_MAX_FUSED_FFT_LEN;
     b->ctx = ctx;
     b->g = g;
@@ -923,46 +927,33 @@ static int batch_alloc(muse_ctx *ctx, muse_group *g, int64_t ref_len, muse_batch
             };
             for (size_t i = 1; i < ctx->pool.size(); i++)
                 if (better(ctx->pool[i], ctx->pool[best])) best = i;
-            static_cast<RunScratch &>(*b) = ctx->pool[best];
+            static_cast<RunScratch &>(*b) = std::move(ctx->pool[best]);
             ctx->pool.erase(ctx->pool.begin() + (long)best);
         }
     }
-    auto bail = [&](int code) {
-        muse_batch_destroy(b);
-        return code;
-    };
-    for (int i = 0; i < 4; i++)
-        if (!b->ev[i] && cudaEventCreate(&b->ev[i]) != cudaSuccess) return bail(fail(MUSE_ERR_CUDA, "cudaEventCreate failed"));
-    int rc = ensure_ref_tables(b, g->ld);
-    if (rc) return bail(rc);
-    cudaError_t e = cudaSuccess;
-    if (!b->d_flag) e = cudaMalloc(&b->d_flag, sizeof(int32_t));
-    if (e == cudaSuccess && !b->d_counters) e = cudaMalloc(&b->d_counters, sizeof(unsigned long long) * 4);
-    if (e == cudaSuccess && !b->d_sel) e = cudaMalloc(&b->d_sel, sizeof(SelectState));
-    if (e == cudaSuccess && !b->d_cut) e = cudaMalloc(&b->d_cut, sizeof(unsigned) * (4 + MUSE_CUT_WORDS));
-    if (e == cudaSuccess && !b->h_pin) {
-        b->h_pin_bytes = (size_t)4 << 20;
-        e = cudaHostAlloc((void **)&b->h_pin, b->h_pin_bytes, cudaHostAllocDefault);
-    }
-    if (e != cudaSuccess) {
-        (void)cudaGetLastError();
-        return bail(fail(e == cudaErrorMemoryAllocation ? MUSE_ERR_OUT_OF_MEMORY : MUSE_ERR_CUDA, "muse_batch_create: %s", cudaGetErrorString(e)));
-    }
-    *out = b;
+    CU(b->ev.create());
+    int rc = ensure_ref_tables(b.get(), g->ld);
+    if (rc) return rc;
+    CU(b->d_flag.grow(1));
+    CU(b->d_counters.grow(4));
+    CU(b->d_sel.grow(1));
+    CU(b->d_cut.grow(4 + MUSE_CUT_WORDS));
+    CU(b->h_pin.grow((int64_t)4 << 20));
+    out = std::move(b);
     return MUSE_OK;
 }
 
-static int batch_create_queue(muse_ctx *ctx, muse_group *g, const double *ref, int64_t ref_len, muse_batch **out,
+static int batch_create_queue(muse_ctx *ctx, muse_group *g, const double *ref, int64_t ref_len, BatchPtr &out,
                               const double *d_ref_row = nullptr) {
     if (!ref) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_create: NULL argument");
-    muse_batch *b = nullptr;
-    int rc = batch_alloc(ctx, g, ref_len, &b);
+    BatchPtr b;
+    int rc = batch_alloc(ctx, g, ref_len, b);
     if (rc) return rc;
     cudaStream_t st = ctx->stream;
     const int64_t M = b->n / 2;
     if (!d_ref_row) {      // (the select state is cleared where it is used)
-        CUB(cudaMemsetAsync(b->d_ref, 0, sizeof(double) * (size_t)g->ld, st));
-        CUB(cudaMemcpyAsync(b->d_ref, ref, sizeof(double) * (size_t)ref_len, cudaMemcpyHostToDevice, st));
+        CU(cudaMemsetAsync(b->d_ref, 0, sizeof(double) * (size_t)g->ld, st));
+        CU(cudaMemcpyAsync(b->d_ref, ref, sizeof(double) * (size_t)ref_len, cudaMemcpyHostToDevice, st));
     }
     // X on the device through the same forward path the series take
     ExactParams p;
@@ -976,30 +967,27 @@ static int batch_create_queue(muse_ctx *ctx, muse_group *g, const double *ref, i
     p.out_X = b->Xt;
     p.out_flag = b->d_flag;
     if (b->is_long) {
-        int rcl = ensure_long_work(b, 1);
-        if (rcl) {
-            muse_batch_destroy(b);
-            return rcl;
-        }
-        LongParams lp = long_params(b, p.slab, 1, nullptr, 0);
+        rc = ensure_long_work(b.get(), 1);
+        if (rc) return rc;
+        LongParams lp = long_params(b.get(), p.slab, 1, nullptr, 0);
         lp.out_X = b->Xt;
-        CUB(launch_long(MODE_REF, lp, b->d_long, b->long_pairs, st));
+        CU(launch_long(MODE_REF, lp, b->d_long, b->long_pairs, st));
     } else {
-        CUB(launch_exact(MODE_REF, b->log2m, p, st));
+        CU(launch_exact(MODE_REF, b->log2m, p, st));
     }
     b->screen_ok = 0;
     const bool screen = b->tab_screen != 0;
     if (screen) {
         screen_tables_kernel<<<(unsigned)((M / 2 + 1 + 255) / 256), 256, 0, st>>>(b->Xt, (int)M, b->swtw, b->sw_f, b->sx_f, b->sb_f, b->d_mid, b->d_flag);
-        CUB(cudaGetLastError());
+        CU(cudaGetLastError());
     }
     // one round trip: the std-zero flag of the reference and the two middle-bin values the kernels take by value
-    int32_t *h_flag = reinterpret_cast<int32_t *>(b->h_pin);
+    int32_t *h_flag = reinterpret_cast<int32_t *>(b->h_pin.get());
     float *h_mid = reinterpret_cast<float *>(b->h_pin + 16);
-    if (screen) CUB(cudaMemcpyAsync(h_mid, b->d_mid, sizeof(float) * 4, cudaMemcpyDeviceToHost, st));      // [0] carries the flag
-    else CUB(cudaMemcpyAsync(h_flag, b->d_flag, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (screen) CU(cudaMemcpyAsync(h_mid, b->d_mid, sizeof(float) * 4, cudaMemcpyDeviceToHost, st));      // [0] carries the flag
+    else CU(cudaMemcpyAsync(h_flag, b->d_flag, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     b->screen_ok = screen ? -1 : 0;      // -1: pending until batch_create_finish
-    *out = b;
+    out = std::move(b);
     return MUSE_OK;
 }
 
@@ -1007,10 +995,8 @@ static int batch_create_finish(muse_batch *b) {
     const float *h_mid = reinterpret_cast<const float *>(b->h_pin + 16);
     int32_t flag;
     memcpy(&flag, b->screen_ok == -1 ? static_cast<const void *>(h_mid) : static_cast<const void *>(b->h_pin), sizeof(flag));
-    if (flag) {   // muse_batch.go:38-41
-        muse_batch_destroy(b);
+    if (flag)   // muse_batch.go:38-41
         return fail(MUSE_ERR_STDDEV_ZERO, "Invalid input query, Standard deviation of zero");
-    }
     if (b->screen_ok == -1) {
         b->a_mid = h_mid[1];
         b->x_mid = cf{h_mid[2], h_mid[3]};
@@ -1019,19 +1005,14 @@ static int batch_create_finish(muse_batch *b) {
     return MUSE_OK;
 }
 
-
 extern "C" int muse_batch_create(muse_ctx *ctx, muse_group *g, const double *ref, int64_t ref_len, muse_batch **out) {
-    muse_batch *b = nullptr;
-    int rc = batch_create_queue(ctx, g, ref, ref_len, &b);
+    BatchPtr b;
+    int rc = batch_create_queue(ctx, g, ref, ref_len, b);
     if (rc) return rc;
-    cudaError_t e = cudaStreamSynchronize(ctx->stream);
-    if (e != cudaSuccess) {
-        muse_batch_destroy(b);
-        return fail(MUSE_ERR_CUDA, "cudaStreamSynchronize failed: %s", cudaGetErrorString(e));
-    }
-    rc = batch_create_finish(b);
+    CU(cudaStreamSynchronize(ctx->stream));
+    rc = batch_create_finish(b.get());
     if (rc) return rc;
-    *out = b;
+    *out = b.release();
     return MUSE_OK;
 }
 
@@ -1042,13 +1023,8 @@ extern "C" void muse_batch_destroy(muse_batch *b) {
     {   // the store-sized scratch goes back to the context (at most MUSE_SCRATCH_POOL sets are kept: a multi-query launch
         // group has 256 batches alive at once)
         std::lock_guard<std::mutex> lk(b->ctx->mu);
-        if (b->ctx->pool.size() < MUSE_SCRATCH_POOL) {
-            b->ctx->pool.push_back(static_cast<RunScratch &>(*b));
-            memset(static_cast<RunScratch *>(b), 0, sizeof(RunScratch));
-        }
+        if (b->ctx->pool.size() < MUSE_SCRATCH_POOL) b->ctx->pool.push_back(std::move(static_cast<RunScratch &>(*b)));
     }
-    scratch_free(*b);
-    cudaFree(b->d_long);
     delete b;
 }
 
@@ -1057,19 +1033,19 @@ extern "C" int64_t muse_batch_fft_len(const muse_batch *b) { return b ? b->n : 0
 static int ensure_scratch(muse_batch *b) {
     const int64_t S = b->g->size;
     if (S <= b->scratch_cap) return MUSE_OK;
-    free_scratch(*b);
     const int64_t cap = std::max<int64_t>(S, 1024);
-    CU(cudaMalloc(&b->d_score, sizeof(double) * (size_t)cap));
-    CU(cudaMalloc(&b->d_lag, sizeof(int32_t) * (size_t)cap));
-    CU(cudaMalloc(&b->d_slot, sizeof(int64_t) * (size_t)cap));
-    CU(cudaMalloc(&b->d_ckey, sizeof(unsigned long long) * (size_t)cap));
-    CU(cudaMalloc(&b->d_skey, sizeof(unsigned long long) * (size_t)cap));
-    CU(cudaMalloc(&b->d_cidx, sizeof(int32_t) * (size_t)cap));
-    CU(cudaMalloc(&b->d_sidx, sizeof(int32_t) * (size_t)cap));
-    CU(cudaMalloc(&b->d_clag, sizeof(int32_t) * (size_t)cap));
-    CU(cudaMalloc(&b->d_slag, sizeof(int32_t) * (size_t)cap));
-    CU(cudaMalloc(&b->d_U, sizeof(float) * (size_t)cap));
-    CU(cudaMalloc(&b->d_list, sizeof(int32_t) * (size_t)cap));
+    b->scratch_cap = 0;      // until every array has grown: a failure part way leaves the next call to retry
+    CU(b->d_score.grow(cap));
+    CU(b->d_lag.grow(cap));
+    CU(b->d_slot.grow(cap));
+    CU(b->d_ckey.grow(cap));
+    CU(b->d_skey.grow(cap));
+    CU(b->d_cidx.grow(cap));
+    CU(b->d_sidx.grow(cap));
+    CU(b->d_clag.grow(cap));
+    CU(b->d_slag.grow(cap));
+    CU(b->d_U.grow(cap));
+    CU(b->d_list.grow(cap));
     b->scratch_cap = cap;
     return MUSE_OK;
 }
@@ -1089,12 +1065,9 @@ static int ensure_long_work(muse_batch *b, int64_t count) {
     static const size_t work_mb = getenv("MUSE_LONG_WORK_MB") ? (size_t)std::max(1, atoi(getenv("MUSE_LONG_WORK_MB"))) : 256;
     long long pairs = std::max<long long>(1, (long long)((work_mb << 20) / per_pair));
     pairs = std::min<long long>(pairs, std::max<long long>(1, (count + 1) / 2));
-    if (b->d_long && b->long_pairs >= pairs) return MUSE_OK;
-    cudaFree(b->d_long);
-    b->d_long = nullptr;
+    if (b->long_pairs >= pairs) return MUSE_OK;
     b->long_pairs = 0;
-    b->d_long_bytes = long_work_bytes(log2n, pairs);
-    CU(cudaMalloc(&b->d_long, b->d_long_bytes));
+    CU(b->d_long.grow((int64_t)long_work_bytes(log2n, pairs)));
     b->long_pairs = pairs;
     return MUSE_OK;
 }
@@ -1169,8 +1142,8 @@ extern "C" int muse_batch_xcorr(muse_batch *b, int64_t local_index, double *cc, 
     if (rc) return rc;
     if (!cc || local_index < 0 || local_index >= b->g->size) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_xcorr: bad argument");
     CU(cudaSetDevice(b->ctx->device));
-    double *d_cc = nullptr;
-    CU(cudaMalloc(&d_cc, sizeof(double) * (size_t)b->n));
+    DevBuf<double> d_cc;
+    CU(d_cc.grow(b->n));
     ExactParams p;
     memset(&p, 0, sizeof(p));
     p.slab = b->g->slab + (size_t)local_index * b->g->ld;
@@ -1182,25 +1155,19 @@ extern "C" int muse_batch_xcorr(muse_batch *b, int64_t local_index, double *cc, 
     p.twn = b->twn;
     p.out_score = d_cc;
     p.out_flag = b->d_flag;
+    if (b->is_long) {
+        rc = ensure_long_work(b, 1);
+        if (rc) return rc;
+        LongParams lp = long_params(b, p.slab, 1, nullptr, 0);
+        lp.out_score = d_cc;
+        CU(launch_long(MODE_CC, lp, b->d_long, b->long_pairs, bstream(b)));
+    } else {
+        CU(launch_exact(MODE_CC, b->log2m, p, bstream(b)));
+    }
     int32_t flag = 0;
-    auto body = [&]() -> int {      // d_cc is freed on every path out of here
-        if (b->is_long) {
-            int rcl = ensure_long_work(b, 1);
-            if (rcl) return rcl;
-            LongParams lp = long_params(b, p.slab, 1, nullptr, 0);
-            lp.out_score = d_cc;
-            CU(launch_long(MODE_CC, lp, b->d_long, b->long_pairs, bstream(b)));
-        } else {
-            CU(launch_exact(MODE_CC, b->log2m, p, bstream(b)));
-        }
-        CU(cudaMemcpyAsync(cc, d_cc, sizeof(double) * (size_t)b->n, cudaMemcpyDeviceToHost, bstream(b)));
-        CU(cudaMemcpyAsync(&flag, b->d_flag, sizeof(flag), cudaMemcpyDeviceToHost, bstream(b)));
-        CU(cudaStreamSynchronize(bstream(b)));
-        return MUSE_OK;
-    };
-    rc = body();
-    cudaFree(d_cc);
-    if (rc) return rc;
+    CU(cudaMemcpyAsync(cc, d_cc, sizeof(double) * (size_t)b->n, cudaMemcpyDeviceToHost, bstream(b)));
+    CU(cudaMemcpyAsync(&flag, b->d_flag, sizeof(flag), cudaMemcpyDeviceToHost, bstream(b)));
+    CU(cudaStreamSynchronize(bstream(b)));
     if (std_zero) *std_zero = flag;
     return MUSE_OK;
 }
@@ -1284,14 +1251,9 @@ static int setup_group_table(muse_batch *b, const RunArgs &a, bool shard, KeyCol
         slots = 1;
         while (slots < 2 * S) slots <<= 1;
     }
-    if (slots > b->table_cap) {
-        cudaFree(b->d_gmax); cudaFree(b->d_gidx); cudaFree(b->d_hkeys);
-        b->d_gmax = b->d_hkeys = nullptr; b->d_gidx = nullptr; b->table_cap = 0;
-        CU(cudaMalloc(&b->d_gmax, sizeof(unsigned long long) * (size_t)slots));
-        CU(cudaMalloc(&b->d_hkeys, sizeof(unsigned long long) * (size_t)slots));
-        CU(cudaMalloc(&b->d_gidx, sizeof(int32_t) * (size_t)slots));
-        b->table_cap = slots;
-    }
+    CU(b->d_gmax.grow(slots));
+    CU(b->d_hkeys.grow(slots));
+    CU(b->d_gidx.grow(slots));
     gt.slots = slots;
     gt.gmax = b->d_gmax;
     gt.gidx = b->d_gidx;
@@ -1356,12 +1318,12 @@ static int run_select(muse_batch *b, const RunArgs &a, int apply_filter, int64_t
     CU(cudaMemsetAsync(b->d_counters, 0, sizeof(unsigned long long) * 2, st));
     FilterArgs f{a.max_lag, a.threshold, a.sign_filter, apply_filter};
     Cand cand{b->d_ckey, b->d_cidx, b->d_clag, b->d_counters};
-    emit_candidates_kernel<<<blocks, 256, 0, st>>>(gt, grouped ? b->d_slot : nullptr, b->d_score, b->d_lag, S, f, cand);
+    emit_candidates_kernel<<<blocks, 256, 0, st>>>(gt, grouped ? b->d_slot.get() : nullptr, b->d_score, b->d_lag, S, f, cand);
     b->timing.n_launches++;
     CU(cudaGetLastError());
     // one round trip: the count and the first CH records together (pinned mailbox)
     const size_t CH = std::min<size_t>((size_t)S, 32768);
-    unsigned long long *h_n = reinterpret_cast<unsigned long long *>(b->h_pin);
+    unsigned long long *h_n = reinterpret_cast<unsigned long long *>(b->h_pin.get());
     unsigned long long *h_key = reinterpret_cast<unsigned long long *>(b->h_pin + 64);
     int32_t *h_idx = reinterpret_cast<int32_t *>(b->h_pin + 64 + CH * 8);
     int32_t *h_lag = reinterpret_cast<int32_t *>(b->h_pin + 64 + CH * 12);
@@ -1396,7 +1358,7 @@ static int run_select(muse_batch *b, const RunArgs &a, int apply_filter, int64_t
             if (limit == 0) return MUSE_OK;
             CU(cudaMemsetAsync(b->d_sel, 0, sizeof(SelectState), st));
             unsigned long long want = (unsigned long long)limit;
-            CU(cudaMemcpyAsync(&b->d_sel->want, &want, sizeof(want), cudaMemcpyHostToDevice, st));
+            CU(cudaMemcpyAsync(&b->d_sel.get()->want, &want, sizeof(want), cudaMemcpyHostToDevice, st));
             const unsigned sblocks = (unsigned)((ncand + 1023ull) / 1024ull);
             for (int r = 0; r < 6; r++) select_round_kernel<<<sblocks, 1024, 0, st>>>(b->d_sel, b->d_ckey, b->d_cidx, ncand, r);
             select_gather_kernel<<<sblocks, 1024, 0, st>>>(b->d_sel, b->d_ckey, b->d_cidx, ncand, b->d_clag, b->d_skey, b->d_sidx,
@@ -1436,17 +1398,8 @@ static cudaError_t launch_screen(const muse_batch *b, const ScreenParams &p, cud
 }
 
 static int ensure_lower(muse_batch *b) {
-    const int64_t S = b->g->size;
-    if (!b->d_L || b->d_L_cap < S) {
-        cudaFree(b->d_L);
-        cudaFree(b->d_W);
-        b->d_L = nullptr;
-        b->d_W = nullptr;
-        b->d_L_cap = 0;
-        CU(cudaMalloc(&b->d_L, sizeof(float) * (size_t)S));
-        CU(cudaMalloc(&b->d_W, (size_t)S));
-        b->d_L_cap = S;
-    }
+    CU(b->d_L.grow(b->g->size));
+    CU(b->d_W.grow(b->g->size));
     return MUSE_OK;
 }
 
@@ -1691,7 +1644,7 @@ static int score_fused_grouped(muse_batch *b, const RunArgs &a) {
     group_contenders_kernel<<<blocks, 256, 0, st>>>(gt, b->d_U, S, b->d_slot, thr_lo, b->d_list, b->d_counters + 2, cut_bits);
     b->timing.n_launches++;
     CU(cudaGetLastError());
-    unsigned long long *h_n = reinterpret_cast<unsigned long long *>(b->h_pin);
+    unsigned long long *h_n = reinterpret_cast<unsigned long long *>(b->h_pin.get());
     CU(cudaMemcpyAsync(h_n, b->d_counters + 2, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));                                 // one small round trip: the list length sizes the launch
     const int64_t n_exact = (int64_t)h_n[0];
@@ -1780,7 +1733,7 @@ static int finish_timing(muse_batch *b) {
 static int finish_pending_timing(muse_batch *b) {
     CU(cudaEventSynchronize(b->ev[3]));
     read_timing_events(b);
-    settle_counters(b, reinterpret_cast<const unsigned long long *>(b->h_pin));
+    settle_counters(b, reinterpret_cast<const unsigned long long *>(b->h_pin.get()));
     b->timing_pending = 0;
     return MUSE_OK;
 }
@@ -1817,7 +1770,7 @@ static bool device_topn_applies(const muse_batch *b, const RunArgs &a) {
 }
 
 static int device_topn_queue(muse_batch *b, const RunArgs &a) {
-    muse_partial *d_rec = reinterpret_cast<muse_partial *>(b->d_skey);      // free scratch in this path
+    muse_partial *d_rec = reinterpret_cast<muse_partial *>(b->d_skey.get());      // free scratch in this path
     int rc = queue_topn_records(b, a, d_rec, a.top_n);
     if (rc) return rc;
     cudaStream_t st = bstream(b);
@@ -1834,7 +1787,7 @@ static int device_topn_finish(muse_batch *b, const RunArgs &a, double *scores, i
         return finish_pending_timing(b);
     }
     b->timing_pending = 0;
-    const unsigned long long *h_n = reinterpret_cast<const unsigned long long *>(b->h_pin);
+    const unsigned long long *h_n = reinterpret_cast<const unsigned long long *>(b->h_pin.get());
     int rc;
     if (b->fused_run == 1) {
         rc = run_fused_overflow(b, (int64_t)h_n[2], true);
@@ -2089,28 +2042,14 @@ extern "C" int muse_merge_partials(const muse_partial *parts, int64_t n_parts, i
 static int tc_bounds_queue(muse_ctx *ctx, muse_group *g, muse_batch **bs, int nq) {
     const int64_t S = g->size;
     cudaStream_t st = ctx->stream;
-    for (int i = 0; i < 5; i++)
-        if (!ctx->mt_ev[i]) CU(cudaEventCreate(&ctx->mt_ev[i]));
+    CU(ctx->mt_ev.create());
     int rc = refresh_row_stats(g);
     if (rc) return rc;
-    const size_t a_bytes = TcCfg::a_bytes(S);
-    if (ctx->tc_a_bytes < a_bytes) {
-        cudaFree(ctx->tc_a);
-        ctx->tc_a = nullptr;
-        ctx->tc_a_bytes = 0;
-        CU(cudaMalloc(&ctx->tc_a, a_bytes));
-        ctx->tc_a_bytes = a_bytes;
-    }
-    if (ctx->tc_mid_cap < S) {
-        cudaFree(ctx->tc_mid);
-        ctx->tc_mid = nullptr;
-        ctx->tc_mid_cap = 0;
-        CU(cudaMalloc(&ctx->tc_mid, sizeof(float) * (size_t)S));
-        ctx->tc_mid_cap = S;
-    }
-    if (!ctx->tc_b) CU(cudaMalloc(&ctx->tc_b, TcCfg::b_bytes()));
-    if (!ctx->tc_amid) CU(cudaMalloc(&ctx->tc_amid, sizeof(float) * TcCfg::TN));
-    if (!ctx->tc_ptrs) CU(cudaMalloc(&ctx->tc_ptrs, sizeof(void *) * 2 * TcCfg::TN));
+    CU(ctx->tc_a.grow((int64_t)TcCfg::a_bytes(S)));
+    CU(ctx->tc_mid.grow(S));
+    CU(ctx->tc_b.grow((int64_t)TcCfg::b_bytes()));
+    CU(ctx->tc_amid.grow(TcCfg::TN));
+    CU(ctx->tc_ptrs.grow(2 * TcCfg::TN));
     void *h_ptrs[2 * TcCfg::TN];
     float h_amid[TcCfg::TN];
     memset(h_ptrs, 0, sizeof(h_ptrs));
@@ -2128,7 +2067,7 @@ static int tc_bounds_queue(muse_ctx *ctx, muse_group *g, muse_batch **bs, int nq
     ScreenParams sp = screen_params(bs[0]);
     CU(cudaEventRecord(ctx->mt_ev[0], st));
     CU(launch_mag_tiles(sp, ctx->tc_a, ctx->tc_mid, ctx->sm_count, st));
-    CU(launch_weight_tiles(reinterpret_cast<const float4 *const *>(ctx->tc_ptrs), nq, ctx->tc_b, st));
+    CU(launch_weight_tiles(reinterpret_cast<const float4 *const *>(ctx->tc_ptrs.get()), nq, ctx->tc_b, st));
     CU(cudaEventRecord(ctx->mt_ev[1], st));
     TcBoundsParams tp;
     memset(&tp, 0, sizeof(tp));
@@ -2148,10 +2087,8 @@ static int tc_bounds_queue(muse_ctx *ctx, muse_group *g, muse_batch **bs, int nq
 // ctx->d_multi_refs for rows of the store's length and pitch: MUSE_MULTI_GROUP reference rows, pad columns zero
 static int ensure_multi_refs(muse_ctx *ctx, const muse_group *g) {
     if (ctx->d_multi_ld == g->ld && ctx->d_multi_n == g->N) return MUSE_OK;
-    cudaFree(ctx->d_multi_refs);
-    ctx->d_multi_refs = nullptr;
     ctx->d_multi_ld = ctx->d_multi_n = 0;
-    CU(cudaMalloc(&ctx->d_multi_refs, sizeof(double) * (size_t)MUSE_MULTI_GROUP * (size_t)g->ld));
+    CU(ctx->d_multi_refs.grow(MUSE_MULTI_GROUP * g->ld));
     CU(cudaMemsetAsync(ctx->d_multi_refs, 0, sizeof(double) * (size_t)MUSE_MULTI_GROUP * (size_t)g->ld, ctx->stream));
     ctx->d_multi_ld = g->ld;
     ctx->d_multi_n = g->N;
@@ -2181,48 +2118,31 @@ struct MultiTables {
 // queries: reference spectra and tables (batched fp64 kernel in MODE_REF, blockIdx.y = query), cut-off states, bounds
 // (bf16 contraction), second stages (one pass over the store), survivors, fp64 re-scoring, filter, top-N -- and two
 // round trips to the host: the std-zero flags after the preparation, the list lengths before the re-scoring.  A query
-// whose lists do not fit the device-side select finishes alone on the single-query path.
+// whose lists do not fit the device-side select finishes alone on the single-query path.  The group's batches go into `bs`
+// (nq entries), which the caller keeps until the work queued on them has run.
 static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, int nq, int64_t ref_len, int64_t max_lag, int64_t top_n,
-                              double threshold, int32_t sign_filter, double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out) {
+                              double threshold, int32_t sign_filter, double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out,
+                              std::vector<BatchPtr> &bs) {
     using MT = MultiTables;
     const int64_t S = g->size;
     cudaStream_t st = ctx->stream;
-    if (!ctx->d_mt || ctx->mt_top_n < top_n) {
-        cudaFree(ctx->d_mt);
-        if (ctx->h_mt) cudaFreeHost(ctx->h_mt);
-        ctx->d_mt = ctx->h_mt = nullptr;
-        ctx->mt_top_n = 0;
-        CU(cudaMalloc(&ctx->d_mt, MT::bytes(top_n)));
-        CU(cudaHostAlloc((void **)&ctx->h_mt, MT::bytes(top_n), cudaHostAllocDefault));
-        ctx->mt_top_n = top_n;
-    }
+    CU(ctx->d_mt.grow((int64_t)MT::bytes(top_n)));
+    CU(ctx->h_mt.grow((int64_t)MT::bytes(top_n)));
     unsigned char *d = ctx->d_mt, *h = ctx->h_mt;
     int rc = ensure_multi_refs(ctx, g);
     if (rc) return rc;
     CU(cudaMemcpy2DAsync(ctx->d_multi_refs, sizeof(double) * (size_t)g->ld, refs, sizeof(double) * (size_t)ref_len,
                          sizeof(double) * (size_t)ref_len, (size_t)nq, cudaMemcpyHostToDevice, st));
-    std::vector<muse_batch *> bs((size_t)nq, nullptr);
-    auto cleanup = [&](int code) {
-        cudaStreamSynchronize(st);
-        for (muse_batch *b : bs)
-            if (b) muse_batch_destroy(b);
-        return code;
-    };
-#define CUM(call)                                                                         \
-    do {                                                                                  \
-        cudaError_t e_ = (call);                                                          \
-        if (e_ != cudaSuccess) return cleanup(cuda_fail(e_, #call, __FILE__, __LINE__)); \
-    } while (0)
 
     // ---- reference preparation: one launch per stage ----
     ExactParams *h_ep = reinterpret_cast<ExactParams *>(h + MT::off_ep());
     TablesArgs *h_ta = reinterpret_cast<TablesArgs *>(h + MT::off_ta());
     unsigned **h_cut = reinterpret_cast<unsigned **>(h + MT::off_cut());
     for (int i = 0; i < nq; i++) {
-        rc = batch_alloc(ctx, g, ref_len, &bs[(size_t)i]);
-        if (rc == MUSE_OK) rc = ensure_scratch(bs[(size_t)i]);
-        if (rc) return cleanup(rc);
-        muse_batch *b = bs[(size_t)i];
+        rc = batch_alloc(ctx, g, ref_len, bs[(size_t)i]);
+        if (rc == MUSE_OK) rc = ensure_scratch(bs[(size_t)i].get());
+        if (rc) return rc;
+        muse_batch *b = bs[(size_t)i].get();
         ExactParams &p = h_ep[i];
         memset(&p, 0, sizeof(p));
         p.slab = ctx->d_multi_refs + (size_t)i * (size_t)g->ld;
@@ -2238,15 +2158,15 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
     }
     const int64_t M = bs[0]->n / 2;
     const float thr_lo = threshold > 0 ? (float)threshold * 0.999999f : 0.f;
-    CUM(cudaMemcpyAsync(d, h, MT::off_tail(), cudaMemcpyHostToDevice, st));
-    CUM(launch_exact_batch(MODE_REF, reinterpret_cast<const ExactParams *>(d + MT::off_ep()), nq, 1, st));
+    CU(cudaMemcpyAsync(d, h, MT::off_tail(), cudaMemcpyHostToDevice, st));
+    CU(launch_exact_batch(MODE_REF, reinterpret_cast<const ExactParams *>(d + MT::off_ep()), nq, 1, st));
     screen_tables_batch_kernel<<<dim3((unsigned)((M / 2 + 1 + 255) / 256), (unsigned)nq), 256, 0, st>>>(
         reinterpret_cast<const TablesArgs *>(d + MT::off_ta()), (int)M, bs[0]->swtw, reinterpret_cast<float *>(d + MT::off_mids()));
     init_cut_batch_kernel<<<dim3((4 + MUSE_CUT_WORDS + 255) / 256, (unsigned)nq), 256, 0, st>>>(
         reinterpret_cast<unsigned *const *>(d + MT::off_cut()), thr_lo);
-    CUM(cudaGetLastError());
-    CUM(cudaMemcpyAsync(h + MT::off_mids(), d + MT::off_mids(), sizeof(float) * 4 * (size_t)nq, cudaMemcpyDeviceToHost, st));
-    CUM(cudaStreamSynchronize(st));
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(h + MT::off_mids(), d + MT::off_mids(), sizeof(float) * 4 * (size_t)nq, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
     const float *h_mids = reinterpret_cast<const float *>(h + MT::off_mids());
     std::vector<int> live;
     for (int i = 0; i < nq; i++) {
@@ -2256,7 +2176,7 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
             n_out[i] = -1;
             continue;
         }
-        muse_batch *b = bs[(size_t)i];
+        muse_batch *b = bs[(size_t)i].get();
         b->a_mid = h_mids[4 * i + 1];
         b->x_mid = cf{h_mids[4 * i + 2], h_mids[4 * i + 3]};
         b->screen_ok = 1;
@@ -2264,17 +2184,17 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
         live.push_back(i);
     }
     const int nl = (int)live.size();
-    if (nl == 0) return cleanup(MUSE_OK);
+    if (nl == 0) return MUSE_OK;
 
     // ---- bounds (tensor cores) and second stages (one pass over the store) ----
     std::vector<muse_batch *> lb((size_t)nl);
     std::vector<MultiQuery> hq((size_t)nl);
     ScreenParams sp0;
     for (int k = 0; k < nl; k++) {
-        muse_batch *b = lb[(size_t)k] = bs[(size_t)live[(size_t)k]];
+        muse_batch *b = lb[(size_t)k] = bs[(size_t)live[(size_t)k]].get();
         ScreenParams sp = screen_params(b);
         rc = arm_refinement(b, sp, thr_lo, max_lag, top_n, threshold, true);
-        if (rc) return cleanup(rc);
+        if (rc) return rc;
         if (k == 0) sp0 = sp;
         MultiQuery &m = hq[(size_t)k];
         memset(&m, 0, sizeof(m));
@@ -2285,14 +2205,14 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
         m.cut = b->d_cut;
         m.out_U = b->d_U;
     }
-    if (!ctx->d_multi_q) CUM(cudaMalloc(&ctx->d_multi_q, sizeof(MultiQuery) * (size_t)MUSE_MULTI_GROUP));
-    if (!ctx->d_multi_next) CUM(cudaMalloc(&ctx->d_multi_next, sizeof(unsigned)));
-    MultiQuery *d_q = static_cast<MultiQuery *>(ctx->d_multi_q);
-    CUM(cudaMemcpyAsync(d_q, hq.data(), sizeof(MultiQuery) * (size_t)nl, cudaMemcpyHostToDevice, st));
+    CU(ctx->d_multi_q.grow(MUSE_MULTI_GROUP));
+    CU(ctx->d_multi_next.grow(1));
+    MultiQuery *d_q = ctx->d_multi_q;
+    CU(cudaMemcpyAsync(d_q, hq.data(), sizeof(MultiQuery) * (size_t)nl, cudaMemcpyHostToDevice, st));
     rc = tc_bounds_queue(ctx, g, lb.data(), nl);
-    if (rc) return cleanup(rc);
-    CUM(launch_refine_multi(sp0, d_q, nl, ctx->sm_count, ctx->d_multi_next, st));
-    CUM(cudaEventRecord(ctx->mt_ev[3], st));
+    if (rc) return rc;
+    CU(launch_refine_multi(sp0, d_q, nl, ctx->sm_count, ctx->d_multi_next, st));
+    CU(cudaEventRecord(ctx->mt_ev[3], st));
 
     // ---- tails: survivors -> fp64 re-scoring -> filter -> top-N, one launch each ----
     MultiTail *h_tail = reinterpret_cast<MultiTail *>(h + MT::off_tail());
@@ -2318,27 +2238,27 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
         p.out_score = b->d_score;
         p.out_lag = b->d_lag;
     }
-    CUM(cudaMemcpyAsync(d + MT::off_tail(), h + MT::off_tail(), MT::off_mids() - MT::off_tail(), cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(d + MT::off_tail(), h + MT::off_tail(), MT::off_mids() - MT::off_tail(), cudaMemcpyHostToDevice, st));
     const MultiTail *d_tail = reinterpret_cast<const MultiTail *>(d + MT::off_tail());
     tail_reset_kernel<<<(nl + 255) / 256, 256, 0, st>>>(d_tail, nl);
     survivors_cut_batch_kernel<<<dim3((unsigned)((S + 255) / 256), (unsigned)nl), 256, 0, st>>>(d_tail, S);
-    CUM(cudaGetLastError());
+    CU(cudaGetLastError());
     unsigned long long *h_cnt = reinterpret_cast<unsigned long long *>(h + MT::off_cnt());
-    CUM(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(unsigned long long) * 4 * (size_t)nl, cudaMemcpyDeviceToHost, st));
-    CUM(cudaStreamSynchronize(st));      // the list lengths size the next launches
+    CU(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(unsigned long long) * 4 * (size_t)nl, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));      // the list lengths size the next launches
     int64_t max_len = 0;
     for (int k = 0; k < nl; k++) max_len = std::max<int64_t>(max_len, std::min<int64_t>((int64_t)h_cnt[4 * k + 2], lim));
     if (max_len > 0) {
-        CUM(launch_exact_batch(MODE_SCORE, reinterpret_cast<const ExactParams *>(d + MT::off_ep2()), nl, max_len, st));
+        CU(launch_exact_batch(MODE_SCORE, reinterpret_cast<const ExactParams *>(d + MT::off_ep2()), nl, max_len, st));
         FilterArgs f{max_lag, threshold, sign_filter, 1};
         emit_listed_batch_kernel<<<dim3((unsigned)((max_len + 255) / 256), (unsigned)nl), 256, 0, st>>>(d_tail, (long long)lim, f);
     }
     partial_topn_batch_kernel<<<dim3(16, (unsigned)nl), 256, 0, st>>>(d_tail, (long long)top_n, (long long)g->global_offset, (long long)lim);
-    CUM(cudaGetLastError());
-    CUM(cudaMemcpyAsync(h + MT::off_recs(), d_recs, sizeof(PartialRec) * (size_t)nl * (size_t)top_n, cudaMemcpyDeviceToHost, st));
-    CUM(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(unsigned long long) * 4 * (size_t)nl, cudaMemcpyDeviceToHost, st));
-    CUM(cudaEventRecord(ctx->mt_ev[4], st));
-    CUM(cudaStreamSynchronize(st));
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(h + MT::off_recs(), d_recs, sizeof(PartialRec) * (size_t)nl * (size_t)top_n, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(unsigned long long) * 4 * (size_t)nl, cudaMemcpyDeviceToHost, st));
+    CU(cudaEventRecord(ctx->mt_ev[4], st));
+    CU(cudaStreamSynchronize(st));
     const muse_partial *h_recs = reinterpret_cast<const muse_partial *>(h + MT::off_recs());
     for (int k = 0; k < nl; k++) {
         const int i = live[(size_t)k];
@@ -2353,13 +2273,12 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
             muse_batch *b = lb[(size_t)k];
             b->prescreened = 1;
             rc = muse_batch_run_ex(b, nullptr, 0, max_lag, top_n, threshold, sign_filter, MUSE_MODE_SCREEN, 0, sc, lg, ix, n_out + i);
-            if (rc) return cleanup(rc);
+            if (rc) return rc;
             continue;
         }
         n_out[i] = records_out(r, top_n, sc, lg, ix);
     }
-#undef CUM
-    return cleanup(MUSE_OK);
+    return MUSE_OK;
 }
 
 extern "C" int muse_multi_last_stats(const muse_ctx *ctx, int64_t *n_refined, int64_t *n_rescored) {
@@ -2388,23 +2307,19 @@ extern "C" int muse_multi_bounds_tc(muse_ctx *ctx, muse_group *g, const double *
     CU(cudaSetDevice(ctx->device));
     const int64_t S = g->size;
     if (S == 0) return MUSE_OK;
-    std::vector<muse_batch *> bs;
-    int rc = MUSE_OK;
-    for (int64_t q = 0; q < n_refs && rc == MUSE_OK; q++) {
-        muse_batch *b = nullptr;
-        rc = muse_batch_create(ctx, g, refs + (size_t)q * (size_t)ref_len, ref_len, &b);
-        if (rc == MUSE_OK) bs.push_back(b);
+    std::vector<BatchPtr> own((size_t)n_refs);
+    std::vector<muse_batch *> bs((size_t)n_refs);
+    for (size_t q = 0; q < bs.size(); q++) {
+        const int rc = muse_batch_create(ctx, g, refs + q * (size_t)ref_len, ref_len, &bs[q]);
+        if (rc) return rc;
+        own[q].reset(bs[q]);
     }
-    if (rc == MUSE_OK) rc = tc_bounds_queue(ctx, g, bs.data(), (int)bs.size());
-    for (size_t q = 0; q < bs.size() && rc == MUSE_OK; q++)
-        if (cudaMemcpyAsync(upper + q * (size_t)S, bs[q]->d_U, sizeof(float) * (size_t)S, cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess)
-            rc = fail(MUSE_ERR_CUDA, "muse_multi_bounds_tc: copy failed");
-    if (cudaStreamSynchronize(ctx->stream) != cudaSuccess && rc == MUSE_OK) {
-        (void)cudaGetLastError();
-        rc = fail(MUSE_ERR_CUDA, "muse_multi_bounds_tc: %s", cudaGetErrorString(cudaPeekAtLastError()));
-    }
-    for (muse_batch *b : bs) muse_batch_destroy(b);
-    return rc;
+    const int rc = tc_bounds_queue(ctx, g, bs.data(), (int)bs.size());
+    if (rc) return rc;
+    for (size_t q = 0; q < bs.size(); q++)
+        CU(cudaMemcpyAsync(upper + q * (size_t)S, bs[q]->d_U, sizeof(float) * (size_t)S, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(cudaStreamSynchronize(ctx->stream));
+    return MUSE_OK;
 }
 
 extern "C" int muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, int64_t n_refs, int64_t ref_len,
@@ -2426,19 +2341,20 @@ extern "C" int muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, 
                           top_n * 4 <= g->size && (g->size >= 16384 || mode == MUSE_MODE_SCREEN) && n_refs > 1;
     ctx->multi_refined = ctx->multi_rescored = 0;
     const int QC = one_pass ? MUSE_MULTI_GROUP : MUSE_MULTI_SEPARATE;
-    std::vector<muse_batch *> bs((size_t)QC), made((size_t)QC);
-    std::vector<int64_t> which((size_t)QC);
     for (int64_t q0 = 0; q0 < n_refs; q0 += QC) {
         const int nq = (int)std::min<int64_t>(QC, n_refs - q0);
         if (one_pass && nq > 1) {
-            int rct = multi_run_tc_group(ctx, g, refs + (size_t)q0 * (size_t)ref_len, nq, ref_len, max_lag, top_n, threshold, sign_filter,
-                                         scores + (size_t)q0 * (size_t)top_n, lags + (size_t)q0 * (size_t)top_n,
-                                         series_idx + (size_t)q0 * (size_t)top_n, n_out + q0);
-            if (rct) return rct;
+            std::vector<BatchPtr> bs((size_t)nq);
+            const int rc = multi_run_tc_group(ctx, g, refs + (size_t)q0 * (size_t)ref_len, nq, ref_len, max_lag, top_n, threshold, sign_filter,
+                                              scores + (size_t)q0 * (size_t)top_n, lags + (size_t)q0 * (size_t)top_n,
+                                              series_idx + (size_t)q0 * (size_t)top_n, n_out + q0, bs);
+            if (rc) {
+                cudaStreamSynchronize(ctx->stream);      // work queued on the batches may still be running: it ends before they go
+                return rc;
+            }
             continue;
         }
-        int live = 0, rc = MUSE_OK;
-        int n_made = 0;
+        int rc = MUSE_OK;
         // the references of the group: ONE upload (rows at the slab's pitch, pad columns zero), then queued back to
         // back, ONE round trip
         const bool rows_on_device = ref_len == g->N;
@@ -2449,36 +2365,30 @@ extern "C" int muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, 
                                  sizeof(double) * (size_t)ref_len, sizeof(double) * (size_t)ref_len, (size_t)nq,
                                  cudaMemcpyHostToDevice, ctx->stream));
         }
-        for (int i = 0; i < nq && rc == MUSE_OK; i++) {
-            rc = batch_create_queue(ctx, g, refs + (size_t)(q0 + i) * (size_t)ref_len, ref_len, &made[n_made],
+        std::vector<BatchPtr> bs((size_t)nq);
+        for (int i = 0; i < nq && rc == MUSE_OK; i++)
+            rc = batch_create_queue(ctx, g, refs + (size_t)(q0 + i) * (size_t)ref_len, ref_len, bs[(size_t)i],
                                     rows_on_device ? ctx->d_multi_refs + (size_t)i * (size_t)g->ld : nullptr);
-            if (rc == MUSE_OK) n_made++;
-        }
         if (cudaStreamSynchronize(ctx->stream) != cudaSuccess && rc == MUSE_OK) rc = fail(MUSE_ERR_CUDA, "cudaStreamSynchronize failed");
-        for (int i = 0; i < n_made; i++) {
-            if (rc != MUSE_OK) {
-                muse_batch_destroy(made[i]);
-                continue;
-            }
-            const int rf = batch_create_finish(made[i]);
-            if (rf == MUSE_ERR_STDDEV_ZERO) {   // muse_batch.go:38-41: this query has no Batch; the others do
-                n_out[q0 + i] = -1;
-            } else if (rf != MUSE_OK) {
-                rc = rf;
-            } else {
-                bs[live] = made[i];
-                which[live++] = q0 + i;
-            }
-        }
-        for (int i = 0; i < live; i++) {
-            const int64_t q = which[i];
-            if (rc == MUSE_OK)
-                rc = muse_batch_run_ex(bs[i], key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0,
-                                       scores ? scores + (size_t)q * (size_t)top_n : nullptr, lags ? lags + (size_t)q * (size_t)top_n : nullptr,
-                                       series_idx ? series_idx + (size_t)q * (size_t)top_n : nullptr, n_out + q);
-            muse_batch_destroy(bs[i]);
-        }
         if (rc) return rc;
+        for (int i = 0; i < nq; i++) {
+            rc = batch_create_finish(bs[(size_t)i].get());
+            if (rc == MUSE_ERR_STDDEV_ZERO) {   // muse_batch.go:38-41: this query has no Batch; the others do
+                n_out[q0 + i] = -1;
+                bs[(size_t)i].reset();
+            } else if (rc) {
+                return rc;
+            }
+        }
+        for (int i = 0; i < nq; i++) {
+            if (!bs[(size_t)i]) continue;
+            const int64_t q = q0 + i;
+            rc = muse_batch_run_ex(bs[(size_t)i].get(), key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0,
+                                   scores ? scores + (size_t)q * (size_t)top_n : nullptr, lags ? lags + (size_t)q * (size_t)top_n : nullptr,
+                                   series_idx ? series_idx + (size_t)q * (size_t)top_n : nullptr, n_out + q);
+            bs[(size_t)i].reset();
+            if (rc) return rc;
+        }
     }
     return MUSE_OK;
 }
@@ -2509,34 +2419,28 @@ extern "C" int muse_xcorr(muse_ctx *ctx, const double *x, int64_t x_len, const d
     if (std_zero) *std_zero = 0;
     // one allocation: x, y, xp, yp, cc (doubles), then lag, value, flag
     const size_t nd = (size_t)x_len + (size_t)y_len + 3 * (size_t)nn;
-    unsigned char *d = nullptr;
-    CU(cudaMalloc(&d, nd * sizeof(double) + 32 + 256 + work_bytes));
+    DevBuf<unsigned char> d;
+    CU(d.grow((int64_t)(nd * sizeof(double) + 32 + 256 + work_bytes)));
     void *d_work = d + ((nd * sizeof(double) + 32 + 255) / 256) * 256;
-    double *dx = reinterpret_cast<double *>(d), *dy = dx + x_len, *dxp = dy + y_len, *dyp = dxp + nn, *dcc = dyp + nn;
+    double *dx = reinterpret_cast<double *>(d.get()), *dy = dx + x_len, *dxp = dy + y_len, *dyp = dxp + nn, *dcc = dyp + nn;
     long long *dlag = reinterpret_cast<long long *>(dcc + nn);
     double *dval = reinterpret_cast<double *>(dlag + 1);
     int *dflag = reinterpret_cast<int *>(dval + 1);
     struct Tail { long long lag; double val; int flag; int pad; } tail;
-    auto body = [&]() -> int {
-        CU(cudaMemcpyAsync(dx, x, sizeof(double) * (size_t)x_len, cudaMemcpyHostToDevice, st));
-        CU(cudaMemcpyAsync(dy, y, sizeof(double) * (size_t)y_len, cudaMemcpyHostToDevice, st));
-        CU(cudaMemsetAsync(dlag, 0, 32, st));
-        xcorr_prepare_kernel<<<2, 256, 0, st>>>(dx, x_len, dy, y_len, nn, normalize ? 1 : 0, dxp, dyp, dflag);
-        // xcorr.go:139-142: gonum's inverse transform is unnormalised (n x the correlation); the reference scales
-        // by 1/(n(n-1)) for z-normalised inputs and by 1/n otherwise -> 1/(n-1) and 1 on a direct sum
-        const double scale = normalize ? 1.0 / (double)(nn - 1) : 1.0;
-        if (by_fft) CU(launch_long_xcorr(dxp, dyp, nn, L, scale, dcc, d_work, st));
-        else xcorr_direct_kernel<<<(unsigned)((nn + XC_LAGS - 1) / XC_LAGS), XC_LAGS, 0, st>>>(dxp, dyp, nn, scale, dcc);
-        xcorr_argmax_kernel<<<1, 256, 0, st>>>(dcc, nn, dlag, dval);
-        CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(&tail, dlag, sizeof(tail), cudaMemcpyDeviceToHost, st));
-        if (cc) CU(cudaMemcpyAsync(cc, dcc, sizeof(double) * (size_t)nn, cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        return MUSE_OK;
-    };
-    const int rc = body();
-    cudaFree(d);
-    if (rc) return rc;
+    CU(cudaMemcpyAsync(dx, x, sizeof(double) * (size_t)x_len, cudaMemcpyHostToDevice, st));
+    CU(cudaMemcpyAsync(dy, y, sizeof(double) * (size_t)y_len, cudaMemcpyHostToDevice, st));
+    CU(cudaMemsetAsync(dlag, 0, 32, st));
+    xcorr_prepare_kernel<<<2, 256, 0, st>>>(dx, x_len, dy, y_len, nn, normalize ? 1 : 0, dxp, dyp, dflag);
+    // xcorr.go:139-142: gonum's inverse transform is unnormalised (n x the correlation); the reference scales
+    // by 1/(n(n-1)) for z-normalised inputs and by 1/n otherwise -> 1/(n-1) and 1 on a direct sum
+    const double scale = normalize ? 1.0 / (double)(nn - 1) : 1.0;
+    if (by_fft) CU(launch_long_xcorr(dxp, dyp, nn, L, scale, dcc, d_work, st));
+    else xcorr_direct_kernel<<<(unsigned)((nn + XC_LAGS - 1) / XC_LAGS), XC_LAGS, 0, st>>>(dxp, dyp, nn, scale, dcc);
+    xcorr_argmax_kernel<<<1, 256, 0, st>>>(dcc, nn, dlag, dval);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(&tail, dlag, sizeof(tail), cudaMemcpyDeviceToHost, st));
+    if (cc) CU(cudaMemcpyAsync(cc, dcc, sizeof(double) * (size_t)nn, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
     if (normalize && tail.flag) {   // xcorr.go:109-126: (nil, 0, 0)
         if (std_zero) *std_zero = 1;
         *n_out = 0;
@@ -2551,25 +2455,27 @@ extern "C" int muse_xcorr(muse_ctx *ctx, const double *x, int64_t x_len, const d
 // multi-GPU exchange over NVLink peer memory (one process per GPU)
 // ------------------------------------------------------------------------------------
 struct muse_exchange {
-    muse_ctx *ctx;
-    int rank, world;
-    int64_t capacity;                 // records per rank per step
-    unsigned char *base;              // local buffer: recs[2][world][capacity] then flags[2][world] (IPC-exported)
-    size_t recs_bytes;                // bytes of ONE parity's records
-    unsigned char *peer_base[MUSE_EXCHANGE_MAX_RANKS];   // every rank's buffer as seen from here (own: base)
-    bool opened;
-    unsigned long long epoch;
-    unsigned *d_done;
-    int *d_status;
-    unsigned char *h_recs;            // pinned: the merged top_n records of one step, then the status word
-    // device-side merge of the gathered records (group max across shards, filter, top-N)
-    MergeState merge;
-    size_t merge_bytes;               // one allocation behind merge.hkeys
-    unsigned long long *d_nlocal;     // grouped runs: representatives of this shard
-    PartialRec *d_out;                // [capacity] merged top_n
+    muse_ctx *ctx = nullptr;
+    int rank = 0, world = 0;
+    int64_t capacity = 0;                 // records per rank per step
+    DevBuf<unsigned char> base;           // local buffer: recs[2][world][capacity] then flags[2][world] (IPC-exported)
+    size_t recs_bytes = 0;                // bytes of ONE parity's records
+    unsigned char *peer_base[MUSE_EXCHANGE_MAX_RANKS] = {};   // every rank's buffer as seen from here (own: base)
+    bool opened = false;
+    unsigned long long epoch = 0;
+    DevBuf<unsigned> d_done;
+    DevBuf<int> d_status;
+    PinnedBuf h_recs;                     // pinned: the merged top_n records of one step, then the status word
+    // device-side merge of the gathered records (group max across shards, filter, top-N), all in merge_buf
+    DevBuf<unsigned char> merge_buf;
+    MergeState merge = {};
+    size_t merge_bytes = 0;               // the hash table at the front of merge_buf: merge.hkeys, gmax, gidx
+    unsigned long long *d_nlocal = nullptr;   // grouped runs: representatives of this shard
+    PartialRec *d_out = nullptr;          // [capacity] merged top_n
     // muse_multi_run_exchange, allocated on its first call: this rank's per-query lists of one step, device and pinned host
     // ([capacity] records, [MUSE_MULTI_GROUP] counts; the host copy then receives the [world] flag words of the step)
-    unsigned char *d_send, *h_send;
+    DevBuf<unsigned char> d_send;
+    PinnedBuf h_send;
 };
 
 // Opens the next step of the exchange: a new epoch, and every rank's receive records and flags of the epoch's parity.
@@ -2602,32 +2508,30 @@ extern "C" int muse_exchange_create(muse_ctx *ctx, int32_t rank, int32_t world, 
     if (world < 1 || world > MUSE_EXCHANGE_MAX_RANKS || rank < 0 || rank >= world || capacity < 1)
         return fail(MUSE_ERR_INVALID_ARG, "muse_exchange_create: rank %d of %d, capacity %lld", rank, world, (long long)capacity);
     CU(cudaSetDevice(ctx->device));
-    muse_exchange *x = new muse_exchange();
-    memset(x, 0, sizeof(*x));
+    std::unique_ptr<muse_exchange> x(new muse_exchange());
     x->ctx = ctx;
     x->rank = rank;
     x->world = world;
     x->capacity = capacity;
     x->recs_bytes = (size_t)world * (size_t)capacity * sizeof(muse_partial);
     const size_t bytes = exchange_bytes(world, capacity);
-    CU(cudaMalloc(&x->base, bytes));
+    CU(x->base.grow((int64_t)bytes));
     CU(cudaMemset(x->base, 0, bytes));
-    CU(cudaMalloc(&x->d_done, sizeof(unsigned)));
+    CU(x->d_done.grow(1));
     CU(cudaMemset(x->d_done, 0, sizeof(unsigned)));
-    CU(cudaMalloc(&x->d_status, sizeof(int)));
+    CU(x->d_status.grow(1));
     CU(cudaMemset(x->d_status, 0, sizeof(int)));
-    CU(cudaHostAlloc((void **)&x->h_recs, (size_t)capacity * sizeof(muse_partial) + 64, cudaHostAllocDefault));
+    CU(x->h_recs.grow((int64_t)((size_t)capacity * sizeof(muse_partial) + 64)));
     {   // merge scratch: hash table of 2 x (records of all shards) slots, candidate arrays, counters, output records
         const long long total = (long long)world * capacity;
         long long slots = 1;
         while (slots < 2 * total) slots <<= 1;
         const size_t tab = sizeof(unsigned long long) * (size_t)slots;
         const size_t bytes_m = 3 * tab + (size_t)total * (8 + 8 + 4) + 64 + (size_t)capacity * sizeof(PartialRec) + 64;
-        unsigned char *m = nullptr;
-        CU(cudaMalloc(&m, bytes_m));
-        CU(cudaMemset(m, 0, bytes_m));
+        CU(x->merge_buf.grow((int64_t)bytes_m));
+        CU(cudaMemset(x->merge_buf, 0, bytes_m));
         x->merge_bytes = 3 * tab;
-        x->merge.hkeys = reinterpret_cast<unsigned long long *>(m);
+        x->merge.hkeys = reinterpret_cast<unsigned long long *>(x->merge_buf.get());
         x->merge.gmax = x->merge.hkeys + slots;
         x->merge.gidx = x->merge.gmax + slots;
         x->merge.slots = slots;
@@ -2643,7 +2547,7 @@ extern "C" int muse_exchange_create(muse_ctx *ctx, int32_t rank, int32_t world, 
     x->peer_base[rank] = x->base;
     x->opened = (world == 1);
     CU(cudaDeviceSynchronize());
-    *out = x;
+    *out = x.release();
     return MUSE_OK;
 }
 
@@ -2680,13 +2584,6 @@ extern "C" void muse_exchange_destroy(muse_exchange *x) {
     cudaStreamSynchronize(x->ctx->stream);
     for (int r = 0; r < x->world; r++)
         if (r != x->rank && x->peer_base[r]) cudaIpcCloseMemHandle(x->peer_base[r]);
-    cudaFree(x->base);
-    cudaFree(x->d_done);
-    cudaFree(x->d_status);
-    cudaFree(x->merge.hkeys);
-    cudaFree(x->d_send);
-    if (x->h_recs) cudaFreeHost(x->h_recs);
-    if (x->h_send) cudaFreeHost(x->h_send);
     delete x;
 }
 
@@ -2760,7 +2657,7 @@ extern "C" int muse_batch_run_exchange_ex(muse_batch *b, muse_exchange *x, const
         CU(cudaMemsetAsync(x->d_status, 0, sizeof(int), st));
         return fail(MUSE_ERR_CUDA, "muse_batch_run_exchange: a peer did not deliver its records within the time limit");
     }
-    const muse_partial *recs = reinterpret_cast<const muse_partial *>(x->h_recs);
+    const muse_partial *recs = reinterpret_cast<const muse_partial *>(x->h_recs.get());
     if (top_n > 0 && recs[0].flags == 2)
         return fail(MUSE_ERR_UNSUPPORTED, "host path needed: a shard's record list was too long for the device-side select or merge");
     *n_out = records_out(recs, top_n, scores, lags, series_idx);
@@ -2781,8 +2678,8 @@ static size_t multi_send_bytes(const muse_exchange *x) {
 }
 
 static int multi_send_alloc(muse_exchange *x) {
-    if (!x->d_send) CU(cudaMalloc(&x->d_send, multi_send_bytes(x)));
-    if (!x->h_send) CU(cudaHostAlloc((void **)&x->h_send, multi_send_bytes(x) + (size_t)x->world * sizeof(unsigned long long), cudaHostAllocDefault));
+    CU(x->d_send.grow((int64_t)multi_send_bytes(x)));
+    CU(x->h_send.grow((int64_t)(multi_send_bytes(x) + (size_t)x->world * sizeof(unsigned long long))));
     return MUSE_OK;
 }
 
@@ -2815,7 +2712,7 @@ extern "C" int muse_multi_run_exchange(muse_group *g, muse_exchange *x, const do
         const int nq = (int)std::min<int64_t>(q_step, n_refs - q0);
         double *sc = scores + (size_t)q0 * (size_t)top_n;
         int64_t *lg = lags + (size_t)q0 * (size_t)top_n, *ix = series_idx + (size_t)q0 * (size_t)top_n, *no = n_out + q0;
-        long long *h_cnt = reinterpret_cast<long long *>(x->h_send);
+        long long *h_cnt = reinterpret_cast<long long *>(x->h_send.get());
         PartialRec *h_tab = reinterpret_cast<PartialRec *>(x->h_send + (size_t)MUSE_MULTI_GROUP * sizeof(long long));
         const unsigned long long *h_flags = reinterpret_cast<const unsigned long long *>(x->h_send + multi_send_bytes(x));
         if (local_rc == MUSE_OK)
@@ -2839,7 +2736,7 @@ extern "C" int muse_multi_run_exchange(muse_group *g, muse_exchange *x, const do
         const ExchangePeers ex = exchange_step(x);
         const long long total = (long long)nq * top_n;
         const unsigned pblocks = (unsigned)std::max<long long>(1, std::min<long long>((total + 255) / 256, (long long)ctx->sm_count * 4));
-        const long long *d_cnt = reinterpret_cast<const long long *>(x->d_send);
+        const long long *d_cnt = reinterpret_cast<const long long *>(x->d_send.get());
         const PartialRec *d_tab = reinterpret_cast<const PartialRec *>(x->d_send + (size_t)MUSE_MULTI_GROUP * sizeof(long long));
         multi_records_push_kernel<<<pblocks, 256, 0, st>>>(d_tab, d_cnt, nq, (long long)top_n, (long long)x->capacity,
                                                            local_rc != MUSE_OK ? 1 : 0, ex);
@@ -2860,7 +2757,7 @@ extern "C" int muse_multi_run_exchange(muse_group *g, muse_exchange *x, const do
         for (int r = 0; r < x->world; r++)
             if ((h_flags[r] & 0xffffffffull) == MUSE_EXCHANGE_RANK_FAILED)
                 return fail(MUSE_ERR_CUDA, "muse_multi_run_exchange: rank %d failed", r);
-        const muse_partial *recs = reinterpret_cast<const muse_partial *>(x->h_recs);
+        const muse_partial *recs = reinterpret_cast<const muse_partial *>(x->h_recs.get());
         for (int q = 0; q < nq; q++) {
             if (no[q] < 0) continue;      // std(ref) == 0 on every rank (muse_batch.go:38-41)
             const size_t row = (size_t)q * (size_t)top_n;
@@ -2884,23 +2781,17 @@ extern "C" int muse_merge_partials_many(muse_ctx *ctx, const muse_partial *d_par
     CU(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const size_t n_rec = (size_t)n_refs * (size_t)top_n;
-    unsigned char *d = nullptr;
-    CU(cudaMalloc(&d, n_rec * sizeof(PartialRec) + (size_t)n_refs * sizeof(long long)));
-    PartialRec *d_out = reinterpret_cast<PartialRec *>(d);
+    DevBuf<unsigned char> d;
+    CU(d.grow((int64_t)(n_rec * sizeof(PartialRec) + (size_t)n_refs * sizeof(long long))));
+    PartialRec *d_out = reinterpret_cast<PartialRec *>(d.get());
     long long *d_n = reinterpret_cast<long long *>(d_out + n_rec);
     std::vector<muse_partial> h(n_rec);
-    auto body = [&]() -> int {
-        multi_merge_kernel<<<(unsigned)n_refs, 256, 0, st>>>(reinterpret_cast<const PartialRec *>(d_parts), world, (long long)(n_refs * top_n),
-                                                             (long long)top_n, d_out, d_n);
-        CU(cudaGetLastError());
-        CU(cudaMemcpyAsync(h.data(), d_out, n_rec * sizeof(PartialRec), cudaMemcpyDeviceToHost, st));
-        CU(cudaMemcpyAsync(n_out, d_n, (size_t)n_refs * sizeof(long long), cudaMemcpyDeviceToHost, st));
-        CU(cudaStreamSynchronize(st));
-        return MUSE_OK;
-    };
-    const int rc = body();
-    cudaFree(d);
-    if (rc) return rc;
+    multi_merge_kernel<<<(unsigned)n_refs, 256, 0, st>>>(reinterpret_cast<const PartialRec *>(d_parts), world, (long long)(n_refs * top_n),
+                                                         (long long)top_n, d_out, d_n);
+    CU(cudaGetLastError());
+    CU(cudaMemcpyAsync(h.data(), d_out, n_rec * sizeof(PartialRec), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(n_out, d_n, (size_t)n_refs * sizeof(long long), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
     for (size_t i = 0; i < n_rec; i++) {
         scores[i] = h[i].score;
         lags[i] = h[i].lag;

@@ -123,6 +123,7 @@ ABI = {
     "muse_ctx_set_stream": (C.c_int, [_vp, _vp]),
     "muse_host_alloc": (C.c_int, [C.POINTER(_vp), C.c_int64]),
     "muse_host_free": (None, [_vp]),
+    "muse_held_bytes": (C.c_int, [_ip64, _ip64]),
     "muse_group_create": (C.c_int, [_vp, C.c_int64, C.c_int32, C.c_int64, C.POINTER(_vp)]),
     "muse_group_destroy": (None, [_vp]),
     "muse_group_append": (C.c_int, [_vp, _vp, C.c_int64, C.c_int64, _vp]),

@@ -91,6 +91,9 @@ int  muse_ctx_set_stream(muse_ctx *ctx, void *cuda_stream);
 /* Page-locked host memory for rows handed to muse_group_append (full-rate DMA). */
 int  muse_host_alloc(void **out, int64_t bytes);
 void muse_host_free(void *p);
+/* Bytes of device and of page-locked host memory the library holds right now, in this process, over every context
+ * (memory of muse_host_alloc belongs to the caller and is not counted).  When every handle is destroyed both are 0. */
+int  muse_held_bytes(int64_t *device_bytes, int64_t *pinned_bytes);
 
 /* ---- series store ----------------------------------------------------------
  * Replaces Group{registry} + Series{y, labels} (group.go:7-56, series.go:8-42):
