@@ -75,6 +75,7 @@ class Buf {
     ~Buf() { release(); }
     T *get() const { return p_; }
     operator T *() const { return p_; }
+    T *operator->() const { return p_; }
     int64_t cap() const { return cap_; }
     // Room for n elements: when n exceeds the capacity, the buffer is freed and reallocated; the contents are not kept.
     cudaError_t grow(int64_t n) {
@@ -157,6 +158,30 @@ extern "C" int muse_held_bytes(int64_t *device_bytes, int64_t *pinned_bytes) {
                                 // of a tensor-core launch group and of a group of separate batches in muse_multi_run
 #define MUSE_MULTI_GROUP 256    // queries of one launch of the tensor-core multi-query path (== TcCfg::TN == RefineMultiCfg::QMAX)
 #define MUSE_MULTI_SEPARATE 16  // queries of one group of separate batches in muse_multi_run (one upload, one round trip)
+#define MUSE_DEVICE_TOPN_MAX 65536   // top_n of a device-side top-N: its records come back through the mailbox
+#define MUSE_SELECT_CHUNK 32768      // candidates that come back with their count (run_select)
+// The pinned mailbox of a batch for the small device->host results (one copy per round trip).
+struct Mailbox {
+    int32_t flag;          // the reference's std-zero flag (no screening tables)
+    float mid[4];          // screening tables: [0] the std-zero flag (as float bits), [1] A[M/2], [2..3] Xt[M/2]
+    RunCounters counters;
+    union {
+        struct {           // run_select: the first candidates
+            unsigned long long key[MUSE_SELECT_CHUNK];
+            int32_t idx[MUSE_SELECT_CHUNK], lagsgn[MUSE_SELECT_CHUNK];
+        } cand;
+        muse_partial recs[MUSE_DEVICE_TOPN_MAX];   // the device-side top-N
+    };
+};
+static_assert(sizeof(Mailbox::cand) <= sizeof(Mailbox::recs) && sizeof(Mailbox::recs) == sizeof(muse_partial) * MUSE_DEVICE_TOPN_MAX,
+              "the device-side top-N records size the mailbox");
+
+// The device-side top-N of top_n records applies when the mailbox holds them and the sort scratch d_skey, 8 bytes per entry
+// of `capacity` entries, holds them as records.
+static bool device_topn_fits(int64_t top_n, int64_t capacity) {
+    return top_n > 0 && top_n <= MUSE_DEVICE_TOPN_MAX && top_n * (int64_t)(sizeof(muse_partial) / 8) <= capacity;
+}
+
 struct RunScratch {
     int64_t scratch_cap = 0;                  // entries of the eleven arrays below (ensure_scratch)
     DevBuf<double> d_score;
@@ -169,12 +194,11 @@ struct RunScratch {
     DevBuf<int32_t> d_list;
     DevBuf<float> d_L;                        // lower bounds (grouped screened runs, diagnostic entry point)
     DevBuf<signed char> d_W;                  // grouped screened runs: lag-window verdict of every refined series (ScreenParams::out_W)
-    PinnedBuf h_pin;                          // pinned mailbox for the small device->host results
-    DevBuf<unsigned long long> d_counters;    // [0] ncand, [1] nselected, [2] exact list length, [3] refined
+    Buf<Mailbox, true> h_pin;
+    DevBuf<RunCounters> d_counters;
     DevBuf<SelectState> d_sel;
     DevBuf<int32_t> d_flag;
-    DevBuf<unsigned> d_cut;                   // fused refinement state: [0] cut bits, [1] series claims of the warp kernel, [2..3] n_refined (u64),
-                                              // [4..] coarse + fine histogram
+    DevBuf<CutState> d_cut;                   // fused refinement state
     // group table
     DevBuf<unsigned long long> d_gmax, d_hkeys;
     DevBuf<int32_t> d_gidx;
@@ -245,7 +269,7 @@ struct muse_batch : RunScratch {
     cf x_mid = {};
     muse_timing timing = {};
     int timing_pending = 0;    // the last run was queued without a final synchronisation (muse_batch_run_partial_device)
-    int fused_run = 0;         // 1: score_fused, 2: score_fused_grouped (d_counters[2] = exact list length, [3] = refined)
+    int fused_run = 0;         // 1: score_fused, 2: score_fused_grouped (d_counters: listed = exact list length)
     int prescreened = 0;       // d_U and the cut-off state were filled by the tensor-core multi-query path: the next fused run starts at its tail
     int signed_run = 0;        // the current run keeps the sign of the scores (muse.go:72-76)
     // n > MUSE_MAX_FUSED_FFT_LEN: Stockham passes through global memory (kernels_long.cu); Xt holds n entries, twM the n twiddles
@@ -805,9 +829,9 @@ static int screen_is_big(int log2m) { return log2m >= 11 && log2m <= 13; }      
 // A[k] = |Xt[k]| * (1 at DC and Nyquist, else 2) rounded UP (the bound must not shrink), one 16-byte entry per
 // mirror pair (k, M-k), k < M/2, with the split twiddle exp(-2*pi*i*k/n); the two reference coefficients of the
 // second stage; and A[M/2], Xt[M/2] for the host (kernel parameters).
-__global__ void screen_tables_kernel(const cd *__restrict__ Xt, int M, const float2 *__restrict__ swtw, float4 *__restrict__ sw,
-                                     float4 *__restrict__ sx, float *__restrict__ sb, float *__restrict__ mid,
-                                     const int32_t *__restrict__ std_zero) {
+__device__ __forceinline__ void screen_tables_body(const cd *__restrict__ Xt, int M, const float2 *__restrict__ swtw, float4 *__restrict__ sw,
+                                                   float4 *__restrict__ sx, float *__restrict__ sb, float *__restrict__ mid,
+                                                   const int32_t *__restrict__ std_zero) {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k > M / 2) return;
     if (k == 0) mid[0] = __int_as_float(*std_zero);      // the reference's std-zero flag rides along: one copy to the host
@@ -824,6 +848,11 @@ __global__ void screen_tables_kernel(const cd *__restrict__ Xt, int M, const flo
     sw[k] = make_float4(w.x, w.y, wa, wc);
     sx[k] = make_float4((float)a.x, (float)a.y, (float)c.x, (float)c.y);
     sb[k] = __double2float_ru(sqrt(2.0 * ((double)wa * (double)wa + (double)wc * (double)wc)) * (1.0 + 1e-15));
+}
+__global__ void screen_tables_kernel(const cd *__restrict__ Xt, int M, const float2 *__restrict__ swtw, float4 *__restrict__ sw,
+                                     float4 *__restrict__ sx, float *__restrict__ sb, float *__restrict__ mid,
+                                     const int32_t *__restrict__ std_zero) {
+    screen_tables_body(Xt, M, swtw, sw, sx, sb, mid, std_zero);
 }
 
 // Twiddle tables of FFT length n (they depend on n alone): filled when the scratch set was last used for another n.
@@ -935,10 +964,10 @@ static int batch_alloc(muse_ctx *ctx, muse_group *g, int64_t ref_len, BatchPtr &
     int rc = ensure_ref_tables(b.get(), g->ld);
     if (rc) return rc;
     CU(b->d_flag.grow(1));
-    CU(b->d_counters.grow(4));
+    CU(b->d_counters.grow(1));
     CU(b->d_sel.grow(1));
-    CU(b->d_cut.grow(4 + MUSE_CUT_WORDS));
-    CU(b->h_pin.grow((int64_t)4 << 20));
+    CU(b->d_cut.grow(1));
+    CU(b->h_pin.grow(1));
     out = std::move(b);
     return MUSE_OK;
 }
@@ -982,19 +1011,17 @@ static int batch_create_queue(muse_ctx *ctx, muse_group *g, const double *ref, i
         CU(cudaGetLastError());
     }
     // one round trip: the std-zero flag of the reference and the two middle-bin values the kernels take by value
-    int32_t *h_flag = reinterpret_cast<int32_t *>(b->h_pin.get());
-    float *h_mid = reinterpret_cast<float *>(b->h_pin + 16);
-    if (screen) CU(cudaMemcpyAsync(h_mid, b->d_mid, sizeof(float) * 4, cudaMemcpyDeviceToHost, st));      // [0] carries the flag
-    else CU(cudaMemcpyAsync(h_flag, b->d_flag, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (screen) CU(cudaMemcpyAsync(b->h_pin->mid, b->d_mid, sizeof(float) * 4, cudaMemcpyDeviceToHost, st));      // [0] carries the flag
+    else CU(cudaMemcpyAsync(&b->h_pin->flag, b->d_flag, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     b->screen_ok = screen ? -1 : 0;      // -1: pending until batch_create_finish
     out = std::move(b);
     return MUSE_OK;
 }
 
 static int batch_create_finish(muse_batch *b) {
-    const float *h_mid = reinterpret_cast<const float *>(b->h_pin + 16);
-    int32_t flag;
-    memcpy(&flag, b->screen_ok == -1 ? static_cast<const void *>(h_mid) : static_cast<const void *>(b->h_pin), sizeof(flag));
+    const float *h_mid = b->h_pin->mid;
+    int32_t flag = b->h_pin->flag;
+    if (b->screen_ok == -1) memcpy(&flag, &h_mid[0], sizeof(flag));
     if (flag)   // muse_batch.go:38-41
         return fail(MUSE_ERR_STDDEV_ZERO, "Invalid input query, Standard deviation of zero");
     if (b->screen_ok == -1) {
@@ -1189,12 +1216,8 @@ struct Rec {
     unsigned long long key;   // |score| bits
     int32_t idx;
     int32_t lagsgn;           // 2*lag + (score < 0)
-    double score() const {
-        double a;
-        memcpy(&a, &key, sizeof(a));
-        return (lagsgn & 1) ? -a : a;
-    }
-    int32_t lag() const { return (lagsgn - (lagsgn & 1)) / 2; }
+    double score() const { return cand_score(key, lagsgn); }
+    int32_t lag() const { return cand_lag(lagsgn); }
 };
 
 // Key bits per group-by column.  64 / ncols each when every column's cardinality fits: that packing does not depend on the
@@ -1287,14 +1310,14 @@ static int queue_group_reps(muse_batch *b, const RunArgs &a, bool shard, KeyCols
 #define MUSE_EXACT_UB 32768
 static int run_fused_overflow(muse_batch *b, int64_t n_exact, bool refill);
 
-// The run's statistics from its counters (d_counters, read back to the host): a fused run's [2] is its exact list and [3]
-// its refined count; any other run re-scores [2] + [3] (screened runs: pilot + second round).
-static void settle_counters(muse_batch *b, const unsigned long long *h_n) {
+// The run's statistics from its counters (d_counters, read back to the host): a fused run's `listed` is its exact list and
+// `refined` its refined count; any other run re-scores listed + refined (screened runs: pilot + second round).
+static void settle_counters(muse_batch *b, const RunCounters &c) {
     if (b->fused_run) {
-        b->timing.n_rescored = (int64_t)h_n[2];
-        b->timing.n_refined = (int64_t)h_n[3];
+        b->timing.n_rescored = (int64_t)c.listed;
+        b->timing.n_refined = (int64_t)c.refined;
     } else {
-        b->timing.n_rescored = (int64_t)(h_n[2] + h_n[3]);
+        b->timing.n_rescored = (int64_t)(c.listed + c.refined);
     }
 }
 
@@ -1315,28 +1338,26 @@ static int run_select(muse_batch *b, const RunArgs &a, int apply_filter, int64_t
         int rc = queue_group_reps(b, a, false, kc, gt);
         if (rc) return rc;
     }
-    CU(cudaMemsetAsync(b->d_counters, 0, sizeof(unsigned long long) * 2, st));
+    CU(cudaMemsetAsync(b->d_counters, 0, sizeof(unsigned long long) * 2, st));      // cand, selected
     FilterArgs f{a.max_lag, a.threshold, a.sign_filter, apply_filter};
-    Cand cand{b->d_ckey, b->d_cidx, b->d_clag, b->d_counters};
+    Cand cand{b->d_ckey, b->d_cidx, b->d_clag, &b->d_counters->cand};
     emit_candidates_kernel<<<blocks, 256, 0, st>>>(gt, grouped ? b->d_slot.get() : nullptr, b->d_score, b->d_lag, S, f, cand);
     b->timing.n_launches++;
     CU(cudaGetLastError());
     // one round trip: the count and the first CH records together (pinned mailbox)
-    const size_t CH = std::min<size_t>((size_t)S, 32768);
-    unsigned long long *h_n = reinterpret_cast<unsigned long long *>(b->h_pin.get());
-    unsigned long long *h_key = reinterpret_cast<unsigned long long *>(b->h_pin + 64);
-    int32_t *h_idx = reinterpret_cast<int32_t *>(b->h_pin + 64 + CH * 8);
-    int32_t *h_lag = reinterpret_cast<int32_t *>(b->h_pin + 64 + CH * 12);
-    CU(cudaMemcpyAsync(h_n, b->d_counters, sizeof(unsigned long long) * 4, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(h_key, b->d_ckey, sizeof(unsigned long long) * CH, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(h_idx, b->d_cidx, sizeof(int32_t) * CH, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(h_lag, b->d_clag, sizeof(int32_t) * CH, cudaMemcpyDeviceToHost, st));
+    const size_t CH = std::min<size_t>((size_t)S, MUSE_SELECT_CHUNK);
+    const RunCounters &h_n = b->h_pin->counters;
+    auto &h_cand = b->h_pin->cand;
+    CU(cudaMemcpyAsync(&b->h_pin->counters, b->d_counters, sizeof(RunCounters), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_cand.key, b->d_ckey, sizeof(unsigned long long) * CH, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_cand.idx, b->d_cidx, sizeof(int32_t) * CH, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_cand.lagsgn, b->d_clag, sizeof(int32_t) * CH, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
-    unsigned long long ncand = h_n[0];
+    unsigned long long ncand = h_n.cand;
     settle_counters(b, h_n);
-    if (b->fused_run == 1 && (int64_t)h_n[2] > std::min<int64_t>(S, MUSE_EXACT_UB)) {
+    if (b->fused_run == 1 && (int64_t)h_n.listed > std::min<int64_t>(S, MUSE_EXACT_UB)) {
         // rare: more exact candidates than the fixed launch covered -> finish them and select again
-        const int64_t n_exact = (int64_t)h_n[2];
+        const int64_t n_exact = (int64_t)h_n.listed;
         int rc = run_fused_overflow(b, n_exact, false);
         if (rc) return rc;
         b->fused_run = 0;
@@ -1345,10 +1366,10 @@ static int run_select(muse_batch *b, const RunArgs &a, int apply_filter, int64_t
         return rc;
     }
     if (ncand == 0) return MUSE_OK;
-    auto better = [](const Rec &x, const Rec &y) { return x.key != y.key ? x.key > y.key : x.idx < y.idx; };
+    auto better = [](const Rec &x, const Rec &y) { return key_precedes(x.key, x.idx, y.key, y.idx); };
     if (ncand <= CH) {
         recs.resize((size_t)ncand);
-        for (size_t i = 0; i < (size_t)ncand; i++) recs[i] = Rec{h_key[i], h_idx[i], h_lag[i]};
+        for (size_t i = 0; i < (size_t)ncand; i++) recs[i] = Rec{h_cand.key[i], h_cand.idx[i], h_cand.lagsgn[i]};
     } else {
         const unsigned long long *src_key = b->d_ckey;
         const int32_t *src_idx = b->d_cidx, *src_lag = b->d_clag;
@@ -1362,10 +1383,10 @@ static int run_select(muse_batch *b, const RunArgs &a, int apply_filter, int64_t
             const unsigned sblocks = (unsigned)((ncand + 1023ull) / 1024ull);
             for (int r = 0; r < 6; r++) select_round_kernel<<<sblocks, 1024, 0, st>>>(b->d_sel, b->d_ckey, b->d_cidx, ncand, r);
             select_gather_kernel<<<sblocks, 1024, 0, st>>>(b->d_sel, b->d_ckey, b->d_cidx, ncand, b->d_clag, b->d_skey, b->d_sidx,
-                                                           b->d_slag, b->d_counters + 1);
+                                                           b->d_slag, &b->d_counters->selected);
             b->timing.n_launches += 7;
             CU(cudaGetLastError());
-            CU(cudaMemcpyAsync(&nsel, b->d_counters + 1, sizeof(nsel), cudaMemcpyDeviceToHost, st));
+            CU(cudaMemcpyAsync(&nsel, &b->d_counters->selected, sizeof(nsel), cudaMemcpyDeviceToHost, st));
             CU(cudaStreamSynchronize(st));
             src_key = b->d_skey;
             src_idx = b->d_sidx;
@@ -1430,24 +1451,30 @@ static ScreenParams screen_params(muse_batch *b) {
     sp.twi = b->twi_f;
     sp.x_mid = b->x_mid;
     sp.row_stat = b->g->row_stat;
-    sp.cut_bits = b->d_cut;
-    sp.n_refined = reinterpret_cast<unsigned long long *>(b->d_cut + 2);
-    sp.next_claim = b->d_cut + 1;
-    sp.cut_hist = b->d_cut + 4;
+    sp.cut_bits = &b->d_cut->bits;
+    sp.n_refined = &b->d_cut->refined;
+    sp.next_claim = &b->d_cut->claims;
+    sp.cut_hist = b->d_cut->hist;
     sp.top_n = 1;
     return sp;
 }
 
 // Arms the fused refinement of the warp kernel: running cut-off = cut0 (+inf: bounds only),
 // counters (series claims, n_refined) and histogram cleared, lag window in the kernel's rotated cc index.
-__device__ __forceinline__ void init_cut_body(unsigned *state, float cut0) {
+#define MUSE_INIT_CUT_BLOCKS ((MUSE_CUT_WORDS + 255) / 256)
+__device__ __forceinline__ void init_cut_body(CutState *state, float cut0) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < 4 + MUSE_CUT_WORDS) state[i] = (i == 0) ? __float_as_uint(cut0) : 0u;
+    if (i == 0) {
+        state->bits = __float_as_uint(cut0);
+        state->claims = 0u;
+        state->refined = 0ull;
+    }
+    if (i < MUSE_CUT_WORDS) state->hist[i] = 0u;
 }
-__global__ void init_cut_kernel(unsigned *state, float cut0) { init_cut_body(state, cut0); }
+__global__ void init_cut_kernel(CutState *state, float cut0) { init_cut_body(state, cut0); }
 
 // the same for the queries of a multi-query launch: blockIdx.y = query
-__global__ void init_cut_batch_kernel(unsigned *const *__restrict__ states, float cut0) { init_cut_body(states[blockIdx.y], cut0); }
+__global__ void init_cut_batch_kernel(CutState *const *__restrict__ states, float cut0) { init_cut_body(states[blockIdx.y], cut0); }
 
 // skip_init: the cut-off state is armed by init_cut_batch_kernel for all the queries of a launch at once
 static int arm_refinement(muse_batch *b, ScreenParams &sp, float cut0, int64_t max_lag, int64_t top_n, double threshold, bool skip_init = false) {
@@ -1456,7 +1483,7 @@ static int arm_refinement(muse_batch *b, ScreenParams &sp, float cut0, int64_t m
     if (rc) return rc;
     sp.row_stat = b->g->row_stat;
     if (!skip_init) {
-        init_cut_kernel<<<(4 + MUSE_CUT_WORDS + 255) / 256, 256, 0, bstream(b)>>>(b->d_cut, cut0);
+        init_cut_kernel<<<MUSE_INIT_CUT_BLOCKS, 256, 0, bstream(b)>>>(b->d_cut, cut0);
         CU(cudaGetLastError());
     }
     const int64_t n = b->n, pad = n - b->N;
@@ -1475,36 +1502,28 @@ static int arm_refinement(muse_batch *b, ScreenParams &sp, float cut0, int64_t m
     return MUSE_OK;
 }
 
-// idx list of every series whose (refined) bound reaches the final cut-off, read from device memory
-// (n = counters + 2: the list length, then the refined count, which rides along)
-__device__ __forceinline__ void survivors_cut_body(const float *__restrict__ U, int64_t S, const unsigned *__restrict__ cut_bits,
-                                                   int32_t *__restrict__ out, unsigned long long *n) {
+// idx list of every series whose (refined) bound reaches the final cut-off, read from device memory, into n->listed (the
+// refined count rides along)
+__device__ __forceinline__ void survivors_cut_body(const float *__restrict__ U, int64_t S, const CutState *__restrict__ cut,
+                                                   int32_t *__restrict__ out, RunCounters *n) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i == 0) n[1] = *reinterpret_cast<const unsigned long long *>(cut_bits + 2);
-    const float lo = __uint_as_float(*cut_bits);
-    const bool take = i < S && U[i] >= lo;
-    const unsigned mask = __ballot_sync(0xffffffffu, take);
-    if (mask == 0u) return;
-    const int lane = threadIdx.x & 31, leader = __ffs(mask) - 1;
-    unsigned long long base = 0;
-    if (lane == leader) base = atomicAdd(n, (unsigned long long)__popc(mask));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (take) out[base + __popc(mask & ((1u << lane) - 1u))] = (int32_t)i;
+    if (i == 0) n->refined = cut->refined;
+    const float lo = __uint_as_float(cut->bits);
+    warp_append(&n->listed, i < S && U[i] >= lo, [&](unsigned long long pos) { out[pos] = (int32_t)i; });
 }
-__global__ void survivors_cut_kernel(const float *__restrict__ U, int64_t S, const unsigned *__restrict__ cut_bits,
-                                     int32_t *__restrict__ out, unsigned long long *n) {
-    survivors_cut_body(U, S, cut_bits, out, n);
+__global__ void survivors_cut_kernel(const float *__restrict__ U, int64_t S, const CutState *__restrict__ cut,
+                                     int32_t *__restrict__ out, RunCounters *n) {
+    survivors_cut_body(U, S, cut, out, n);
 }
 
 // the batched tails of muse_multi_run: blockIdx.y = query (MultiTail, muse_select.cuh)
 __global__ void tail_reset_kernel(const MultiTail *__restrict__ tails, int nq) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
-    if (q < nq)
-        for (int i = 0; i < 4; i++) tails[q].counters[i] = 0ull;
+    if (q < nq) *tails[q].counters = RunCounters{0ull, 0ull, 0ull, 0ull};
 }
 __global__ void survivors_cut_batch_kernel(const MultiTail *__restrict__ tails, int64_t S) {
     const MultiTail t = tails[blockIdx.y];
-    survivors_cut_body(t.U, S, t.cut, t.list, t.counters + 2);
+    survivors_cut_body(t.U, S, t.cut, t.list, t.counters);
 }
 // reference preparation of a launch's queries: screen_tables_kernel with blockIdx.y = query; the 4 floats of every query
 // (std-zero flag, A[M/2], Xt[M/2]) land in ONE array for one copy to the host
@@ -1516,23 +1535,7 @@ struct TablesArgs {
 };
 __global__ void screen_tables_batch_kernel(const TablesArgs *__restrict__ args, int M, const float2 *__restrict__ swtw, float *__restrict__ mids) {
     const TablesArgs a = args[blockIdx.y];
-    const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k > M / 2) return;
-    float *mid = mids + 4 * blockIdx.y;
-    if (k == 0) mid[0] = __int_as_float(*a.std_zero);
-    const cd x = a.Xt[k], c = a.Xt[M - k];
-    if (k == M / 2) {
-        mid[1] = __double2float_ru(hypot(x.x, x.y) * 2.0);
-        mid[2] = (float)x.x;
-        mid[3] = (float)x.y;
-        return;
-    }
-    const float wa = __double2float_ru(hypot(x.x, x.y) * (k == 0 ? 1.0 : 2.0));
-    const float wc = __double2float_ru(hypot(c.x, c.y) * (k == 0 ? 1.0 : 2.0));
-    const float2 w = swtw[k];
-    a.sw[k] = make_float4(w.x, w.y, wa, wc);
-    a.sx[k] = make_float4((float)x.x, (float)x.y, (float)c.x, (float)c.y);
-    a.sb[k] = __double2float_ru(sqrt(2.0 * ((double)wa * (double)wa + (double)wc * (double)wc)) * (1.0 + 1e-15));
+    screen_tables_body(a.Xt, M, swtw, a.sw, a.sx, a.sb, mids + 4 * blockIdx.y, a.std_zero);
 }
 
 extern "C" int muse_batch_screen_bounds(muse_batch *b, int32_t refine, int64_t max_lag, float *upper, float *lower) {
@@ -1586,9 +1589,9 @@ static int score_fused(muse_batch *b, const RunArgs &a) {
     CU(cudaEventRecord(b->ev[1], st));
     if (!a.list_only) CU(cudaMemsetAsync(b->d_score, 0xff, sizeof(double) * (size_t)S, st));      // NaN = "cannot be in the result"
     const unsigned blocks = (unsigned)((S + 255) / 256);
-    survivors_cut_kernel<<<blocks, 256, 0, st>>>(b->d_U, S, b->d_cut, b->d_list, b->d_counters + 2);
+    survivors_cut_kernel<<<blocks, 256, 0, st>>>(b->d_U, S, b->d_cut, b->d_list, b->d_counters);
     b->timing.n_launches++;
-    rc = score_exact_all(b, b->signed_run, b->d_list, std::min<int64_t>(S, MUSE_EXACT_UB), b->d_counters + 2);
+    rc = score_exact_all(b, b->signed_run, b->d_list, std::min<int64_t>(S, MUSE_EXACT_UB), &b->d_counters->listed);
     if (rc) return rc;
     return MUSE_OK;
 }
@@ -1636,21 +1639,21 @@ static int score_fused_grouped(muse_batch *b, const RunArgs &a) {
     const unsigned *cut_bits = nullptr;
     if (running && a.group_cut && a.top_n > 0 && a.top_n < 0x7fffffff) {
         group_uncertain_kernel<<<blocks, 256, 0, st>>>(gt, b->d_U, b->d_W, S, b->d_slot);
-        group_cut_count_kernel<<<(unsigned)((gt.slots + 255) / 256), 256, 0, st>>>(gt, a.threshold, b->d_cut + 4);
-        group_cut_find_kernel<<<1, 32, 0, st>>>(b->d_cut + 4, (int)a.top_n, b->d_cut);
+        group_cut_count_kernel<<<(unsigned)((gt.slots + 255) / 256), 256, 0, st>>>(gt, a.threshold, b->d_cut->hist);
+        group_cut_find_kernel<<<1, 32, 0, st>>>(b->d_cut->hist, (int)a.top_n, &b->d_cut->bits);
         b->timing.n_launches += 3;
-        cut_bits = b->d_cut;
+        cut_bits = &b->d_cut->bits;
     }
-    group_contenders_kernel<<<blocks, 256, 0, st>>>(gt, b->d_U, S, b->d_slot, thr_lo, b->d_list, b->d_counters + 2, cut_bits);
+    group_contenders_kernel<<<blocks, 256, 0, st>>>(gt, b->d_U, S, b->d_slot, thr_lo, b->d_list, &b->d_counters->listed, cut_bits);
     b->timing.n_launches++;
     CU(cudaGetLastError());
-    unsigned long long *h_n = reinterpret_cast<unsigned long long *>(b->h_pin.get());
-    CU(cudaMemcpyAsync(h_n, b->d_counters + 2, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    unsigned long long *h_listed = &b->h_pin->counters.listed;
+    CU(cudaMemcpyAsync(h_listed, &b->d_counters->listed, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));                                 // one small round trip: the list length sizes the launch
-    const int64_t n_exact = (int64_t)h_n[0];
+    const int64_t n_exact = (int64_t)*h_listed;
     rc = score_exact_all(b, b->signed_run, b->d_list, n_exact);
     if (rc) return rc;
-    CU(cudaMemcpyAsync(b->d_counters + 3, b->d_cut + 2, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, st));
+    CU(cudaMemcpyAsync(&b->d_counters->refined, &b->d_cut->refined, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, st));
     return MUSE_OK;
 }
 
@@ -1676,7 +1679,7 @@ static int run_scores(muse_batch *b, const RunArgs &a) {
     b->signed_run = a.signed_scores ? 1 : 0;
     cudaStream_t st = bstream(b);
     CU(cudaEventRecord(b->ev[0], st));
-    CU(cudaMemsetAsync(b->d_counters, 0, sizeof(unsigned long long) * 4, st));
+    CU(cudaMemsetAsync(b->d_counters, 0, sizeof(RunCounters), st));
     // screening needs: a kernel for this FFT size, an ungrouped unsigned run, a sign filter that
     // unsigned scores can pass, and a store big enough to be worth two extra round trips
     // grouped runs are screened only by the fused kernels (the bound of a member says nothing about the
@@ -1733,7 +1736,7 @@ static int finish_timing(muse_batch *b) {
 static int finish_pending_timing(muse_batch *b) {
     CU(cudaEventSynchronize(b->ev[3]));
     read_timing_events(b);
-    settle_counters(b, reinterpret_cast<const unsigned long long *>(b->h_pin.get()));
+    settle_counters(b, b->h_pin->counters);
     b->timing_pending = 0;
     return MUSE_OK;
 }
@@ -1766,7 +1769,7 @@ static int queue_topn_records(muse_batch *b, const RunArgs &a, muse_partial *d_o
 // candidate list was too long for the device-side select, or the fused path's exact launch did not cover its list --
 // finish on the host path from the scores already on the device.
 static bool device_topn_applies(const muse_batch *b, const RunArgs &a) {
-    return a.n_key_cols == 0 && a.top_n > 0 && a.top_n <= 65536 && b->g->size > 0;
+    return a.n_key_cols == 0 && b->g->size > 0 && device_topn_fits(a.top_n, b->scratch_cap);
 }
 
 static int device_topn_queue(muse_batch *b, const RunArgs &a) {
@@ -1774,23 +1777,22 @@ static int device_topn_queue(muse_batch *b, const RunArgs &a) {
     int rc = queue_topn_records(b, a, d_rec, a.top_n);
     if (rc) return rc;
     cudaStream_t st = bstream(b);
-    CU(cudaMemcpyAsync(b->h_pin + 64, d_rec, sizeof(muse_partial) * (size_t)a.top_n, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(b->h_pin->recs, d_rec, sizeof(muse_partial) * (size_t)a.top_n, cudaMemcpyDeviceToHost, st));
     CU(cudaEventRecord(b->ev[3], st));
     return MUSE_OK;
 }
 
 static int device_topn_finish(muse_batch *b, const RunArgs &a, double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out) {
     const int64_t top_n = a.top_n;
-    const muse_partial *h_rec = reinterpret_cast<const muse_partial *>(b->h_pin + 64);
+    const muse_partial *h_rec = b->h_pin->recs;
     if (h_rec[0].flags != 2) {
         *n_out = records_out(h_rec, top_n, scores, lags, series_idx);
         return finish_pending_timing(b);
     }
     b->timing_pending = 0;
-    const unsigned long long *h_n = reinterpret_cast<const unsigned long long *>(b->h_pin.get());
     int rc;
     if (b->fused_run == 1) {
-        rc = run_fused_overflow(b, (int64_t)h_n[2], true);
+        rc = run_fused_overflow(b, (int64_t)b->h_pin->counters.listed, true);
         if (rc) return rc;
         b->fused_run = 0;
     }
@@ -1813,16 +1815,14 @@ extern "C" int muse_batch_run_ex(muse_batch *b, const int32_t *key_cols, int32_t
     RunArgs a{key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores};
     a.group_cut = 1;
     *n_out = 0;
+    rc = ensure_scratch(b);
+    if (rc) return rc;
     if (device_topn_applies(b, a)) {
         // ungrouped: filter and top-N on the device, ONE copy of top_n records to the host
-        rc = ensure_scratch(b);
+        rc = device_topn_queue(b, a);
         if (rc) return rc;
-        if (top_n * 4 <= b->scratch_cap) {
-            rc = device_topn_queue(b, a);
-            if (rc) return rc;
-            CU(cudaStreamSynchronize(bstream(b)));
-            return device_topn_finish(b, a, scores, lags, series_idx, n_out);
-        }
+        CU(cudaStreamSynchronize(bstream(b)));
+        return device_topn_finish(b, a, scores, lags, series_idx, n_out);
     }
     rc = run_scores(b, a);
     if (rc) return rc;
@@ -1856,18 +1856,18 @@ struct TopnLaunch {
     unsigned blocks;
 };
 
-// Queues the filter of an ungrouped run's exact scores into the candidate list (counters[0]).  counters[0..1] (candidates,
-// selected) are still zero: run_scores cleared all four and ungrouped scoring writes only [2..3].
+// Queues the filter of an ungrouped run's exact scores into the candidate list (counters.cand).  The candidate and selected
+// counts are still zero: run_scores cleared all four counters and ungrouped scoring writes only `listed` and `refined`.
 static TopnLaunch queue_candidates(muse_batch *b, const RunArgs &a) {
     const int64_t S = b->g->size;
     cudaStream_t st = bstream(b);
     if (S > 0) {
         FilterArgs f{a.max_lag, a.threshold, a.sign_filter, 1};
-        Cand cand{b->d_ckey, b->d_cidx, b->d_clag, b->d_counters};
+        Cand cand{b->d_ckey, b->d_cidx, b->d_clag, &b->d_counters->cand};
         if (b->fused_run == 1) {
             // only the listed series have scores: filter those (the list's length stays on the device)
             const int64_t lim = std::min<int64_t>(S, MUSE_EXACT_UB);
-            emit_listed_kernel<<<(unsigned)((lim + 255) / 256), 256, 0, st>>>(b->d_list, b->d_counters + 2, lim, b->d_score, b->d_lag, f, cand);
+            emit_listed_kernel<<<(unsigned)((lim + 255) / 256), 256, 0, st>>>(b->d_list, &b->d_counters->listed, lim, b->d_score, b->d_lag, f, cand);
         } else {
             GroupTable gt;
             memset(&gt, 0, sizeof(gt));
@@ -1901,7 +1901,7 @@ static int queue_topn_records(muse_batch *b, const RunArgs &a_in, muse_partial *
     b->timing.n_launches++;
     CU(cudaGetLastError());
     // statistics and the end-of-run event are picked up by muse_batch_last_timing
-    CU(cudaMemcpyAsync(b->h_pin, b->d_counters, sizeof(unsigned long long) * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&b->h_pin->counters, b->d_counters, sizeof(RunCounters), cudaMemcpyDeviceToHost, st));
     CU(cudaEventRecord(b->ev[3], st));
     b->timing_pending = 1;
     return MUSE_OK;
@@ -1995,30 +1995,22 @@ extern "C" int muse_merge_partials(const muse_partial *parts, int64_t n_parts, i
     if (top_n < 0) top_n = 0;
     if (top_n > 0 && (!scores || !lags || !series_idx)) return fail(MUSE_ERR_INVALID_ARG, "muse_merge_partials: NULL output");
     // group max across shards first (muse_batch.go:87-89), ties -> lowest global series index
-    std::unordered_map<uint64_t, muse_partial> best;
+    const PartialRec *recs = reinterpret_cast<const PartialRec *>(parts);
+    std::unordered_map<uint64_t, PartialRec> best;
     best.reserve((size_t)n_parts * 2 + 1);
     for (int64_t i = 0; i < n_parts; i++) {
-        const muse_partial &p = parts[i];
+        const PartialRec &p = recs[i];
         if ((p.flags & 1) || p.score != p.score) continue;
         auto it = best.find(p.group_key);
         if (it == best.end()) best.emplace(p.group_key, p);
-        else {
-            muse_partial &q = it->second;
-            if (fabs(p.score) > fabs(q.score) || (fabs(p.score) == fabs(q.score) && p.series_idx < q.series_idx)) q = p;
-        }
+        else if (rec_precedes(p, it->second)) it->second = p;
     }
-    std::vector<muse_partial> v;
+    const FilterArgs f{max_lag, threshold, sign_filter, 1};
+    std::vector<PartialRec> v;
     v.reserve(best.size());
-    for (auto &kv : best) {
-        const muse_partial &p = kv.second;
-        const int64_t al = p.lag < 0 ? -(int64_t)p.lag : (int64_t)p.lag;   // results.go:46-52
-        const bool ok = al <= max_lag && fabs(p.score) >= threshold &&
-                        (sign_filter == 0 || (p.score > 0 && sign_filter == 1) || (p.score < 0 && sign_filter == -1));
-        if (ok) v.push_back(p);
-    }
-    auto better = [](const muse_partial &x, const muse_partial &y) {
-        return fabs(x.score) != fabs(y.score) ? fabs(x.score) > fabs(y.score) : x.series_idx < y.series_idx;
-    };
+    for (auto &kv : best)
+        if (passed(f, kv.second.score, kv.second.lag)) v.push_back(kv.second);
+    auto better = [](const PartialRec &x, const PartialRec &y) { return rec_precedes(x, y); };
     if ((int64_t)v.size() > top_n) {
         std::nth_element(v.begin(), v.begin() + top_n, v.end(), better);
         v.resize((size_t)top_n);
@@ -2105,12 +2097,12 @@ struct MultiTables {
     static constexpr int Q = MUSE_MULTI_GROUP;
     static size_t off_ep() { return 0; }                                                  // ExactParams[Q]: reference spectra
     static size_t off_ta() { return off_ep() + sizeof(ExactParams) * Q; }                 // TablesArgs[Q]
-    static size_t off_cut() { return off_ta() + sizeof(TablesArgs) * Q; }                 // unsigned*[Q]: cut-off states
+    static size_t off_cut() { return off_ta() + sizeof(TablesArgs) * Q; }                 // CutState*[Q]: cut-off states
     static size_t off_tail() { return off_cut() + sizeof(void *) * Q; }                   // MultiTail[Q]
     static size_t off_ep2() { return off_tail() + sizeof(MultiTail) * Q; }                // ExactParams[Q]: fp64 re-scoring
     static size_t off_mids() { return off_ep2() + sizeof(ExactParams) * Q; }              // float[Q][4]
-    static size_t off_cnt() { return off_mids() + sizeof(float) * 4 * Q; }                // u64[Q][4]
-    static size_t off_recs() { return (off_cnt() + sizeof(unsigned long long) * 4 * Q + 255) / 256 * 256; }      // PartialRec[Q][top_n]
+    static size_t off_cnt() { return off_mids() + sizeof(float) * 4 * Q; }                // RunCounters[Q]
+    static size_t off_recs() { return (off_cnt() + sizeof(RunCounters) * Q + 255) / 256 * 256; }      // PartialRec[Q][top_n]
     static size_t bytes(int64_t top_n) { return off_recs() + sizeof(PartialRec) * (size_t)Q * (size_t)std::max<int64_t>(top_n, 1); }
 };
 
@@ -2137,7 +2129,7 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
     // ---- reference preparation: one launch per stage ----
     ExactParams *h_ep = reinterpret_cast<ExactParams *>(h + MT::off_ep());
     TablesArgs *h_ta = reinterpret_cast<TablesArgs *>(h + MT::off_ta());
-    unsigned **h_cut = reinterpret_cast<unsigned **>(h + MT::off_cut());
+    CutState **h_cut = reinterpret_cast<CutState **>(h + MT::off_cut());
     for (int i = 0; i < nq; i++) {
         rc = batch_alloc(ctx, g, ref_len, bs[(size_t)i]);
         if (rc == MUSE_OK) rc = ensure_scratch(bs[(size_t)i].get());
@@ -2162,8 +2154,7 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
     CU(launch_exact_batch(MODE_REF, reinterpret_cast<const ExactParams *>(d + MT::off_ep()), nq, 1, st));
     screen_tables_batch_kernel<<<dim3((unsigned)((M / 2 + 1 + 255) / 256), (unsigned)nq), 256, 0, st>>>(
         reinterpret_cast<const TablesArgs *>(d + MT::off_ta()), (int)M, bs[0]->swtw, reinterpret_cast<float *>(d + MT::off_mids()));
-    init_cut_batch_kernel<<<dim3((4 + MUSE_CUT_WORDS + 255) / 256, (unsigned)nq), 256, 0, st>>>(
-        reinterpret_cast<unsigned *const *>(d + MT::off_cut()), thr_lo);
+    init_cut_batch_kernel<<<dim3(MUSE_INIT_CUT_BLOCKS, (unsigned)nq), 256, 0, st>>>(reinterpret_cast<CutState *const *>(d + MT::off_cut()), thr_lo);
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(h + MT::off_mids(), d + MT::off_mids(), sizeof(float) * 4 * (size_t)nq, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
@@ -2217,19 +2208,19 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
     // ---- tails: survivors -> fp64 re-scoring -> filter -> top-N, one launch each ----
     MultiTail *h_tail = reinterpret_cast<MultiTail *>(h + MT::off_tail());
     ExactParams *h_ep2 = reinterpret_cast<ExactParams *>(h + MT::off_ep2());
-    unsigned long long *d_cnt = reinterpret_cast<unsigned long long *>(d + MT::off_cnt());
+    RunCounters *d_cnt = reinterpret_cast<RunCounters *>(d + MT::off_cnt());
     PartialRec *d_recs = reinterpret_cast<PartialRec *>(d + MT::off_recs());
     const int64_t lim = std::min<int64_t>(S, MUSE_EXACT_UB);
     for (int k = 0; k < nl; k++) {
         muse_batch *b = lb[(size_t)k];
-        h_tail[k] = MultiTail{b->d_U, b->d_cut, b->d_list, d_cnt + 4 * k, b->d_score, b->d_lag, b->d_ckey, b->d_cidx, b->d_clag,
+        h_tail[k] = MultiTail{b->d_U, b->d_cut, b->d_list, d_cnt + k, b->d_score, b->d_lag, b->d_ckey, b->d_cidx, b->d_clag,
                               d_recs + (size_t)k * (size_t)top_n};
         ExactParams &p = h_ep2[k];
         memset(&p, 0, sizeof(p));
         p.slab = g->slab;
         p.ld = g->ld;
         p.count = lim;
-        p.count_ptr = d_cnt + 4 * k + 2;
+        p.count_ptr = &d_cnt[k].listed;
         p.idx = b->d_list;
         p.N = (int)ref_len;
         p.Xt = b->Xt;
@@ -2243,11 +2234,11 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
     tail_reset_kernel<<<(nl + 255) / 256, 256, 0, st>>>(d_tail, nl);
     survivors_cut_batch_kernel<<<dim3((unsigned)((S + 255) / 256), (unsigned)nl), 256, 0, st>>>(d_tail, S);
     CU(cudaGetLastError());
-    unsigned long long *h_cnt = reinterpret_cast<unsigned long long *>(h + MT::off_cnt());
-    CU(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(unsigned long long) * 4 * (size_t)nl, cudaMemcpyDeviceToHost, st));
+    RunCounters *h_cnt = reinterpret_cast<RunCounters *>(h + MT::off_cnt());
+    CU(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(RunCounters) * (size_t)nl, cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));      // the list lengths size the next launches
     int64_t max_len = 0;
-    for (int k = 0; k < nl; k++) max_len = std::max<int64_t>(max_len, std::min<int64_t>((int64_t)h_cnt[4 * k + 2], lim));
+    for (int k = 0; k < nl; k++) max_len = std::max<int64_t>(max_len, std::min<int64_t>((int64_t)h_cnt[k].listed, lim));
     if (max_len > 0) {
         CU(launch_exact_batch(MODE_SCORE, reinterpret_cast<const ExactParams *>(d + MT::off_ep2()), nl, max_len, st));
         FilterArgs f{max_lag, threshold, sign_filter, 1};
@@ -2256,7 +2247,7 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
     partial_topn_batch_kernel<<<dim3(16, (unsigned)nl), 256, 0, st>>>(d_tail, (long long)top_n, (long long)g->global_offset, (long long)lim);
     CU(cudaGetLastError());
     CU(cudaMemcpyAsync(h + MT::off_recs(), d_recs, sizeof(PartialRec) * (size_t)nl * (size_t)top_n, cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(unsigned long long) * 4 * (size_t)nl, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(RunCounters) * (size_t)nl, cudaMemcpyDeviceToHost, st));
     CU(cudaEventRecord(ctx->mt_ev[4], st));
     CU(cudaStreamSynchronize(st));
     const muse_partial *h_recs = reinterpret_cast<const muse_partial *>(h + MT::off_recs());
@@ -2265,8 +2256,8 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
         const muse_partial *r = h_recs + (size_t)k * (size_t)top_n;
         double *sc = scores + (size_t)i * (size_t)top_n;
         int64_t *lg = lags + (size_t)i * (size_t)top_n, *ix = series_idx + (size_t)i * (size_t)top_n;
-        ctx->multi_rescored += (int64_t)h_cnt[4 * k + 2];
-        ctx->multi_refined += (int64_t)h_cnt[4 * k + 3];
+        ctx->multi_rescored += (int64_t)h_cnt[k].listed;
+        ctx->multi_refined += (int64_t)h_cnt[k].refined;
         if (r[0].flags == 2) {
             // the list did not fit the device-side select (or the re-scoring launch): this query finishes alone, from its
             // bounds and cut-off on the device (the fused run skips the screening of a prescreened batch)
@@ -2337,8 +2328,8 @@ extern "C" int muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, 
     // NewBatch + Run per reference on the resident store: the store, its row statistics and the run scratch (context
     // pool) are shared, and results of query q land in row q of the outputs
     const bool one_pass = n_key_cols == 0 && mode != MUSE_MODE_EXACT && sign_filter != MUSE_SIGN_NEG && ref_len == g->N &&
-                          next_pow2(ref_len) == 2048 && top_n > 0 && top_n <= 65536 &&
-                          top_n * 4 <= g->size && (g->size >= 16384 || mode == MUSE_MODE_SCREEN) && n_refs > 1;
+                          next_pow2(ref_len) == 2048 && device_topn_fits(top_n, g->size) &&
+                          (g->size >= 16384 || mode == MUSE_MODE_SCREEN) && n_refs > 1;
     ctx->multi_refined = ctx->multi_rescored = 0;
     const int QC = one_pass ? MUSE_MULTI_GROUP : MUSE_MULTI_SEPARATE;
     for (int64_t q0 = 0; q0 < n_refs; q0 += QC) {
@@ -2649,7 +2640,7 @@ extern "C" int muse_batch_run_exchange_ex(muse_batch *b, muse_exchange *x, const
     int *h_status = reinterpret_cast<int *>(x->h_recs + (size_t)x->capacity * sizeof(muse_partial));
     if (top_n > 0) CU(cudaMemcpyAsync(x->h_recs, x->d_out, sizeof(muse_partial) * (size_t)top_n, cudaMemcpyDeviceToHost, st));
     CU(cudaMemcpyAsync(h_status, x->d_status, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CU(cudaMemcpyAsync(b->h_pin, b->d_counters, sizeof(unsigned long long) * 4, cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&b->h_pin->counters, b->d_counters, sizeof(RunCounters), cudaMemcpyDeviceToHost, st));
     CU(cudaEventRecord(b->ev[3], st));
     b->timing_pending = 1;
     CU(cudaStreamSynchronize(st));

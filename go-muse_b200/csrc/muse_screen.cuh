@@ -59,6 +59,14 @@ typedef cx<float> cf;
 #define MUSE_CUT_BINS 262144
 #define MUSE_CUT_WORDS (64 + 64 * 64 + MUSE_CUT_BINS)
 
+// The running cut-off of a run (of one query of a multi-query run), armed by init_cut_kernel / init_cut_batch_kernel.
+struct CutState {
+    unsigned bits;                    // running lower bound on the final top-N cut-off (float bits, only ever raised)
+    unsigned claims;                  // warp kernel: claims of series handed out so far
+    unsigned long long refined;       // series that took the fused second stage
+    unsigned hist[MUSE_CUT_WORDS];    // 64 coarse, 64*64 middle, 64^3 fine counts of lower bounds
+};
+
 // Per-row statistics of the store, computed once per appended row (the batched mean/std kernel of the
 // z-normalisation, xcorr.go:84-95): the fp64 mean, and 1/std in fp32 -- or NaN when no fp32 statement may be
 // made about the row (constant row, variance outside [MUSE_SCREEN_VAR_MIN, MUSE_SCREEN_VAR_MAX], non-finite
@@ -221,16 +229,20 @@ __device__ __forceinline__ int cut_level(const unsigned *cnt, int t, unsigned &n
 
 // cut_bits / cut_hist / top_n: the cut-off state of ScreenParams, or of one query of a multi-query run.  Arguments that
 // are kernel parameters are taken by reference here and in the blocks below, so that they are read where they are used.
-__device__ __forceinline__ void cut_count_and_raise(unsigned *const &cut_bits, unsigned *const &cut_hist, const int &top_n, float L, int t) {
+// Counts the lower bound L in the three levels of the histogram.
+__device__ __forceinline__ void cut_hist_add(unsigned *const &cut_hist, float L) {
     int bin = (int)(L * (float)MUSE_CUT_BINS);
     bin = bin < 0 ? 0 : (bin >= MUSE_CUT_BINS ? MUSE_CUT_BINS - 1 : bin);
     unsigned *coarse = cut_hist, *mid = coarse + 64, *fine = mid + 64 * 64;
-    if (t == 0) {
-        atomicAdd(&fine[bin], 1u);
-        atomicAdd(&mid[bin >> 6], 1u);
-        atomicAdd(&coarse[bin >> 12], 1u);
-    }
-    __syncwarp();
+    atomicAdd(&fine[bin], 1u);
+    atomicAdd(&mid[bin >> 6], 1u);
+    atomicAdd(&coarse[bin >> 12], 1u);
+}
+
+// Warp-collective: raises the cut-off to the lower edge of the bin that holds the top_n-th largest count (nothing when
+// fewer were counted).
+__device__ __forceinline__ void cut_walk(unsigned *const &cut_bits, const unsigned *const &cut_hist, const int &top_n, int t) {
+    const unsigned *coarse = cut_hist, *mid = coarse + 64, *fine = mid + 64 * 64;
     unsigned need = (unsigned)top_n;
     const int c = cut_level(coarse, t, need);
     if (c < 0) return;
@@ -239,6 +251,12 @@ __device__ __forceinline__ void cut_count_and_raise(unsigned *const &cut_bits, u
     const int f = cut_level(fine + (c * 64 + m) * 64, t, need);
     if (f < 0) return;
     if (t == 0) atomicMax(cut_bits, __float_as_uint((float)((c * 64 + m) * 64 + f) / (float)MUSE_CUT_BINS));
+}
+
+__device__ __forceinline__ void cut_count_and_raise(unsigned *const &cut_bits, unsigned *const &cut_hist, const int &top_n, float L, int t) {
+    if (t == 0) cut_hist_add(cut_hist, L);
+    __syncwarp();
+    cut_walk(cut_bits, cut_hist, top_n, t);
 }
 
 // Refined decision for one series from the fp32 maxima of |cc| inside / outside the lag window

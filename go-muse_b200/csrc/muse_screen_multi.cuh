@@ -17,7 +17,7 @@ struct MultiQuery {
     cf x_mid;             // Xt[M/2]
     float a_mid;          // A[M/2]
     int pad;
-    unsigned *cut;        // the query's cut-off state: [0] running cut-off bits, [2..3] refined count, [4..] histogram
+    CutState *cut;        // the query's cut-off state
     float *out_U;         // [count] upper bound on the score for this query
 };
 
@@ -79,7 +79,7 @@ refine_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queri
     const cd *rowc = reinterpret_cast<const cd *>(buf);
     cf *stash = reinterpret_cast<cf *>(buf);                                  // slot j of lane t at [32 j + t]
     cf *ex = reinterpret_cast<cf *>(buf + C::STASH_BYTES);                    // this warp's FFT exchange buffer
-    unsigned **s_cut = reinterpret_cast<unsigned **>(smem_raw + (size_t)nwarps * warp_bytes);      // [QMAX] cut-off words
+    CutState **s_cut = reinterpret_cast<CutState **>(smem_raw + (size_t)nwarps * warp_bytes);      // [QMAX] cut-off states
     float **s_out = reinterpret_cast<float **>(s_cut + C::QMAX);                                   // [QMAX] bound arrays
     cf *s_tw = reinterpret_cast<cf *>(s_out + C::QMAX);                                            // pass twiddles W_1024^(j t)
     cf *s_sw = reinterpret_cast<cf *>(reinterpret_cast<unsigned char *>(s_tw) + C::TW_BYTES);      // split twiddles exp(-2 pi i k / n)
@@ -119,7 +119,7 @@ refine_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queri
             cutr[i] = 0x7f800000u;          // +inf: no such query
             if (i < nqi && t + 32 * i < nq) {
                 U[i] = s_out[t + 32 * i][pos];
-                cutr[i] = ld_relaxed_u32(s_cut[t + 32 * i]);
+                cutr[i] = ld_relaxed_u32(&s_cut[t + 32 * i]->bits);
             }
         }
         const RowStat rs = prm.row_stat[pos];
@@ -187,8 +187,8 @@ refine_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queri
                 window_maxima<32>(u, t, prm.win_lo, prm.win_len, m_in, m_out);
                 float L = -1.f;
                 Uq = refine_decide(Uq, m_in * rs.rstd, m_out * rs.rstd, L, 0);
-                if (t == 0) atomicAdd(reinterpret_cast<unsigned long long *>(mq.cut + 2), 1ull);
-                if (L >= prm.thr && L >= cut_now) cut_count_and_raise(mq.cut, mq.cut + 4, prm.top_n, L, t);
+                if (t == 0) atomicAdd(&mq.cut->refined, 1ull);
+                if (L >= prm.thr && L >= cut_now) cut_count_and_raise(&mq.cut->bits, mq.cut->hist, prm.top_n, L, t);
 #pragma unroll
                 for (int i = 0; i < QI; i++)
                     if (i == gi && t == ql) {

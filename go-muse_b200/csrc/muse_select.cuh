@@ -10,6 +10,9 @@
 #pragma once
 
 #include <stdint.h>
+#include <string.h>
+
+#include <type_traits>
 
 #if defined(__CUDACC__)
 #include <cuda_runtime.h>
@@ -53,25 +56,43 @@ struct GroupTable {
     int64_t radix[MUSE_MAX_KEY_COLS];   // dense: cardinality (max id + 2) per column
 };
 
+// slot of `key` (!= 0) in an open-addressing table of `slots` (a power of two) keys, 0 = empty: the slot that holds it,
+// or the empty slot it claims
+__device__ __forceinline__ long long hash_slot(unsigned long long *hkeys, long long slots, unsigned long long key) {
+    unsigned long long h = key * 0x9E3779B97F4A7C15ull;
+    h ^= h >> 32;
+    long long s = (long long)(h & (unsigned long long)(slots - 1));
+    for (;;) {
+        const unsigned long long cur = hkeys[s];
+        if (cur == key) return s;
+        if (cur == 0ull) {
+            const unsigned long long old = atomicCAS(&hkeys[s], 0ull, key);
+            if (old == 0ull || old == key) return s;
+        }
+        s = (s + 1) & (slots - 1);
+    }
+}
+
 __device__ __forceinline__ int64_t table_slot(const GroupTable &gt, const KeyCols &kc, int64_t i) {
     if (gt.dense) {
         int64_t s = 0;
         for (int c = 0; c < kc.ncols; c++) s = s * gt.radix[c] + (int64_t)(kc.col[c][i] + 1);
         return s;
     }
-    const unsigned long long key = canonical_key(kc, i) + 1ull;
-    unsigned long long h = key * 0x9E3779B97F4A7C15ull;
-    h ^= h >> 32;
-    int64_t s = (int64_t)(h & (unsigned long long)(gt.slots - 1));
-    for (;;) {
-        const unsigned long long cur = gt.hkeys[s];
-        if (cur == key) return s;
-        if (cur == 0ull) {
-            const unsigned long long old = atomicCAS(&gt.hkeys[s], 0ull, key);
-            if (old == 0ull || old == key) return s;
-        }
-        s = (s + 1) & (gt.slots - 1);
-    }
+    return hash_slot(gt.hkeys, gt.slots, canonical_key(kc, i) + 1ull);
+}
+
+// Warp-aggregated append: every lane whose `take` is set gets its own position in a list whose length is *n, with one
+// atomic per warp, and calls store(position).  All 32 lanes of the warp call it.
+template <typename Store>
+__device__ __forceinline__ void warp_append(unsigned long long *n, bool take, Store store) {
+    const unsigned mask = __ballot_sync(0xffffffffu, take);
+    if (mask == 0u) return;
+    const int lane = threadIdx.x & 31, leader = __ffs(mask) - 1;
+    unsigned long long base = 0;
+    if (lane == leader) base = atomicAdd(n, (unsigned long long)__popc(mask));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (take) store(base + (unsigned long long)__popc(mask & ((1u << lane) - 1u)));
 }
 
 // pass 1: slot per series + atomicMax of |score| bits
@@ -122,13 +143,7 @@ __global__ void group_contenders_kernel(GroupTable gt, const float *__restrict__
         // results.go:46-48 whatever the exact scores are (flags of group_uncertain_kernel; only set in that mode)
         if (cut_bits && !((g >> 33) & 1ull)) take = false;
     }
-    const unsigned mask = __ballot_sync(0xffffffffu, take);
-    if (mask == 0u) return;
-    const int lane = threadIdx.x & 31, leader = __ffs(mask) - 1;
-    unsigned long long base = 0;
-    if (lane == leader) base = atomicAdd(n, (unsigned long long)__popc(mask));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (take) out[base + __popc(mask & ((1u << lane) - 1u))] = (int32_t)i;
+    warp_append(n, take, [&](unsigned long long pos) { out[pos] = (int32_t)i; });
 }
 
 // ---- a cut-off for grouped single-GPU runs -----------------------------------------------------------------------
@@ -153,32 +168,18 @@ __global__ void group_uncertain_kernel(GroupTable gt, const float *__restrict__ 
     }
 }
 // 2. count the certain groups' lower bounds in the three-level histogram of the running cut-off (muse_screen.cuh)
-__global__ void group_cut_count_kernel(GroupTable gt, double threshold, unsigned *__restrict__ hist) {
+__global__ void group_cut_count_kernel(GroupTable gt, double threshold, unsigned *hist) {
     const int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= gt.slots) return;
     const unsigned long long g = gt.gmax[s];
     if ((g >> 32) & 1ull) return;
     const float L = __uint_as_float((unsigned)g);
     if (!(L > 0.f) || (double)L < threshold) return;
-    int bin = (int)(L * (float)MUSE_CUT_BINS);
-    bin = bin < 0 ? 0 : (bin >= MUSE_CUT_BINS ? MUSE_CUT_BINS - 1 : bin);
-    unsigned *coarse = hist, *mid = coarse + 64, *fine = mid + 64 * 64;
-    atomicAdd(&fine[bin], 1u);
-    atomicAdd(&mid[bin >> 6], 1u);
-    atomicAdd(&coarse[bin >> 12], 1u);
+    cut_hist_add(hist, L);
 }
 // 3. one warp: the lower edge of the bin that holds the top_n-th largest counted bound (nothing when fewer were counted)
-__global__ void group_cut_find_kernel(const unsigned *__restrict__ hist, int top_n, unsigned *__restrict__ cut_bits) {
-    const int t = threadIdx.x;
-    const unsigned *coarse = hist, *mid = coarse + 64, *fine = mid + 64 * 64;
-    unsigned need = (unsigned)top_n;
-    const int c = cut_level(coarse, t, need);
-    if (c < 0) return;
-    const int m = cut_level(mid + c * 64, t, need);
-    if (m < 0) return;
-    const int f = cut_level(fine + (c * 64 + m) * 64, t, need);
-    if (f < 0) return;
-    if (t == 0) atomicMax(cut_bits, __float_as_uint((float)((c * 64 + m) * 64 + f) / (float)MUSE_CUT_BINS));
+__global__ void group_cut_find_kernel(const unsigned *hist, int top_n, unsigned *cut_bits) {
+    cut_walk(cut_bits, hist, top_n, threadIdx.x);
 }
 
 // pass 2: lowest series index among the members that hold the group max
@@ -199,12 +200,20 @@ struct FilterArgs {
     int apply;   // 0: emit every representative unfiltered (multi-GPU grouped partials)
 };
 
-__device__ __forceinline__ bool passed(const FilterArgs &f, double sc, int lag) {
+MUSE_HD bool passed(const FilterArgs &f, double sc, int lag) {
     // results.go:46-52
     const int64_t al = lag < 0 ? -(int64_t)lag : (int64_t)lag;
     return al <= f.max_lag && fabs(sc) >= f.threshold &&
            (f.sign_filter == 0 || (sc > 0.0 && f.sign_filter == 1) || (sc < 0.0 && f.sign_filter == -1));
 }
+
+// The counters of a run (d_counters, and one set per query of a multi-query launch).
+struct RunCounters {
+    unsigned long long cand;       // candidates (Cand::n)
+    unsigned long long selected;   // candidates the radix select gathered
+    unsigned long long listed;     // length of the exact list (fused runs) / series re-scored in the pilot round
+    unsigned long long refined;    // series that took the fused second stage / re-scored in the second round
+};
 
 // Candidate = a group representative that passed the filter.
 struct Cand {
@@ -213,6 +222,28 @@ struct Cand {
     int32_t *lagsgn;           // 2*lag + (score < 0)
     unsigned long long *n;     // counter
 };
+
+// score and lag of a candidate from its |score| bits and 2*lag + (score < 0)
+MUSE_HD double cand_score(unsigned long long key, int lagsgn) {
+    double a;
+    memcpy(&a, &key, sizeof(a));
+    return (lagsgn & 1) ? -a : a;
+}
+MUSE_HD int cand_lag(int lagsgn) { return (lagsgn - (lagsgn & 1)) / 2; }
+
+// candidate a precedes candidate b in (|score| desc, index asc) -- on |score| bits, which order like the non-negative scores
+template <typename Idx>
+MUSE_HD bool key_precedes(unsigned long long ka, Idx ia, unsigned long long kb, Idx ib) {
+    return ka > kb || (ka == kb && ia < ib);
+}
+
+__device__ __forceinline__ void emit_candidate(const Cand &out, bool emit, double sc, int32_t idx, const int32_t *__restrict__ lag) {
+    warp_append(out.n, emit, [&](unsigned long long pos) {
+        out.key[pos] = score_bits(sc);
+        out.idx[pos] = idx;
+        out.lagsgn[pos] = 2 * lag[idx] + (sc < 0.0 ? 1 : 0);
+    });
+}
 
 // Emit candidates.  slot_of == NULL: ungrouped (every series is its own representative).
 __global__ void emit_candidates_kernel(GroupTable gt, const int64_t *__restrict__ slot_of,
@@ -227,20 +258,7 @@ __global__ void emit_candidates_kernel(GroupTable gt, const int64_t *__restrict_
         if (emit && slot_of) emit = (gt.gidx[slot_of[i]] == (int32_t)i);
         if (emit && f.apply) emit = passed(f, sc, lag[i]);
     }
-    // warp-aggregated append
-    const unsigned mask = __ballot_sync(0xffffffffu, emit);
-    if (mask == 0u) return;
-    const int lane = threadIdx.x & 31;
-    const int leader = __ffs(mask) - 1;
-    unsigned long long base = 0;
-    if (lane == leader) base = atomicAdd(out.n, (unsigned long long)__popc(mask));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (emit) {
-        const unsigned long long pos = base + (unsigned long long)__popc(mask & ((1u << lane) - 1u));
-        out.key[pos] = score_bits(sc);
-        out.idx[pos] = (int32_t)i;
-        out.lagsgn[pos] = 2 * lag[i] + (sc < 0.0 ? 1 : 0);
-    }
+    emit_candidate(out, emit, sc, (int32_t)i, lag);
 }
 
 // Emit candidates from a LIST of series (the fused path's exact list): entry i < min(*n_list, limit) is a
@@ -258,19 +276,7 @@ __device__ __forceinline__ void emit_listed_body(const int32_t *__restrict__ lis
         sc = score[idx];
         emit = (sc == sc) && (!f.apply || passed(f, sc, lag[idx]));
     }
-    const unsigned mask = __ballot_sync(0xffffffffu, emit);
-    if (mask == 0u) return;
-    const int lane = threadIdx.x & 31;
-    const int leader = __ffs(mask) - 1;
-    unsigned long long base = 0;
-    if (lane == leader) base = atomicAdd(out.n, (unsigned long long)__popc(mask));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (emit) {
-        const unsigned long long pos = base + (unsigned long long)__popc(mask & ((1u << lane) - 1u));
-        out.key[pos] = score_bits(sc);
-        out.idx[pos] = idx;
-        out.lagsgn[pos] = 2 * lag[idx] + (sc < 0.0 ? 1 : 0);
-    }
+    emit_candidate(out, emit, sc, idx, lag);
 }
 
 __global__ void emit_listed_kernel(const int32_t *__restrict__ list, const unsigned long long *__restrict__ n_list,
@@ -282,9 +288,9 @@ __global__ void emit_listed_kernel(const int32_t *__restrict__ list, const unsig
 // Per-query pointers of the batched tails of muse_multi_run (one launch per stage, blockIdx.y = query).
 struct MultiTail {
     const float *U;                 // [S] the query's bounds after the second stages
-    const unsigned *cut;            // the query's cut-off state ([0] final cut-off bits, [2..3] refined count)
+    const CutState *cut;            // the query's cut-off state
     int32_t *list;                  // series whose bound reaches the cut-off
-    unsigned long long *counters;   // [0] candidates, [1] selected, [2] list length, [3] refined
+    RunCounters *counters;
     double *score;                  // [S] exact scores of the listed series
     int32_t *lag;
     unsigned long long *ckey;       // candidates
@@ -294,7 +300,7 @@ struct MultiTail {
 
 __global__ void emit_listed_batch_kernel(const MultiTail *__restrict__ tails, long long limit, FilterArgs f) {
     const MultiTail t = tails[blockIdx.y];
-    emit_listed_body(t.list, t.counters + 2, limit, t.score, t.lag, f, Cand{t.ckey, t.cidx, t.clag, t.counters});
+    emit_listed_body(t.list, &t.counters->listed, limit, t.score, t.lag, f, Cand{t.ckey, t.cidx, t.clag, &t.counters->cand});
 }
 
 // ---- device-side top-N of a short candidate list, written as muse_partial records ------
@@ -318,57 +324,75 @@ struct PartialRec {           // == muse_partial (include/muse_b200.h)
 // Position of candidate (k, ix) in the (|score| desc, index asc) order: the number of the n candidates that come before it,
 // counted by the calling warp.  Its lanes stride over the list, four independent loads in flight per lane (the list is 48 KB
 // at C3: L1/L2 resident, but one dependent load per step made this kernel 31 us).
-__device__ __forceinline__ unsigned rank_of(const unsigned long long *__restrict__ ckey, const int32_t *__restrict__ cidx, unsigned long long n,
-                                            unsigned long long k, unsigned ix, int lane) {
+template <typename Idx>
+__device__ __forceinline__ unsigned rank_of(const unsigned long long *__restrict__ ckey, const Idx *__restrict__ cidx, unsigned long long n,
+                                            unsigned long long k, typename std::make_unsigned<Idx>::type ix, int lane) {
+    using U = decltype(ix);      // indices compare unsigned: they are >= 0
     unsigned before = 0;
     unsigned long long j = lane;
     for (; j + 96 < n; j += 128) {
         const unsigned long long k0 = ckey[j], k1 = ckey[j + 32], k2 = ckey[j + 64], k3 = ckey[j + 96];
-        const unsigned i0 = (unsigned)cidx[j], i1 = (unsigned)cidx[j + 32], i2 = (unsigned)cidx[j + 64], i3 = (unsigned)cidx[j + 96];
-        before += (k0 > k || (k0 == k && i0 < ix)) ? 1u : 0u;
-        before += (k1 > k || (k1 == k && i1 < ix)) ? 1u : 0u;
-        before += (k2 > k || (k2 == k && i2 < ix)) ? 1u : 0u;
-        before += (k3 > k || (k3 == k && i3 < ix)) ? 1u : 0u;
+        const U i0 = (U)cidx[j], i1 = (U)cidx[j + 32], i2 = (U)cidx[j + 64], i3 = (U)cidx[j + 96];
+        before += key_precedes(k0, i0, k, ix) ? 1u : 0u;
+        before += key_precedes(k1, i1, k, ix) ? 1u : 0u;
+        before += key_precedes(k2, i2, k, ix) ? 1u : 0u;
+        before += key_precedes(k3, i3, k, ix) ? 1u : 0u;
     }
     for (; j < n; j += 32) {
         const unsigned long long kj = ckey[j];
-        before += (kj > k || (kj == k && (unsigned)cidx[j] < ix)) ? 1u : 0u;
+        before += (kj > k || (kj == k && (U)cidx[j] < ix)) ? 1u : 0u;      // the index is loaded only on a tie
     }
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) before += __shfl_xor_sync(0xffffffffu, before, off);
     return before;
 }
 
-__device__ __forceinline__ void partial_topn_body(const unsigned long long *__restrict__ ckey, const int32_t *__restrict__ cidx,
-                                                  const int32_t *__restrict__ clag, const unsigned long long *__restrict__ counters, long long top_n,
-                                                  long long global_offset, long long exact_list_bound, PartialRec *__restrict__ out, long long capacity) {
-    const unsigned long long n = counters[0];
-    const bool overflow = n > MUSE_PARTIAL_RANK_CAP || (exact_list_bound >= 0 && counters[2] > (unsigned long long)exact_list_bound);
+// The top_n of the n candidates (ckey, cidx, clag) by rank, as records in slots 0 .. top_n - 1 and padding up to `capacity`
+// (record 0 flagged 2 instead when `overflow`).  Candidate indices are global_offset + cidx; the series index is the
+// group key of an ungrouped run.  store(d, slot, rec) writes a record to destination d < ndest: the padding by every
+// thread to all destinations, a ranked record by the lanes of its warp, one destination each.
+template <typename Idx, typename Store>
+__device__ __forceinline__ void rank_topn(const unsigned long long *__restrict__ ckey, const Idx *__restrict__ cidx,
+                                          const int32_t *__restrict__ clag, unsigned long long n, bool overflow, long long top_n,
+                                          long long global_offset, long long capacity, int ndest, Store store) {
     const long long gtid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     const long long take = overflow ? 0 : ((long long)n < top_n ? (long long)n : top_n);
-    // padding (and the overflow signal) by the first threads of the grid
-    for (long long r = take + gtid; r < capacity; r += (long long)gridDim.x * blockDim.x)
-        out[r] = PartialRec{0ull, 0.0, 0ll, 0, (overflow && r == 0) ? 2 : 1};
+    for (long long r = take + gtid; r < capacity; r += (long long)gridDim.x * blockDim.x) {
+        const PartialRec pad{0ull, 0.0, 0ll, 0, (overflow && r == 0) ? 2 : 1};
+        for (int d = 0; d < ndest; d++) store(d, r, pad);
+    }
     if (overflow) return;
     // one warp per candidate
     const int lane = threadIdx.x & 31;
     const unsigned long long nwarps = ((unsigned long long)gridDim.x * blockDim.x) >> 5;
     for (unsigned long long i = (unsigned long long)gtid >> 5; i < n; i += nwarps) {
         const unsigned long long k = ckey[i];
-        const unsigned ix = (unsigned)cidx[i];
+        const Idx ix = cidx[i];
         const unsigned before = rank_of(ckey, cidx, n, k, ix, lane);
-        if (lane == 0 && (long long)before < top_n) {
+        if ((long long)before < top_n) {
             const int ls = clag[i];
-            const double a = __longlong_as_double((long long)k);
             const long long gi = global_offset + (long long)ix;
-            out[before] = PartialRec{(unsigned long long)gi, (ls & 1) ? -a : a, gi, (ls - (ls & 1)) / 2, 0};
+            const PartialRec rec{(unsigned long long)gi, cand_score(k, ls), gi, cand_lag(ls), 0};
+            for (int d = lane; d < ndest; d += 32) store(d, (long long)before, rec);
         }
     }
 }
 
+// the list is too long for rank_topn, or (exact_list_bound >= 0) the fused path's exact launch did not cover its list
+__device__ __forceinline__ bool topn_overflow(const RunCounters &c, long long exact_list_bound) {
+    return c.cand > MUSE_PARTIAL_RANK_CAP || (exact_list_bound >= 0 && c.listed > (unsigned long long)exact_list_bound);
+}
+
+__device__ __forceinline__ void partial_topn_body(const unsigned long long *__restrict__ ckey, const int32_t *__restrict__ cidx,
+                                                  const int32_t *__restrict__ clag, const RunCounters *__restrict__ counters, long long top_n,
+                                                  long long global_offset, long long exact_list_bound, PartialRec *__restrict__ out, long long capacity) {
+    rank_topn(ckey, cidx, clag, counters->cand, topn_overflow(*counters, exact_list_bound), top_n, global_offset, capacity, 1,
+              [&](int, long long r, const PartialRec &rec) { out[r] = rec; });
+}
+
 __global__ void __launch_bounds__(256)
 partial_topn_kernel(const unsigned long long *__restrict__ ckey, const int32_t *__restrict__ cidx,
-                    const int32_t *__restrict__ clag, const unsigned long long *__restrict__ counters, long long top_n,
+                    const int32_t *__restrict__ clag, const RunCounters *__restrict__ counters, long long top_n,
                     long long global_offset, long long exact_list_bound, PartialRec *__restrict__ out, long long capacity) {
     partial_topn_body(ckey, cidx, clag, counters, top_n, global_offset, exact_list_bound, out, capacity);
 }
@@ -422,33 +446,12 @@ __device__ __forceinline__ void release_flags(const ExchangePeers &ex, unsigned 
 
 __global__ void __launch_bounds__(256)
 partial_topn_push_kernel(const unsigned long long *__restrict__ ckey, const int32_t *__restrict__ cidx,
-                         const int32_t *__restrict__ clag, const unsigned long long *__restrict__ counters, long long top_n,
+                         const int32_t *__restrict__ clag, const RunCounters *__restrict__ counters, long long top_n,
                          long long global_offset, long long exact_list_bound, long long capacity, ExchangePeers ex) {
-    const unsigned long long n = counters[0];
-    const bool overflow = n > MUSE_PARTIAL_RANK_CAP || (exact_list_bound >= 0 && counters[2] > (unsigned long long)exact_list_bound);
-    const long long gtid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long take = overflow ? 0 : ((long long)n < top_n ? (long long)n : top_n);
+    const bool overflow = topn_overflow(*counters, exact_list_bound);
     const long long slot0 = (long long)ex.rank * capacity;
-    for (long long r = take + gtid; r < capacity; r += (long long)gridDim.x * blockDim.x) {
-        const PartialRec pad{0ull, 0.0, 0ll, 0, (overflow && r == 0) ? 2 : 1};
-        for (int d = 0; d < ex.world; d++) ex.recs[d][slot0 + r] = pad;
-    }
-    if (!overflow) {
-        const int lane = threadIdx.x & 31;
-        const unsigned long long nwarps = ((unsigned long long)gridDim.x * blockDim.x) >> 5;
-        for (unsigned long long i = (unsigned long long)gtid >> 5; i < n; i += nwarps) {
-            const unsigned long long k = ckey[i];
-            const unsigned ix = (unsigned)cidx[i];
-            const unsigned before = rank_of(ckey, cidx, n, k, ix, lane);
-            if ((long long)before < top_n) {
-                const int ls = clag[i];
-                const double a = __longlong_as_double((long long)k);
-                const long long gi = global_offset + (long long)ix;
-                const PartialRec rec{(unsigned long long)gi, (ls & 1) ? -a : a, gi, (ls - (ls & 1)) / 2, 0};
-                for (int d = lane; d < ex.world; d += 32) ex.recs[d][slot0 + before] = rec;      // one lane per destination
-            }
-        }
-    }
+    rank_topn(ckey, cidx, clag, counters->cand, overflow, top_n, global_offset, capacity, ex.world,
+              [&](int d, long long r, const PartialRec &rec) { ex.recs[d][slot0 + r] = rec; });
     if (!last_block_fenced(ex.done_blocks)) return;
     // flag word: (epoch << 32) | records in the slot (the whole slot: it is padded), 0xffffffff = take the host path
     release_flags(ex, (ex.epoch << 32) | (overflow ? 0xffffffffull : (unsigned long long)capacity));
@@ -497,7 +500,7 @@ multi_records_push_kernel(const PartialRec *__restrict__ table, const long long 
 }
 
 // a precedes b in (|score| desc, global series index asc), the order of results.go:81-85 with ties by index
-__device__ __forceinline__ bool rec_precedes(const PartialRec &a, const PartialRec &b) {
+MUSE_HD bool rec_precedes(const PartialRec &a, const PartialRec &b) {
     const double sa = fabs(a.score), sb = fabs(b.score);
     return sa > sb || (sa == sb && a.series_idx < b.series_idx);
 }
@@ -598,19 +601,7 @@ struct MergeState {
 };
 
 __device__ __forceinline__ long long merge_slot(const MergeState &m, unsigned long long group_key) {
-    const unsigned long long key = group_key + 1ull;
-    unsigned long long h = key * 0x9E3779B97F4A7C15ull;
-    h ^= h >> 32;
-    long long s = (long long)(h & (unsigned long long)(m.slots - 1));
-    for (;;) {
-        const unsigned long long cur = m.hkeys[s];
-        if (cur == key) return s;
-        if (cur == 0ull) {
-            const unsigned long long old = atomicCAS(&m.hkeys[s], 0ull, key);
-            if (old == 0ull || old == key) return s;
-        }
-        s = (s + 1) & (m.slots - 1);
-    }
+    return hash_slot(m.hkeys, m.slots, group_key + 1ull);
 }
 
 // record j of shard r is live when j < the count its flag word carries
@@ -649,48 +640,19 @@ __global__ void merge_emit_kernel(MergeState m, const PartialRec *__restrict__ r
         const long long s = merge_slot(m, p.group_key);
         emit = score_bits(p.score) == m.gmax[s] && (unsigned long long)p.series_idx == m.gidx[s] && passed(f, p.score, p.lag);
     }
-    const unsigned mask = __ballot_sync(0xffffffffu, emit);
-    if (mask == 0u) return;
-    const int lane = threadIdx.x & 31, leader = __ffs(mask) - 1;
-    unsigned long long base = 0;
-    if (lane == leader) base = atomicAdd(&m.counters[0], (unsigned long long)__popc(mask));
-    base = __shfl_sync(0xffffffffu, base, leader);
-    if (emit) {
-        const unsigned long long pos = base + (unsigned long long)__popc(mask & ((1u << lane) - 1u));
+    warp_append(&m.counters[0], emit, [&](unsigned long long pos) {
         m.ckey[pos] = score_bits(p.score);
         m.cidx[pos] = p.series_idx;
         m.clag[pos] = 2 * p.lag + (p.score < 0.0 ? 1 : 0);
-    }
+    });
 }
 // rank by counting, as partial_topn_kernel, on (|score| desc, GLOBAL series index asc); out[0 .. top_n) padded with flags = 1,
 // out[0].flags = 2 when the list is too long for this kernel or a shard overflowed (the caller takes the host path)
 __global__ void __launch_bounds__(256)
 merged_topn_kernel(MergeState m, long long top_n, PartialRec *__restrict__ out) {
     const unsigned long long n = m.counters[0];
-    const bool overflow = n > MUSE_PARTIAL_RANK_CAP || m.counters[1] != 0ull;
-    const long long gtid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long take = overflow ? 0 : ((long long)n < top_n ? (long long)n : top_n);
-    for (long long r = take + gtid; r < top_n; r += (long long)gridDim.x * blockDim.x)
-        out[r] = PartialRec{0ull, 0.0, 0ll, 0, (overflow && r == 0) ? 2 : 1};
-    if (overflow) return;
-    const int lane = threadIdx.x & 31;
-    const unsigned long long nwarps = ((unsigned long long)gridDim.x * blockDim.x) >> 5;
-    for (unsigned long long i = (unsigned long long)gtid >> 5; i < n; i += nwarps) {
-        const unsigned long long k = m.ckey[i];
-        const long long ix = m.cidx[i];
-        unsigned before = 0;
-        for (unsigned long long j = lane; j < n; j += 32) {
-            const unsigned long long kj = m.ckey[j];
-            before += (kj > k || (kj == k && m.cidx[j] < ix)) ? 1u : 0u;
-        }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) before += __shfl_xor_sync(0xffffffffu, before, off);
-        if (lane == 0 && (long long)before < top_n) {
-            const int ls = m.clag[i];
-            const double a = __longlong_as_double((long long)k);
-            out[before] = PartialRec{(unsigned long long)ix, (ls & 1) ? -a : a, ix, (ls - (ls & 1)) / 2, 0};
-        }
-    }
+    rank_topn(m.ckey, m.cidx, m.clag, n, n > MUSE_PARTIAL_RANK_CAP || m.counters[1] != 0ull, top_n, 0ll, top_n, 1,
+              [&](int, long long r, const PartialRec &rec) { out[r] = rec; });
 }
 
 // ---- radix select of the top_n candidates by (key desc, idx asc) ---------------------

@@ -287,23 +287,25 @@ def test_run_matches_oracle_ungrouped_and_grouped(ctx):
 
 
 def test_top_n_device_select_with_ties(ctx):
-    # > 4096 candidates and heavy ties: many exact duplicates of a few rows -> the device
-    # radix select must cut by (score desc, index asc)
+    # heavy ties: many exact duplicates of a few rows, so the top-N must cut by (score desc, index asc).  Every series
+    # passes the filter: a store of 20000 takes the device-side rank-by-counting top-N; one of 300000 has more candidates
+    # than that ranks (32768) and than run_select leaves to the host (262144), so it takes the device radix select, whose
+    # last digits are the ~index ones
     rng = np.random.default_rng(2)
     N = 64
     ref, base = _siggen(rng, 8, N, pulse_every=1)
-    S = 20000
-    Y = base[rng.integers(0, 8, S)]
-    store = mb.DeviceStore(ctx, N, 0, S)
-    store.append(Y)
-    b = mb.DeviceBatch(ctx, store, ref)
-    sl = mo.score_series_batch(ref, Y)
-    for top_n in (1, 100, 4500, 12345):
-        sc, lg, ix = b.run([], N, top_n, 0.0, mode=mb.MODE_EXACT)
-        wsc, wlg, wix = mo.batch_run_arrays(ref, Y, None, N, top_n, 0.0, scores_lags=sl)
-        assert len(sc) == len(wsc)
-        np.testing.assert_array_equal(ix, wix)
-        assert np.max(np.abs(sc - wsc), initial=0.0) <= SCORE_TOL
+    for S in (20000, 300000):
+        Y = base[rng.integers(0, 8, S)]
+        store = mb.DeviceStore(ctx, N, 0, S)
+        store.append(Y)
+        b = mb.DeviceBatch(ctx, store, ref)
+        sl = mo.score_series_batch(ref, Y)
+        for top_n in (1, 100, 4500, 12345):
+            sc, lg, ix = b.run([], N, top_n, 0.0, mode=mb.MODE_EXACT)
+            wsc, wlg, wix = mo.batch_run_arrays(ref, Y, None, N, top_n, 0.0, scores_lags=sl)
+            assert len(sc) == len(wsc), (S, top_n)
+            np.testing.assert_array_equal(ix, wix, err_msg="S = %d, top_n = %d" % (S, top_n))
+            assert np.max(np.abs(sc - wsc), initial=0.0) <= SCORE_TOL, (S, top_n)
 
 
 def test_hash_group_table(ctx):
