@@ -183,7 +183,7 @@ static bool device_topn_fits(int64_t top_n, int64_t capacity) {
 }
 
 struct RunScratch {
-    int64_t scratch_cap = 0;                  // entries of the eleven arrays below (ensure_scratch)
+    int64_t scratch_cap = 0;                  // entries of the twelve arrays below (ensure_scratch)
     DevBuf<double> d_score;
     DevBuf<int32_t> d_lag;
     DevBuf<int64_t> d_slot;
@@ -194,6 +194,8 @@ struct RunScratch {
     DevBuf<int32_t> d_list;
     DevBuf<float> d_L;                        // lower bounds (grouped screened runs, diagnostic entry point)
     DevBuf<signed char> d_W;                  // grouped screened runs: lag-window verdict of every refined series (ScreenParams::out_W)
+    DevBuf<int32_t> d_rows;                   // filtered runs: the selected local rows in ascending order (muse_batch_run_where)
+    DevBuf<int32_t> d_where_off;              // filtered runs: per-block offsets of the selection, then its length
     Buf<Mailbox, true> h_pin;
     DevBuf<RunCounters> d_counters;
     DevBuf<SelectState> d_sel;
@@ -272,6 +274,8 @@ struct muse_batch : RunScratch {
     int fused_run = 0;         // 1: score_fused, 2: score_fused_grouped (d_counters: listed = exact list length)
     int prescreened = 0;       // d_U and the cut-off state were filled by the tensor-core multi-query path: the next fused run starts at its tail
     int signed_run = 0;        // the current run keeps the sign of the scores (muse.go:72-76)
+    int64_t where_m = -1;      // a filtered run (muse_batch_run_where) is under way over the where_m rows of d_rows; -1: none
+    int pre_launches = -1;     // launches muse_batch_run_where queued (after recording ev[0]) before the run it starts; -1: none
     // n > MUSE_MAX_FUSED_FFT_LEN: Stockham passes through global memory (kernels_long.cu); Xt holds n entries, twM the n twiddles
     int is_long = 0;
     DevBuf<unsigned char> d_long;   // work buffer of launch_long
@@ -285,6 +289,12 @@ struct BatchDestroy {
 using BatchPtr = std::unique_ptr<muse_batch, BatchDestroy>;   // a batch that goes back through muse_batch_destroy
 
 static inline cudaStream_t bstream(const muse_batch *b) { return b->ctx->stream; }
+
+// The rows the current run scores: a filtered run's selection (d_rows[0 .. where_m)), else every row of the store (NULL).
+// Everything that depends on the size of the store -- the AUTO rule, launch bounds, what a fallback scores -- uses
+// run_count, so a filtered run takes the path a store of just its rows would take.
+static inline int64_t run_count(const muse_batch *b) { return b->where_m >= 0 ? b->where_m : b->g->size; }
+static inline const int32_t *run_rows(const muse_batch *b) { return b->where_m >= 0 ? b->d_rows.get() : nullptr; }
 
 // ------------------------------------------------------------------------------------
 // context
@@ -1073,6 +1083,7 @@ static int ensure_scratch(muse_batch *b) {
     CU(b->d_slag.grow(cap));
     CU(b->d_U.grow(cap));
     CU(b->d_list.grow(cap));
+    CU(b->d_rows.grow(cap));
     b->scratch_cap = cap;
     return MUSE_OK;
 }
@@ -1355,7 +1366,7 @@ static int run_select(muse_batch *b, const RunArgs &a, int apply_filter, int64_t
     CU(cudaStreamSynchronize(st));
     unsigned long long ncand = h_n.cand;
     settle_counters(b, h_n);
-    if (b->fused_run == 1 && (int64_t)h_n.listed > std::min<int64_t>(S, MUSE_EXACT_UB)) {
+    if (b->fused_run == 1 && (int64_t)h_n.listed > std::min<int64_t>(run_count(b), MUSE_EXACT_UB)) {
         // rare: more exact candidates than the fixed launch covered -> finish them and select again
         const int64_t n_exact = (int64_t)h_n.listed;
         int rc = run_fused_overflow(b, n_exact, false);
@@ -1440,7 +1451,8 @@ static ScreenParams screen_params(muse_batch *b) {
     memset(&sp, 0, sizeof(sp));
     sp.slab = b->g->slab;
     sp.ld = b->g->ld;
-    sp.count = b->g->size;
+    sp.count = run_count(b);
+    sp.rows = run_rows(b);
     sp.N = (int)b->N;
     sp.twp = b->twp_f;
     sp.sw = b->sw_f;
@@ -1591,7 +1603,7 @@ static int score_fused(muse_batch *b, const RunArgs &a) {
     const unsigned blocks = (unsigned)((S + 255) / 256);
     survivors_cut_kernel<<<blocks, 256, 0, st>>>(b->d_U, S, b->d_cut, b->d_list, b->d_counters);
     b->timing.n_launches++;
-    rc = score_exact_all(b, b->signed_run, b->d_list, std::min<int64_t>(S, MUSE_EXACT_UB), &b->d_counters->listed);
+    rc = score_exact_all(b, b->signed_run, b->d_list, std::min<int64_t>(run_count(b), MUSE_EXACT_UB), &b->d_counters->listed);
     if (rc) return rc;
     return MUSE_OK;
 }
@@ -1666,7 +1678,7 @@ static int run_fused_overflow(muse_batch *b, int64_t n_exact, bool refill) {
         CU(cudaMemsetAsync(b->d_score, 0xff, sizeof(double) * (size_t)S, bstream(b)));
         return score_exact_all(b, b->signed_run, b->d_list, n_exact);
     }
-    if (n_exact <= std::min<int64_t>(S, MUSE_EXACT_UB)) return MUSE_OK;
+    if (n_exact <= std::min<int64_t>(run_count(b), MUSE_EXACT_UB)) return MUSE_OK;
     return score_exact_all(b, b->signed_run, b->d_list + MUSE_EXACT_UB, n_exact - MUSE_EXACT_UB);
 }
 
@@ -1678,7 +1690,8 @@ static int run_scores(muse_batch *b, const RunArgs &a) {
     b->timing_pending = 0;
     b->signed_run = a.signed_scores ? 1 : 0;
     cudaStream_t st = bstream(b);
-    CU(cudaEventRecord(b->ev[0], st));
+    if (b->pre_launches >= 0) b->timing.n_launches = b->pre_launches;      // the run began with the caller's work (ev[0] recorded)
+    else CU(cudaEventRecord(b->ev[0], st));
     CU(cudaMemsetAsync(b->d_counters, 0, sizeof(RunCounters), st));
     // screening needs: a kernel for this FFT size, an ungrouped unsigned run, a sign filter that
     // unsigned scores can pass, and a store big enough to be worth two extra round trips
@@ -1688,7 +1701,7 @@ static int run_scores(muse_batch *b, const RunArgs &a) {
     // top-N rank by; the survivors are re-scored signed.  A sign filter on signed scores needs the sign, which no bound has.
     const bool can_screen = b->screen_ok && (a.n_key_cols == 0 || screen_is_fused(b->log2m)) &&
                             (a.signed_scores ? a.sign_filter == MUSE_SIGN_ANY : a.sign_filter != MUSE_SIGN_NEG);
-    bool screen = can_screen && (a.mode == MUSE_MODE_SCREEN || (a.mode == MUSE_MODE_AUTO && b->g->size >= 16384));
+    bool screen = can_screen && (a.mode == MUSE_MODE_SCREEN || (a.mode == MUSE_MODE_AUTO && run_count(b) >= 16384));
     if (screen && a.n_key_cols > 0) {
         b->timing.mode = MUSE_MODE_SCREEN;
         b->fused_run = 2;          // statistics as a fused run; its exact list is already complete
@@ -1706,7 +1719,7 @@ static int run_scores(muse_batch *b, const RunArgs &a) {
         return MUSE_OK;
     }
     b->timing.mode = MUSE_MODE_EXACT;
-    rc = score_exact_all(b, a.signed_scores, nullptr, b->g->size);
+    rc = score_exact_all(b, a.signed_scores, run_rows(b), run_count(b));
     if (rc) return rc;
     CU(cudaEventRecord(b->ev[1], st));
     CU(cudaEventRecord(b->ev[2], st));
@@ -1769,7 +1782,9 @@ static int queue_topn_records(muse_batch *b, const RunArgs &a, muse_partial *d_o
 // candidate list was too long for the device-side select, or the fused path's exact launch did not cover its list --
 // finish on the host path from the scores already on the device.
 static bool device_topn_applies(const muse_batch *b, const RunArgs &a) {
-    return a.n_key_cols == 0 && b->g->size > 0 && device_topn_fits(a.top_n, b->scratch_cap);
+    // a filtered run: as on a store of its rows, whose scratch holds max(rows, 1024) entries (ensure_scratch)
+    const int64_t cap = b->where_m >= 0 ? std::max<int64_t>(b->where_m, 1024) : b->scratch_cap;
+    return a.n_key_cols == 0 && run_count(b) > 0 && device_topn_fits(a.top_n, cap);
 }
 
 static int device_topn_queue(muse_batch *b, const RunArgs &a) {
@@ -1841,6 +1856,195 @@ extern "C" int muse_batch_run(muse_batch *b, const int32_t *key_cols, int32_t n_
 }
 
 // ------------------------------------------------------------------------------------
+// Filtered runs: Batch.Run over the series whose label ids match (Group.FilterByLabelValues, group.go:60-71)
+// ------------------------------------------------------------------------------------
+#define MUSE_WHERE_MAX 16        // equalities of one predicate
+#define MUSE_WHERE_TILE 1024     // rows per block of the selection kernels: 256 threads x 4 rows
+struct WherePred {
+    const int32_t *col[MUSE_WHERE_MAX];   // label-id column of each equality
+    int32_t id[MUSE_WHERE_MAX];
+    int n;
+};
+__device__ __forceinline__ bool where_match(const WherePred &p, int64_t i) {
+    for (int j = 0; j < p.n; j++)
+        if (p.col[j][i] != p.id[j]) return false;
+    return true;
+}
+
+// 1. matching rows per tile of MUSE_WHERE_TILE rows
+__global__ void __launch_bounds__(256) where_count_kernel(WherePred p, int64_t S, int32_t *__restrict__ block_count) {
+    __shared__ int wsum[8];
+    const int64_t base = (int64_t)blockIdx.x * MUSE_WHERE_TILE;
+    int c = 0;
+#pragma unroll
+    for (int k = 0; k < MUSE_WHERE_TILE / 256; k++) {
+        const int64_t i = base + k * 256 + threadIdx.x;
+        c += (i < S && where_match(p, i)) ? 1 : 0;
+    }
+    c = __reduce_add_sync(0xffffffffu, c);
+    if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = c;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int total = 0;
+        for (int w = 0; w < 8; w++) total += wsum[w];
+        block_count[blockIdx.x] = total;
+    }
+}
+
+// 2. one block: exclusive scan of the nb tile counts in place, the selection's length into off[nb]
+__global__ void __launch_bounds__(1024) where_scan_kernel(int32_t *__restrict__ off, int64_t nb) {
+    __shared__ int wsum[32];
+    __shared__ int carry;
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    if (threadIdx.x == 0) carry = 0;
+    __syncthreads();
+    for (int64_t base = 0; base < nb; base += 1024) {
+        const int64_t i = base + threadIdx.x;
+        const int v = i < nb ? off[i] : 0;
+        int x = v;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) {
+            const int y = __shfl_up_sync(0xffffffffu, x, d);
+            if (lane >= d) x += y;
+        }
+        if (lane == 31) wsum[w] = x;
+        __syncthreads();
+        if (w == 0) {
+            int s = wsum[lane];
+#pragma unroll
+            for (int d = 1; d < 32; d <<= 1) {
+                const int y = __shfl_up_sync(0xffffffffu, s, d);
+                if (lane >= d) s += y;
+            }
+            wsum[lane] = s;
+        }
+        __syncthreads();
+        const int excl = carry + (w > 0 ? wsum[w - 1] : 0) + x - v;
+        if (i < nb) off[i] = excl;
+        __syncthreads();                    // every thread has read carry
+        if (threadIdx.x == 1023) carry = excl + v;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) off[nb] = carry;
+}
+
+// 3. the matching rows of each tile at the tile's offset, in ascending order (the same list on every run)
+__global__ void __launch_bounds__(256) where_write_kernel(WherePred p, int64_t S, const int32_t *__restrict__ off, int32_t *__restrict__ rows) {
+    __shared__ int wsum[8];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int64_t base = (int64_t)blockIdx.x * MUSE_WHERE_TILE;
+    int out = off[blockIdx.x];
+#pragma unroll
+    for (int k = 0; k < MUSE_WHERE_TILE / 256; k++) {
+        const int64_t i = base + k * 256 + threadIdx.x;
+        const bool m = i < S && where_match(p, i);
+        const unsigned ball = __ballot_sync(0xffffffffu, m);
+        if (lane == 0) wsum[w] = __popc(ball);
+        __syncthreads();
+        int before = 0, total = 0;
+        for (int v = 0; v < 8; v++) {
+            before += v < w ? wsum[v] : 0;
+            total += wsum[v];
+        }
+        if (m) rows[out + before + __popc(ball & ((1u << lane) - 1u))] = (int32_t)i;
+        out += total;
+        __syncthreads();                    // wsum is rewritten by the next slice
+    }
+}
+
+// Rows outside the selection get the values that already mean "cannot be in the result" to the per-series kernels that
+// walk the whole store (survivors_cut, group_*, emit_candidates): score NaN (group max / rep and the candidates skip it),
+// upper bound -1 (never a survivor or contender, never marks its group uncertain) and lower bound -1 (never a group's
+// bound).  The pass over the selection then overwrites its own rows.
+__global__ void where_neutral_kernel(double *__restrict__ score, float *__restrict__ U, float *__restrict__ L, int64_t S) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= S) return;
+    score[i] = __longlong_as_double(-1ll);      // all bits set: a NaN, what the NaN fills of the other paths write
+    U[i] = -1.f;
+    L[i] = -1.f;
+}
+
+// The selection of a predicate into d_rows (ascending local rows); its length.
+static int select_where(muse_batch *b, const WherePred &p, int64_t &m) {
+    const int64_t S = b->g->size;
+    cudaStream_t st = bstream(b);
+    const int64_t nb = (S + MUSE_WHERE_TILE - 1) / MUSE_WHERE_TILE;
+    CU(b->d_where_off.grow(nb + 1));
+    where_count_kernel<<<(unsigned)nb, 256, 0, st>>>(p, S, b->d_where_off);
+    where_scan_kernel<<<1, 1024, 0, st>>>(b->d_where_off, nb);
+    where_write_kernel<<<(unsigned)nb, 256, 0, st>>>(p, S, b->d_where_off, b->d_rows);
+    CU(cudaGetLastError());
+    int32_t h_m = 0;                      // one small copy: the host sizes the launches and takes the AUTO decision on it
+    CU(cudaMemcpyAsync(&h_m, b->d_where_off.get() + nb, sizeof(h_m), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    m = h_m;
+    return MUSE_OK;
+}
+
+extern "C" int muse_batch_run_where(muse_batch *b, const int32_t *where_cols, const int32_t *where_ids, int32_t n_where,
+                                    const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n, double threshold,
+                                    int32_t sign_filter, int32_t mode, int32_t signed_scores, double *scores, int64_t *lags,
+                                    int64_t *series_idx, int64_t *n_out) {
+    int rc = check_batch(b);
+    if (rc) return rc;
+    if (n_where < 0 || n_where > MUSE_WHERE_MAX)
+        return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: %d where columns (0 .. %d)", (int)n_where, MUSE_WHERE_MAX);
+    if (n_where > 0 && (!where_cols || !where_ids)) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: NULL where arrays");
+    muse_group *g = b->g;
+    WherePred p;
+    memset(&p, 0, sizeof(p));
+    p.n = n_where;
+    for (int j = 0; j < n_where; j++) {
+        if (where_cols[j] < 0 || where_cols[j] >= g->nkeys)
+            return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: where column %d not in [0,%d)", (int)where_cols[j], g->nkeys);
+        if (where_ids[j] < 0) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: negative label id %d", (int)where_ids[j]);
+        p.col[j] = g->labels + (size_t)where_cols[j] * g->cap;
+        p.id[j] = where_ids[j];
+    }
+    if (n_where == 0 || g->size == 0)
+        return muse_batch_run_ex(b, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores, scores, lags,
+                                 series_idx, n_out);
+    if (!n_out || (top_n > 0 && (!scores || !lags || !series_idx))) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: NULL output");
+    if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: bad key columns");
+    CU(cudaSetDevice(b->ctx->device));
+    *n_out = 0;
+    rc = ensure_scratch(b);
+    if (rc) return rc;
+    rc = ensure_lower(b);
+    if (rc) return rc;
+    // The timing of a filtered run starts here, before the selection, and counts its launches in every case below.
+    cudaStream_t st = bstream(b);
+    CU(cudaEventRecord(b->ev[0], st));
+    int launches = 3;      // the selection: count, scan, write
+    int64_t m = 0;
+    rc = select_where(b, p, m);
+    if (rc) return rc;
+    const int64_t S = g->size;
+    if (m == 0) {          // nothing matches: no records and nothing scored
+        memset(&b->timing, 0, sizeof(b->timing));
+        b->timing_pending = 0;
+        b->timing.mode = MUSE_MODE_EXACT;
+        b->timing.n_launches = launches;
+        CU(cudaEventRecord(b->ev[1], st));      // no scoring pass, no re-scoring
+        CU(cudaEventRecord(b->ev[2], st));
+        return finish_timing(b);
+    }
+    struct EndWhere {      // every path out of the run leaves the batch unfiltered
+        muse_batch *b;
+        ~EndWhere() { b->where_m = -1; b->pre_launches = -1; }
+    } end_where{b};
+    if (m < S) {           // m == S: every row matches, the run of the whole store
+        where_neutral_kernel<<<(unsigned)((S + 255) / 256), 256, 0, st>>>(b->d_score, b->d_U, b->d_L, S);
+        CU(cudaGetLastError());
+        launches++;
+        b->where_m = m;
+    }
+    b->pre_launches = launches;
+    return muse_batch_run_ex(b, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores, scores, lags,
+                             series_idx, n_out);
+}
+
+// ------------------------------------------------------------------------------------
 // multi-GPU partials
 // ------------------------------------------------------------------------------------
 extern "C" int64_t muse_batch_partial_capacity(muse_batch *b, const int32_t *key_cols, int32_t n_key_cols, int64_t top_n) {
@@ -1866,7 +2070,7 @@ static TopnLaunch queue_candidates(muse_batch *b, const RunArgs &a) {
         Cand cand{b->d_ckey, b->d_cidx, b->d_clag, &b->d_counters->cand};
         if (b->fused_run == 1) {
             // only the listed series have scores: filter those (the list's length stays on the device)
-            const int64_t lim = std::min<int64_t>(S, MUSE_EXACT_UB);
+            const int64_t lim = std::min<int64_t>(run_count(b), MUSE_EXACT_UB);
             emit_listed_kernel<<<(unsigned)((lim + 255) / 256), 256, 0, st>>>(b->d_list, &b->d_counters->listed, lim, b->d_score, b->d_lag, f, cand);
         } else {
             GroupTable gt;
@@ -1876,8 +2080,8 @@ static TopnLaunch queue_candidates(muse_batch *b, const RunArgs &a) {
         b->timing.n_launches++;
     }
     // the grid covers MUSE_PARTIAL_RANK_CAP candidates; blocks past the real count (device side) leave at once
-    const long long exact_bound = b->fused_run == 1 ? (long long)std::min<int64_t>(S, MUSE_EXACT_UB) : -1;
-    const unsigned pblocks = (unsigned)std::min<int64_t>((std::max<int64_t>(S, 1) + 7) / 8, (int64_t)b->ctx->sm_count * 8);   // 8 warps per block, one warp per candidate
+    const long long exact_bound = b->fused_run == 1 ? (long long)std::min<int64_t>(run_count(b), MUSE_EXACT_UB) : -1;
+    const unsigned pblocks = (unsigned)std::min<int64_t>((std::max<int64_t>(run_count(b), 1) + 7) / 8, (int64_t)b->ctx->sm_count * 8);   // 8 warps per block, one warp per candidate
     return TopnLaunch{exact_bound, pblocks};
 }
 

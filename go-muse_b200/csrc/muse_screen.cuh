@@ -106,6 +106,9 @@ struct ScreenParams {
     const int64_t *slot_of;           // grouped runs: group-table slot of every series
     unsigned long long *group_L;      // grouped runs: [slots] running best lower bound of each group (float bits, low word)
     signed char *out_W;   // grouped runs: [count] 1 = peak certainly inside the lag window, -1 = certainly outside, 0 = undecided
+    // filtered runs (muse_batch_run_where): work item pos < count is the series rows[pos] (ascending local row numbers); the
+    // per-series arrays above (slab, row_stat, slot_of, out_U, out_L, out_W) are indexed by that row.  NULL: row = pos
+    const int32_t *rows;
 };
 
 // ---- maxima of |cc'| inside / outside the lag window (rotated index: (idx - win_lo) mod n <= win_len) ----
@@ -616,7 +619,7 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
     if (t == 0) {
         mbar_init(bar, 1);
         mbar_init_fence();
-        if (pos0 < count) bulk_load(smem_u32(buf), prm.slab + (int64_t)pos0 * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
+        if (pos0 < count) bulk_load(smem_u32(buf), prm.slab + (int64_t)(prm.rows ? prm.rows[pos0] : pos0) * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
     }
     __syncthreads();
 
@@ -639,7 +642,8 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
             // count / CLAIM times.
             if (claim_ends) claim = atomicInc(prm.next_claim, (unsigned)count);
         }
-        const RowStat rs = prm.row_stat[pos];   // fp64 mean and 1/std from the ingest pass (xcorr.go:84-95); in flight with the row
+        const int row = prm.rows ? prm.rows[pos] : pos;
+        const RowStat rs = prm.row_stat[row];   // fp64 mean and 1/std from the ingest pass (xcorr.go:84-95); in flight with the row
         const double mu = rs.mean;
         mbar_wait(bar, phase);      // every lane waits itself (one polling lane + __syncwarp measured 3x slower)
 
@@ -659,7 +663,7 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
                 asm volatile("" ::"r"(__float_as_uint(v[P - 1].y)) : "memory");
                 // the generic-proxy reads and writes of the exchange are ordered before the async-proxy write of the copy
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                bulk_load(smem_u32(buf), prm.slab + (int64_t)next * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
+                bulk_load(smem_u32(buf), prm.slab + (int64_t)(prm.rows ? prm.rows[next] : next) * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
             }
         }
         screen_pass1<32>(v);                            // v[Perm(j)] = Z[t + 32*j]
@@ -728,8 +732,8 @@ score_screen_warp_kernel(const ScreenParams prm, const unsigned warp_bytes, cons
             if (L >= prm.thr && L >= cut_now) cut_count_and_raise(prm.cut_bits, prm.cut_hist, prm.top_n, L, t);
         }
         if (t == 0) {
-            prm.out_U[pos] = U;
-            if (prm.out_L) prm.out_L[pos] = L;
+            prm.out_U[row] = U;
+            if (prm.out_L) prm.out_L[row] = L;
         }
         __syncwarp();                       // next_of[w] of lane 0's re-arm
         pp = (unsigned)next_of[w] | (~pp & 0x80000000u);

@@ -417,21 +417,24 @@ score_screen_big_kernel(const ScreenParams prm) {
     const int chunk = (count + (int)gridDim.x - 1) / (int)gridDim.x;
     const int pos_lo = (int)blockIdx.x * chunk;
     const int pos_hi = min(pos_lo + chunk, count);
-    if (t == 0 && pos_lo < pos_hi) big_l2_prefetch(prm.slab + (int64_t)pos_lo * prm.ld, row_bytes);
+    // the series of work item pos (filtered runs: the listed rows, so the prefetch fetches listed rows, not a range)
+    auto row_of = [&](int pos) { return prm.rows ? prm.rows[pos] : pos; };
+    if (t == 0 && pos_lo < pos_hi) big_l2_prefetch(prm.slab + (int64_t)row_of(pos_lo) * prm.ld, row_bytes);
 
     for (int pos = pos_lo; pos < pos_hi; pos++) {
-        const double *rowp = prm.slab + (int64_t)pos * prm.ld;
+        const int row = row_of(pos);
+        const double *rowp = prm.slab + (int64_t)row * prm.ld;
         unsigned cut_raw = 0u, lg_raw = 0u;
         unsigned long long *gslot = nullptr;
         if (t == 0) {
-            if (pos + 1 < pos_hi) big_l2_prefetch(rowp + prm.ld, row_bytes);
+            if (pos + 1 < pos_hi) big_l2_prefetch(prm.slab + (int64_t)row_of(pos + 1) * prm.ld, row_bytes);
             cut_raw = ld_relaxed_u32(prm.cut_bits);
             if (prm.group_L) {
-                gslot = prm.group_L + prm.slot_of[pos];
+                gslot = prm.group_L + prm.slot_of[row];
                 lg_raw = ld_relaxed_u32(reinterpret_cast<const unsigned *>(gslot));      // low word: float bits of the best lower bound so far
             }
         }
-        const RowStat rs = prm.row_stat[pos];
+        const RowStat rs = prm.row_stat[row];
         const double mu = rs.mean;
 
         // ---- centred samples -> fp32 registers, LB x 16 bytes in flight per thread ----
@@ -533,9 +536,9 @@ if constexpr (NZ > 0) {
             if (!prm.grouped && t < 32 && L >= prm.thr && L >= cut_now) cut_count_and_raise(prm.cut_bits, prm.cut_hist, prm.top_n, L, t);
         }
         if (t == 0) {
-            prm.out_U[pos] = U;
-            if (prm.out_L) prm.out_L[pos] = L;
-            if (prm.out_W) prm.out_W[pos] = W;
+            prm.out_U[row] = U;
+            if (prm.out_L) prm.out_L[row] = L;
+            if (prm.out_W) prm.out_W[row] = W;
         }
         // no barrier here: the exchange buffer was last read before the reduction barrier of whichever path ran, and
         // red_f / bc_word are next written three barriers into the next iteration

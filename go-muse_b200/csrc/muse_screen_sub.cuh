@@ -96,6 +96,7 @@ score_screen_sub_kernel(const ScreenParams prm, const unsigned warp_bytes, const
         for (int gg = 0; gg < GS; gg++) {
             int s = unit * GS + gg;
             s = s < count ? s : count - 1;
+            if (prm.rows) s = prm.rows[s];
             bulk_copy(smem_u32(wbuf + (size_t)gg * row_bytes), prm.slab + (int64_t)s * prm.ld, bytes, bar);
         }
     };
@@ -112,7 +113,8 @@ score_screen_sub_kernel(const ScreenParams prm, const unsigned warp_bytes, const
     for (int pos = pos0; pos < units; pos += stride, phase ^= 1u) {
         const int sraw = pos * GS + g;
         const bool valid = sraw < count;
-        const int s = valid ? sraw : count - 1;
+        const int spos = valid ? sraw : count - 1;
+        const int s = prm.rows ? prm.rows[spos] : spos;      // the series (row of the store) of this work item
         unsigned cut_raw = 0u;
         if (lane == 0) cut_raw = ld_relaxed_u32(prm.cut_bits);
         const RowStat rs = prm.row_stat[s];

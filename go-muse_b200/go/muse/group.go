@@ -304,4 +304,23 @@ func (g *Group) keyCols(groupByLabels []string) []int32 {
 	return cols
 }
 
+// whereCols maps the label set of FilterByLabelValues to device columns and value ids; ok == false when no series can match
+// (a key or a value the dictionary does not know).
+func (g *Group) whereCols(labels *Labels) (cols, ids []int32, ok bool) {
+	for _, k := range labels.Keys() {
+		v, _ := labels.Get(k)
+		c := sort.SearchStrings(g.cols, k)
+		if c == len(g.cols) || g.cols[c] != k {
+			return nil, nil, false
+		}
+		id, seen := g.dict[k][v]
+		if !seen {
+			return nil, nil, false
+		}
+		cols = append(cols, int32(c))
+		ids = append(ids, id)
+	}
+	return cols, ids, len(cols) > 0
+}
+
 var errNoSeries = errors.New("comparison group is empty")

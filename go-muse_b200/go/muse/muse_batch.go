@@ -88,15 +88,43 @@ func (b *Batch) bind() error {
 // the groupByLabels values, or per series when none are given.  Always returns nil, like go-muse; Err() tells
 // whether the run could be carried out.
 func (b *Batch) Run(groupByLabels []string) error {
-	comp := b.Comparison
 	b.err = nil
-	if len(comp.series) == 0 {
+	if len(b.Comparison.series) == 0 {
 		return nil
 	}
 	if err := b.bind(); err != nil {
 		b.err = err
 		return nil
 	}
+	b.err = b.run(groupByLabels, nil, nil)
+	return nil
+}
+
+// RunWhere is Run over the series of Comparison.FilterByLabelValues(labels) only, on the resident device store (no second
+// store, no upload): Results end up as NewBatch(ref, <a Group of those series>, ...).Run(groupByLabels) leaves them.  When
+// nothing can match -- empty labels, a key or a value no series of the group has -- it returns at once and Results are
+// untouched.  Always returns nil, like Run; Err() tells whether the run could be carried out.
+func (b *Batch) RunWhere(labels *Labels, groupByLabels []string) error {
+	b.err = nil
+	if len(b.Comparison.series) == 0 || labels == nil || labels.Len() == 0 {
+		return nil
+	}
+	if err := b.bind(); err != nil { // uploads series added since the last call: the dictionary then knows every value
+		b.err = err
+		return nil
+	}
+	cols, ids, ok := b.Comparison.whereCols(labels)
+	if !ok {
+		return nil
+	}
+	b.err = b.run(groupByLabels, cols, ids)
+	return nil
+}
+
+// run scores the bound store (whereCols / whereIDs: only the series with those label ids, muse_batch_run_where) and pushes
+// the device's records through Results.Update.
+func (b *Batch) run(groupByLabels []string, whereCols, whereIDs []int32) error {
+	comp := b.Comparison
 	r := b.Results
 	cols := comp.keyCols(groupByLabels)
 	topN := r.TopN
@@ -111,13 +139,21 @@ func (b *Batch) Run(groupByLabels []string) error {
 	if len(cols) > 0 {
 		colPtr = (*C.int32_t)(unsafe.Pointer(&cols[0]))
 	}
-	rc := C.muse_batch_run(b.batch, colPtr, C.int32_t(len(cols)), C.int64_t(r.MaxLag), C.int64_t(topN),
-		C.double(r.Threshold), C.int32_t(r.SignFilter),
-		(*C.double)(unsafe.Pointer(&scores[0])), (*C.int64_t)(unsafe.Pointer(&lags[0])),
-		(*C.int64_t)(unsafe.Pointer(&idx[0])), &nOut)
+	var rc C.int
+	if len(whereCols) > 0 {
+		rc = C.muse_batch_run_where(b.batch, (*C.int32_t)(unsafe.Pointer(&whereCols[0])), (*C.int32_t)(unsafe.Pointer(&whereIDs[0])),
+			C.int32_t(len(whereCols)), colPtr, C.int32_t(len(cols)), C.int64_t(r.MaxLag), C.int64_t(topN),
+			C.double(r.Threshold), C.int32_t(r.SignFilter), C.MUSE_MODE_AUTO, 0,
+			(*C.double)(unsafe.Pointer(&scores[0])), (*C.int64_t)(unsafe.Pointer(&lags[0])),
+			(*C.int64_t)(unsafe.Pointer(&idx[0])), &nOut)
+	} else {
+		rc = C.muse_batch_run(b.batch, colPtr, C.int32_t(len(cols)), C.int64_t(r.MaxLag), C.int64_t(topN),
+			C.double(r.Threshold), C.int32_t(r.SignFilter),
+			(*C.double)(unsafe.Pointer(&scores[0])), (*C.int64_t)(unsafe.Pointer(&lags[0])),
+			(*C.int64_t)(unsafe.Pointer(&idx[0])), &nOut)
+	}
 	if rc != C.MUSE_OK {
-		b.err = lastError(rc)
-		return nil
+		return lastError(rc)
 	}
 	// the device applied the Results filter and kept the TopN best; pushing those through
 	// Results.Update leaves the heap exactly as pushing every group score would

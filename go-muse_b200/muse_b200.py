@@ -149,6 +149,8 @@ ABI = {
                                  _dp, _ip64, _ip64, _ip64]),
     "muse_batch_run_ex": (C.c_int, [_vp, _ip32, C.c_int32, C.c_int64, C.c_int64, C.c_double, C.c_int32,
                                     C.c_int32, C.c_int32, _dp, _ip64, _ip64, _ip64]),
+    "muse_batch_run_where": (C.c_int, [_vp, _ip32, _ip32, C.c_int32, _ip32, C.c_int32, C.c_int64, C.c_int64, C.c_double,
+                                       C.c_int32, C.c_int32, C.c_int32, _dp, _ip64, _ip64, _ip64]),
     "muse_batch_score_all": (C.c_int, [_vp, C.c_int32, _dp, _ip32]),
     "muse_batch_xcorr": (C.c_int, [_vp, C.c_int64, _dp, _ip32]),
     "muse_batch_screen_bounds": (C.c_int, [_vp, C.c_int32, C.c_int64, _vp, _vp]),
@@ -368,6 +370,28 @@ class DeviceBatch:
         _check(lib().muse_batch_run_ex(self.h, kc.ctypes.data_as(_ip32) if kc.size else None, kc.size, max_lag, top_n,
                                        threshold, sign_filter, mode, int(signed_scores), _d(sc),
                                        lg.ctypes.data_as(_ip64), ix.ctypes.data_as(_ip64), C.byref(n_out)))
+        k = int(n_out.value)
+        return sc[:k], lg[:k], ix[:k]
+
+    def run_where(self, where_cols: Sequence[int], where_ids: Sequence[int], key_cols: Sequence[int], max_lag: int, top_n: int,
+                  threshold: float, sign_filter: int = 0, mode: int = MODE_AUTO, signed_scores: bool = False):
+        """muse_batch_run_where: run() over the series whose label id in column where_cols[j] is where_ids[j] for every j;
+        indices are those of the whole store."""
+        wc = np.asarray(list(where_cols), dtype=np.int32)
+        wi = np.asarray(list(where_ids), dtype=np.int32)
+        if wc.size != wi.size:
+            raise MuseError(MUSE_ERR_INVALID_ARG, "run_where: %d where columns, %d ids" % (wc.size, wi.size))
+        cap = max(1, int(top_n))
+        sc = np.zeros(cap)
+        lg = np.zeros(cap, dtype=np.int64)
+        ix = np.zeros(cap, dtype=np.int64)
+        n_out = C.c_int64(0)
+        kc = np.asarray(list(key_cols), dtype=np.int32)
+        _check(lib().muse_batch_run_where(self.h, wc.ctypes.data_as(_ip32) if wc.size else None,
+                                          wi.ctypes.data_as(_ip32) if wi.size else None, wc.size,
+                                          kc.ctypes.data_as(_ip32) if kc.size else None, kc.size, max_lag, top_n, threshold,
+                                          sign_filter, mode, int(signed_scores), _d(sc), lg.ctypes.data_as(_ip64),
+                                          ix.ctypes.data_as(_ip64), C.byref(n_out)))
         k = int(n_out.value)
         return sc[:k], lg[:k], ix[:k]
 
@@ -707,6 +731,21 @@ class Group:
             self._uploaded = len(self.series)
         return self._store
 
+    def _where(self, labels: Labels) -> Optional[Tuple[List[int], List[int]]]:
+        """(columns, ids) of the equalities of FilterByLabelValues(labels) on the device store; None when no series can
+        match: empty labels, or a key or value no series of the store has."""
+        keys = labels.Keys()
+        if not keys:
+            return None
+        cols, ids = [], []
+        for k in keys:
+            v, _ = labels.Get(k)
+            if k not in self._cols or v not in self._dict[k]:
+                return None
+            cols.append(self._cols.index(k))
+            ids.append(self._dict[k][v])
+        return cols, ids
+
     def _key_cols(self, group_by: Optional[List[str]]) -> List[int]:
         if not group_by:
             return []
@@ -850,6 +889,28 @@ class Batch:
         # the device applies the Results filter and keeps the TopN best; pushing those through
         # Results.Update leaves the heap exactly as pushing every group score would
         sc, lg, ix = self._batch.run(cols, r.MaxLag, r.TopN, r.Threshold, r.SignFilter, mode=self.mode)
+        for s, l, i in zip(sc, lg, ix):
+            r.Update(Score(comp.series[int(i)].Labels(), int(l), float(s)))
+        return None
+
+
+    def RunWhere(self, labels: Labels, groupByLabels: Optional[List[str]] = None):
+        """Run over the series of Comparison.FilterByLabelValues(labels) only, on the resident store: Results end up as
+        NewBatch(ref, <a Group of those series>, ...).Run(groupByLabels) leaves them.  Nothing matches (empty labels, a key
+        or value no series has): no device call, Results untouched.  Always returns None (nil)."""
+        comp = self.Comparison
+        if not comp.series or not labels.Keys():
+            return None
+        store = comp._sync_device()          # uploads series added since the last call; the dictionary then knows every value
+        where = comp._where(labels)
+        if where is None:
+            return None
+        if self._batch is None or self._batch.store is not store:
+            self._batch = DeviceBatch(store.ctx, store, self._ref)
+        r = self.Results
+        cols = comp._key_cols(groupByLabels)
+        sc, lg, ix = self._batch.run_where(where[0], where[1], cols, r.MaxLag, r.TopN, r.Threshold, r.SignFilter,
+                                           mode=self.mode)
         for s, l, i in zip(sc, lg, ix):
             r.Update(Score(comp.series[int(i)].Labels(), int(l), float(s)))
         return None

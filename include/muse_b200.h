@@ -200,6 +200,20 @@ int  muse_batch_run_ex(muse_batch *b, const int32_t *key_cols, int32_t n_key_col
                        int32_t mode, int32_t signed_scores,
                        double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out);
 
+/* Batch.Run restricted to the series of the store whose label ids match: series i takes part when
+ * labels[where_cols[j]][i] == where_ids[j] for every j < n_where (go-muse's Group.FilterByLabelValues, group.go:60-71:
+ * a series that lacks a key does not match it).  Returns what muse_batch_run_ex returns on a store that holds only the
+ * matching series in the same order, with each record's series_idx the index of that series in THIS store (plus the
+ * global offset).  n_where == 0: the whole store, exactly muse_batch_run_ex.  Nothing matches: *n_out = 0, MUSE_OK.
+ * Argument errors (n_where < 0 or > 16, NULL where arrays with n_where > 0, a column outside [0, n_label_keys),
+ * a negative id) return MUSE_ERR_INVALID_ARG before any device work.  Timings: muse_batch_last_timing.
+ * The selection (ascending local rows) is built on the device from the n_where label columns alone; only the selected
+ * rows are read by the scoring pass, and the run takes the path (muse_timing.mode) a store of just those rows would take. */
+int  muse_batch_run_where(muse_batch *b, const int32_t *where_cols, const int32_t *where_ids, int32_t n_where,
+                          const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n, double threshold,
+                          int32_t sign_filter, int32_t mode, int32_t signed_scores,
+                          double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out);
+
 /* Per-series (score, lag) of every series in the store, exact fp64 path
  * (xCorrWithX + abs/clamp per series; what scoreSingle's loop computes,
  * muse_batch.go:68-77).  Host outputs of muse_group_size() entries. */
