@@ -232,6 +232,7 @@ struct muse_ctx {
     PinnedBuf h_stage[3];           // pinned staging ring for rows that arrive in pageable host memory (muse_group_append, muse_group_roll)
     Events<3> stage_ev;
     DevBuf<double> d_roll;          // device buffer of the new samples of muse_group_roll: at most MUSE_STAGE_BYTES
+    DevBuf<int2> d_moves;           // (from, to) row pairs of muse_group_remove: MUSE_MOVE_CHUNK entries once the first row moves
     // multi-query bounds on the tensor cores (muse_bounds_tc.cuh): magnitudes of the store and weights of a launch's queries
     DevBuf<unsigned char> tc_a, tc_b;     // bf16 tiles: [S/128][16][16 KB] and [16][32 KB]
     DevBuf<float> tc_mid, tc_amid;        // [S] |2Y_(M/2)| per series, [256] A_q[M/2] per query
@@ -817,6 +818,69 @@ extern "C" int muse_group_roll(muse_group *g, int64_t first, int64_t n_rows, con
         if (rc != MUSE_OK) return rc;
     }
     CU(cudaStreamSynchronize(st));
+    return MUSE_OK;
+}
+
+static int refresh_row_stats(muse_group *g);
+
+// Removal moves only as many rows as were removed below the new size m: the removed rows below m ("holes", ascending) take
+// the kept rows at or above m ("fillers", ascending), the j-th hole the j-th filler.  Finding them is O(n_rows) on the host
+// (the fillers are [m, size) minus the listed rows there).  The pairs reach the device in chunks of MUSE_MOVE_CHUNK through
+// ctx->d_moves (one buffer: the copy of chunk c + 1 is queued behind the kernel of chunk c on the same stream).
+#define MUSE_MOVE_CHUNK ((int64_t)1 << 20)
+extern "C" int muse_group_remove(muse_group *g, const int64_t *rows, int64_t n_rows, int64_t *moved_from, int64_t *moved_to,
+                                 int64_t *n_moved) {
+    if (!g || !n_moved) return fail(MUSE_ERR_INVALID_ARG, "muse_group_remove: NULL argument");
+    *n_moved = 0;
+    if (n_rows < 0 || n_rows > g->size)
+        return fail(MUSE_ERR_INVALID_ARG, "muse_group_remove: %lld rows of a store of %lld", (long long)n_rows, (long long)g->size);
+    if (!rows && n_rows > 0) return fail(MUSE_ERR_INVALID_ARG, "muse_group_remove: rows is NULL");
+    if (!moved_from != !moved_to) return fail(MUSE_ERR_INVALID_ARG, "muse_group_remove: one of moved_from / moved_to is NULL");
+    for (int64_t i = 0; i < n_rows; i++)
+        if (rows[i] < 0 || rows[i] >= g->size || (i > 0 && rows[i] <= rows[i - 1]))
+            return fail(MUSE_ERR_INVALID_ARG, "muse_group_remove: rows[%lld] = %lld is outside [0, %lld), repeated or out of order",
+                        (long long)i, (long long)rows[i], (long long)g->size);
+    if (n_rows == 0) return MUSE_OK;
+    const int64_t m = g->size - n_rows;
+    const int64_t holes = std::lower_bound(rows, rows + n_rows, m) - rows;
+    std::vector<int2> mv((size_t)holes);
+    for (int64_t j = 0, k = holes, r = m; j < holes; r++) {
+        if (k < n_rows && rows[k] == r) {
+            k++;      // a removed row at or above m: not a filler
+        } else {
+            mv[(size_t)j] = make_int2((int)r, (int)rows[j]);
+            j++;
+        }
+    }
+    muse_ctx *c = g->ctx;
+    CU(cudaSetDevice(c->device));
+    cudaStream_t st = c->stream;
+    int rc = refresh_row_stats(g);      // the moved rows carry their statistics: all of them must exist first
+    if (rc) return rc;
+    if (holes > 0) CU(c->d_moves.grow(MUSE_MOVE_CHUNK));
+    for (int64_t c0 = 0; c0 < holes; c0 += MUSE_MOVE_CHUNK) {
+        const int64_t nc = std::min<int64_t>(MUSE_MOVE_CHUNK, holes - c0);
+        CU(cudaMemcpyAsync(c->d_moves, mv.data() + c0, sizeof(int2) * (size_t)nc, cudaMemcpyHostToDevice, st));
+        CU(launch_move_rows(g->slab, g->ld, g->row_stat, g->labels, g->nkeys, g->cap, c->d_moves, nc, c->sm_count, st));
+    }
+    g->size = g->stats_upto = m;
+    // max_id over the rows that remain, as a fresh store of them has it (group-key widths depend on it); the old values stay
+    // if that fails: they are still upper bounds
+    int32_t old[MUSE_MAX_LABEL_KEYS];
+    memcpy(old, g->max_id, sizeof(old));
+    for (int k = 0; k < MUSE_MAX_LABEL_KEYS; k++) g->max_id[k] = -1;
+    rc = refresh_max_ids(g, 0, m);
+    if (rc) {
+        memcpy(g->max_id, old, sizeof(old));
+        return rc;
+    }
+    CU(cudaStreamSynchronize(st));
+    if (moved_from)
+        for (int64_t j = 0; j < holes; j++) {
+            moved_from[j] = mv[(size_t)j].x;
+            moved_to[j] = mv[(size_t)j].y;
+        }
+    *n_moved = holes;
     return MUSE_OK;
 }
 

@@ -83,6 +83,11 @@ cudaError_t launch_bounds_tc(const TcBoundsParams &p, cudaStream_t st);
 cudaError_t launch_roll_rows(double *slab, int64_t ld, int N, int64_t first, int64_t count, const double *d_add, int k,
                              RowStat *stat, int sm_count, cudaStream_t st);
 
+// local row d_moves[i].x -> local row d_moves[i].y for i < count: the whole ld-wide row, its RowStat and its id in each of the
+// nkeys label columns [nkeys][cap]; no source may be a destination (kernels_remove.cu)
+cudaError_t launch_move_rows(double *slab, int64_t ld, RowStat *stat, int32_t *labels, int nkeys, int64_t cap, const int2 *d_moves,
+                             int64_t count, int sm_count, cudaStream_t st);
+
 // ---- series above n = 16384 (kernels_long.cu): Stockham passes through global memory, two series per transform ----
 struct LongParams {
     const double *slab;      // [rows][ld] fp64

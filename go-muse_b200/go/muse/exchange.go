@@ -90,6 +90,7 @@ func (e *Exchange) Close() {
 // process, so that the int32 ids the device groups by mean the same labels everywhere.  Call before the first
 // NewBatch on the group.
 func (g *Group) SetShard(first int64, dictionary map[string][]string) {
+	g.sharded = true
 	g.shardFirst = first
 	g.fixedDict = dictionary
 	if g.store != nil { // re-encode with the fixed ids

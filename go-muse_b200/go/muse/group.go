@@ -66,6 +66,7 @@ type Group struct {
 
 	// sharded groups (exchange.go): index of this block's first series in the whole group, and the label dictionary
 	// every process agreed on
+	sharded    bool
 	shardFirst int64
 	fixedDict  map[string][]string
 }
@@ -146,11 +147,14 @@ func (g *Group) syncDevice() error {
 		keys = append(keys, k)
 	}
 	sort.Strings(keys)
-	same := len(keys) == len(g.cols)
-	for i := 0; same && i < len(keys); i++ {
-		same = keys[i] == g.cols[i]
+	// a new key needs a column; a key that Remove took from every series keeps its column (all ids -1 now), which groups
+	// and filters as an absent key does, so the store is not rebuilt
+	known := true
+	for _, k := range keys {
+		c := sort.SearchStrings(g.cols, k)
+		known = known && c < len(g.cols) && g.cols[c] == k
 	}
-	if g.store == nil || !same {
+	if g.store == nil || !known {
 		if g.store != nil {
 			C.muse_group_destroy(g.store)
 			g.store = nil
@@ -275,6 +279,93 @@ func (g *Group) Roll(samples [][]float64) error {
 		s.vals = append(v, samples[i]...)
 	}
 	return nil
+}
+
+// Remove takes series out of the group, matched by UID (go-muse has no counterpart).  A series that is not a member is an
+// error and nothing is removed; a series named twice is removed once.  With a device store the removal is in place
+// (muse_group_remove): the remaining series keep their positions, except that the last ones move into the places of
+// removed ones, and the Group's series make the same moves (the library's pairs).  Batches stay bound: the store is not
+// replaced.  Without a store, or when the device call fails (the store is then dropped and rebuilt by the next call that
+// needs it), the remaining series keep their order.  A group that becomes empty forgets its length, as a new Group.
+// Remove then Add of the same UID replaces a series; g.Remove(g.FilterByLabelValues(l)...) removes a label set.
+// A sharded group (SetShard) cannot remove: ShardScore.Index counts over all shards.
+func (g *Group) Remove(series ...*Series) error {
+	if g.sharded {
+		return errors.New("Remove: a sharded group cannot remove series")
+	}
+	idx := make(map[int]bool, len(series))
+	for _, s := range series {
+		i, ok := g.registry[s.UID()]
+		if !ok {
+			return fmt.Errorf("Series with label:values, %v, is not within group, %s", s.UID(), g.Name)
+		}
+		idx[i] = true
+	}
+	if len(idx) == 0 {
+		return nil
+	}
+	if len(idx) == len(g.series) || g.store == nil {
+		if g.store != nil {
+			C.muse_group_destroy(g.store)
+			g.store = nil
+		}
+		g.removeInOrder(idx)
+		return nil
+	}
+	if err := g.syncDevice(); err != nil {
+		return err
+	}
+	rows := make([]int64, 0, len(idx))
+	for i := range idx {
+		rows = append(rows, int64(i))
+	}
+	sort.Slice(rows, func(a, b int) bool { return rows[a] < rows[b] })
+	from := make([]int64, len(rows))
+	to := make([]int64, len(rows))
+	var moved C.int64_t
+	if rc := C.muse_group_remove(g.store, (*C.int64_t)(unsafe.Pointer(&rows[0])), C.int64_t(len(rows)), (*C.int64_t)(unsafe.Pointer(&from[0])),
+		(*C.int64_t)(unsafe.Pointer(&to[0])), &moved); rc != C.MUSE_OK {
+		err := lastError(rc)
+		C.muse_group_destroy(g.store)
+		g.store = nil
+		g.removeInOrder(idx)
+		return err
+	}
+	for _, r := range rows {
+		delete(g.registry, g.series[r].UID())
+	}
+	for j := 0; j < int(moved); j++ {
+		g.series[to[j]] = g.series[from[j]]
+		g.registry[g.series[to[j]].UID()] = int(to[j])
+	}
+	m := len(g.series) - len(rows)
+	for i := m; i < len(g.series); i++ {
+		g.series[i] = nil
+	}
+	g.series = g.series[:m]
+	g.uploaded = m
+	return nil
+}
+
+// removeInOrder drops the series at the indices in idx from the host lists, keeping the order of the others.
+func (g *Group) removeInOrder(idx map[int]bool) {
+	kept := g.series[:0]
+	for i, s := range g.series {
+		if !idx[i] {
+			kept = append(kept, s)
+		}
+	}
+	for i := len(kept); i < len(g.series); i++ {
+		g.series[i] = nil
+	}
+	g.series = kept
+	g.registry = make(map[string]int, len(kept))
+	for i, s := range kept {
+		g.registry[s.UID()] = i
+	}
+	if len(kept) == 0 {
+		g.n = 0
+	}
 }
 
 // keyCols maps label names to device columns; unknown names mean "no series has it", which

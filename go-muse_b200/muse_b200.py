@@ -47,7 +47,8 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", 
 # translation units of libmuse_b200.so: the C ABI and one file per family of kernel instantiations
 SOURCES = ["muse_api.cu", "kernels_exact.cu", "kernels_screen_warp.cu", "kernels_screen_big.cu", "kernels_screen_big13_a.cu", "kernels_screen_big13_b.cu", "kernels_screen_big13_c.cu",
            "kernels_screen_big13_d.cu", "kernels_screen_multi.cu", "kernels_bounds_tc.cu", "kernels_long.cu",
-           "kernels_screen_sub1.cu", "kernels_screen_sub2.cu", "kernels_screen_sub3.cu", "kernels_screen_sub4.cu", "kernels_roll.cu"]
+           "kernels_screen_sub1.cu", "kernels_screen_sub2.cu", "kernels_screen_sub3.cu", "kernels_screen_sub4.cu", "kernels_roll.cu",
+           "kernels_remove.cu"]
 
 
 class MuseError(Exception):
@@ -142,6 +143,7 @@ ABI = {
     "muse_group_read_rows": (C.c_int, [_vp, C.c_int64, C.c_int64, _vp]),
     "muse_group_roll": (C.c_int, [_vp, C.c_int64, C.c_int64, _vp, C.c_int64]),
     "muse_group_roll_device": (C.c_int, [_vp, C.c_int64, C.c_int64, _vp, C.c_int64]),
+    "muse_group_remove": (C.c_int, [_vp, _ip64, C.c_int64, _ip64, _ip64, _ip64]),
     "muse_batch_create": (C.c_int, [_vp, _vp, _dp, C.c_int64, C.POINTER(_vp)]),
     "muse_batch_destroy": (None, [_vp]),
     "muse_batch_fft_len": (C.c_int64, [_vp]),
@@ -313,6 +315,17 @@ class DeviceStore:
     def roll_device(self, ptr: int, first: int, n_rows: int, k: int):
         """muse_group_roll_device: as roll, the [n_rows][k] samples in DEVICE memory at address ptr."""
         _check(lib().muse_group_roll_device(self.h, first, n_rows, _vp(ptr), k))
+
+    def remove(self, rows) -> Tuple[np.ndarray, np.ndarray]:
+        """muse_group_remove: the local rows `rows` (strictly ascending) leave the store, in place.  Returns (moved_from,
+        moved_to): the kept rows at or above the new size that took the places of removed rows below it, in that order."""
+        r = np.ascontiguousarray(rows, dtype=np.int64).reshape(-1)
+        moved_from = np.zeros(max(r.size, 1), dtype=np.int64)
+        moved_to = np.zeros(max(r.size, 1), dtype=np.int64)
+        n_moved = C.c_int64(0)
+        _check(lib().muse_group_remove(self.h, r.ctypes.data_as(_ip64) if r.size else None, r.size, moved_from.ctypes.data_as(_ip64),
+                                       moved_to.ctypes.data_as(_ip64), C.byref(n_moved)))
+        return moved_from[:n_moved.value], moved_to[:n_moved.value]
 
     def read_rows_ptr(self, first: int, n_rows: int, ptr: int):
         _check(lib().muse_group_read_rows(self.h, first, n_rows, _vp(ptr)))
@@ -696,6 +709,51 @@ class Group:
             s.y = np.concatenate([s.y[k:], r])
         return None
 
+    def Remove(self, *series: Series):
+        """Takes series out of the group, matched by UID(); a series that is not a member raises MuseError and nothing is
+        removed (a series named twice is removed once).  With a device store the removal is in place (muse_group_remove):
+        the remaining series keep their positions, except that the last ones move into the places of removed ones, and
+        self.series makes the same moves (the library's pairs).  Without a store, or when the device call fails (the store
+        is then dropped and rebuilt by the next call that needs it), the remaining series keep their order.  A group that
+        becomes empty forgets its length, as a new Group.  Remove then Add of the same UID replaces a series."""
+        idx = set()
+        for s in series:
+            i = self.registry.get(s.UID())
+            if i is None:
+                raise MuseError(MUSE_ERR_INVALID_ARG, "Series with label:values, %s, is not within group, %s" % (s.UID(), self.Name))
+            idx.add(i)
+        if not idx:
+            return None
+        if len(idx) == len(self.series) or self._store is None:
+            if self._store is not None:
+                self._store.close()
+                self._store = None
+            self._remove_in_order(idx)
+            return None
+        store = self._sync_device()
+        rows = sorted(idx)
+        try:
+            moved_from, moved_to = store.remove(rows)
+        except MuseError:
+            store.close()
+            self._store = None
+            self._remove_in_order(idx)
+            raise
+        for i in rows:
+            del self.registry[self.series[i].UID()]
+        for f, t in zip(moved_from.tolist(), moved_to.tolist()):
+            self.series[t] = self.series[f]
+            self.registry[self.series[t].UID()] = t
+        del self.series[len(self.series) - len(rows):]
+        self._uploaded = len(self.series)
+        return None
+
+    def _remove_in_order(self, idx):
+        self.series = [s for i, s in enumerate(self.series) if i not in idx]
+        self.registry = {s.UID(): i for i, s in enumerate(self.series)}
+        if not self.series:
+            self.n = 0
+
     def FilterByLabelValues(self, labels: Labels) -> List[Series]:
         """group.go:60-71: members whose values match on every key of `labels`."""
         keys = labels.Keys()
@@ -709,7 +767,9 @@ class Group:
     def _sync_device(self) -> DeviceStore:
         ctx = self._ctx or default_context()
         keys = sorted({k for s in self.series for k in s.labels.Keys()})
-        if self._store is None or keys != self._cols:
+        # a new key needs a column; a key that Remove took from every series keeps its column (all ids -1 now), which groups
+        # and filters as an absent key does, so the store is not rebuilt
+        if self._store is None or not set(keys) <= set(self._cols):
             if self._store is not None:
                 self._store.close()
             self._cols = keys

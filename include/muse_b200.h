@@ -161,6 +161,21 @@ int  muse_group_read_rows(muse_group *g, int64_t first, int64_t n_rows, double *
 int  muse_group_roll(muse_group *g, int64_t first, int64_t n_rows, const double *samples, int64_t k);
 int  muse_group_roll_device(muse_group *g, int64_t first, int64_t n_rows, const double *d_samples, int64_t k);
 
+/* Remove rows[0 .. n_rows) from the store, in place.  rows: local indices, strictly ascending, in [0, size).
+ * The store keeps m = size - n_rows rows.  Kept rows below m stay where they are.  The removed rows below m ("holes",
+ * ascending) take the kept rows at or above m ("fillers", ascending): the j-th hole receives the j-th filler, with its
+ * label ids and row statistics.  So a removal moves as many rows as it removes below m, never the rest of the store, and
+ * the order of the remaining series changes exactly as the pairs say.  moved_from / moved_to (host, capacity n_rows each;
+ * both NULL or both non-NULL) receive the *n_moved pairs (old local index -> new local index) in that order.  Capacity,
+ * global offset and every batch of the store are kept; batches see the new rows, and every run, label-key width and
+ * MUSE_ERR_UNSUPPORTED answer is what a fresh store that appended the remaining rows in their new order gives.  A later
+ * muse_group_append writes at index m.  Everything is complete when the call returns.  Argument errors (NULL g or n_moved;
+ * NULL rows with n_rows > 0; n_rows outside [0, size]; an index out of range, repeated or out of order; exactly one of
+ * moved_from / moved_to NULL) return MUSE_ERR_INVALID_ARG before any device work and leave the store untouched;
+ * n_rows == 0 does nothing and sets *n_moved = 0.  After any other error the store's rows are unspecified: destroy it. */
+int  muse_group_remove(muse_group *g, const int64_t *rows, int64_t n_rows, int64_t *moved_from, int64_t *moved_to,
+                       int64_t *n_moved);
+
 /* ---- batch -----------------------------------------------------------------
  * NewBatch (muse_batch.go:23-52): checks ref_len against the group
  * (MUSE_ERR_LENGTH_MISMATCH), n = nextPowOf2(ref_len), computes on the device
