@@ -1,4 +1,4 @@
-// kernels_screen_multi.cu -- instantiations of refine_multi_kernel<NZ> (muse_screen_multi.cuh), n = 2048.
+// kernels_screen_multi.cu -- instantiations of refine_multi_kernel<NZ, LIST> (muse_screen_multi.cuh), n = 2048.
 #include "muse_launch.h"
 
 namespace muse {
@@ -6,7 +6,7 @@ namespace muse {
 cudaError_t launch_refine_multi(const ScreenParams &p, const MultiQuery *d_queries, int nq, int sm_count, unsigned *d_next, cudaStream_t st) {
     using C = RefineMultiCfg;
     return dispatch_nz(ScreenWarpCfg::nz(p.N), [&](auto nz) {
-        auto kern = refine_multi_kernel<decltype(nz)::value>;
+        auto kern = p.rows ? refine_multi_kernel<decltype(nz)::value, true> : refine_multi_kernel<decltype(nz)::value, false>;
         const int warps = C::warps(p.N);
         const size_t smem = C::smem_bytes(p.N);
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);

@@ -245,6 +245,8 @@ struct muse_ctx {
     DevBuf<MultiQuery> d_multi_q;   // query table of refine_multi_kernel (MUSE_MULTI_GROUP entries)
     DevBuf<double> d_multi_refs;    // [MUSE_MULTI_GROUP][d_multi_ld] reference rows of a muse_multi_run group, pad columns kept zero
     int64_t d_multi_ld = 0, d_multi_n = 0;
+    DevBuf<int32_t> d_where_rows;   // muse_multi_run_where: the selection shared by every reference of the call (ascending local rows)
+    DevBuf<int32_t> d_where_off;    // its per-tile offsets, then its length
 };
 
 struct muse_group {
@@ -275,7 +277,8 @@ struct muse_batch : RunScratch {
     int fused_run = 0;         // 1: score_fused, 2: score_fused_grouped (d_counters: listed = exact list length)
     int prescreened = 0;       // d_U and the cut-off state were filled by the tensor-core multi-query path: the next fused run starts at its tail
     int signed_run = 0;        // the current run keeps the sign of the scores (muse.go:72-76)
-    int64_t where_m = -1;      // a filtered run (muse_batch_run_where) is under way over the where_m rows of d_rows; -1: none
+    int64_t where_m = -1;      // a filtered run (muse_batch_run_where) is under way over the where_m rows of where_rows; -1: none
+    const int32_t *where_rows = nullptr;   // that run's selection: d_rows, or the selection of muse_multi_run_where (muse_ctx)
     int pre_launches = -1;     // launches muse_batch_run_where queued (after recording ev[0]) before the run it starts; -1: none
     // n > MUSE_MAX_FUSED_FFT_LEN: Stockham passes through global memory (kernels_long.cu); Xt holds n entries, twM the n twiddles
     int is_long = 0;
@@ -291,11 +294,11 @@ using BatchPtr = std::unique_ptr<muse_batch, BatchDestroy>;   // a batch that go
 
 static inline cudaStream_t bstream(const muse_batch *b) { return b->ctx->stream; }
 
-// The rows the current run scores: a filtered run's selection (d_rows[0 .. where_m)), else every row of the store (NULL).
+// The rows the current run scores: a filtered run's selection (where_rows[0 .. where_m)), else every row of the store (NULL).
 // Everything that depends on the size of the store -- the AUTO rule, launch bounds, what a fallback scores -- uses
 // run_count, so a filtered run takes the path a store of just its rows would take.
 static inline int64_t run_count(const muse_batch *b) { return b->where_m >= 0 ? b->where_m : b->g->size; }
-static inline const int32_t *run_rows(const muse_batch *b) { return b->where_m >= 0 ? b->d_rows.get() : nullptr; }
+static inline const int32_t *run_rows(const muse_batch *b) { return b->where_m >= 0 ? b->where_rows : nullptr; }
 
 // ------------------------------------------------------------------------------------
 // context
@@ -1579,17 +1582,18 @@ static int arm_refinement(muse_batch *b, ScreenParams &sp, float cut0, int64_t m
 }
 
 // idx list of every series whose (refined) bound reaches the final cut-off, read from device memory, into n->listed (the
-// refined count rides along)
+// refined count rides along).  rows: bound i belongs to the store's row rows[i] (a selection), which goes into the list;
+// NULL: row i
 __device__ __forceinline__ void survivors_cut_body(const float *__restrict__ U, int64_t S, const CutState *__restrict__ cut,
-                                                   int32_t *__restrict__ out, RunCounters *n) {
+                                                   int32_t *__restrict__ out, RunCounters *n, const int32_t *__restrict__ rows) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i == 0) n->refined = cut->refined;
     const float lo = __uint_as_float(cut->bits);
-    warp_append(&n->listed, i < S && U[i] >= lo, [&](unsigned long long pos) { out[pos] = (int32_t)i; });
+    warp_append(&n->listed, i < S && U[i] >= lo, [&](unsigned long long pos) { out[pos] = rows ? rows[i] : (int32_t)i; });
 }
 __global__ void survivors_cut_kernel(const float *__restrict__ U, int64_t S, const CutState *__restrict__ cut,
                                      int32_t *__restrict__ out, RunCounters *n) {
-    survivors_cut_body(U, S, cut, out, n);
+    survivors_cut_body(U, S, cut, out, n, nullptr);
 }
 
 // the batched tails of muse_multi_run: blockIdx.y = query (MultiTail, muse_select.cuh)
@@ -1597,9 +1601,9 @@ __global__ void tail_reset_kernel(const MultiTail *__restrict__ tails, int nq) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q < nq) *tails[q].counters = RunCounters{0ull, 0ull, 0ull, 0ull};
 }
-__global__ void survivors_cut_batch_kernel(const MultiTail *__restrict__ tails, int64_t S) {
+__global__ void survivors_cut_batch_kernel(const MultiTail *__restrict__ tails, int64_t S, const int32_t *__restrict__ rows) {
     const MultiTail t = tails[blockIdx.y];
-    survivors_cut_body(t.U, S, t.cut, t.list, t.counters);
+    survivors_cut_body(t.U, S, t.cut, t.list, t.counters, rows);
 }
 // reference preparation of a launch's queries: screen_tables_kernel with blockIdx.y = query; the 4 floats of every query
 // (std-zero flag, A[M/2], Xt[M/2]) land in ONE array for one copy to the host
@@ -2028,62 +2032,55 @@ __global__ void where_neutral_kernel(double *__restrict__ score, float *__restri
     L[i] = -1.f;
 }
 
-// The selection of a predicate into d_rows (ascending local rows); its length.
-static int select_where(muse_batch *b, const WherePred &p, int64_t &m) {
-    const int64_t S = b->g->size;
-    cudaStream_t st = bstream(b);
+// The predicate where_cols[j] == where_ids[j] (j < n_where) on the label columns of g, after the argument checks of a
+// filtered run (fn names the entry point in the message).
+static int where_pred(const muse_group *g, const int32_t *where_cols, const int32_t *where_ids, int32_t n_where, const char *fn,
+                      WherePred &p) {
+    if (n_where < 0 || n_where > MUSE_WHERE_MAX)
+        return fail(MUSE_ERR_INVALID_ARG, "%s: %d where columns (0 .. %d)", fn, (int)n_where, MUSE_WHERE_MAX);
+    if (n_where > 0 && (!where_cols || !where_ids)) return fail(MUSE_ERR_INVALID_ARG, "%s: NULL where arrays", fn);
+    memset(&p, 0, sizeof(p));
+    p.n = n_where;
+    for (int j = 0; j < n_where; j++) {
+        if (where_cols[j] < 0 || where_cols[j] >= g->nkeys)
+            return fail(MUSE_ERR_INVALID_ARG, "%s: where column %d not in [0,%d)", fn, (int)where_cols[j], g->nkeys);
+        if (where_ids[j] < 0) return fail(MUSE_ERR_INVALID_ARG, "%s: negative label id %d", fn, (int)where_ids[j]);
+        p.col[j] = g->labels + (size_t)where_cols[j] * g->cap;
+        p.id[j] = where_ids[j];
+    }
+    return MUSE_OK;
+}
+
+// The selection of a predicate over the store's size() rows into rows (room for size() entries; ascending local rows), queued
+// on the context's stream with off as the per-tile scratch; its length.
+static int select_where(muse_ctx *ctx, const muse_group *g, const WherePred &p, int32_t *rows, DevBuf<int32_t> &off, int64_t &m) {
+    const int64_t S = g->size;
+    cudaStream_t st = ctx->stream;
     const int64_t nb = (S + MUSE_WHERE_TILE - 1) / MUSE_WHERE_TILE;
-    CU(b->d_where_off.grow(nb + 1));
-    where_count_kernel<<<(unsigned)nb, 256, 0, st>>>(p, S, b->d_where_off);
-    where_scan_kernel<<<1, 1024, 0, st>>>(b->d_where_off, nb);
-    where_write_kernel<<<(unsigned)nb, 256, 0, st>>>(p, S, b->d_where_off, b->d_rows);
+    CU(off.grow(nb + 1));
+    where_count_kernel<<<(unsigned)nb, 256, 0, st>>>(p, S, off);
+    where_scan_kernel<<<1, 1024, 0, st>>>(off, nb);
+    where_write_kernel<<<(unsigned)nb, 256, 0, st>>>(p, S, off, rows);
     CU(cudaGetLastError());
     int32_t h_m = 0;                      // one small copy: the host sizes the launches and takes the AUTO decision on it
-    CU(cudaMemcpyAsync(&h_m, b->d_where_off.get() + nb, sizeof(h_m), cudaMemcpyDeviceToHost, st));
+    CU(cudaMemcpyAsync(&h_m, off.get() + nb, sizeof(h_m), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     m = h_m;
     return MUSE_OK;
 }
 
-extern "C" int muse_batch_run_where(muse_batch *b, const int32_t *where_cols, const int32_t *where_ids, int32_t n_where,
-                                    const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n, double threshold,
-                                    int32_t sign_filter, int32_t mode, int32_t signed_scores, double *scores, int64_t *lags,
-                                    int64_t *series_idx, int64_t *n_out) {
-    int rc = check_batch(b);
-    if (rc) return rc;
-    if (n_where < 0 || n_where > MUSE_WHERE_MAX)
-        return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: %d where columns (0 .. %d)", (int)n_where, MUSE_WHERE_MAX);
-    if (n_where > 0 && (!where_cols || !where_ids)) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: NULL where arrays");
-    muse_group *g = b->g;
-    WherePred p;
-    memset(&p, 0, sizeof(p));
-    p.n = n_where;
-    for (int j = 0; j < n_where; j++) {
-        if (where_cols[j] < 0 || where_cols[j] >= g->nkeys)
-            return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: where column %d not in [0,%d)", (int)where_cols[j], g->nkeys);
-        if (where_ids[j] < 0) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: negative label id %d", (int)where_ids[j]);
-        p.col[j] = g->labels + (size_t)where_cols[j] * g->cap;
-        p.id[j] = where_ids[j];
-    }
-    if (n_where == 0 || g->size == 0)
-        return muse_batch_run_ex(b, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores, scores, lags,
-                                 series_idx, n_out);
-    if (!n_out || (top_n > 0 && (!scores || !lags || !series_idx))) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: NULL output");
-    if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: bad key columns");
-    CU(cudaSetDevice(b->ctx->device));
+// The run of b over the m ascending local rows of `rows`, selected on the stream before this call.  The run's timing starts at
+// ev[0], which the caller recorded, and counts the caller's `launches` since then.
+static int run_selected(muse_batch *b, const int32_t *rows, int64_t m, int launches, const int32_t *key_cols, int32_t n_key_cols,
+                        int64_t max_lag, int64_t top_n, double threshold, int32_t sign_filter, int32_t mode, int32_t signed_scores,
+                        double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out) {
     *n_out = 0;
-    rc = ensure_scratch(b);
+    int rc = ensure_scratch(b);
     if (rc) return rc;
     rc = ensure_lower(b);
     if (rc) return rc;
-    // The timing of a filtered run starts here, before the selection, and counts its launches in every case below.
     cudaStream_t st = bstream(b);
-    CU(cudaEventRecord(b->ev[0], st));
-    int launches = 3;      // the selection: count, scan, write
-    int64_t m = 0;
-    rc = select_where(b, p, m);
-    if (rc) return rc;
-    const int64_t S = g->size;
+    const int64_t S = b->g->size;
     if (m == 0) {          // nothing matches: no records and nothing scored
         memset(&b->timing, 0, sizeof(b->timing));
         b->timing_pending = 0;
@@ -2095,17 +2092,48 @@ extern "C" int muse_batch_run_where(muse_batch *b, const int32_t *where_cols, co
     }
     struct EndWhere {      // every path out of the run leaves the batch unfiltered
         muse_batch *b;
-        ~EndWhere() { b->where_m = -1; b->pre_launches = -1; }
+        ~EndWhere() { b->where_m = -1; b->where_rows = nullptr; b->pre_launches = -1; }
     } end_where{b};
     if (m < S) {           // m == S: every row matches, the run of the whole store
         where_neutral_kernel<<<(unsigned)((S + 255) / 256), 256, 0, st>>>(b->d_score, b->d_U, b->d_L, S);
         CU(cudaGetLastError());
         launches++;
         b->where_m = m;
+        b->where_rows = rows;
     }
     b->pre_launches = launches;
     return muse_batch_run_ex(b, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores, scores, lags,
                              series_idx, n_out);
+}
+
+extern "C" int muse_batch_run_where(muse_batch *b, const int32_t *where_cols, const int32_t *where_ids, int32_t n_where,
+                                    const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n, double threshold,
+                                    int32_t sign_filter, int32_t mode, int32_t signed_scores, double *scores, int64_t *lags,
+                                    int64_t *series_idx, int64_t *n_out) {
+    int rc = check_batch(b);
+    if (rc) return rc;
+    muse_group *g = b->g;
+    WherePred p;
+    rc = where_pred(g, where_cols, where_ids, n_where, "muse_batch_run_where", p);
+    if (rc) return rc;
+    if (n_where == 0 || g->size == 0)
+        return muse_batch_run_ex(b, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores, scores, lags,
+                                 series_idx, n_out);
+    if (!n_out || (top_n > 0 && (!scores || !lags || !series_idx))) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: NULL output");
+    if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: bad key columns");
+    CU(cudaSetDevice(b->ctx->device));
+    *n_out = 0;
+    rc = ensure_scratch(b);
+    if (rc) return rc;
+    rc = ensure_lower(b);
+    if (rc) return rc;
+    // The timing of a filtered run starts here, before the selection, and counts its launches in every case.
+    CU(cudaEventRecord(b->ev[0], bstream(b)));
+    int64_t m = 0;
+    rc = select_where(b->ctx, g, p, b->d_rows, b->d_where_off, m);
+    if (rc) return rc;
+    return run_selected(b, b->d_rows, m, 3, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores,
+                        scores, lags, series_idx, n_out);      // 3 launches: the selection's count, scan, write
 }
 
 // ------------------------------------------------------------------------------------
@@ -2298,9 +2326,9 @@ extern "C" int muse_merge_partials(const muse_partial *parts, int64_t n_parts, i
 // ------------------------------------------------------------------------------------
 // The bounds of up to TcCfg::TN queries (batches bs[0 .. nq), FFT length 2048, tables built) against the whole store, as
 // one bf16 contraction on the tensor cores: magnitudes of every series -> tiles, the queries' weights -> tiles, GEMM with
-// the bound's epilogue into every batch's d_U.  Everything is queued on the context's stream.
-static int tc_bounds_queue(muse_ctx *ctx, muse_group *g, muse_batch **bs, int nq) {
-    const int64_t S = g->size;
+// the bound's epilogue into every batch's d_U.  Everything is queued on the context's stream.  rows: the S series are the
+// store's rows rows[0 .. S) (a selection; bound s is that of rows[s]), NULL: the store's S = size() rows.
+static int tc_bounds_queue(muse_ctx *ctx, muse_group *g, muse_batch **bs, int nq, const int32_t *rows, int64_t S) {
     cudaStream_t st = ctx->stream;
     CU(ctx->mt_ev.create());
     int rc = refresh_row_stats(g);
@@ -2325,6 +2353,8 @@ static int tc_bounds_queue(muse_ctx *ctx, muse_group *g, muse_batch **bs, int nq
     CU(cudaMemcpyAsync(ctx->tc_ptrs, h_ptrs, sizeof(h_ptrs), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(ctx->tc_amid, h_amid, sizeof(h_amid), cudaMemcpyHostToDevice, st));
     ScreenParams sp = screen_params(bs[0]);
+    sp.count = S;
+    sp.rows = rows;
     CU(cudaEventRecord(ctx->mt_ev[0], st));
     CU(launch_mag_tiles(sp, ctx->tc_a, ctx->tc_mid, ctx->sm_count, st));
     CU(launch_weight_tiles(reinterpret_cast<const float4 *const *>(ctx->tc_ptrs.get()), nq, ctx->tc_b, st));
@@ -2336,6 +2366,7 @@ static int tc_bounds_queue(muse_ctx *ctx, muse_group *g, muse_batch **bs, int nq
     tp.mid = ctx->tc_mid;
     tp.amid = ctx->tc_amid;
     tp.row_stat = g->row_stat;
+    tp.rows = rows;
     tp.out_U = reinterpret_cast<float *const *>(ctx->tc_ptrs + TcCfg::TN);
     tp.S = S;
     tp.nq = nq;
@@ -2374,17 +2405,28 @@ struct MultiTables {
     static size_t bytes(int64_t top_n) { return off_recs() + sizeof(PartialRec) * (size_t)Q * (size_t)std::max<int64_t>(top_n, 1); }
 };
 
+// The run of batch b over the m ascending local rows `rows` that muse_multi_run_where selected for all its references: what
+// muse_batch_run_where runs after its selection (its timing starts here).
+static int run_multi_selected(muse_batch *b, const int32_t *rows, int64_t m, const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag,
+                              int64_t top_n, double threshold, int32_t sign_filter, int32_t mode, double *scores, int64_t *lags,
+                              int64_t *series_idx, int64_t *n_out) {
+    CU(cudaEventRecord(b->ev[0], bstream(b)));
+    return run_selected(b, rows, m, 0, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0, scores, lags, series_idx,
+                        n_out);
+}
+
 // One launch group (<= 256 references) of muse_multi_run on the tensor-core path, with ONE launch per stage for all its
 // queries: reference spectra and tables (batched fp64 kernel in MODE_REF, blockIdx.y = query), cut-off states, bounds
 // (bf16 contraction), second stages (one pass over the store), survivors, fp64 re-scoring, filter, top-N -- and two
 // round trips to the host: the std-zero flags after the preparation, the list lengths before the re-scoring.  A query
 // whose lists do not fit the device-side select finishes alone on the single-query path.  The group's batches go into `bs`
-// (nq entries), which the caller keeps until the work queued on them has run.
-static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, int nq, int64_t ref_len, int64_t max_lag, int64_t top_n,
-                              double threshold, int32_t sign_filter, double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out,
-                              std::vector<BatchPtr> &bs) {
+// (nq entries), which the caller keeps until the work queued on them has run.  rows: the run covers the S series rows[0 .. S)
+// of the store (a selection, muse_multi_run_where): the magnitudes, bounds and second stages are compact over them and the
+// survivors' lists carry store rows, so the tails are those of a whole-store run.  NULL: the store's S = size() rows.
+static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const int32_t *rows, int64_t S, const double *refs, int nq, int64_t ref_len,
+                              int64_t max_lag, int64_t top_n, double threshold, int32_t sign_filter, double *scores, int64_t *lags,
+                              int64_t *series_idx, int64_t *n_out, std::vector<BatchPtr> &bs) {
     using MT = MultiTables;
-    const int64_t S = g->size;
     cudaStream_t st = ctx->stream;
     CU(ctx->d_mt.grow((int64_t)MT::bytes(top_n)));
     CU(ctx->h_mt.grow((int64_t)MT::bytes(top_n)));
@@ -2454,6 +2496,8 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
         ScreenParams sp = screen_params(b);
         rc = arm_refinement(b, sp, thr_lo, max_lag, top_n, threshold, true);
         if (rc) return rc;
+        sp.count = S;
+        sp.rows = rows;
         if (k == 0) sp0 = sp;
         MultiQuery &m = hq[(size_t)k];
         memset(&m, 0, sizeof(m));
@@ -2468,7 +2512,7 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
     CU(ctx->d_multi_next.grow(1));
     MultiQuery *d_q = ctx->d_multi_q;
     CU(cudaMemcpyAsync(d_q, hq.data(), sizeof(MultiQuery) * (size_t)nl, cudaMemcpyHostToDevice, st));
-    rc = tc_bounds_queue(ctx, g, lb.data(), nl);
+    rc = tc_bounds_queue(ctx, g, lb.data(), nl, rows, S);
     if (rc) return rc;
     CU(launch_refine_multi(sp0, d_q, nl, ctx->sm_count, ctx->d_multi_next, st));
     CU(cudaEventRecord(ctx->mt_ev[3], st));
@@ -2500,7 +2544,7 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
     CU(cudaMemcpyAsync(d + MT::off_tail(), h + MT::off_tail(), MT::off_mids() - MT::off_tail(), cudaMemcpyHostToDevice, st));
     const MultiTail *d_tail = reinterpret_cast<const MultiTail *>(d + MT::off_tail());
     tail_reset_kernel<<<(nl + 255) / 256, 256, 0, st>>>(d_tail, nl);
-    survivors_cut_batch_kernel<<<dim3((unsigned)((S + 255) / 256), (unsigned)nl), 256, 0, st>>>(d_tail, S);
+    survivors_cut_batch_kernel<<<dim3((unsigned)((S + 255) / 256), (unsigned)nl), 256, 0, st>>>(d_tail, S, rows);
     CU(cudaGetLastError());
     RunCounters *h_cnt = reinterpret_cast<RunCounters *>(h + MT::off_cnt());
     CU(cudaMemcpyAsync(h_cnt, d_cnt, sizeof(RunCounters) * (size_t)nl, cudaMemcpyDeviceToHost, st));
@@ -2528,10 +2572,16 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const double *refs, 
         ctx->multi_refined += (int64_t)h_cnt[k].refined;
         if (r[0].flags == 2) {
             // the list did not fit the device-side select (or the re-scoring launch): this query finishes alone, from its
-            // bounds and cut-off on the device (the fused run skips the screening of a prescreened batch)
+            // bounds and cut-off on the device (the fused run skips the screening of a prescreened batch) -- or, over a
+            // selection, whose bounds are compact and not those of the store's rows, screened again as a filtered run
             muse_batch *b = lb[(size_t)k];
-            b->prescreened = 1;
-            rc = muse_batch_run_ex(b, nullptr, 0, max_lag, top_n, threshold, sign_filter, MUSE_MODE_SCREEN, 0, sc, lg, ix, n_out + i);
+            if (rows) {
+                rc = run_multi_selected(b, rows, S, nullptr, 0, max_lag, top_n, threshold, sign_filter, MUSE_MODE_SCREEN, sc, lg, ix,
+                                        n_out + i);
+            } else {
+                b->prescreened = 1;
+                rc = muse_batch_run_ex(b, nullptr, 0, max_lag, top_n, threshold, sign_filter, MUSE_MODE_SCREEN, 0, sc, lg, ix, n_out + i);
+            }
             if (rc) return rc;
             continue;
         }
@@ -2573,7 +2623,7 @@ extern "C" int muse_multi_bounds_tc(muse_ctx *ctx, muse_group *g, const double *
         if (rc) return rc;
         own[q].reset(bs[q]);
     }
-    const int rc = tc_bounds_queue(ctx, g, bs.data(), (int)bs.size());
+    const int rc = tc_bounds_queue(ctx, g, bs.data(), (int)bs.size(), nullptr, S);
     if (rc) return rc;
     for (size_t q = 0; q < bs.size(); q++)
         CU(cudaMemcpyAsync(upper + q * (size_t)S, bs[q]->d_U, sizeof(float) * (size_t)S, cudaMemcpyDeviceToHost, ctx->stream));
@@ -2581,31 +2631,39 @@ extern "C" int muse_multi_bounds_tc(muse_ctx *ctx, muse_group *g, const double *
     return MUSE_OK;
 }
 
-extern "C" int muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, int64_t n_refs, int64_t ref_len,
-                              const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n, double threshold,
-                              int32_t sign_filter, int32_t mode, double *scores, int64_t *lags, int64_t *series_idx,
-                              int64_t *n_out) {
-    if (!ctx || !g || (!refs && n_refs > 0) || !n_out) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run: NULL argument");
-    if (n_refs < 0 || top_n < 0) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run: n_refs %lld, top_n %lld", (long long)n_refs, (long long)top_n);
-    if (top_n > 0 && (!scores || !lags || !series_idx)) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run: NULL output");
-    if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run: bad key columns");
-    CU(cudaSetDevice(ctx->device));
+// The argument checks of muse_multi_run (fn names the entry point in the message).
+static int multi_check(const muse_ctx *ctx, const muse_group *g, const double *refs, int64_t n_refs, const int32_t *key_cols,
+                       int32_t n_key_cols, int64_t top_n, const double *scores, const int64_t *lags, const int64_t *series_idx,
+                       const int64_t *n_out, const char *fn) {
+    if (!ctx || !g || (!refs && n_refs > 0) || !n_out) return fail(MUSE_ERR_INVALID_ARG, "%s: NULL argument", fn);
+    if (n_refs < 0 || top_n < 0) return fail(MUSE_ERR_INVALID_ARG, "%s: n_refs %lld, top_n %lld", fn, (long long)n_refs, (long long)top_n);
+    if (top_n > 0 && (!scores || !lags || !series_idx)) return fail(MUSE_ERR_INVALID_ARG, "%s: NULL output", fn);
+    if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "%s: bad key columns", fn);
+    return MUSE_OK;
+}
+
+// muse_multi_run over the m store rows rows[0 .. m) (ascending; a selection of muse_multi_run_where), or over the whole store
+// (rows NULL, m = size()).  Every decision that depends on the size of the store takes m, so the call takes the path, and
+// returns the records, of a store that holds only those rows.
+static int multi_run(muse_ctx *ctx, muse_group *g, const int32_t *rows, int64_t m, const double *refs, int64_t n_refs, int64_t ref_len,
+                     const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n, double threshold, int32_t sign_filter,
+                     int32_t mode, double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out) {
     // the tensor-core path (multi_run_tc_group, up to MUSE_MULTI_GROUP queries per pass over the store) exists for the
     // shape the single-query warp kernel serves (FFT length 2048, ungrouped, unsigned scores, a sign filter unsigned
     // scores can pass, a store worth screening, a device-side top-N); everything else -- and a group of one query -- is
     // NewBatch + Run per reference on the resident store: the store, its row statistics and the run scratch (context
     // pool) are shared, and results of query q land in row q of the outputs
     const bool one_pass = n_key_cols == 0 && mode != MUSE_MODE_EXACT && sign_filter != MUSE_SIGN_NEG && ref_len == g->N &&
-                          next_pow2(ref_len) == 2048 && device_topn_fits(top_n, g->size) &&
-                          (g->size >= 16384 || mode == MUSE_MODE_SCREEN) && n_refs > 1;
+                          next_pow2(ref_len) == 2048 && device_topn_fits(top_n, m) &&
+                          (m >= 16384 || mode == MUSE_MODE_SCREEN) && n_refs > 1;
     ctx->multi_refined = ctx->multi_rescored = 0;
     const int QC = one_pass ? MUSE_MULTI_GROUP : MUSE_MULTI_SEPARATE;
     for (int64_t q0 = 0; q0 < n_refs; q0 += QC) {
         const int nq = (int)std::min<int64_t>(QC, n_refs - q0);
         if (one_pass && nq > 1) {
             std::vector<BatchPtr> bs((size_t)nq);
-            const int rc = multi_run_tc_group(ctx, g, refs + (size_t)q0 * (size_t)ref_len, nq, ref_len, max_lag, top_n, threshold, sign_filter,
-                                              scores + (size_t)q0 * (size_t)top_n, lags + (size_t)q0 * (size_t)top_n,
+            const int rc = multi_run_tc_group(ctx, g, rows, m, refs + (size_t)q0 * (size_t)ref_len, nq, ref_len, max_lag, top_n, threshold,
+                                              sign_filter, scores + (size_t)q0 * (size_t)top_n, lags + (size_t)q0 * (size_t)top_n,
                                               series_idx + (size_t)q0 * (size_t)top_n, n_out + q0, bs);
             if (rc) {
                 cudaStreamSynchronize(ctx->stream);      // work queued on the batches may still be running: it ends before they go
@@ -2642,14 +2700,54 @@ extern "C" int muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, 
         for (int i = 0; i < nq; i++) {
             if (!bs[(size_t)i]) continue;
             const int64_t q = q0 + i;
-            rc = muse_batch_run_ex(bs[(size_t)i].get(), key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0,
-                                   scores ? scores + (size_t)q * (size_t)top_n : nullptr, lags ? lags + (size_t)q * (size_t)top_n : nullptr,
-                                   series_idx ? series_idx + (size_t)q * (size_t)top_n : nullptr, n_out + q);
+            double *sc = scores ? scores + (size_t)q * (size_t)top_n : nullptr;
+            int64_t *lg = lags ? lags + (size_t)q * (size_t)top_n : nullptr, *ix = series_idx ? series_idx + (size_t)q * (size_t)top_n : nullptr;
+            if (rows)      // every query of the call reads the one selection
+                rc = run_multi_selected(bs[(size_t)i].get(), rows, m, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode,
+                                        sc, lg, ix, n_out + q);
+            else
+                rc = muse_batch_run_ex(bs[(size_t)i].get(), key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0, sc, lg,
+                                       ix, n_out + q);
             bs[(size_t)i].reset();
             if (rc) return rc;
         }
     }
     return MUSE_OK;
+}
+
+extern "C" int muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, int64_t n_refs, int64_t ref_len,
+                              const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n, double threshold,
+                              int32_t sign_filter, int32_t mode, double *scores, int64_t *lags, int64_t *series_idx,
+                              int64_t *n_out) {
+    const int rc = multi_check(ctx, g, refs, n_refs, key_cols, n_key_cols, top_n, scores, lags, series_idx, n_out, "muse_multi_run");
+    if (rc) return rc;
+    CU(cudaSetDevice(ctx->device));
+    return multi_run(ctx, g, nullptr, g->size, refs, n_refs, ref_len, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode,
+                     scores, lags, series_idx, n_out);
+}
+
+extern "C" int muse_multi_run_where(muse_ctx *ctx, muse_group *g, const double *refs, int64_t n_refs, int64_t ref_len,
+                                    const int32_t *where_cols, const int32_t *where_ids, int32_t n_where, const int32_t *key_cols,
+                                    int32_t n_key_cols, int64_t max_lag, int64_t top_n, double threshold, int32_t sign_filter,
+                                    int32_t mode, double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out) {
+    int rc = multi_check(ctx, g, refs, n_refs, key_cols, n_key_cols, top_n, scores, lags, series_idx, n_out, "muse_multi_run_where");
+    if (rc) return rc;
+    WherePred p;
+    rc = where_pred(g, where_cols, where_ids, n_where, "muse_multi_run_where", p);
+    if (rc) return rc;
+    if (n_where == 0 || g->size == 0 || n_refs == 0)
+        return muse_multi_run(ctx, g, refs, n_refs, ref_len, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, scores,
+                              lags, series_idx, n_out);
+    if (g->ctx != ctx) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run_where: group belongs to another context");
+    CU(cudaSetDevice(ctx->device));
+    // ONE selection for every reference of the call
+    CU(ctx->d_where_rows.grow(g->size));
+    int64_t m = 0;
+    rc = select_where(ctx, g, p, ctx->d_where_rows, ctx->d_where_off, m);
+    if (rc) return rc;
+    const int32_t *rows = m < g->size ? ctx->d_where_rows.get() : nullptr;      // every row matches: the run of the whole store
+    return multi_run(ctx, g, rows, m, refs, n_refs, ref_len, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, scores,
+                     lags, series_idx, n_out);
 }
 
 // ------------------------------------------------------------------------------------

@@ -63,9 +63,10 @@ struct TcBoundsParams {
     const unsigned char *b_tiles;     // [16][hi 32 KB, lo 32 KB] bf16 weights of up to 256 queries (weight_tiles_kernel), zero rows beyond nq
     const float *mid;                 // [S] |2Y_(M/2)| of every series
     const float *amid;                // [256] A_q[M/2]
-    const RowStat *row_stat;          // [S] (1/std of every series)
+    const RowStat *row_stat;          // (1/std of every series of the store)
+    const int32_t *rows;              // [S] the store's row of tile row s (a selection), NULL: row s
     float *const *out_U;              // [nq] per-query bound arrays [S]
-    int64_t S;
+    int64_t S;                        // tile rows (series of the contraction)
     int nq;
 };
 
@@ -81,7 +82,8 @@ __device__ __forceinline__ void bf16_split(float x, unsigned &hi, unsigned &lo) 
 
 // ---- 1. magnitudes of every series in tile layout ----------------------------------------------------------------
 // The transform is score_screen_warp_kernel's (one warp per series, row by cp.async.bulk, radix-32 x radix-32 through the
-// row buffer); lane t ends with the mirror pairs k = t + 32 j, j < 16.
+// row buffer); lane t ends with the mirror pairs k = t + 32 j, j < 16.  Work item pos is the series prm.rows[pos] (NULL: pos);
+// the tiles and mid stay compact over the work items, so a selection of m rows is a contraction over ceil(m / 128) tiles.
 template <int NZ>
 __global__ void __launch_bounds__(ScreenWarpCfg::MAX_WARPS * 32, 1)
 mag_tiles_kernel(const ScreenParams prm, unsigned char *__restrict__ a_tiles, float *__restrict__ mid, const unsigned warp_bytes) {
@@ -108,13 +110,13 @@ mag_tiles_kernel(const ScreenParams prm, unsigned char *__restrict__ a_tiles, fl
     if (t == 0) {
         mbar_init(bar, 1);
         mbar_init_fence();
-        if (pos0 < count) bulk_load(smem_u32(buf), prm.slab + (int64_t)pos0 * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
+        if (pos0 < count) bulk_load(smem_u32(buf), prm.slab + (int64_t)(prm.rows ? prm.rows[pos0] : pos0) * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
     }
     __syncthreads();
 
     unsigned phase = 0;
     for (int pos = pos0; pos < count; pos += stride, phase ^= 1u) {
-        const double mu = prm.row_stat[pos].mean;
+        const double mu = prm.row_stat[prm.rows ? prm.rows[pos] : pos].mean;
         mbar_wait(bar, phase);
         cf v[P];
         load_centred<NZ, 32>(v, rowc, t, mu, last_in);
@@ -125,7 +127,7 @@ mag_tiles_kernel(const ScreenParams prm, unsigned char *__restrict__ a_tiles, fl
         __syncwarp();
         if (t == 0 && next < count) {       // the exchange is over: the buffer goes back to the copy engine
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            bulk_load(smem_u32(buf), prm.slab + (int64_t)next * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
+            bulk_load(smem_u32(buf), prm.slab + (int64_t)(prm.rows ? prm.rows[next] : next) * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
         }
         screen_pass1<32>(v);                            // v[Perm(j)] = Z[t + 32*j]
 
@@ -305,7 +307,7 @@ bounds_tc_kernel(const TcBoundsParams prm) {
         const bool live = srow < prm.S;
         float rstd = 0.f, midv = 0.f;
         if (live) {
-            rstd = prm.row_stat[srow].rstd;
+            rstd = prm.row_stat[prm.rows ? prm.rows[srow] : srow].rstd;
             midv = prm.mid[srow];
         }
         mbar_wait(smem_u32(&done_bar), 0u);

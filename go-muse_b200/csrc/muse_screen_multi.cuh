@@ -30,7 +30,9 @@ struct MultiQuery {
 // stage of muse_screen.cuh (conj(Y) X_q, inverse FFT_1024, maxima inside / outside the lag window), which replaces the
 // bound by the tight fp32 one and feeds the query's cut-off histogram.  Afterwards every query is exactly where a
 // single-query run is after its screening kernel.  Each warp owns its exchange buffer: with ~10 refinements per series a
-// shared, locked buffer would serialise the block.
+// shared, locked buffer would serialise the block.  LIST: work item pos is the series prm.rows[pos], else pos; the bound
+// arrays are indexed by pos, so a selection of m rows has bound arrays of m entries.  (A template parameter rather than a
+// test of prm.rows: the whole-store instantiation stays the code it was, and this kernel is sensitive to code size.)
 struct RefineMultiCfg {
     using G = Geo<10, 5>;
 #ifndef MUSE_REFINE_WARPS
@@ -58,7 +60,7 @@ struct RefineMultiCfg {
     static size_t smem_bytes(int N) { return (size_t)warps(N) * warp_bytes(N) + table_bytes(); }
 };
 
-template <int NZ>
+template <int NZ, bool LIST>
 __global__ void __launch_bounds__(RefineMultiCfg::MAX_WARPS * 32, 1)
 refine_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queries, const int nq, const unsigned warp_bytes,
                     unsigned *__restrict__ next_series) {
@@ -94,7 +96,7 @@ refine_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queri
     if (t == 0) {
         mbar_init(bar, 1);
         mbar_init_fence();
-        if (pos0 < count) bulk_load(smem_u32(buf), prm.slab + (int64_t)pos0 * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
+        if (pos0 < count) bulk_load(smem_u32(buf), prm.slab + (int64_t)(LIST ? prm.rows[pos0] : pos0) * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
     }
     for (int q = threadIdx.x; q < C::QMAX; q += blockDim.x) {
         s_cut[q] = q < nq ? queries[q].cut : nullptr;
@@ -122,7 +124,7 @@ refine_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queri
                 cutr[i] = ld_relaxed_u32(&s_cut[t + 32 * i]->bits);
             }
         }
-        const RowStat rs = prm.row_stat[pos];
+        const RowStat rs = prm.row_stat[LIST ? prm.rows[pos] : pos];
         const double mu = rs.mean;
         mbar_wait(bar, phase);
 
@@ -204,7 +206,7 @@ refine_multi_kernel(const ScreenParams prm, const MultiQuery *__restrict__ queri
         __syncwarp();
         if (t == 0 && next < count) {
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            bulk_load(smem_u32(buf), prm.slab + (int64_t)next * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
+            bulk_load(smem_u32(buf), prm.slab + (int64_t)(LIST ? prm.rows[next] : next) * prm.ld, (unsigned)(N + (N & 1)) * 8u, bar);
         }
     }
 }

@@ -17,6 +17,21 @@ import (
 // scores of refs[q]; a constant reference gets NewBatch's error in errs[q] and leaves results[q] untouched.
 // Not part of go-muse's API: the reference builds one Batch per query.
 func RunMany(refs []*Series, comp *Group, results []*Results, groupByLabels []string) (errs []error, err error) {
+	return runMany(refs, comp, results, false, nil, groupByLabels)
+}
+
+// RunManyWhere is RunMany over the series of comp.FilterByLabelValues(labels) only, on the resident device store (one
+// selection for every reference, no second store): results[q] ends up as RunMany on a Group of those series leaves it --
+// what a loop of NewBatch(ref_q, comp, results_q, cc).RunWhere(labels, groupByLabels) computes (muse_multi_run_where).
+// It makes the checks of RunMany.  When nothing can match -- empty labels, a key or a value no series of the group has --
+// there is no device call: every results[q] is untouched and every errs[q] nil, as Batch.RunWhere does.
+// Not part of go-muse's API.
+func RunManyWhere(refs []*Series, comp *Group, results []*Results, labels *Labels, groupByLabels []string) (errs []error, err error) {
+	return runMany(refs, comp, results, true, labels, groupByLabels)
+}
+
+// runMany is RunMany, or RunManyWhere when filter is set.
+func runMany(refs []*Series, comp *Group, results []*Results, filter bool, labels *Labels, groupByLabels []string) (errs []error, err error) {
 	if len(refs) != len(results) {
 		return nil, fmt.Errorf("%d references but %d results", len(refs), len(results))
 	}
@@ -36,11 +51,18 @@ func RunMany(refs []*Series, comp *Group, results []*Results, groupByLabels []st
 		}
 		rows = append(rows, ref.Values()...)
 	}
-	if r0.TopN < 1 {
+	if r0.TopN < 1 || (filter && (labels == nil || labels.Len() == 0)) {
 		return errs, nil
 	}
-	if err := comp.syncDevice(); err != nil {
+	if err := comp.syncDevice(); err != nil { // uploads series added since the last call: the dictionary then knows every value
 		return nil, err
+	}
+	var whereCols, whereIDs []int32
+	if filter {
+		var ok bool
+		if whereCols, whereIDs, ok = comp.whereCols(labels); !ok {
+			return errs, nil
+		}
 	}
 	c, err := deviceContext()
 	if err != nil {
@@ -56,11 +78,21 @@ func RunMany(refs []*Series, comp *Group, results []*Results, groupByLabels []st
 	lags := make([]int64, len(refs)*topN)
 	idx := make([]int64, len(refs)*topN)
 	nOut := make([]int64, len(refs))
-	rc := C.muse_multi_run(c, comp.store, (*C.double)(unsafe.Pointer(&rows[0])), C.int64_t(len(refs)), C.int64_t(n),
-		colPtr, C.int32_t(len(cols)), C.int64_t(r0.MaxLag), C.int64_t(topN), C.double(r0.Threshold),
-		C.int32_t(r0.SignFilter), C.MUSE_MODE_AUTO,
-		(*C.double)(unsafe.Pointer(&scores[0])), (*C.int64_t)(unsafe.Pointer(&lags[0])),
-		(*C.int64_t)(unsafe.Pointer(&idx[0])), (*C.int64_t)(unsafe.Pointer(&nOut[0])))
+	var rc C.int
+	if filter {
+		rc = C.muse_multi_run_where(c, comp.store, (*C.double)(unsafe.Pointer(&rows[0])), C.int64_t(len(refs)), C.int64_t(n),
+			(*C.int32_t)(unsafe.Pointer(&whereCols[0])), (*C.int32_t)(unsafe.Pointer(&whereIDs[0])), C.int32_t(len(whereCols)),
+			colPtr, C.int32_t(len(cols)), C.int64_t(r0.MaxLag), C.int64_t(topN), C.double(r0.Threshold),
+			C.int32_t(r0.SignFilter), C.MUSE_MODE_AUTO,
+			(*C.double)(unsafe.Pointer(&scores[0])), (*C.int64_t)(unsafe.Pointer(&lags[0])),
+			(*C.int64_t)(unsafe.Pointer(&idx[0])), (*C.int64_t)(unsafe.Pointer(&nOut[0])))
+	} else {
+		rc = C.muse_multi_run(c, comp.store, (*C.double)(unsafe.Pointer(&rows[0])), C.int64_t(len(refs)), C.int64_t(n),
+			colPtr, C.int32_t(len(cols)), C.int64_t(r0.MaxLag), C.int64_t(topN), C.double(r0.Threshold),
+			C.int32_t(r0.SignFilter), C.MUSE_MODE_AUTO,
+			(*C.double)(unsafe.Pointer(&scores[0])), (*C.int64_t)(unsafe.Pointer(&lags[0])),
+			(*C.int64_t)(unsafe.Pointer(&idx[0])), (*C.int64_t)(unsafe.Pointer(&nOut[0])))
+	}
 	if rc != C.MUSE_OK {
 		return nil, lastError(rc)
 	}

@@ -161,6 +161,8 @@ ABI = {
     "muse_batch_run_partial_device": (C.c_int, [_vp, C.c_int64, C.c_int64, C.c_double, C.c_int32, C.c_int32, _vp, C.c_int64]),
     "muse_multi_run": (C.c_int, [_vp, _vp, _dp, C.c_int64, C.c_int64, _ip32, C.c_int32, C.c_int64, C.c_int64, C.c_double,
                                  C.c_int32, C.c_int32, _dp, _ip64, _ip64, _ip64]),
+    "muse_multi_run_where": (C.c_int, [_vp, _vp, _dp, C.c_int64, C.c_int64, _ip32, _ip32, C.c_int32, _ip32, C.c_int32, C.c_int64,
+                                       C.c_int64, C.c_double, C.c_int32, C.c_int32, _dp, _ip64, _ip64, _ip64]),
     "muse_multi_last_stats": (C.c_int, [_vp, _ip64, _ip64]),
     "muse_multi_bounds_tc": (C.c_int, [_vp, _vp, _dp, C.c_int64, C.c_int64, _vp]),
     "muse_xcorr": (C.c_int, [_vp, _dp, C.c_int64, _dp, C.c_int64, C.c_int64, C.c_int32, _dp, C.c_int64, _ip64, _ip64,
@@ -501,6 +503,32 @@ def multi_run(store: "DeviceStore", refs, key_cols: Sequence[int], max_lag: int,
         return sc[:Q], lg[:Q], ix[:Q], n_out[:Q]
     return [None if n_out[q] < 0 else (sc[q, :n_out[q]].copy(), lg[q, :n_out[q]].copy(), ix[q, :n_out[q]].copy())
             for q in range(Q)]
+
+
+def multi_run_where(store: "DeviceStore", refs, where_cols: Sequence[int], where_ids: Sequence[int], key_cols: Sequence[int],
+                    max_lag: int, top_n: int, threshold: float, sign_filter: int = 0, mode: int = MODE_AUTO, raw: bool = False):
+    """muse_multi_run_where: multi_run over the series whose label id in column where_cols[j] is where_ids[j] for every j (one
+    selection for all references); indices are those of the whole store.  Returns as multi_run."""
+    R = np.ascontiguousarray(refs, dtype=np.float64)
+    assert R.ndim == 2
+    wc = np.asarray(list(where_cols), dtype=np.int32)
+    wi = np.asarray(list(where_ids), dtype=np.int32)
+    if wc.size != wi.size:
+        raise MuseError(MUSE_ERR_INVALID_ARG, "multi_run_where: %d where columns, %d ids" % (wc.size, wi.size))
+    Q, cap = R.shape[0], max(1, int(top_n))
+    kc = np.asarray(list(key_cols), dtype=np.int32)
+    sc = np.zeros((max(Q, 1), cap))
+    lg = np.zeros((max(Q, 1), cap), dtype=np.int64)
+    ix = np.zeros((max(Q, 1), cap), dtype=np.int64)
+    n_out = np.zeros(max(Q, 1), dtype=np.int64)
+    _check(lib().muse_multi_run_where(store.ctx.h, store.h, _d(R), Q, R.shape[1], wc.ctypes.data_as(_ip32) if wc.size else None,
+                                      wi.ctypes.data_as(_ip32) if wi.size else None, wc.size,
+                                      kc.ctypes.data_as(_ip32) if kc.size else None, kc.size, max_lag, top_n, threshold,
+                                      sign_filter, mode, _d(sc), lg.ctypes.data_as(_ip64), ix.ctypes.data_as(_ip64),
+                                      n_out.ctypes.data_as(_ip64)))
+    if raw:
+        return sc[:Q], lg[:Q], ix[:Q], n_out[:Q]
+    return _triples(sc[:Q], lg[:Q], ix[:Q], n_out[:Q])
 
 
 def multi_records(sc: np.ndarray, lg: np.ndarray, ix: np.ndarray, n_out: np.ndarray) -> np.ndarray:
@@ -978,6 +1006,59 @@ class Batch:
 
 def NewBatch(ref: Series, comp: Group, results: Results, cc: int) -> Batch:
     return Batch(ref, comp, results, cc)
+
+
+def RunMany(refs: Sequence[Series], comp: Group, results: Sequence[Results], groupByLabels: Optional[List[str]] = None):
+    """go/muse/multi.go RunMany: a loop of NewBatch(refs[q], comp, results[q], cc).Run(groupByLabels) in one call
+    (muse_multi_run).  Returns (errs, err) as the Go function: err a MuseError (nothing was run), else errs[q] the
+    MuseError of a constant reference (results[q] untouched) or None."""
+    return _run_many(refs, comp, results, False, None, groupByLabels)
+
+
+def RunManyWhere(refs: Sequence[Series], comp: Group, results: Sequence[Results], labels: Optional[Labels],
+                 groupByLabels: Optional[List[str]] = None):
+    """go/muse/multi.go RunManyWhere: RunMany over comp.FilterByLabelValues(labels) only, on the resident store
+    (muse_multi_run_where) -- a loop of NewBatch(refs[q], comp, results[q], cc).RunWhere(labels, groupByLabels).  The checks
+    of RunMany; nothing can match (empty labels, a key or value no series has): no device call, results untouched and
+    every errs[q] None."""
+    return _run_many(refs, comp, results, True, labels, groupByLabels)
+
+
+def _run_many(refs, comp: Group, results, filter_: bool, labels: Optional[Labels], groupByLabels):
+    if len(refs) != len(results):
+        return None, MuseError(MUSE_ERR_INVALID_ARG, "%d references but %d results" % (len(refs), len(results)))
+    errs: List[Optional[MuseError]] = [None] * len(refs)
+    if len(refs) == 0 or len(comp.series) == 0:
+        return errs, None
+    n = comp.Length()
+    r0 = results[0]
+    for ref, rq in zip(refs, results):
+        if ref.Length() != n:
+            return None, MuseError(MUSE_ERR_INVALID_ARG, "%s does not have the same length as the comparison group" % ref.UID())
+        if (rq.MaxLag, rq.TopN, rq.Threshold, rq.SignFilter) != (r0.MaxLag, r0.TopN, r0.Threshold, r0.SignFilter):
+            return None, MuseError(MUSE_ERR_INVALID_ARG, "RunMany needs the same MaxLag, TopN, Threshold and SignFilter on every Results")
+    if r0.TopN < 1 or (filter_ and (labels is None or not labels.Keys())):
+        return errs, None
+    R = np.stack([np.asarray(ref.Values(), dtype=np.float64) for ref in refs])
+    try:
+        store = comp._sync_device()      # uploads series added since the last call: the dictionary then knows every value
+        cols = comp._key_cols(groupByLabels)
+        if filter_:
+            where = comp._where(labels)
+            if where is None:
+                return errs, None
+            out = multi_run_where(store, R, where[0], where[1], cols, r0.MaxLag, r0.TopN, r0.Threshold, r0.SignFilter)
+        else:
+            out = multi_run(store, R, cols, r0.MaxLag, r0.TopN, r0.Threshold, r0.SignFilter)
+    except MuseError as e:
+        return None, e
+    for q, got in enumerate(out):
+        if got is None:
+            errs[q] = MuseError(MUSE_ERR_STDDEV_ZERO, "Invalid input query, Standard deviation of zero")
+            continue
+        for s, l, i in zip(*got):
+            results[q].Update(Score(comp.series[int(i)].Labels(), int(l), float(s)))
+    return errs, None
 
 
 class Muse:

@@ -262,6 +262,22 @@ int  muse_multi_run(muse_ctx *ctx, muse_group *g, const double *refs, int64_t n_
                     int32_t sign_filter, int32_t mode,
                     double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out);
 
+/* muse_multi_run restricted to the series whose label ids match, with the predicate of muse_batch_run_where (every
+ * j < n_where: labels[where_cols[j]][i] == where_ids[j]; a series that lacks a key does not match it) shared by every
+ * reference.  Row q of the outputs is what muse_multi_run writes for reference q on a store that holds only the matching
+ * series in the same order -- equivalently, what muse_batch_run_where returns for reference q -- with series_idx the index
+ * of the series in THIS store (plus the global offset); n_out[q] = -1 for a reference with std == 0.  n_where == 0: exactly
+ * muse_multi_run.  Nothing matches: n_out[q] = 0 for every other reference, and nothing is scored.  Argument errors (those of
+ * muse_multi_run and of muse_batch_run_where) return MUSE_ERR_INVALID_ARG before any device work.
+ * The selection is built once per call on the device; the path (tensor-core or separate batches) is the one muse_multi_run
+ * takes for a store of the selected size, and the tensor-core path reads only the selected rows.  muse_multi_last_stats and
+ * muse_multi_last_timing describe this call. */
+int  muse_multi_run_where(muse_ctx *ctx, muse_group *g, const double *refs, int64_t n_refs, int64_t ref_len,
+                          const int32_t *where_cols, const int32_t *where_ids, int32_t n_where,
+                          const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n, double threshold,
+                          int32_t sign_filter, int32_t mode,
+                          double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out);
+
 /* Totals of the context's last muse_multi_run over all its queries: (series, query) pairs that took the fp32 second stage and
  * pairs re-scored by the fp64 kernel (tensor-core path only; 0 otherwise). */
 int  muse_multi_last_stats(const muse_ctx *ctx, int64_t *n_refined, int64_t *n_rescored);
