@@ -273,13 +273,9 @@ struct muse_batch : RunScratch {
     float a_mid = 0.f;
     cf x_mid = {};
     muse_timing timing = {};
+    // the last run's state that muse_batch_last_timing reads after the call has returned (finish_pending_timing, settle_counters)
     int timing_pending = 0;    // the last run was queued without a final synchronisation (muse_batch_run_partial_device)
     int fused_run = 0;         // 1: score_fused, 2: score_fused_grouped (d_counters: listed = exact list length)
-    int prescreened = 0;       // d_U and the cut-off state were filled by the tensor-core multi-query path: the next fused run starts at its tail
-    int signed_run = 0;        // the current run keeps the sign of the scores (muse.go:72-76)
-    int64_t where_m = -1;      // a filtered run (muse_batch_run_where) is under way over the where_m rows of where_rows; -1: none
-    const int32_t *where_rows = nullptr;   // that run's selection: d_rows, or the selection of muse_multi_run_where (muse_ctx)
-    int pre_launches = -1;     // launches muse_batch_run_where queued (after recording ev[0]) before the run it starts; -1: none
     // n > MUSE_MAX_FUSED_FFT_LEN: Stockham passes through global memory (kernels_long.cu); Xt holds n entries, twM the n twiddles
     int is_long = 0;
     DevBuf<unsigned char> d_long;   // work buffer of launch_long
@@ -293,12 +289,6 @@ struct BatchDestroy {
 using BatchPtr = std::unique_ptr<muse_batch, BatchDestroy>;   // a batch that goes back through muse_batch_destroy
 
 static inline cudaStream_t bstream(const muse_batch *b) { return b->ctx->stream; }
-
-// The rows the current run scores: a filtered run's selection (where_rows[0 .. where_m)), else every row of the store (NULL).
-// Everything that depends on the size of the store -- the AUTO rule, launch bounds, what a fallback scores -- uses
-// run_count, so a filtered run takes the path a store of just its rows would take.
-static inline int64_t run_count(const muse_batch *b) { return b->where_m >= 0 ? b->where_m : b->g->size; }
-static inline const int32_t *run_rows(const muse_batch *b) { return b->where_m >= 0 ? b->where_rows : nullptr; }
 
 // ------------------------------------------------------------------------------------
 // context
@@ -1288,7 +1278,35 @@ struct RunArgs {
     int32_t sign_filter, mode, signed_scores;
     int32_t list_only;   // fused runs: the caller reads scores only through the exact list (no NaN fill of the score array)
     int32_t group_cut;   // grouped fused runs whose top-N is final here (one GPU): members below the top_n-th certain group need no exact score
+    // The rows the run scores: rows[0 .. count), ascending store rows (a selection), or every row of the store (rows NULL,
+    // count = size()).  Everything that depends on the size of the store -- the AUTO rule, launch bounds, what a fallback
+    // scores -- uses count, so a filtered run takes the path a store of just its rows would take.
+    const int32_t *rows;
+    int64_t count;
+    int32_t pre_launches;   // launches the caller queued since it recorded ev[0]; -1: the run records ev[0] itself
+    int32_t prescreened;    // d_U and the cut-off state come from the tensor-core launch group: the fused run starts at its tail
 };
+
+// The arguments of a run over every row of g's store.
+static RunArgs run_args(const muse_group *g, const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n,
+                        double threshold, int32_t sign_filter, int32_t mode, int32_t signed_scores) {
+    RunArgs a{key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores};
+    a.count = g->size;
+    a.pre_launches = -1;
+    return a;
+}
+
+// The checks of a run entry point's outputs (n_out, top_n records in scores, lags and series_idx) and group-by columns; fn
+// names the entry point in the message.
+static int check_run_outputs(const char *fn, const int64_t *n_out, int64_t top_n, const double *scores, const int64_t *lags,
+                             const int64_t *series_idx, const int32_t *key_cols, int32_t n_key_cols) {
+    if (!n_out || (top_n > 0 && (!scores || !lags || !series_idx))) return fail(MUSE_ERR_INVALID_ARG, "%s: NULL output", fn);
+    if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "%s: bad key columns", fn);
+    return MUSE_OK;
+}
+
+// The fp32 threshold of the screening passes: never above the fp64 threshold.
+static float threshold_floor(double threshold) { return threshold > 0 ? (float)threshold * 0.999999f : 0.f; }
 
 struct Rec {
     unsigned long long key;   // |score| bits
@@ -1386,7 +1404,7 @@ static int queue_group_reps(muse_batch *b, const RunArgs &a, bool shard, KeyCols
 // fused screened runs launch the exact kernel over at most this many listed series without knowing
 // the list length on the host; run_fused_overflow finishes a longer list after the fact
 #define MUSE_EXACT_UB 32768
-static int run_fused_overflow(muse_batch *b, int64_t n_exact, bool refill);
+static int run_fused_overflow(muse_batch *b, const RunArgs &a, int64_t n_exact, bool refill);
 
 // The run's statistics from its counters (d_counters, read back to the host): a fused run's `listed` is its exact list and
 // `refined` its refined count; any other run re-scores listed + refined (screened runs: pilot + second round).
@@ -1433,10 +1451,10 @@ static int run_select(muse_batch *b, const RunArgs &a, int apply_filter, int64_t
     CU(cudaStreamSynchronize(st));
     unsigned long long ncand = h_n.cand;
     settle_counters(b, h_n);
-    if (b->fused_run == 1 && (int64_t)h_n.listed > std::min<int64_t>(run_count(b), MUSE_EXACT_UB)) {
+    if (b->fused_run == 1 && (int64_t)h_n.listed > std::min<int64_t>(a.count, MUSE_EXACT_UB)) {
         // rare: more exact candidates than the fixed launch covered -> finish them and select again
         const int64_t n_exact = (int64_t)h_n.listed;
-        int rc = run_fused_overflow(b, n_exact, false);
+        int rc = run_fused_overflow(b, a, n_exact, false);
         if (rc) return rc;
         b->fused_run = 0;
         rc = run_select(b, a, apply_filter, limit, recs);
@@ -1513,13 +1531,14 @@ static int refresh_row_stats(muse_group *g) {
     return MUSE_OK;
 }
 
-static ScreenParams screen_params(muse_batch *b) {
+// The screening parameters of b over the store rows rows[0 .. count) (rows NULL: the first count rows).
+static ScreenParams screen_params(muse_batch *b, const int32_t *rows, int64_t count) {
     ScreenParams sp;
     memset(&sp, 0, sizeof(sp));
     sp.slab = b->g->slab;
     sp.ld = b->g->ld;
-    sp.count = run_count(b);
-    sp.rows = run_rows(b);
+    sp.count = count;
+    sp.rows = rows;
     sp.N = (int)b->N;
     sp.twp = b->twp_f;
     sp.sw = b->sw_f;
@@ -1630,7 +1649,7 @@ extern "C" int muse_batch_screen_bounds(muse_batch *b, int32_t refine, int64_t m
     const int64_t S = b->g->size;
     if (S == 0) return MUSE_OK;
     cudaStream_t st = bstream(b);
-    ScreenParams sp = screen_params(b);
+    ScreenParams sp = screen_params(b, nullptr, S);
     if (refine) {
         rc = ensure_lower(b);
         if (rc) return rc;
@@ -1655,13 +1674,9 @@ extern "C" int muse_batch_screen_bounds(muse_batch *b, int32_t refine, int64_t m
 static int score_fused(muse_batch *b, const RunArgs &a) {
     const int64_t S = b->g->size;
     cudaStream_t st = bstream(b);
-    ScreenParams sp = screen_params(b);
-    const float thr_lo = a.threshold > 0 ? (float)a.threshold * 0.999999f : 0.f;   // never above the fp64 threshold
-    int rc = MUSE_OK;
-    if (b->prescreened) {      // muse_multi_run: this query's bounds and cut-off came out of the tensor-core launch group
-        b->prescreened = 0;
-    } else {
-        rc = arm_refinement(b, sp, thr_lo, a.max_lag, a.top_n, a.threshold);
+    if (!a.prescreened) {      // prescreened (muse_multi_run): the bounds and cut-off came out of the tensor-core launch group
+        ScreenParams sp = screen_params(b, a.rows, a.count);
+        int rc = arm_refinement(b, sp, threshold_floor(a.threshold), a.max_lag, a.top_n, a.threshold);
         if (rc) return rc;
         CU(launch_screen(b, sp, st));
         b->timing.n_launches += 2;
@@ -1671,9 +1686,7 @@ static int score_fused(muse_batch *b, const RunArgs &a) {
     const unsigned blocks = (unsigned)((S + 255) / 256);
     survivors_cut_kernel<<<blocks, 256, 0, st>>>(b->d_U, S, b->d_cut, b->d_list, b->d_counters);
     b->timing.n_launches++;
-    rc = score_exact_all(b, b->signed_run, b->d_list, std::min<int64_t>(run_count(b), MUSE_EXACT_UB), &b->d_counters->listed);
-    if (rc) return rc;
-    return MUSE_OK;
+    return score_exact_all(b, a.signed_scores, b->d_list, std::min<int64_t>(a.count, MUSE_EXACT_UB), &b->d_counters->listed);
 }
 
 // Grouped runs on the fused kernels: every series takes the fp32 second stage (bounds on the score
@@ -1684,13 +1697,13 @@ static int score_fused(muse_batch *b, const RunArgs &a) {
 static int score_fused_grouped(muse_batch *b, const RunArgs &a) {
     const int64_t S = b->g->size;
     cudaStream_t st = bstream(b);
-    ScreenParams sp = screen_params(b);
+    ScreenParams sp = screen_params(b, a.rows, a.count);
     int rc = ensure_lower(b);
     if (rc) return rc;
     sp.out_L = b->d_L;
     sp.grouped = 1;
     // a member below the threshold cannot be the representative of a group that passes results.go:46-52
-    const float thr_lo = a.threshold > 0 ? (float)a.threshold * 0.999999f : 0.f;
+    const float thr_lo = threshold_floor(a.threshold);
     rc = arm_refinement(b, sp, thr_lo, a.max_lag, 0x7fffffff, 0.0);      // a cut-off that never rises
     if (rc) return rc;
     GroupTable gt;
@@ -1731,7 +1744,7 @@ static int score_fused_grouped(muse_batch *b, const RunArgs &a) {
     CU(cudaMemcpyAsync(h_listed, &b->d_counters->listed, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));                                 // one small round trip: the list length sizes the launch
     const int64_t n_exact = (int64_t)*h_listed;
-    rc = score_exact_all(b, b->signed_run, b->d_list, n_exact);
+    rc = score_exact_all(b, a.signed_scores, b->d_list, n_exact);
     if (rc) return rc;
     CU(cudaMemcpyAsync(&b->d_counters->refined, &b->d_cut->refined, sizeof(unsigned long long), cudaMemcpyDeviceToDevice, st));
     return MUSE_OK;
@@ -1740,25 +1753,24 @@ static int score_fused_grouped(muse_batch *b, const RunArgs &a) {
 // The exact list was longer than the launch bound: score the rest now that its length is known.
 // refill: the run skipped the NaN fill of the score array (list_only) and the caller is about to
 // read it as a whole -- fill it and score the complete list again.
-static int run_fused_overflow(muse_batch *b, int64_t n_exact, bool refill) {
+static int run_fused_overflow(muse_batch *b, const RunArgs &a, int64_t n_exact, bool refill) {
     const int64_t S = b->g->size;
     if (refill) {
         CU(cudaMemsetAsync(b->d_score, 0xff, sizeof(double) * (size_t)S, bstream(b)));
-        return score_exact_all(b, b->signed_run, b->d_list, n_exact);
+        return score_exact_all(b, a.signed_scores, b->d_list, n_exact);
     }
-    if (n_exact <= std::min<int64_t>(run_count(b), MUSE_EXACT_UB)) return MUSE_OK;
-    return score_exact_all(b, b->signed_run, b->d_list + MUSE_EXACT_UB, n_exact - MUSE_EXACT_UB);
+    if (n_exact <= std::min<int64_t>(a.count, MUSE_EXACT_UB)) return MUSE_OK;
+    return score_exact_all(b, a.signed_scores, b->d_list + MUSE_EXACT_UB, n_exact - MUSE_EXACT_UB);
 }
 
+// The scores of a run (its scratch grown: ensure_scratch) queued on the stream.
 static int run_scores(muse_batch *b, const RunArgs &a) {
-    int rc = ensure_scratch(b);
-    if (rc) return rc;
+    int rc;
     memset(&b->timing, 0, sizeof(b->timing));
     b->fused_run = 0;
     b->timing_pending = 0;
-    b->signed_run = a.signed_scores ? 1 : 0;
     cudaStream_t st = bstream(b);
-    if (b->pre_launches >= 0) b->timing.n_launches = b->pre_launches;      // the run began with the caller's work (ev[0] recorded)
+    if (a.pre_launches >= 0) b->timing.n_launches = a.pre_launches;      // the run began with the caller's work (ev[0] recorded)
     else CU(cudaEventRecord(b->ev[0], st));
     CU(cudaMemsetAsync(b->d_counters, 0, sizeof(RunCounters), st));
     // screening needs: a kernel for this FFT size, an ungrouped unsigned run, a sign filter that
@@ -1769,7 +1781,7 @@ static int run_scores(muse_batch *b, const RunArgs &a) {
     // top-N rank by; the survivors are re-scored signed.  A sign filter on signed scores needs the sign, which no bound has.
     const bool can_screen = b->screen_ok && (a.n_key_cols == 0 || screen_is_fused(b->log2m)) &&
                             (a.signed_scores ? a.sign_filter == MUSE_SIGN_ANY : a.sign_filter != MUSE_SIGN_NEG);
-    bool screen = can_screen && (a.mode == MUSE_MODE_SCREEN || (a.mode == MUSE_MODE_AUTO && run_count(b) >= 16384));
+    bool screen = can_screen && (a.mode == MUSE_MODE_SCREEN || (a.mode == MUSE_MODE_AUTO && a.count >= 16384));
     if (screen && a.n_key_cols > 0) {
         b->timing.mode = MUSE_MODE_SCREEN;
         b->fused_run = 2;          // statistics as a fused run; its exact list is already complete
@@ -1787,7 +1799,7 @@ static int run_scores(muse_batch *b, const RunArgs &a) {
         return MUSE_OK;
     }
     b->timing.mode = MUSE_MODE_EXACT;
-    rc = score_exact_all(b, a.signed_scores, run_rows(b), run_count(b));
+    rc = score_exact_all(b, a.signed_scores, a.rows, a.count);
     if (rc) return rc;
     CU(cudaEventRecord(b->ev[1], st));
     CU(cudaEventRecord(b->ev[2], st));
@@ -1851,8 +1863,8 @@ static int queue_topn_records(muse_batch *b, const RunArgs &a, muse_partial *d_o
 // finish on the host path from the scores already on the device.
 static bool device_topn_applies(const muse_batch *b, const RunArgs &a) {
     // a filtered run: as on a store of its rows, whose scratch holds max(rows, 1024) entries (ensure_scratch)
-    const int64_t cap = b->where_m >= 0 ? std::max<int64_t>(b->where_m, 1024) : b->scratch_cap;
-    return a.n_key_cols == 0 && run_count(b) > 0 && device_topn_fits(a.top_n, cap);
+    const int64_t cap = a.rows ? std::max<int64_t>(a.count, 1024) : b->scratch_cap;
+    return a.n_key_cols == 0 && a.count > 0 && device_topn_fits(a.top_n, cap);
 }
 
 static int device_topn_queue(muse_batch *b, const RunArgs &a) {
@@ -1875,7 +1887,7 @@ static int device_topn_finish(muse_batch *b, const RunArgs &a, double *scores, i
     b->timing_pending = 0;
     int rc;
     if (b->fused_run == 1) {
-        rc = run_fused_overflow(b, (int64_t)b->h_pin->counters.listed, true);
+        rc = run_fused_overflow(b, a, (int64_t)b->h_pin->counters.listed, true);
         if (rc) return rc;
         b->fused_run = 0;
     }
@@ -1886,20 +1898,9 @@ static int device_topn_finish(muse_batch *b, const RunArgs &a, double *scores, i
     return finish_timing(b);
 }
 
-extern "C" int muse_batch_run_ex(muse_batch *b, const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n,
-                                 double threshold, int32_t sign_filter, int32_t mode, int32_t signed_scores, double *scores,
-                                 int64_t *lags, int64_t *series_idx, int64_t *n_out) {
-    int rc = check_batch(b);
-    if (rc) return rc;
-    if (!n_out || (top_n > 0 && (!scores || !lags || !series_idx))) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run: NULL output");
-    if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run: bad key columns");
-    if (top_n < 0) top_n = 0;
-    CU(cudaSetDevice(b->ctx->device));
-    RunArgs a{key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores};
-    a.group_cut = 1;
-    *n_out = 0;
-    rc = ensure_scratch(b);
-    if (rc) return rc;
+// The run of b that `a` describes (the device set, the scratch grown: ensure_scratch): its records into the caller's arrays.
+static int batch_run(muse_batch *b, const RunArgs &a, double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out) {
+    int rc;
     if (device_topn_applies(b, a)) {
         // ungrouped: filter and top-N on the device, ONE copy of top_n records to the host
         rc = device_topn_queue(b, a);
@@ -1910,10 +1911,27 @@ extern "C" int muse_batch_run_ex(muse_batch *b, const int32_t *key_cols, int32_t
     rc = run_scores(b, a);
     if (rc) return rc;
     std::vector<Rec> recs;
-    rc = run_select(b, a, 1, top_n, recs);
+    rc = run_select(b, a, 1, a.top_n, recs);
     if (rc) return rc;
     *n_out = records_out(b, recs, scores, lags, series_idx);
     return finish_timing(b);
+}
+
+extern "C" int muse_batch_run_ex(muse_batch *b, const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n,
+                                 double threshold, int32_t sign_filter, int32_t mode, int32_t signed_scores, double *scores,
+                                 int64_t *lags, int64_t *series_idx, int64_t *n_out) {
+    int rc = check_batch(b);
+    if (rc) return rc;
+    rc = check_run_outputs("muse_batch_run", n_out, top_n, scores, lags, series_idx, key_cols, n_key_cols);
+    if (rc) return rc;
+    if (top_n < 0) top_n = 0;
+    CU(cudaSetDevice(b->ctx->device));
+    RunArgs a = run_args(b->g, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores);
+    a.group_cut = 1;
+    *n_out = 0;
+    rc = ensure_scratch(b);
+    if (rc) return rc;
+    return batch_run(b, a, scores, lags, series_idx, n_out);
 }
 
 extern "C" int muse_batch_run(muse_batch *b, const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag, int64_t top_n,
@@ -2051,59 +2069,53 @@ static int where_pred(const muse_group *g, const int32_t *where_cols, const int3
     return MUSE_OK;
 }
 
-// The selection of a predicate over the store's size() rows into rows (room for size() entries; ascending local rows), queued
-// on the context's stream with off as the per-tile scratch; its length.
-static int select_where(muse_ctx *ctx, const muse_group *g, const WherePred &p, int32_t *rows, DevBuf<int32_t> &off, int64_t &m) {
+// The selection of a predicate over the store's size() rows into buf (room for size() entries; ascending local rows), queued
+// on the context's stream with off as the per-tile scratch: rows = buf and its length m, or rows = NULL when every row matches
+// (the run of the whole store).
+static int select_where(muse_ctx *ctx, const muse_group *g, const WherePred &p, int32_t *buf, DevBuf<int32_t> &off,
+                        const int32_t *&rows, int64_t &m) {
     const int64_t S = g->size;
     cudaStream_t st = ctx->stream;
     const int64_t nb = (S + MUSE_WHERE_TILE - 1) / MUSE_WHERE_TILE;
     CU(off.grow(nb + 1));
     where_count_kernel<<<(unsigned)nb, 256, 0, st>>>(p, S, off);
     where_scan_kernel<<<1, 1024, 0, st>>>(off, nb);
-    where_write_kernel<<<(unsigned)nb, 256, 0, st>>>(p, S, off, rows);
+    where_write_kernel<<<(unsigned)nb, 256, 0, st>>>(p, S, off, buf);
     CU(cudaGetLastError());
     int32_t h_m = 0;                      // one small copy: the host sizes the launches and takes the AUTO decision on it
     CU(cudaMemcpyAsync(&h_m, off.get() + nb, sizeof(h_m), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     m = h_m;
+    rows = m < S ? buf : nullptr;
     return MUSE_OK;
 }
 
-// The run of b over the m ascending local rows of `rows`, selected on the stream before this call.  The run's timing starts at
-// ev[0], which the caller recorded, and counts the caller's `launches` since then.
-static int run_selected(muse_batch *b, const int32_t *rows, int64_t m, int launches, const int32_t *key_cols, int32_t n_key_cols,
-                        int64_t max_lag, int64_t top_n, double threshold, int32_t sign_filter, int32_t mode, int32_t signed_scores,
-                        double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out) {
+// The run of b over the selection a.rows[0 .. a.count), made on the stream before this call (a.rows NULL: the whole store).
+// Its timing starts at ev[0]: recorded by the caller, who queued a.pre_launches launches since, or here (a.pre_launches < 0).
+static int run_selected(muse_batch *b, RunArgs a, double *scores, int64_t *lags, int64_t *series_idx, int64_t *n_out) {
     *n_out = 0;
-    int rc = ensure_scratch(b);
-    if (rc) return rc;
-    rc = ensure_lower(b);
+    if (!a.rows) return batch_run(b, a, scores, lags, series_idx, n_out);
+    int rc = ensure_lower(b);
     if (rc) return rc;
     cudaStream_t st = bstream(b);
-    const int64_t S = b->g->size;
-    if (m == 0) {          // nothing matches: no records and nothing scored
+    if (a.pre_launches < 0) {
+        CU(cudaEventRecord(b->ev[0], st));
+        a.pre_launches = 0;
+    }
+    if (a.count == 0) {    // nothing matches: no records and nothing scored
         memset(&b->timing, 0, sizeof(b->timing));
         b->timing_pending = 0;
         b->timing.mode = MUSE_MODE_EXACT;
-        b->timing.n_launches = launches;
+        b->timing.n_launches = a.pre_launches;
         CU(cudaEventRecord(b->ev[1], st));      // no scoring pass, no re-scoring
         CU(cudaEventRecord(b->ev[2], st));
         return finish_timing(b);
     }
-    struct EndWhere {      // every path out of the run leaves the batch unfiltered
-        muse_batch *b;
-        ~EndWhere() { b->where_m = -1; b->where_rows = nullptr; b->pre_launches = -1; }
-    } end_where{b};
-    if (m < S) {           // m == S: every row matches, the run of the whole store
-        where_neutral_kernel<<<(unsigned)((S + 255) / 256), 256, 0, st>>>(b->d_score, b->d_U, b->d_L, S);
-        CU(cudaGetLastError());
-        launches++;
-        b->where_m = m;
-        b->where_rows = rows;
-    }
-    b->pre_launches = launches;
-    return muse_batch_run_ex(b, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores, scores, lags,
-                             series_idx, n_out);
+    const int64_t S = b->g->size;
+    where_neutral_kernel<<<(unsigned)((S + 255) / 256), 256, 0, st>>>(b->d_score, b->d_U, b->d_L, S);
+    CU(cudaGetLastError());
+    a.pre_launches++;
+    return batch_run(b, a, scores, lags, series_idx, n_out);
 }
 
 extern "C" int muse_batch_run_where(muse_batch *b, const int32_t *where_cols, const int32_t *where_ids, int32_t n_where,
@@ -2116,24 +2128,22 @@ extern "C" int muse_batch_run_where(muse_batch *b, const int32_t *where_cols, co
     WherePred p;
     rc = where_pred(g, where_cols, where_ids, n_where, "muse_batch_run_where", p);
     if (rc) return rc;
-    if (n_where == 0 || g->size == 0)
-        return muse_batch_run_ex(b, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores, scores, lags,
-                                 series_idx, n_out);
-    if (!n_out || (top_n > 0 && (!scores || !lags || !series_idx))) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: NULL output");
-    if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_where: bad key columns");
+    rc = check_run_outputs("muse_batch_run_where", n_out, top_n, scores, lags, series_idx, key_cols, n_key_cols);
+    if (rc) return rc;
+    if (top_n < 0) top_n = 0;
     CU(cudaSetDevice(b->ctx->device));
+    RunArgs a = run_args(g, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores);
+    a.group_cut = 1;
     *n_out = 0;
     rc = ensure_scratch(b);
     if (rc) return rc;
-    rc = ensure_lower(b);
-    if (rc) return rc;
+    if (n_where == 0 || g->size == 0) return batch_run(b, a, scores, lags, series_idx, n_out);      // the run of the whole store
     // The timing of a filtered run starts here, before the selection, and counts its launches in every case.
     CU(cudaEventRecord(b->ev[0], bstream(b)));
-    int64_t m = 0;
-    rc = select_where(b->ctx, g, p, b->d_rows, b->d_where_off, m);
+    rc = select_where(b->ctx, g, p, b->d_rows, b->d_where_off, a.rows, a.count);
     if (rc) return rc;
-    return run_selected(b, b->d_rows, m, 3, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, signed_scores,
-                        scores, lags, series_idx, n_out);      // 3 launches: the selection's count, scan, write
+    a.pre_launches = 3;      // the selection's count, scan, write
+    return run_selected(b, a, scores, lags, series_idx, n_out);
 }
 
 // ------------------------------------------------------------------------------------
@@ -2162,7 +2172,7 @@ static TopnLaunch queue_candidates(muse_batch *b, const RunArgs &a) {
         Cand cand{b->d_ckey, b->d_cidx, b->d_clag, &b->d_counters->cand};
         if (b->fused_run == 1) {
             // only the listed series have scores: filter those (the list's length stays on the device)
-            const int64_t lim = std::min<int64_t>(run_count(b), MUSE_EXACT_UB);
+            const int64_t lim = std::min<int64_t>(a.count, MUSE_EXACT_UB);
             emit_listed_kernel<<<(unsigned)((lim + 255) / 256), 256, 0, st>>>(b->d_list, &b->d_counters->listed, lim, b->d_score, b->d_lag, f, cand);
         } else {
             GroupTable gt;
@@ -2172,8 +2182,8 @@ static TopnLaunch queue_candidates(muse_batch *b, const RunArgs &a) {
         b->timing.n_launches++;
     }
     // the grid covers MUSE_PARTIAL_RANK_CAP candidates; blocks past the real count (device side) leave at once
-    const long long exact_bound = b->fused_run == 1 ? (long long)std::min<int64_t>(run_count(b), MUSE_EXACT_UB) : -1;
-    const unsigned pblocks = (unsigned)std::min<int64_t>((std::max<int64_t>(run_count(b), 1) + 7) / 8, (int64_t)b->ctx->sm_count * 8);   // 8 warps per block, one warp per candidate
+    const long long exact_bound = b->fused_run == 1 ? (long long)std::min<int64_t>(a.count, MUSE_EXACT_UB) : -1;
+    const unsigned pblocks = (unsigned)std::min<int64_t>((std::max<int64_t>(a.count, 1) + 7) / 8, (int64_t)b->ctx->sm_count * 8);   // 8 warps per block, one warp per candidate
     return TopnLaunch{exact_bound, pblocks};
 }
 
@@ -2211,8 +2221,9 @@ extern "C" int muse_batch_run_partial_device(muse_batch *b, int64_t max_lag, int
     if (top_n < 0) top_n = 0;
     if (top_n > capacity) return fail(MUSE_ERR_INVALID_ARG, "partial capacity %lld < top_n %lld", (long long)capacity, (long long)top_n);
     CU(cudaSetDevice(b->ctx->device));
-    RunArgs a{nullptr, 0, max_lag, top_n, threshold, sign_filter, mode, 0};
-    return queue_topn_records(b, a, d_out, capacity);
+    rc = ensure_scratch(b);
+    if (rc) return rc;
+    return queue_topn_records(b, run_args(b->g, nullptr, 0, max_lag, top_n, threshold, sign_filter, mode, 0), d_out, capacity);
 }
 
 static int host_keys(muse_batch *b, const RunArgs &a, const std::vector<Rec> &recs, std::vector<uint64_t> &keys) {
@@ -2254,12 +2265,15 @@ extern "C" int muse_batch_run_partial(muse_batch *b, const int32_t *key_cols, in
                                       int64_t *n_out) {
     int rc = check_batch(b);
     if (rc) return rc;
-    if (!n_out || (!out && capacity > 0)) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_partial: NULL output");
-    if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_partial: bad key columns");
+    if (!out && capacity > 0) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_partial: NULL output");
+    rc = check_run_outputs("muse_batch_run_partial", n_out, 0, nullptr, nullptr, nullptr, key_cols, n_key_cols);
+    if (rc) return rc;
     if (top_n < 0) top_n = 0;
     CU(cudaSetDevice(b->ctx->device));
-    RunArgs a{key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0};
+    const RunArgs a = run_args(b->g, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0);
     *n_out = 0;
+    rc = ensure_scratch(b);
+    if (rc) return rc;
     rc = run_scores(b, a);
     if (rc) return rc;
     std::vector<Rec> recs;
@@ -2352,9 +2366,7 @@ static int tc_bounds_queue(muse_ctx *ctx, muse_group *g, muse_batch **bs, int nq
     // pageable sources: the copies have left the host buffers when the calls return
     CU(cudaMemcpyAsync(ctx->tc_ptrs, h_ptrs, sizeof(h_ptrs), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(ctx->tc_amid, h_amid, sizeof(h_amid), cudaMemcpyHostToDevice, st));
-    ScreenParams sp = screen_params(bs[0]);
-    sp.count = S;
-    sp.rows = rows;
+    const ScreenParams sp = screen_params(bs[0], rows, S);
     CU(cudaEventRecord(ctx->mt_ev[0], st));
     CU(launch_mag_tiles(sp, ctx->tc_a, ctx->tc_mid, ctx->sm_count, st));
     CU(launch_weight_tiles(reinterpret_cast<const float4 *const *>(ctx->tc_ptrs.get()), nq, ctx->tc_b, st));
@@ -2405,16 +2417,6 @@ struct MultiTables {
     static size_t bytes(int64_t top_n) { return off_recs() + sizeof(PartialRec) * (size_t)Q * (size_t)std::max<int64_t>(top_n, 1); }
 };
 
-// The run of batch b over the m ascending local rows `rows` that muse_multi_run_where selected for all its references: what
-// muse_batch_run_where runs after its selection (its timing starts here).
-static int run_multi_selected(muse_batch *b, const int32_t *rows, int64_t m, const int32_t *key_cols, int32_t n_key_cols, int64_t max_lag,
-                              int64_t top_n, double threshold, int32_t sign_filter, int32_t mode, double *scores, int64_t *lags,
-                              int64_t *series_idx, int64_t *n_out) {
-    CU(cudaEventRecord(b->ev[0], bstream(b)));
-    return run_selected(b, rows, m, 0, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0, scores, lags, series_idx,
-                        n_out);
-}
-
 // One launch group (<= 256 references) of muse_multi_run on the tensor-core path, with ONE launch per stage for all its
 // queries: reference spectra and tables (batched fp64 kernel in MODE_REF, blockIdx.y = query), cut-off states, bounds
 // (bf16 contraction), second stages (one pass over the store), survivors, fp64 re-scoring, filter, top-N -- and two
@@ -2459,7 +2461,7 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const int32_t *rows,
         h_cut[i] = b->d_cut;
     }
     const int64_t M = bs[0]->n / 2;
-    const float thr_lo = threshold > 0 ? (float)threshold * 0.999999f : 0.f;
+    const float thr_lo = threshold_floor(threshold);
     CU(cudaMemcpyAsync(d, h, MT::off_tail(), cudaMemcpyHostToDevice, st));
     CU(launch_exact_batch(MODE_REF, reinterpret_cast<const ExactParams *>(d + MT::off_ep()), nq, 1, st));
     screen_tables_batch_kernel<<<dim3((unsigned)((M / 2 + 1 + 255) / 256), (unsigned)nq), 256, 0, st>>>(
@@ -2493,11 +2495,9 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const int32_t *rows,
     ScreenParams sp0;
     for (int k = 0; k < nl; k++) {
         muse_batch *b = lb[(size_t)k] = bs[(size_t)live[(size_t)k]].get();
-        ScreenParams sp = screen_params(b);
+        ScreenParams sp = screen_params(b, rows, S);
         rc = arm_refinement(b, sp, thr_lo, max_lag, top_n, threshold, true);
         if (rc) return rc;
-        sp.count = S;
-        sp.rows = rows;
         if (k == 0) sp0 = sp;
         MultiQuery &m = hq[(size_t)k];
         memset(&m, 0, sizeof(m));
@@ -2572,16 +2572,13 @@ static int multi_run_tc_group(muse_ctx *ctx, muse_group *g, const int32_t *rows,
         ctx->multi_refined += (int64_t)h_cnt[k].refined;
         if (r[0].flags == 2) {
             // the list did not fit the device-side select (or the re-scoring launch): this query finishes alone, from its
-            // bounds and cut-off on the device (the fused run skips the screening of a prescreened batch) -- or, over a
+            // bounds and cut-off on the device (the fused run skips the screening of a prescreened run) -- or, over a
             // selection, whose bounds are compact and not those of the store's rows, screened again as a filtered run
-            muse_batch *b = lb[(size_t)k];
-            if (rows) {
-                rc = run_multi_selected(b, rows, S, nullptr, 0, max_lag, top_n, threshold, sign_filter, MUSE_MODE_SCREEN, sc, lg, ix,
-                                        n_out + i);
-            } else {
-                b->prescreened = 1;
-                rc = muse_batch_run_ex(b, nullptr, 0, max_lag, top_n, threshold, sign_filter, MUSE_MODE_SCREEN, 0, sc, lg, ix, n_out + i);
-            }
+            RunArgs a = run_args(g, nullptr, 0, max_lag, top_n, threshold, sign_filter, MUSE_MODE_SCREEN, 0);
+            a.rows = rows;
+            a.count = S;
+            a.prescreened = rows ? 0 : 1;
+            rc = run_selected(lb[(size_t)k], a, sc, lg, ix, n_out + i);
             if (rc) return rc;
             continue;
         }
@@ -2637,9 +2634,7 @@ static int multi_check(const muse_ctx *ctx, const muse_group *g, const double *r
                        const int64_t *n_out, const char *fn) {
     if (!ctx || !g || (!refs && n_refs > 0) || !n_out) return fail(MUSE_ERR_INVALID_ARG, "%s: NULL argument", fn);
     if (n_refs < 0 || top_n < 0) return fail(MUSE_ERR_INVALID_ARG, "%s: n_refs %lld, top_n %lld", fn, (long long)n_refs, (long long)top_n);
-    if (top_n > 0 && (!scores || !lags || !series_idx)) return fail(MUSE_ERR_INVALID_ARG, "%s: NULL output", fn);
-    if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "%s: bad key columns", fn);
-    return MUSE_OK;
+    return check_run_outputs(fn, n_out, top_n, scores, lags, series_idx, key_cols, n_key_cols);
 }
 
 // muse_multi_run over the m store rows rows[0 .. m) (ascending; a selection of muse_multi_run_where), or over the whole store
@@ -2697,17 +2692,17 @@ static int multi_run(muse_ctx *ctx, muse_group *g, const int32_t *rows, int64_t 
                 return rc;
             }
         }
+        RunArgs a = run_args(g, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0);
+        a.group_cut = 1;
+        a.rows = rows;      // every query of the call reads the one selection
+        a.count = m;
         for (int i = 0; i < nq; i++) {
             if (!bs[(size_t)i]) continue;
             const int64_t q = q0 + i;
             double *sc = scores ? scores + (size_t)q * (size_t)top_n : nullptr;
             int64_t *lg = lags ? lags + (size_t)q * (size_t)top_n : nullptr, *ix = series_idx ? series_idx + (size_t)q * (size_t)top_n : nullptr;
-            if (rows)      // every query of the call reads the one selection
-                rc = run_multi_selected(bs[(size_t)i].get(), rows, m, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode,
-                                        sc, lg, ix, n_out + q);
-            else
-                rc = muse_batch_run_ex(bs[(size_t)i].get(), key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0, sc, lg,
-                                       ix, n_out + q);
+            rc = ensure_scratch(bs[(size_t)i].get());
+            if (rc == MUSE_OK) rc = run_selected(bs[(size_t)i].get(), a, sc, lg, ix, n_out + q);
             bs[(size_t)i].reset();
             if (rc) return rc;
         }
@@ -2742,10 +2737,10 @@ extern "C" int muse_multi_run_where(muse_ctx *ctx, muse_group *g, const double *
     CU(cudaSetDevice(ctx->device));
     // ONE selection for every reference of the call
     CU(ctx->d_where_rows.grow(g->size));
+    const int32_t *rows = nullptr;
     int64_t m = 0;
-    rc = select_where(ctx, g, p, ctx->d_where_rows, ctx->d_where_off, m);
+    rc = select_where(ctx, g, p, ctx->d_where_rows, ctx->d_where_off, rows, m);
     if (rc) return rc;
-    const int32_t *rows = m < g->size ? ctx->d_where_rows.get() : nullptr;      // every row matches: the run of the whole store
     return multi_run(ctx, g, rows, m, refs, n_refs, ref_len, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, scores,
                      lags, series_idx, n_out);
 }
@@ -2955,18 +2950,20 @@ extern "C" int muse_batch_run_exchange_ex(muse_batch *b, muse_exchange *x, const
                                           int64_t *series_idx, int64_t *n_out) {
     int rc = check_batch(b);
     if (rc) return rc;
-    if (!x || !n_out) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_exchange: NULL argument");
+    if (!x) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_exchange: NULL argument");
     if (x->ctx != b->ctx) return fail(MUSE_ERR_INVALID_ARG, "exchange belongs to another context");
     if (!x->opened) return fail(MUSE_ERR_INVALID_ARG, "muse_exchange_open_peers has not been called");
-    if (n_key_cols < 0 || (n_key_cols > 0 && !key_cols)) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_exchange: bad key columns");
+    rc = check_run_outputs("muse_batch_run_exchange", n_out, top_n, scores, lags, series_idx, key_cols, n_key_cols);
+    if (rc) return rc;
     if (top_n < 0) top_n = 0;
     if (top_n > x->capacity) return fail(MUSE_ERR_INVALID_ARG, "exchange capacity %lld < top_n %lld", (long long)x->capacity, (long long)top_n);
-    if (top_n > 0 && (!scores || !lags || !series_idx)) return fail(MUSE_ERR_INVALID_ARG, "muse_batch_run_exchange: NULL output");
     CU(cudaSetDevice(b->ctx->device));
     *n_out = 0;
     const bool grouped = n_key_cols > 0;
-    RunArgs a{key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0};
+    RunArgs a = run_args(b->g, key_cols, n_key_cols, max_lag, top_n, threshold, sign_filter, mode, 0);
     a.list_only = grouped ? 0 : 1;
+    rc = ensure_scratch(b);
+    if (rc) return rc;
     rc = run_scores(b, a);
     if (rc) return rc;
     const int64_t S = b->g->size;
@@ -3051,7 +3048,8 @@ extern "C" int muse_multi_run_exchange(muse_group *g, muse_exchange *x, const do
     if (!g || !x || (!refs && n_refs > 0) || !n_out) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run_exchange: NULL argument");
     if (n_refs < 0 || top_n < 0)
         return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run_exchange: n_refs %lld, top_n %lld", (long long)n_refs, (long long)top_n);
-    if (top_n > 0 && (!scores || !lags || !series_idx)) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run_exchange: NULL output");
+    int rc = check_run_outputs("muse_multi_run_exchange", n_out, top_n, scores, lags, series_idx, nullptr, 0);
+    if (rc) return rc;
     if (x->ctx != g->ctx) return fail(MUSE_ERR_INVALID_ARG, "muse_multi_run_exchange: exchange and store belong to different contexts");
     if (!x->opened) return fail(MUSE_ERR_INVALID_ARG, "muse_exchange_open_peers has not been called");
     if (top_n > x->capacity) return fail(MUSE_ERR_INVALID_ARG, "exchange capacity %lld < top_n %lld", (long long)x->capacity, (long long)top_n);
